@@ -3,7 +3,7 @@
 Benchmark of the hot path: predict_y + UCB + arg-max over leaf candidates (BASELINE.json metric, config C3:
 N=4096 training points, d=10, 1e7 candidates, Matern-5/2, fp64).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one full scoring pass over the candidate set (a `gp_eval_best_ucb` call at C3 size).  With N > 1 GPUs
@@ -278,8 +278,10 @@ def run_reference(args, rank):
         cpu_reference_step(X, y, theta, Xc, VARSIGMA)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_reference_step(X, y, theta, Xc, VARSIGMA)
+        result = cpu_reference_step(X, y, theta, Xc, VARSIGMA)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_record(args.dump_outputs, result)
     cores, blas = blas_threads()
     value = sample * args.steps / dt
     line = {
@@ -337,6 +339,14 @@ def verify_result(session, cuda, X, y, theta, xc_dev, m_local, varsigma, stream,
     return out
 
 
+def dump_record(out_dir, result):
+    """The arg-max record a caller of the scoring path receives, one float64 array per field (the index is exact in float64
+    up to 2^53 candidates)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, value in zip(("index", "mean", "var", "ucb"), result):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.array([value], dtype=np.float64))
+
+
 def side_leg(fn, *a, **kw):
     """Run a side measurement; a failure there must not cost the headline line (the error text is reported instead)."""
     try:
@@ -362,7 +372,12 @@ def main():
     ap.add_argument("--no-bound", action="store_true", help="skip the bound-and-refine side measurement (screen mode 5)")
     ap.add_argument("--no-overlap", action="store_true", help="int8 engine: run cross-covariance and product back to back")
     ap.add_argument("--slices", type=int, default=0, help="8-bit digits per operand for the int8 engine (0 = automatic)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the record the last timed step returned (index, mean, var, ucb) as DIR/<name>.npy in float64, "
+                         "so that two builds can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -484,6 +499,8 @@ def main():
     dev_ms = max_over_ranks(ev0.elapsed_time(ev1))
     launches = session.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_record(args.dump_outputs, result)
     product_ms = stage_ms[2]  # summed duration of all variance-product launches (event pairs on their stream)
     engine = session.predict_info()
     screened = bool(screen["paths"]) and all(p == "screened" for p in screen["paths"])

@@ -44,14 +44,17 @@ def build_library(force=False, verbose=False):
     if not force and not needs_build():
         return LIB_PATH
     cmd = [find_nvcc()] + NVCC_FLAGS + [os.path.join(CSRC, s) for s in SOURCES] + ["-o", LIB_PATH]
-    proc = subprocess.run(cmd, capture_output=True, text=True)
+    # C locale: the host compiler's diagnostics (quote characters, translations) are then the same for every caller
+    proc = subprocess.run(cmd, capture_output=True, text=True, env=dict(os.environ, LC_ALL="C"))
     if verbose or proc.returncode != 0:
         sys.stderr.write(proc.stdout + proc.stderr)
     if proc.returncode != 0:
         raise RuntimeError("nvcc failed building libgpso_b200.so")
     with open(os.path.join(HERE, "csrc", "ptxas_report.txt"), "w") as handle:
-        # registers / spills / shared memory per kernel; the compile times would change the file on every build
-        handle.write("".join(line for line in (proc.stdout + proc.stderr).splitlines(True) if "Compile time" not in line))
+        # registers / spills / shared memory per kernel; the compile times, and the directory of the checkout in the
+        # diagnostics, would change the file on every build
+        text = (proc.stdout + proc.stderr).replace(os.path.dirname(HERE) + os.sep, "")
+        handle.write("".join(line for line in text.splitlines(True) if "Compile time" not in line))
     return LIB_PATH
 
 
