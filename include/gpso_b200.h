@@ -73,6 +73,23 @@ int gpso_predict_y_host(gpso_handle* h, const double* Xc_host, int64_t M, double
 int gpso_predict_y_dev(gpso_handle* h, const double* Xc_dev, int64_t M, double* mean_dev, double* var_dev,
                        void* stream);
 
+/* ---- joint posterior: model.predict_f(Xnew, full_cov=True) and model.predict_f_samples(Xnew, S) (GPflow 2 GPR) ---- */
+/* Candidates per call of the joint entry points: the M x M covariance, its Cholesky factor and V = L^-1 K(X, X*) stay on the
+ * device (~2.5 GB at M = N = 8192); more candidates are drawn in batches. */
+#define GPSO_MAX_JOINT 8192
+/* model.predict_f(Xnew, full_cov=True): mean[M], cov[M*M] row-major, both triangles written (exactly symmetric).
+ * cov = K(X*, X*) - A^T A, A = L^-1 K(X, X*) (no noise variance).  Valid after gpso_factorize; 1 <= M <= GPSO_MAX_JOINT.
+ * The fitted state of the handle is not modified; the FP64 L^-1 is used whatever gpso_set_predict_mode selected. */
+int gpso_predict_f_cov_host(gpso_handle* h, const double* Xc_host, int64_t M, double* mean_host, double* cov_host);
+int gpso_predict_f_cov_dev(gpso_handle* h, const double* Xc_dev, int64_t M, double* mean_dev, double* cov_dev, void* stream);
+/* model.predict_f_samples(Xnew, S): out[s*M + m] = mean[m] + sum_k Lc[m][k] * z[s*M + k],  Lc = chol(cov + jitter*I).
+ * z[S,M] standard normals supplied by the caller; jitter >= 0.  Returns info > 0 (LAPACK pivot) when cov + jitter*I is
+ * not positive definite.  The _dev form is synchronous on `stream` at return (it reads the pivot status). */
+int gpso_predict_f_samples_host(gpso_handle* h, const double* Xc_host, int64_t M, int S, double jitter, const double* z_host,
+                                double* out_host);
+int gpso_predict_f_samples_dev(gpso_handle* h, const double* Xc_dev, int64_t M, int S, double jitter, const double* z_dev,
+                               double* out_dev, void* stream);
+
 /* ---- exploitation step: gp_eval_best_ucb(normed_coords), gp_surrogate.py:313-328 ------------------------------ */
 /* ucb = mean + varsigma * var ; winner = FIRST index of the maximum (np.argmax; a NaN wins like in numpy).
  * result_host[4] = { (double)index, mean, var, ucb }.  The cross-covariance is never materialised beyond a

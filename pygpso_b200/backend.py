@@ -17,6 +17,7 @@ _LIB_NAME = "libgpso_b200.so"
 _ABI_VERSION = 1
 
 _c_double_p = ctypes.POINTER(ctypes.c_double)
+MAX_JOINT = 8192  # GPSO_MAX_JOINT: candidates per joint-posterior call (predict_f_cov / predict_f_samples)
 
 
 class GpsoBackendError(RuntimeError):
@@ -84,6 +85,10 @@ def load_library():
         "gpso_factor_lml": (i32, [H, _c_double_p]),
         "gpso_predict_y_host": (i32, [H, _c_double_p, i64, _c_double_p, _c_double_p]),
         "gpso_predict_y_dev": (i32, [H, ctypes.c_void_p, i64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+        "gpso_predict_f_cov_host": (i32, [H, _c_double_p, i64, _c_double_p, _c_double_p]),
+        "gpso_predict_f_cov_dev": (i32, [H, ctypes.c_void_p, i64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+        "gpso_predict_f_samples_host": (i32, [H, _c_double_p, i64, i32, dbl, _c_double_p, _c_double_p]),
+        "gpso_predict_f_samples_dev": (i32, [H, ctypes.c_void_p, i64, i32, dbl, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
         "gpso_ucb_argmax_host": (i32, [H, _c_double_p, i64, dbl, _c_double_p]),
         "gpso_ucb_argmax_dev": (i32, [H, ctypes.c_void_p, i64, dbl, _c_double_p, ctypes.c_void_p]),
         "gpso_ucb_topk_host": (i32, [H, _c_double_p, i64, dbl, i32, _c_double_p, ctypes.POINTER(ctypes.c_int)]),
@@ -142,6 +147,7 @@ EXPORTED_SYMBOLS = (
     "gpso_version gpso_last_error gpso_device_count gpso_create gpso_destroy gpso_set_data gpso_neg_lml_grad "
     "gpso_factorize gpso_factor_lml gpso_predict_y_host gpso_predict_y_dev gpso_ucb_argmax_host gpso_ucb_argmax_dev "
     "gpso_ucb_topk_host gpso_ucb_topk_dev "
+    "gpso_predict_f_cov_host gpso_predict_f_cov_dev gpso_predict_f_samples_host gpso_predict_f_samples_dev "
     "gpso_grow_count gpso_grow_leaves_host gpso_grow_leaves_dev gpso_grow_ucb_argmax gpso_grow_ucb_argmax_range gpso_state_bytes "
     "gpso_export_state_dev gpso_import_state_dev gpso_launch_count gpso_debug_fetch gpso_last_timing gpso_set_window "
     "gpso_set_profile gpso_last_windows gpso_set_predict_mode gpso_predict_info gpso_set_overlap "
@@ -157,6 +163,13 @@ def _check(lib, rc, what):
     if rc > 0:
         raise NotPositiveDefiniteError(f"{what}: {text}")
     raise GpsoBackendError(f"{what} failed (status {rc}): {text}")
+
+
+def _joint_candidates(xnew):
+    xnew = np.ascontiguousarray(xnew, dtype=np.float64)
+    if not 1 <= xnew.shape[0] <= MAX_JOINT:
+        raise ValueError(f"the joint posterior takes 1..{MAX_JOINT} candidates per call, got {xnew.shape[0]}; draw larger sets in batches")
+    return xnew
 
 
 def default_device():
@@ -226,6 +239,28 @@ class CudaSession:
                    "gpso_predict_y_host")
         return mean, var
 
+    def predict_f_cov(self, xnew):
+        """Joint posterior of the latent function: mean[M] and the full covariance cov[M,M] (no noise variance)."""
+        xnew = _joint_candidates(xnew)
+        m = xnew.shape[0]
+        mean = np.empty(m)
+        cov = np.empty((m, m))
+        _check(self._lib, self._lib.gpso_predict_f_cov_host(self._h, _dptr(xnew), m, _dptr(mean), _dptr(cov)),
+               "gpso_predict_f_cov_host")
+        return mean, cov
+
+    def predict_f_samples(self, xnew, z, jitter):
+        """Posterior draws [S,M] = mean + z chol(cov + jitter I)^T for standard normals z[S,M]; a covariance that is not
+        positive definite raises NotPositiveDefiniteError."""
+        xnew = _joint_candidates(xnew)
+        z = np.ascontiguousarray(z, dtype=np.float64)
+        if z.ndim != 2 or z.shape[1] != xnew.shape[0] or z.shape[0] < 1:
+            raise ValueError(f"z must be [S,{xnew.shape[0]}] with S >= 1, got {z.shape}")
+        out = np.empty(z.shape)
+        _check(self._lib, self._lib.gpso_predict_f_samples_host(self._h, _dptr(xnew), xnew.shape[0], z.shape[0], float(jitter),
+                                                                _dptr(z), _dptr(out)), "gpso_predict_f_samples_host")
+        return out
+
     def ucb_argmax(self, xnew, varsigma):
         xnew = np.ascontiguousarray(xnew, dtype=np.float64)
         out = np.empty(4)
@@ -265,6 +300,13 @@ class CudaSession:
     # -- device-pointer variants (benchmarks, multi-GPU sharding): pointers are ints (e.g. torch.Tensor.data_ptr()) -----
     def predict_y_dev(self, xc_ptr, m, mean_ptr, var_ptr, stream=0):
         _check(self._lib, self._lib.gpso_predict_y_dev(self._h, xc_ptr, m, mean_ptr, var_ptr, stream), "gpso_predict_y_dev")
+
+    def predict_f_cov_dev(self, xc_ptr, m, mean_ptr, cov_ptr, stream=0):
+        _check(self._lib, self._lib.gpso_predict_f_cov_dev(self._h, xc_ptr, m, mean_ptr, cov_ptr, stream), "gpso_predict_f_cov_dev")
+
+    def predict_f_samples_dev(self, xc_ptr, m, s, jitter, z_ptr, out_ptr, stream=0):
+        _check(self._lib, self._lib.gpso_predict_f_samples_dev(self._h, xc_ptr, m, int(s), float(jitter), z_ptr, out_ptr, stream),
+               "gpso_predict_f_samples_dev")
 
     def ucb_argmax_dev(self, xc_ptr, m, varsigma, stream=0):
         out = np.empty(4)

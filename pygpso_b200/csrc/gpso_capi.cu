@@ -25,6 +25,7 @@
 #include "kern_leaves.cuh"
 #include "kern_ozaki.cuh"
 #include "kern_predict.cuh"
+#include "kern_joint.cuh"
 #include "kern_screen.cuh"
 #include "kern_probe.cuh"
 
@@ -219,6 +220,11 @@ struct gpso_handle {
     // predict workspaces
     DevBuf KsT, part, blockbest, running, cand[2], leaves, omean, ovar, topk;
     int topk_k = 0;         // records per window of the top-k pass in flight
+    // joint posterior (kern_joint.cuh): scaled candidates, cross-covariance, mean, V^T, Sigma; for the samples the factor's
+    // scratch (inverse diagonal blocks and their transposes, log-determinant, pivot status, scheduler state) and the padded
+    // normals; host staging of candidates, normals and outputs.  Separate from the fit's buffers, which a joint call never touches.
+    DevBuf jXcs, jKsT, jmean, jVT, jSigma, jLinv, jLinvT, jlogdet, jinfo, jstate, jcounter, jZ, jcand, jzin, jout;
+    int jLinv_mp = 0;       // row pitch jLinv was cleared for (its zero sub-blocks above the diagonal are never written)
     // int8 tensor-core (tcgen05) variance product: digit tiles of L^-1 and of the cross-covariance window
     DevBuf ozA, ozBb[2], wmeanb[2], rowscale, rowmax, rowl2;
     // int8 tensor-core K_y^-1 = L^-T L^-1 (fit path): digit tiles of L^-T, its row scales, the tile -> CTA table
@@ -551,6 +557,12 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(dense_gemm_kernel<MODE_LAUUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(dense_gemm_kernel<MODE_LAUUM_PART>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(predict_trmm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_v_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN12>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN32>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN52>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_SE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(diag_factor_inverse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(factor_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(diag_transpose_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_TRANSPOSE_SMEM));
@@ -2537,6 +2549,185 @@ extern "C" int gpso_ucb_topk_host(gpso_handle* h, const double* Xc_host, int64_t
     GP_TRY(predict_common_checks(h, Xc_host, M, "gpso_ucb_topk_host"));
     if (!result_host) return fail(GPSO_E_BADARG, "gpso_ucb_topk_host: null output");
     return topk_common(h, h->stream, nullptr, Xc_host, M, varsigma, k, result_host, found);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// joint posterior (kern_joint.cuh): a fixed number of launches per call, on one stream, into the handle's j* buffers
+// ---------------------------------------------------------------------------------------------------------------------
+static int joint_checks(gpso_handle* h, const void* xc, long long M, const void* out1, const void* out2, const char* who) {
+    if (M < 1 || M > GPSO_MAX_JOINT) return fail(GPSO_E_BADARG, std::string(who) + ": M must be in 1..8192 (draw larger batches in parts)");
+    if (!h || !xc || !out1 || !out2) return fail(GPSO_E_BADARG, std::string(who) + ": null argument");
+    return 0;
+}
+
+static int joint_ready(gpso_handle* h, const char* who) {
+    if (!h->factorized) return fail(GPSO_E_STATE, std::string(who) + ": call gpso_factorize first");
+    return set_device(h);
+}
+
+template <int KID>
+static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, int M, int Mp) {
+    size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
+    crosscov_kernel<KID><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
+                                                              h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
+                                                              h->jKsT.as<double>(), h->jmean.as<double>());
+}
+
+template <int KID>
+static void launch_joint_syrk(gpso_handle* h, cudaStream_t st, int M, int Mp, double jitter) {
+    const int mb = Mp / TB;
+    joint_syrk_kernel<KID><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp, h->Np,
+                                                                               h->d, h->variance, jitter, h->jSigma.as<double>());
+}
+
+// scaled candidates -> cross-covariance + mean -> V^T = (L^-1 K*)^T -> lower triangle of K** - V^T V (+ jitter I) in jSigma
+static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M, double jitter) {
+    const int Mp = (M + TB - 1) / TB * TB, Np = h->Np;
+    GP_TRY(h->jXcs.ensure((size_t)h->d * Mp * sizeof(double)));
+    GP_TRY(h->jKsT.ensure((size_t)Mp * Np * sizeof(double)));
+    GP_TRY(h->jmean.ensure((size_t)Mp * sizeof(double)));
+    GP_TRY(h->jVT.ensure((size_t)Mp * Np * sizeof(double)));
+    GP_TRY(h->jSigma.ensure((size_t)Mp * Mp * sizeof(double)));
+    GP_TRY(h->jcounter.ensure(sizeof(int)));
+    scale_inputs_kernel<<<(Mp + 255) / 256, 256, 0, st>>>(Xc, h->ls.as<double>(), h->n_ls(), M, h->d, Mp, h->jXcs.as<double>());
+    GP_TRY(check_launch(h, "scale_inputs"));
+    DISPATCH_KID(h, launch_joint_crosscov, h, st, Xc, M, Mp);
+    GP_TRY(check_launch(h, "crosscov"));
+    JointVParams P;
+    P.Linv = h->Linv.as<double>();
+    P.KsT = h->jKsT.as<double>();
+    P.VT = h->jVT.as<double>();
+    P.Np = Np;
+    P.nb = h->nb;
+    P.nct = Mp / TB;
+    P.counter = h->jcounter.as<int>();
+    CU_TRY(cudaMemsetAsync(h->jcounter.p, 0, sizeof(int), st));
+    joint_v_kernel<<<std::min(h->nsm > 0 ? h->nsm : 148, P.nct * P.nb), GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
+    GP_TRY(check_launch(h, "joint_v"));
+    DISPATCH_KID(h, launch_joint_syrk, h, st, M, Mp, jitter);
+    return check_launch(h, "joint_syrk");
+}
+
+static int joint_cov(gpso_handle* h, cudaStream_t st, const double* Xc, int M, double* mean, double* cov, bool host) {
+    GP_TRY(joint_sigma(h, st, Xc, M, 0.0));
+    const int Mp = (M + TB - 1) / TB * TB;
+    double* dst = cov;
+    if (host) {
+        GP_TRY(h->jout.ensure((size_t)M * M * sizeof(double)));
+        dst = h->jout.as<double>();
+    }
+    joint_mirror_kernel<<<dim3((M + 31) / 32, (M + 31) / 32), dim3(32, 8), 0, st>>>(h->jSigma.as<double>(), M, Mp, dst);
+    GP_TRY(check_launch(h, "joint_mirror"));
+    const cudaMemcpyKind kind = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+    CU_TRY(cudaMemcpyAsync(mean, h->jmean.p, (size_t)M * sizeof(double), kind, st));
+    if (host) CU_TRY(cudaMemcpyAsync(cov, dst, (size_t)M * M * sizeof(double), kind, st));
+    return 0;
+}
+
+// Sigma = cov + jitter I -> Lc (in place, Cholesky tasks of the persistent kernel on the joint scratch) -> out = mean + Z Lc^T
+static int joint_samples(gpso_handle* h, cudaStream_t st, const double* Xc, int M, int S, double jitter, const double* z, double* out) {
+    GP_TRY(joint_sigma(h, st, Xc, M, jitter));
+    const int Mp = (M + TB - 1) / TB * TB, mb = Mp / TB;
+    const int Sp = (S + TB - 1) / TB * TB, nsb = Sp / TB;
+    const size_t mat = (size_t)Mp * Mp * sizeof(double);
+    gpso_handle::FactorPlan* plan = nullptr;
+    GP_TRY(get_factor_plan(h, mb, 0, &plan));
+    GP_TRY(h->jLinv.ensure(mat));
+    GP_TRY(h->jLinvT.ensure(mat));
+    GP_TRY(h->jlogdet.ensure((size_t)mb * sizeof(double)));
+    GP_TRY(h->jinfo.ensure(sizeof(int)));
+    GP_TRY(h->jstate.ensure((size_t)(2 + plan->ncounters) * sizeof(int)));
+    GP_TRY(h->jZ.ensure((size_t)Sp * Mp * sizeof(double)));
+    // the panel solves read whole diagonal blocks of the inverse, whose zero sub-blocks above the diagonal the diagonal task
+    // never writes: cleared on every call (Mp^2 doubles, ~1 % of the factorisation's time at any size)
+    CU_TRY(cudaMemsetAsync(h->jLinv.p, 0, mat, st));
+    CU_TRY(cudaMemsetAsync(h->jstate.p, 0, (size_t)(2 + plan->ncounters) * sizeof(int), st));
+    CU_TRY(cudaMemsetAsync(h->jinfo.p, 0, sizeof(int), st));
+    DenseParams P;
+    P.K = h->jSigma.as<double>();
+    P.Linv = h->jLinv.as<double>();
+    P.LinvT = h->jLinvT.as<double>();
+    P.T = nullptr;
+    P.Kinv = nullptr;
+    P.Np = Mp;
+    P.nb = mb;
+    P.p = 0;
+    P.s = 0;
+    const int grid = std::min(plan->ntasks, h->nsm > 0 ? h->nsm : 148);
+    factor_persistent_kernel<<<grid, GTHREADS, DIAG_SMEM_BYTES, st>>>(P, M, plan->tasks.as<int>(), plan->ntasks, h->jstate.as<int>(),
+                                                                       h->jlogdet.as<double>(), h->jinfo.as<int>());
+    GP_TRY(check_launch(h, "factor_persistent"));
+    joint_tril_kernel<<<mb, 256, 0, st>>>(h->jSigma.as<double>(), Mp);
+    GP_TRY(check_launch(h, "joint_tril"));
+    const long long nz = (long long)Sp * Mp;
+    joint_pad_kernel<<<(unsigned)std::min<long long>((nz + 255) / 256, 4096), 256, 0, st>>>(z, S, M, Sp, Mp, h->jZ.as<double>());
+    GP_TRY(check_launch(h, "joint_pad"));
+    joint_sample_kernel<<<mb * nsb, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jSigma.as<double>(), h->jZ.as<double>(), h->jmean.as<double>(), M,
+                                                                     Mp, S, mb, nsb, out);
+    return check_launch(h, "joint_sample");
+}
+
+// waits for the stream and reports the pivot status of the last joint_samples
+static int joint_pivot_status(gpso_handle* h, cudaStream_t st) {
+    int info = 0;
+    CU_TRY(cudaMemcpyAsync(&info, h->jinfo.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    if (info < 0) return fail(GPSO_E_CUDA, "Cholesky tile scheduler timed out waiting for a dependency");
+    if (info > 0) {
+        char b[128];
+        snprintf(b, sizeof b, "posterior covariance + jitter is not positive definite (pivot %d)", info);
+        fail(info, b);
+        return info;
+    }
+    return 0;
+}
+
+static int joint_sample_checks(gpso_handle* h, const void* xc, long long M, int S, double jitter, const void* z, const void* out,
+                               const char* who) {
+    GP_TRY(joint_checks(h, xc, M, z, out, who));
+    if (S < 1) return fail(GPSO_E_BADARG, std::string(who) + ": S must be positive");
+    if (!(jitter >= 0.0)) return fail(GPSO_E_BADARG, std::string(who) + ": jitter must be a non-negative number");
+    return joint_ready(h, who);
+}
+
+extern "C" int gpso_predict_f_cov_dev(gpso_handle* h, const double* Xc_dev, int64_t M, double* mean_dev, double* cov_dev, void* stream) {
+    GP_TRY(joint_checks(h, Xc_dev, M, mean_dev, cov_dev, "gpso_predict_f_cov_dev"));
+    GP_TRY(joint_ready(h, "gpso_predict_f_cov_dev"));
+    return joint_cov(h, (cudaStream_t)stream, Xc_dev, (int)M, mean_dev, cov_dev, false);
+}
+
+extern "C" int gpso_predict_f_cov_host(gpso_handle* h, const double* Xc_host, int64_t M, double* mean_host, double* cov_host) {
+    GP_TRY(joint_checks(h, Xc_host, M, mean_host, cov_host, "gpso_predict_f_cov_host"));
+    GP_TRY(joint_ready(h, "gpso_predict_f_cov_host"));
+    cudaStream_t st = h->stream;
+    GP_TRY(h->jcand.ensure((size_t)M * h->d * sizeof(double)));
+    CU_TRY(cudaMemcpyAsync(h->jcand.p, Xc_host, (size_t)M * h->d * sizeof(double), cudaMemcpyHostToDevice, st));
+    GP_TRY(joint_cov(h, st, h->jcand.as<double>(), (int)M, mean_host, cov_host, true));
+    CU_TRY(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int gpso_predict_f_samples_dev(gpso_handle* h, const double* Xc_dev, int64_t M, int S, double jitter, const double* z_dev,
+                                          double* out_dev, void* stream) {
+    GP_TRY(joint_sample_checks(h, Xc_dev, M, S, jitter, z_dev, out_dev, "gpso_predict_f_samples_dev"));
+    cudaStream_t st = (cudaStream_t)stream;
+    GP_TRY(joint_samples(h, st, Xc_dev, (int)M, S, jitter, z_dev, out_dev));
+    return joint_pivot_status(h, st);
+}
+
+extern "C" int gpso_predict_f_samples_host(gpso_handle* h, const double* Xc_host, int64_t M, int S, double jitter, const double* z_host,
+                                           double* out_host) {
+    GP_TRY(joint_sample_checks(h, Xc_host, M, S, jitter, z_host, out_host, "gpso_predict_f_samples_host"));
+    cudaStream_t st = h->stream;
+    const size_t zbytes = (size_t)S * M * sizeof(double);
+    GP_TRY(h->jcand.ensure((size_t)M * h->d * sizeof(double)));
+    GP_TRY(h->jzin.ensure(zbytes));
+    GP_TRY(h->jout.ensure(zbytes));
+    CU_TRY(cudaMemcpyAsync(h->jcand.p, Xc_host, (size_t)M * h->d * sizeof(double), cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->jzin.p, z_host, zbytes, cudaMemcpyHostToDevice, st));
+    GP_TRY(joint_samples(h, st, h->jcand.as<double>(), (int)M, S, jitter, h->jzin.as<double>(), h->jout.as<double>()));
+    CU_TRY(cudaMemcpyAsync(out_host, h->jout.p, zbytes, cudaMemcpyDeviceToHost, st));
+    return joint_pivot_status(h, st);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -40,6 +40,20 @@ __device__ __forceinline__ void predict_tile_decode(int t, int nb, int nct, int&
     ct = grp * PRED_GROUP + r % gsize;
 }
 
+// tile -> (row block I, candidate tile ct) over all nct * nb tiles, the short last group included: tiles of full groups first
+__device__ __forceinline__ void predict_tile_of(int tile, int nb, int nct, int& I, int& ct) {
+    int full_groups = nct / PRED_GROUP;
+    int full_tiles = full_groups * PRED_GROUP * nb;
+    if (tile < full_tiles) {
+        predict_tile_decode(tile, nb, nct, I, ct);
+    } else {
+        int r = tile - full_tiles;
+        int gsize = nct - full_groups * PRED_GROUP;
+        I = nb - 1 - r / gsize;
+        ct = full_groups * PRED_GROUP + r % gsize;
+    }
+}
+
 __global__ void __launch_bounds__(GTHREADS, 1) predict_trmm_kernel(PredictParams P) {
     extern __shared__ double smem[];
     __shared__ int s_tile;
@@ -56,19 +70,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) predict_trmm_kernel(PredictParams
         const int tile = s_tile;
         if (tile >= ntiles) break;
         int I, ct;
-        {
-            // decode with short last group handled: tiles of full groups first
-            int full_groups = nct / PRED_GROUP;
-            int full_tiles = full_groups * PRED_GROUP * nb;
-            if (tile < full_tiles) {
-                predict_tile_decode(tile, nb, nct, I, ct);
-            } else {
-                int r = tile - full_tiles;
-                int gsize = nct - full_groups * PRED_GROUP;
-                I = nb - 1 - r / gsize;
-                ct = full_groups * PRED_GROUP + r % gsize;
-            }
-        }
+        predict_tile_of(tile, nb, nct, I, ct);
         TileOperands w;
         w.A = P.Linv + (size_t)I * TB * Np;
         w.B = P.KsT + (size_t)ct * TB * Np;

@@ -7,6 +7,7 @@ and ``gpflow.models.GPR`` (gpso/gp_surrogate.py:138,165-169,397,424-429,463-473,
     model.data = (x, y)                      gp_surrogate.py:498
     optimiser.minimize(model.training_loss, model.trainable_variables)     :500-503
     model.predict_y(Xnew) -> (mean[M,1], var[M,1]) with ``.numpy()``      :298,325; plotting.py:351-356
+    model.predict_f(Xnew, full_cov=True), model.predict_f_samples(Xnew, S)   (joint posterior, user code)
     model.kernel.lengthscales / .variance, model.likelihood.variance, model.mean_function.c   (summaries, save)
     gpflow.utilities.parameter_dict / multiple_assign / freeze            :462-473,514-519
 
@@ -27,6 +28,7 @@ import scipy.optimize
 from . import backend as _backend
 
 NOISE_VARIANCE_FLOOR = 1.0e-6
+SAMPLE_JITTER = 1.0e-6  # gpflow.config.default_jitter(): added to the posterior covariance before its Cholesky in predict_f_samples
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -298,18 +300,49 @@ class GPR(GPModel):
             self._session.factorize(theta)
             self._factor_key = key
 
-    def predict_y(self, Xnew):
-        """Posterior mean and variance *including* the noise variance, both ``[M,1]``."""
+    def _candidates(self, Xnew):
         Xnew = np.ascontiguousarray(Xnew, dtype=np.float64)
         if Xnew.ndim != 2 or Xnew.shape[1] != self._data[0].shape[1]:
             raise ValueError(f"Xnew must be [M,{self._data[0].shape[1]}], got {Xnew.shape}")
+        return Xnew
+
+    def predict_y(self, Xnew):
+        """Posterior mean and variance *including* the noise variance, both ``[M,1]``."""
+        Xnew = self._candidates(Xnew)
         self._ensure_factor()
         mean, var = self._session.predict_y(Xnew)
         return _as_host_tensor(mean).reshape(-1, 1), _as_host_tensor(var).reshape(-1, 1)
 
-    def predict_f(self, Xnew):
-        mean, var = self.predict_y(Xnew)
-        return mean, _as_host_tensor(var - float(self.likelihood.variance))
+    def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
+        """Posterior of the latent function: mean ``[M,1]`` and variance ``[M,1]``, or with ``full_cov`` the covariance
+        ``[1,M,M]`` of the M candidates jointly (no noise variance; at most ``backend.MAX_JOINT`` candidates per call).
+        ``full_output_cov`` has no effect: the model has a single output."""
+        if not full_cov:
+            mean, var = self.predict_y(Xnew)
+            return mean, _as_host_tensor(var - float(self.likelihood.variance))
+        Xnew = self._candidates(Xnew)
+        self._ensure_factor()
+        mean, cov = self._session.predict_f_cov(Xnew)
+        return _as_host_tensor(mean).reshape(-1, 1), _as_host_tensor(cov).reshape(1, Xnew.shape[0], Xnew.shape[0])
+
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """Draws of the latent function at ``Xnew``: ``[S,M,1]``, or ``[M,1]`` when ``num_samples`` is None.
+        ``full_cov``: joint draws ``mean + chol(cov + SAMPLE_JITTER I) z``; otherwise independent ``mean + sqrt(var) z``.
+        The standard normals ``z[S,M]`` come from ``np.random.default_rng(seed)`` (the one keyword GPflow lacks: its
+        TensorFlow random stream cannot be reproduced, a seed makes draws reproducible)."""
+        Xnew = self._candidates(Xnew)
+        S = 1 if num_samples is None else int(num_samples)
+        if S < 1:
+            raise ValueError(f"num_samples must be positive, got {num_samples}")
+        z = np.random.default_rng(seed).standard_normal((S, Xnew.shape[0]))
+        if full_cov:
+            self._ensure_factor()
+            f = self._session.predict_f_samples(Xnew, z, SAMPLE_JITTER)
+        else:
+            mean, var = self.predict_f(Xnew)
+            f = mean[:, 0] + np.sqrt(var[:, 0]) * z
+        f = _as_host_tensor(f)
+        return f[0].reshape(-1, 1) if num_samples is None else f.reshape(S, -1, 1)
 
     def ucb_argmax(self, Xnew, varsigma):
         """Fused predict_y + ``mean + varsigma*var`` + first-max argmax.  Returns (index, mean, var, ucb)."""
