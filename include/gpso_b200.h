@@ -18,6 +18,8 @@
  *                (1-based); <0 = GPSO_E_* below.  No exception crosses the ABI; gpso_last_error() gives the text.
  *   - hyper-parameter vectors are packed in GPflow's trainable_variables order:
  *         [ lengthscale(s) (1, or d when ard) , kernel variance , likelihood (noise) variance , mean constant (if any) ]
+ *     GPSO_KERNEL_RQ puts its shape parameter alpha first (tf.Module lists kernel.alpha before kernel.lengthscales):
+ *         [ alpha , lengthscale(s) , kernel variance , likelihood (noise) variance , mean constant (if any) ]
  *     `u`     = unconstrained (softplus pre-image; noise variance has the 1e-6 floor of gpflow.likelihoods.Gaussian),
  *     `theta` = constrained values.
  */
@@ -42,7 +44,8 @@ enum {
 };
 
 /* gpflow.kernels.* accepted by GPRSurrogate(gp_kernel=...), gp_surrogate.py:393-402, default Matern52 (:424) */
-enum { GPSO_KERNEL_MATERN12 = 0, GPSO_KERNEL_MATERN32 = 1, GPSO_KERNEL_MATERN52 = 2, GPSO_KERNEL_SE = 3 };
+enum { GPSO_KERNEL_MATERN12 = 0, GPSO_KERNEL_MATERN32 = 1, GPSO_KERNEL_MATERN52 = 2, GPSO_KERNEL_SE = 3, GPSO_KERNEL_RQ = 4 };
+/* GPSO_KERNEL_RQ = gpflow.kernels.RationalQuadratic: variance * (1 + r2 / (2 alpha))^-alpha, alpha > 0 (softplus) */
 /* gpflow.mean_functions.*: None/Zero or Constant (:167, :427) */
 enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1 };
 

@@ -12,7 +12,7 @@ import os
 
 import numpy as np
 
-KERNEL_IDS = {"Matern12": 0, "Matern32": 1, "Matern52": 2, "SquaredExponential": 3}
+KERNEL_IDS = {"Matern12": 0, "Matern32": 1, "Matern52": 2, "SquaredExponential": 3, "RationalQuadratic": 4}
 _LIB_NAME = "libgpso_b200.so"
 _ABI_VERSION = 1
 

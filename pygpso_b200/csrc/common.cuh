@@ -10,6 +10,7 @@ constexpr int KERNEL_MATERN12 = 0;
 constexpr int KERNEL_MATERN32 = 1;
 constexpr int KERNEL_MATERN52 = 2;
 constexpr int KERNEL_SE = 3;
+constexpr int KERNEL_RQ = 4;  // gpflow.kernels.RationalQuadratic: one more hyper-parameter, the shape alpha
 
 constexpr int TB = 128;           // tile / panel edge: every dense matrix is padded to a multiple of TB
 constexpr double R2_CLIP = 1e-36; // GPflow clips the scaled squared distance before the sqrt (Matern kernels)
@@ -84,11 +85,90 @@ __device__ __forceinline__ double sqrt_pos(double x) {
     return fma(q, pl, t);
 }
 
+// exp_neg's constants for the W-wide forms below (the first object in constant memory: its bank offsets stay put)
+__constant__ double EXPNEG_C[16] = {
+    1.4426950408889634074,        // 0: log2(e)
+    6.93147180369123816490e-01,   // 1: ln2 high
+    1.90821492927058770002e-10,   // 2: ln2 low
+    1.0 / 6227020800.0, 1.0 / 479001600.0, 1.0 / 39916800.0, 1.0 / 3628800.0, 1.0 / 362880.0, 1.0 / 40320.0, 1.0 / 5040.0,
+    1.0 / 720.0, 1.0 / 120.0, 1.0 / 24.0, 1.0 / 6.0,  // 3..13: 1/13! .. 1/3!
+    2.23606797749978969641,       // 14: sqrt(5)
+    1.73205080756887729353,       // 15: sqrt(3)
+};
+
+// ---- log(1 + z) for z >= 0 --------------------------------------------------------------------------------------------
+// The RationalQuadratic covariance is var * exp(-alpha log1p(z)), z = r2 / (2 alpha): an absolute error d of log1p costs
+// k * alpha * d, unbounded in alpha, so log1p must be accurate RELATIVE to its result, also near z = 0.  Branch-free:
+//   z < sqrt2 - 1:  f = z exactly (no rounding of 1 + z), e = 0
+//   otherwise:      1 + z = u + c exactly (Fast2Sum of max(1, z) and min(1, z)), u = 2^e m, m in [sqrt(1/2), sqrt(2)), f = m - 1
+// and log1p(f) by fdlibm's e_log.c kernel: s = f / (2 + f), R(s^2) degree-7 minimax (error < 2^-58.45),
+//   log1p(z) = e ln2_hi - ((f^2/2 - (s (f^2/2 + R) + (e ln2_lo + c / u))) - f).
+// The reciprocal 1/(2 + f) is the MUFU.RCP64H seed with a third-order correction (as sqrt_pos); c / u <= 2^-53 is a
+// correction only where the result is >= log(sqrt 2), so the bare seed serves there.  Result within a few ulp relative
+// (tests/rq_oracle.py emulates it); exactly 0 at z = 0; +inf -> +inf; NaN -> NaN.  22 FP64-pipe operations.
+__constant__ double LOG1P_C[7] = {
+    6.666666666666735130e-01, 3.999999999940941908e-01, 2.857142874366239149e-01, 2.222219843214978396e-01,
+    1.818357216161805012e-01, 1.531383769920937332e-01, 1.479819860511658591e-01,  // fdlibm Lg1 .. Lg7
+};
+constexpr double LOG1P_SPLIT = 0.41421356237309503;  // sqrt(2) - 1
+
+__device__ __forceinline__ double rcp_pos(double x) {  // 1/x for x in [1, 3]: seed + third-order correction
+    double y;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
+    const double e = fma(-x, y, 1.0);
+    return fma(y, fma(e, e, e), y);
+}
+
+__device__ __forceinline__ double log1p_pos(double z) {
+    const bool big = z >= LOG1P_SPLIT;
+    const double a = big ? fmax(z, 1.0) : 1.0;
+    const double b = big ? fmin(z, 1.0) : z;
+    const double u = a + b;
+    const double c = b - (u - a);
+    int hx = __double2hiint(u) + (0x3ff00000 - 0x3fe6a09e);
+    const int e = big ? (hx >> 20) - 0x3ff : 0;
+    hx = (hx & 0x000fffff) + 0x3fe6a09e;
+    const double f = big ? __hiloint2double(hx, __double2loint(u)) - 1.0 : z;
+    double cu;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(cu) : "d"(u));
+    cu = big ? c * cu : 0.0;
+    const double s = f * rcp_pos(2.0 + f);
+    const double w = s * s;
+    double R = LOG1P_C[6];
+#pragma unroll
+    for (int i = 5; i >= 0; i--) R = fma(R, w, LOG1P_C[i]);
+    R *= w;
+    const double hfsq = 0.5 * f * f;
+    const double ed = (double)e;
+    const double v = fma(ed, 6.93147180369123816490e-01, -((hfsq - fma(s, hfsq + R, fma(ed, 1.90821492927058770002e-10, cu))) - f));
+    return (z > 1.7976931348623157e308) ? z : v;
+}
+
+// ---- z = r2 / (2 alpha) of the RationalQuadratic kernel ---------------------------------------------------------------
+// z = (r2 * ia) * sc with ia = 0.5 / (alpha / sc), both factors formed once per thread (rq_scale): two multiplications per
+// element instead of a division, within an ulp or two of GPflow's 0.5 * r2 / alpha.  sc = 1 while 0.5 / alpha is finite;
+// below alpha = 2^-1000 (softplus(u_alpha) for u_alpha < -693, which L-BFGS-B line searches do probe) 0.5 / alpha alone would
+// overflow and r2 = 0 would give 0 * inf = NaN, so alpha is scaled by 2^600 first: r2 = 0 gives z = 0 and z overflows to inf
+// where GPflow's quotient does.  alpha = 0 gives ia = inf; the callers select k = var there.
+__device__ __forceinline__ void rq_scale(double alpha, double& ia, double& sc) {
+    const bool tiny = alpha < 0x1p-1000;
+    sc = tiny ? 0x1p600 : 1.0;
+    ia = 0.5 / (tiny ? alpha * 0x1p600 : alpha);
+}
+__device__ __forceinline__ double rq_z(double r2, double ia, double sc) { return (r2 * ia) * sc; }
+
 // ---- covariance functions (gpflow.kernels.stationaries) ----------------------------------------------------------
-// r2 = scaled squared distance (inputs already divided by the lengthscale), var = kernel variance
+// r2 = scaled squared distance (inputs already divided by the lengthscale), var = kernel variance, alpha = the
+// RationalQuadratic shape (read by KERNEL_RQ only).  RQ: var * (1 + r2 / (2 alpha))^-alpha = var * exp(-alpha log1p(z));
+// alpha = 0 (softplus underflow) gives var for every pair, as pow(x, -0) = 1 does in GPflow.
 template <int KID>
-__device__ __forceinline__ double cov_from_r2(double r2, double var) {
-    if (KID == KERNEL_SE) {
+__device__ __forceinline__ double cov_from_r2(double r2, double var, double alpha) {
+    if (KID == KERNEL_RQ) {
+        double ia, sc;
+        rq_scale(alpha, ia, sc);
+        const double E = alpha * log1p_pos(rq_z(r2, ia, sc));
+        return var * exp_neg(alpha > 0.0 ? E : 0.0);
+    } else if (KID == KERNEL_SE) {
         return var * exp_neg(0.5 * r2);
     } else {
         double r = sqrt_pos(clip_r2(r2));
@@ -112,15 +192,6 @@ __device__ __forceinline__ double cov_from_r2(double r2, double var) {
 // arguments so that the W dependent chains interleave in the instruction stream (the scalar forms compile to one serial
 // chain per element, ~8 clk between dependent DFMAs), with the 64-bit polynomial coefficients read from the constant bank
 // as DFMA operands instead of being rebuilt by two UMOV / IMAD.MOV per use (28 of 140 instructions per element before).
-__constant__ double EXPNEG_C[16] = {
-    1.4426950408889634074,        // 0: log2(e)
-    6.93147180369123816490e-01,   // 1: ln2 high
-    1.90821492927058770002e-10,   // 2: ln2 low
-    1.0 / 6227020800.0, 1.0 / 479001600.0, 1.0 / 39916800.0, 1.0 / 3628800.0, 1.0 / 362880.0, 1.0 / 40320.0, 1.0 / 5040.0,
-    1.0 / 720.0, 1.0 / 120.0, 1.0 / 24.0, 1.0 / 6.0,  // 3..13: 1/13! .. 1/3!
-    2.23606797749978969641,       // 14: sqrt(5)
-    1.73205080756887729353,       // 15: sqrt(3)
-};
 
 template <int W>
 __device__ __forceinline__ void exp_neg_v(const double (&s)[W], double (&v)[W]) {
@@ -175,10 +246,62 @@ __device__ __forceinline__ void sqrt_pos_v(const double (&x)[W], double (&out)[W
     }
 }
 
+// log1p_pos over W arguments, the same operation sequence stage by stage
+template <int W>
+__device__ __forceinline__ void log1p_pos_v(const double (&z)[W], double (&out)[W]) {
+    double u[W], cu[W], f[W], ed[W], s[W], w[W], R[W];
+#pragma unroll
+    for (int i = 0; i < W; i++) {
+        const bool big = z[i] >= LOG1P_SPLIT;
+        const double a = big ? fmax(z[i], 1.0) : 1.0;
+        const double b = big ? fmin(z[i], 1.0) : z[i];
+        u[i] = a + b;
+        const double c = b - (u[i] - a);
+        int hx = __double2hiint(u[i]) + (0x3ff00000 - 0x3fe6a09e);
+        ed[i] = (double)(big ? (hx >> 20) - 0x3ff : 0);
+        hx = (hx & 0x000fffff) + 0x3fe6a09e;
+        f[i] = big ? __hiloint2double(hx, __double2loint(u[i])) - 1.0 : z[i];
+        double r;
+        asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(u[i]));
+        cu[i] = big ? c * r : 0.0;
+    }
+#pragma unroll
+    for (int i = 0; i < W; i++) s[i] = f[i] * rcp_pos(2.0 + f[i]);
+#pragma unroll
+    for (int i = 0; i < W; i++) {
+        w[i] = s[i] * s[i];
+        R[i] = LOG1P_C[6];
+    }
+#pragma unroll
+    for (int c = 5; c >= 0; c--) {
+#pragma unroll
+        for (int i = 0; i < W; i++) R[i] = fma(R[i], w[i], LOG1P_C[c]);
+    }
+#pragma unroll
+    for (int i = 0; i < W; i++) {
+        R[i] *= w[i];
+        const double hfsq = 0.5 * f[i] * f[i];
+        const double v = fma(ed[i], 6.93147180369123816490e-01,
+                             -((hfsq - fma(s[i], hfsq + R[i], fma(ed[i], 1.90821492927058770002e-10, cu[i]))) - f[i]));
+        out[i] = (z[i] > 1.7976931348623157e308) ? z[i] : v;
+    }
+}
+
 template <int KID, int W>
-__device__ __forceinline__ void cov_from_r2_v(const double (&r2)[W], double var, double (&k)[W]) {
+__device__ __forceinline__ void cov_from_r2_v(const double (&r2)[W], double var, double alpha, double (&k)[W]) {
     double s[W], e[W];
-    if (KID == KERNEL_SE) {
+    if (KID == KERNEL_RQ) {
+        double ia, sc;
+        rq_scale(alpha, ia, sc);
+#pragma unroll
+        for (int i = 0; i < W; i++) s[i] = rq_z(r2[i], ia, sc);
+        log1p_pos_v<W>(s, e);
+#pragma unroll
+        for (int i = 0; i < W; i++) s[i] = alpha > 0.0 ? alpha * e[i] : 0.0;
+        exp_neg_v<W>(s, e);
+#pragma unroll
+        for (int i = 0; i < W; i++) k[i] = var * e[i];
+    } else if (KID == KERNEL_SE) {
 #pragma unroll
         for (int i = 0; i < W; i++) s[i] = 0.5 * r2[i];
         exp_neg_v<W>(s, e);
@@ -211,9 +334,21 @@ __device__ __forceinline__ void cov_from_r2_v(const double (&r2)[W], double var,
 
 // covariance value and the radial factor g with  dK/d(ls_j) = g * Delta_j^2 / ls_j^3  (Delta in UNscaled units),
 // i.e. for a scalar lengthscale dK/d(ls) = g * r2 / ls.  g = 0 where r2 was clipped (GPflow: zero gradient there).
+// RQ also gives ka = dk/dalpha = k (z / (1 + z) - log1p(z)), 0 where k = 0; g = k / (1 + z).  alpha = 0: k = var, g = ka = 0 (the host
+// zeroes the alpha entry there: its chain factor sigmoid(u) is 0).
 template <int KID>
-__device__ __forceinline__ void cov_and_radial(double r2, double var, double& k, double& g) {
-    if (KID == KERNEL_SE) {
+__device__ __forceinline__ void cov_and_radial(double r2, double var, double alpha, double& k, double& g, double& ka) {
+    if (KID == KERNEL_RQ) {
+        double ia, sc;
+        rq_scale(alpha, ia, sc);
+        const double z = rq_z(r2, ia, sc);
+        const double l = log1p_pos(z);
+        const bool live = alpha > 0.0;
+        k = var * exp_neg(live ? alpha * l : 0.0);
+        const double iu = 1.0 / (1.0 + z);
+        g = live ? k * iu : 0.0;
+        ka = (live && k != 0.0) ? k * (z * iu - l) : 0.0;  // k = 0 (z = inf): the limit 0, not 0 * (inf * 0 - inf)
+    } else if (KID == KERNEL_SE) {
         k = var * exp_neg(0.5 * r2);
         g = k;
     } else {

@@ -276,6 +276,7 @@ struct gpso_handle {
     size_t scr_prod_marks = 0;
     // host copies of the hyper-parameters in force
     double ls_host[MAX_LS] = {0}, variance = 1.0, noise = 1.0, c0 = 0.0;
+    double rq_alpha = 1.0;  // RationalQuadratic shape (KERNEL_RQ only; the other kernels never read it)
     bool have_data = false, factorized = false;
     double factor_nlml = 0.0;
     double* host_rec = nullptr;  // pinned: results of an evaluation come back in one record without staging copies
@@ -297,7 +298,8 @@ struct gpso_handle {
     size_t trace_used = 0;
     std::vector<double> trace_out;
     int n_ls() const { return ard ? d : 1; }
-    int n_params() const { return n_ls() + 2 + (mean_id == GPSO_MEAN_CONSTANT ? 1 : 0); }
+    int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
+    int n_params() const { return n_rq() + n_ls() + 2 + (mean_id == GPSO_MEAN_CONSTANT ? 1 : 0); }
 };
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -335,7 +337,8 @@ static int l2_setaside(gpso_handle* h, size_t bytes) {
 template <int KID>
 static void launch_gram(gpso_handle* h, cudaStream_t st) {
     dim3 grid(h->Np / CT, h->Np / CT);
-    gram_kernel<KID><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->d, h->Np, h->variance, h->noise, h->K.as<double>());
+    gram_kernel<KID><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->d, h->Np, h->variance, h->noise, h->K.as<double>(),
+                                               h->rq_alpha);
 }
 
 template <int KID>
@@ -343,7 +346,7 @@ static void launch_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, l
     size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
     crosscov_kernel<KID><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
                                                                   h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                                  h->KsT.as<double>(), h->wmeanb[0].as<double>());
+                                                                  h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha);
 }
 
 template <int S>
@@ -356,10 +359,12 @@ static int oz_configure() {
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN32, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN52, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_SE, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_RQ, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN12, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN32, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN52, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_SE, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
+    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_RQ, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     return 0;
 }
 
@@ -377,10 +382,12 @@ static int screen_configure() {
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN32, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN52, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_SE, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
+    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_RQ, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN12, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN32, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN52, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_SE, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_RQ, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     return 0;
 }
 
@@ -394,7 +401,7 @@ static void launch_screen_crosscov(gpso_handle* h, cudaStream_t st, const double
                                    uint8_t* B, double* wmean) {
     crosscov_screen_kernel<KID, S, SCR_NT><<<(unsigned)ngroups, 256, screen_xcov_smem(h->d), st>>>(
         Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs32.as<float>(), h->alpha32.as<float>(), h->N, h->Np, (float)h->variance, h->c0,
-        bscale, h->Np / 32, B, wmean);
+        bscale, h->Np / 32, B, wmean, (float)h->rq_alpha);
 }
 
 template <int S>
@@ -404,6 +411,7 @@ static void launch_screen_crosscov_s(gpso_handle* h, cudaStream_t st, const doub
         case KERNEL_MATERN12: launch_screen_crosscov<KERNEL_MATERN12, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
         case KERNEL_MATERN32: launch_screen_crosscov<KERNEL_MATERN32, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
         case KERNEL_MATERN52: launch_screen_crosscov<KERNEL_MATERN52, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
+        case KERNEL_RQ: launch_screen_crosscov<KERNEL_RQ, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
         default: launch_screen_crosscov<KERNEL_SE, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
     }
 }
@@ -470,7 +478,7 @@ static void launch_oz_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc
                                uint8_t* B, double* wmean) {
     crosscov_slices_kernel<KID, S><<<(unsigned)nct, 256, oz_xcov_smem(h->d), st>>>(
         Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(), h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0, bscale,
-        h->Np / 32, B, wmean);
+        h->Np / 32, B, wmean, h->rq_alpha);
 }
 
 template <int S>
@@ -480,6 +488,7 @@ static void launch_oz_crosscov_s(gpso_handle* h, cudaStream_t st, const double* 
         case KERNEL_MATERN12: launch_oz_crosscov<KERNEL_MATERN12, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
         case KERNEL_MATERN32: launch_oz_crosscov<KERNEL_MATERN32, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
         case KERNEL_MATERN52: launch_oz_crosscov<KERNEL_MATERN52, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
+        case KERNEL_RQ: launch_oz_crosscov<KERNEL_RQ, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
         default: launch_oz_crosscov<KERNEL_SE, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
     }
 }
@@ -523,14 +532,14 @@ template <int KID>
 static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride) {
     if (!h->ard) {
         lml_grad_kernel<KID, false><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
-                                                         h->d, h->Np, h->variance, 0, 1, h->gpart.as<double>(), stride);
+                                                         h->d, h->Np, h->variance, 0, 1, h->gpart.as<double>(), stride, h->rq_alpha);
         h->launches++;
     } else {
         for (int dim0 = 0; dim0 < h->d; dim0 += GRAD_DCH) {
             int nd = std::min(GRAD_DCH, h->d - dim0);
             lml_grad_kernel<KID, true><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(),
                                                             h->N, h->d, h->Np, h->variance, dim0, nd, h->gpart.as<double>(),
-                                                            stride);
+                                                            stride, h->rq_alpha);
             h->launches++;
         }
     }
@@ -541,6 +550,7 @@ static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride) {
         case KERNEL_MATERN12: fn<KERNEL_MATERN12>(__VA_ARGS__); break;     \
         case KERNEL_MATERN32: fn<KERNEL_MATERN32>(__VA_ARGS__); break;     \
         case KERNEL_MATERN52: fn<KERNEL_MATERN52>(__VA_ARGS__); break;     \
+        case KERNEL_RQ: fn<KERNEL_RQ>(__VA_ARGS__); break;                 \
         default: fn<KERNEL_SE>(__VA_ARGS__); break;                        \
     }
 
@@ -562,6 +572,7 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN32>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN52>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_SE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_RQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(joint_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(diag_factor_inverse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(factor_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM_BYTES));
@@ -574,6 +585,7 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN32, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN52, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_SE, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
+    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_RQ, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(ozaki_screen_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ScrPairCfg::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_screen_pair_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     GP_TRY(screen_configure<2>());
@@ -1520,7 +1532,7 @@ extern "C" int gpso_destroy(gpso_handle* h);
 extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** out) {
     if (!out) return fail(GPSO_E_BADARG, "gpso_create: out is null");
     *out = nullptr;
-    if (kernel_id < 0 || kernel_id > 3) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
+    if (kernel_id < 0 || kernel_id > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
     if (mean_id != GPSO_MEAN_ZERO && mean_id != GPSO_MEAN_CONSTANT) return fail(GPSO_E_BADARG, "gpso_create: unknown mean id");
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) return fail(GPSO_E_NOGPU, "gpso_create: no CUDA device available");
@@ -1597,6 +1609,12 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
         snprintf(b, sizeof b, "%s: expected %d hyper-parameters, got %d", who, h->n_params(), p);
         return fail(GPSO_E_BADARG, b);
     }
+    if (h->n_rq()) {
+        if (!(theta[0] > 0.0) && !(allow_zero && theta[0] == 0.0))
+            return fail(GPSO_E_BADARG, std::string(who) + ": alpha must be positive");
+        h->rq_alpha = theta[0];
+        theta++;
+    }
     int nl = h->n_ls();
     for (int i = 0; i < nl; i++) {
         if (!(theta[i] > 0.0) && !(allow_zero && theta[i] == 0.0))
@@ -1616,12 +1634,15 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     if (!h->have_data) return fail(GPSO_E_STATE, "gpso_neg_lml_grad: call gpso_set_data first");
     if (p != h->n_params()) return fail(GPSO_E_BADARG, "gpso_neg_lml_grad: wrong number of hyper-parameters");
     GP_TRY(set_device(h));
-    const int nl = h->n_ls();
+    const int nl = h->n_ls(), na = h->n_rq();
     std::vector<double> theta(p);
-    for (int i = 0; i < nl; i++) theta[i] = softplus(u[i]);
-    theta[nl] = softplus(u[nl]);
-    theta[nl + 1] = NOISE_FLOOR + softplus(u[nl + 1]);
-    if (h->mean_id == GPSO_MEAN_CONSTANT) theta[nl + 2] = u[nl + 2];
+    for (int i = 0; i < na; i++) theta[i] = softplus(u[i]);  // alpha: positive, no floor
+    grad_host += na;  // the shared layout after alpha
+    u += na;
+    for (int i = 0; i < nl; i++) theta[na + i] = softplus(u[i]);
+    theta[na + nl] = softplus(u[nl]);
+    theta[na + nl + 1] = NOISE_FLOOR + softplus(u[nl + 1]);
+    if (h->mean_id == GPSO_MEAN_CONSTANT) theta[na + nl + 2] = u[nl + 2];
     // softplus(u) underflows to exactly 0 for u < -745 and L-BFGS-B line searches do probe such points: like GPflow, evaluate
     // them (kernel variance 0 -> K_y = noise * I; lengthscale 0 -> NaN objective) instead of rejecting the call
     GP_TRY(load_theta(h, theta.data(), p, "gpso_neg_lml_grad", true));
@@ -1631,7 +1652,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     GP_TRY(factor_pipeline(h, st, true));
     const int nb64 = h->Np / CT;
     const int nblk = nb64 * (nb64 + 1) / 2;
-    const int stride = 2 + nl;
+    const int stride = 2 + nl + na;
     GP_TRY(h->gpart.ensure((size_t)nblk * stride * sizeof(double)));
     GP_TRY(h->gout.ensure((size_t)(stride + 4) * sizeof(double)));
     DISPATCH_KID(h, launch_grad, h, st, nblk, stride);
@@ -1667,6 +1688,8 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     grad_host[nl] = h->variance > 0.0 ? -(0.5 * g[0] / h->variance) * sigmoid(u[nl]) : 0.0;
     grad_host[nl + 1] = -(0.5 * g[1]) * sigmoid(u[nl + 1]);
     if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[nl + 2] = -sc[2];
+    // alpha (slot stride - 1 of the partial sums); alpha == 0 only when softplus underflowed: the entry is 0, as for the variance
+    if (na) grad_host[-1] = h->rq_alpha > 0.0 ? -(0.5 * g[stride - 1]) * sigmoid(u[-1]) : 0.0;
     return 0;
 }
 
@@ -2011,6 +2034,9 @@ static void screen_error_model(const ScreenFit& f, int S, int full, double varsi
         est_var1 = 2.0 * sigma_f * unit * f.rho_max;   // first order:  2 sum_i v_i dv_i,  |v|_2 <= sigma_f
         est_var2 = unit * unit * f.rho_l2sq;           // second order: sum_i dv_i^2 (a bias; matters at 2 digits only)
     }
+    // the fp32 covariance contract of kern_screen.cuh, for every kernel family and, for RationalQuadratic, every alpha.  The
+    // rest of the model (pick_slices' digit scale, the mean bound of bound_argmax, the int8 engines) relies only on
+    // 0 <= k* <= variance, which RationalQuadratic satisfies too: no kernel-specific term anywhere else.
     const double eps_k32 = 2.0e-6 * f.variance;
     const double var_b = 2.0 * eps_k32 * sigma_f / sqrt(f.noise);
     const double var_epi = 1.0e-6 * f.variance;
@@ -2055,6 +2081,7 @@ static bool screen_applicable(const gpso_handle* h, long long M) {
     if (h->Np < min_np || M < SCREEN_MIN_M) return false;
     // the fp32 path needs the kernel variance and the lengthscales well inside the float range
     if (!(h->variance > 1e-30 && h->variance < 1e30)) return false;
+    if (h->n_rq() && !(h->rq_alpha > 1e-30 && h->rq_alpha < 1e30)) return false;
     for (int i = 0; i < h->n_ls(); i++)
         if (!(h->ls_host[i] > 1e-30 && h->ls_host[i] < 1e30)) return false;
     return true;
@@ -2570,14 +2597,15 @@ static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double*
     size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
     crosscov_kernel<KID><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
                                                               h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                              h->jKsT.as<double>(), h->jmean.as<double>());
+                                                              h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha);
 }
 
 template <int KID>
 static void launch_joint_syrk(gpso_handle* h, cudaStream_t st, int M, int Mp, double jitter) {
     const int mb = Mp / TB;
     joint_syrk_kernel<KID><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp, h->Np,
-                                                                               h->d, h->variance, jitter, h->jSigma.as<double>());
+                                                                               h->d, h->variance, jitter, h->jSigma.as<double>(),
+                                                                               h->rq_alpha);
 }
 
 // scaled candidates -> cross-covariance + mean -> V^T = (L^-1 K*)^T -> lower triangle of K** - V^T V (+ jitter I) in jSigma
@@ -2834,6 +2862,8 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 
 // ---------------------------------------------------------------------------------------------------------------------
 // multi-GPU state exchange: [ header (128 doubles) | Xs (d*Np) | alpha (Np) | Linv (Np*Np) ]
+// header: N, d, kernel variance, noise variance, mean constant, -LML, kernel id, ard, RationalQuadratic alpha (0 for the
+// other kernels), lengthscales from slot 16
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int STATE_HEADER = 128;
 
@@ -2861,6 +2891,7 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     hdr[5] = h->factor_nlml;
     hdr[6] = h->kernel_id;
     hdr[7] = h->ard;
+    if (h->n_rq()) hdr[8] = h->rq_alpha;
     for (int i = 0; i < h->n_ls(); i++) hdr[16 + i] = h->ls_host[i];
     double* dst = (double*)dst_dev;
     CU_TRY(cudaStreamSynchronize(h->stream));
@@ -2893,6 +2924,7 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     h->noise = hdr[3];
     h->c0 = hdr[4];
     h->factor_nlml = hdr[5];
+    if (h->n_rq()) h->rq_alpha = hdr[8];
     for (int i = 0; i < h->n_ls(); i++) h->ls_host[i] = hdr[16 + i];
     size_t Np = h->Np;
     CU_TRY(cudaMemcpyAsync(h->Xs.p, src + STATE_HEADER, sizeof(double) * d * Np, cudaMemcpyDeviceToDevice, st));

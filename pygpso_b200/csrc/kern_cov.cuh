@@ -23,7 +23,7 @@ constexpr int CDCH = 32;  // dimensions staged in shared memory per pass
 
 template <int KID>
 __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs, int N, int d, int Np, double var,
-                                                   double noise, double* __restrict__ K) {
+                                                   double noise, double* __restrict__ K, double rq_alpha) {
     const int bj = blockIdx.x, bi = blockIdx.y;
     if (bj > bi) return;
     __shared__ double sXi[CDCH][CT];
@@ -51,7 +51,7 @@ __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs
         int i = bi * CT + ty + 4 * r;
         double v;
         if (i < N && j < N) {
-            v = cov_from_r2<KID>(r2[r], var);
+            v = cov_from_r2<KID>(r2[r], var, rq_alpha);
             if (i == j) v += noise;
         } else {
             v = (i == j) ? 1.0 : 0.0;
@@ -73,7 +73,7 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
                                                        const double* __restrict__ ls, int n_ls,
                                                        const double* __restrict__ Xs, const double* __restrict__ alpha,
                                                        int N, int Np, double var, double c0, double* __restrict__ KsT,
-                                                       double* __restrict__ mean) {
+                                                       double* __restrict__ mean, double rq_alpha) {
     extern __shared__ double sm[];  // [XG][d] scaled candidate coords, then [8 warps][XG] reduction scratch
     double* sC = sm;
     double* sR = sm + XG * d;
@@ -102,7 +102,7 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
         double a = alpha[j];  // zero for j >= N
 #pragma unroll
         for (int c = 0; c < XG; c++) {
-            double k = (j < N && cbase + c < Mw) ? cov_from_r2<KID>(r2[c], var) : 0.0;
+            double k = (j < N && cbase + c < Mw) ? cov_from_r2<KID>(r2[c], var, rq_alpha) : 0.0;
             KsT[(size_t)(cbase + c) * Np + j] = k;
             macc[c] = fma(k, a, macc[c]);
         }
@@ -128,12 +128,14 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
 //   part[blk][0] = sum W*k            (-> d/d variance after / variance)
 //   part[blk][1] = sum_i W_ii         (-> d/d noise)
 //   part[blk][2 + q] = sum W*g*r2     (scalar lengthscale, q = 0)  or  sum W*g*(xs_i - xs_j)_dim^2 for dim = dim0+q
+//   part[blk][stride - 1] = sum W*dk/dalpha   (RationalQuadratic only: stride = 3 + n_ls)
 constexpr int GRAD_DCH = 4;  // ARD dimensions reduced per launch
 
 template <int KID, bool ARD>
 __global__ void __launch_bounds__(256) lml_grad_kernel(const double* __restrict__ Xs, const double* __restrict__ alpha,
                                                        const double* __restrict__ Kinv, int N, int d, int Np, double var,
-                                                       int dim0, int ndim, double* __restrict__ part, int part_stride) {
+                                                       int dim0, int ndim, double* __restrict__ part, int part_stride,
+                                                       double rq_alpha) {
     // triangular block index -> (bi, bj)
     int blk = blockIdx.x;
     int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
@@ -173,7 +175,7 @@ __global__ void __launch_bounds__(256) lml_grad_kernel(const double* __restrict_
             }
         }
     }
-    double s_k = 0.0, s_tr = 0.0, s_l[ARD ? GRAD_DCH : 1];
+    double s_k = 0.0, s_tr = 0.0, s_a = 0.0, s_l[ARD ? GRAD_DCH : 1];
 #pragma unroll
     for (int q = 0; q < (ARD ? GRAD_DCH : 1); q++) s_l[q] = 0.0;
     const double aj = alpha[j];
@@ -185,9 +187,10 @@ __global__ void __launch_bounds__(256) lml_grad_kernel(const double* __restrict_
         if (i < N && j < N) {
             double kin = (j <= i) ? Kinv[(size_t)i * Np + j] : Kinv[(size_t)j * Np + i];
             double W = fma(alpha[i], aj, -kin) * wsym;
-            double k, g;
-            cov_and_radial<KID>(r2[r], var, k, g);
+            double k, g, ka;
+            cov_and_radial<KID>(r2[r], var, rq_alpha, k, g, ka);
             s_k = fma(W, k, s_k);
+            if (KID == KERNEL_RQ) s_a = fma(W, ka, s_a);
             if (i == j) s_tr += W;
             double wg = W * g;
             if (ARD) {
@@ -203,6 +206,10 @@ __global__ void __launch_bounds__(256) lml_grad_kernel(const double* __restrict_
     if (threadIdx.x == 0 && dim0 == 0) part[(size_t)blk * part_stride + 0] = v;
     v = block_sum<256>(s_tr, sRed);
     if (threadIdx.x == 0 && dim0 == 0) part[(size_t)blk * part_stride + 1] = v;
+    if (KID == KERNEL_RQ) {
+        v = block_sum<256>(s_a, sRed);
+        if (threadIdx.x == 0 && dim0 == 0) part[(size_t)blk * part_stride + part_stride - 1] = v;
+    }
 #pragma unroll
     for (int q = 0; q < (ARD ? GRAD_DCH : 1); q++) {
         v = block_sum<256>(s_l[q], sRed);

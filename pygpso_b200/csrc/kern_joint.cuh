@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_v_kernel(JointVParams P) {
 template <int KID>
 __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* __restrict__ VT, const double* __restrict__ Xcs, int M,
                                                                  int Mp, int Np, int d, double var, double jitter,
-                                                                 double* __restrict__ Sigma) {
+                                                                 double* __restrict__ Sigma, double rq_alpha) {
     extern __shared__ double smem[];
     int a, b;
     tri_index(blockIdx.x, a, b);
@@ -115,7 +115,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* _
                 const double df = Xcs[(size_t)dim * Mp + gi] - Xcs[(size_t)dim * Mp + gj];
                 r2 = fma(df, df, r2);
             }
-            v = cov_from_r2<KID>(r2, var) - smem[r * JST + c];
+            v = cov_from_r2<KID>(r2, var, rq_alpha) - smem[r * JST + c];
             if (gi == gj) v += jitter;
         }
         Sigma[(size_t)gi * Mp + gj] = v;

@@ -379,7 +379,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                                                               const double* __restrict__ ls, int n_ls,
                                                               const double* __restrict__ Xs, const double* __restrict__ alpha, int N,
                                                               int Np, double var, double c0, double bscale, int nks,
-                                                              uint8_t* __restrict__ B, double* __restrict__ mean) {
+                                                              uint8_t* __restrict__ B, double* __restrict__ mean, double rq_alpha) {
     extern __shared__ double sm[];
     double* sC = sm;                      // [d][64]       scaled candidate coordinates, dimension-major
     double* sX = sC + d * OZ_NT;          // [2][d][128]   scaled training coordinates of the current / next super-step
@@ -446,7 +446,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                 double rr[XW], kk[XW];
 #pragma unroll
                 for (int i = 0; i < XW; i++) rr[i] = r2[a][g + i];
-                cov_from_r2_v<KID, XW>(rr, var, kk);
+                cov_from_r2_v<KID, XW>(rr, var, rq_alpha, kk);
 #pragma unroll
                 for (int i = 0; i < XW; i++) {
                     const double k = (cvalid[a] && j0 + g + i < N) ? kk[i] : 0.0;

@@ -69,9 +69,28 @@ struct ScrParams {
 // ---- FP32 covariance (screening only) -----------------------------------------------------------------------------------
 // Absolute error against the fp64 evaluation below 2e-6 * variance for every kernel family (tests/test_screen_model.py
 // checks the same formulas in numpy float32; MUFU.EX2 / MUFU.RSQ add ~2 ulp each).  NaN propagates.
+//
+// RationalQuadratic: k = var * 2^(-alpha log2(1 + z)), z = r2 / (2 alpha).  An absolute error d of log2(1 + z) costs
+// k * alpha * ln2 * d, unbounded in alpha, so log2(1 + z) must be accurate relative to its result:
+//   z <  1/4:  z * P(z), P the degree-5 relative-minimax fit of log2(1 + z) / z (fit error 9e-9, 1.2e-7 after fp32 Horner)
+//   z >= 1/4:  MUFU.LG2 of fl(1 + z): absolute error ~1.6e-7 plus the rounding of 1 + z, on a result >= log2(1.25) = 0.32
+// i.e. a relative error rho < 8e-7, and since x e^-x <= 1/e the covariance error stays below var * rho / e for every alpha.
+// tests/rq_oracle.py emulates this evaluation in numpy float32.
+constexpr float RQ32_SPLIT = 0.25f;
+__constant__ float RQ32_P[6] = {  // log2(e) times the fit of log1p(z) / z on [0, 1/4]
+    1.4426950216293335f, -0.7213437557220459f, 0.48071789741516113f, -0.357472687959671f, 0.26215097308158875f, -0.1332305371761322f,
+};
+
 template <int KID>
-__device__ __forceinline__ float cov32_from_r2(float r2, float var) {
-    if (KID == KERNEL_SE) {
+__device__ __forceinline__ float cov32_from_r2(float r2, float var, float alpha) {
+    if (KID == KERNEL_RQ) {
+        const float z = r2 * __fdividef(0.5f, alpha);
+        float p = RQ32_P[5];
+#pragma unroll
+        for (int i = 4; i >= 0; i--) p = fmaf(p, z, RQ32_P[i]);
+        const float l2 = (z < RQ32_SPLIT) ? z * p : __log2f(1.0f + z);
+        return var * exp2f(-alpha * l2);
+    } else if (KID == KERNEL_SE) {
         return var * __expf(-0.5f * r2);
     } else {
         const float c = (r2 < 1e-36f) ? 1e-36f : r2;
@@ -130,12 +149,34 @@ __device__ __forceinline__ float scr_rsqrt(float x) {
 }
 
 // cov32_from_r2 for the two halves of a packed pair (same formulas; exp(-s) = 2^(-s log2 e))
+__device__ __forceinline__ float scr_lg2(float x) {
+    float y;
+    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+
 template <int KID>
-__device__ __forceinline__ f32x2_t cov32x2_from_r2(f32x2_t r2, float var) {
+__device__ __forceinline__ f32x2_t cov32x2_from_r2(f32x2_t r2, float var, float alpha) {
     const float L2E = 1.4426950408889634f;
     const f32x2_t var2 = f2_pack(var, var);
     float a, b;
-    if (KID == KERNEL_SE) {
+    if (KID == KERNEL_RQ) {
+        const float ia = __fdividef(0.5f, alpha);
+        const f32x2_t z = f2_mul(r2, f2_pack(ia, ia));
+        f32x2_t p = f2_pack(RQ32_P[5], RQ32_P[5]);
+#pragma unroll
+        for (int i = 4; i >= 0; i--) p = f2_fma(p, z, f2_pack(RQ32_P[i], RQ32_P[i]));
+        p = f2_mul(p, z);
+        const f32x2_t u = f2_add(z, f2_pack(1.0f, 1.0f));
+        float za, zb, pa, pb, ua, ub;
+        f2_unpack(z, za, zb);
+        f2_unpack(p, pa, pb);
+        f2_unpack(u, ua, ub);
+        // z < 1/4 (and not NaN): the polynomial; otherwise the MUFU logarithm (NaN propagates through it)
+        const f32x2_t l2 = f2_pack((za < RQ32_SPLIT) ? pa : scr_lg2(ua), (zb < RQ32_SPLIT) ? pb : scr_lg2(ub));
+        f2_unpack(f2_mul(l2, f2_pack(-alpha, -alpha)), a, b);
+        return f2_mul(var2, f2_pack(scr_ex2(a), scr_ex2(b)));
+    } else if (KID == KERNEL_SE) {
         const f32x2_t t = f2_mul(r2, f2_pack(-0.5f * L2E, -0.5f * L2E));
         f2_unpack(t, a, b);
         return f2_mul(var2, f2_pack(scr_ex2(a), scr_ex2(b)));
@@ -194,7 +235,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                                                                  const double* __restrict__ ls, int n_ls,
                                                                  const float* __restrict__ Xs32, const float* __restrict__ alpha32,
                                                                  int N, int Np, float var, double c0, float bscale, int nks,
-                                                                 uint8_t* __restrict__ B, double* __restrict__ mean) {
+                                                                 uint8_t* __restrict__ B, double* __restrict__ mean, float rq_alpha) {
     extern __shared__ __align__(16) float smf[];
     float* sC = smf;                       // [d][64]
     float* sX = sC + d * 64;               // [2][d][128]
@@ -273,7 +314,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
         const bool tail = j0 + 16 > N;
 #pragma unroll
         for (int g = 0; g < 16; g++) {
-            f32x2_t k2 = cov32x2_from_r2<KID>(r2[g], var);
+            f32x2_t k2 = cov32x2_from_r2<KID>(r2[g], var, rq_alpha);
             float k0, k1;
             f2_unpack(k2, k0, k1);
             k0 = cvalid[0] ? k0 : 0.0f;

@@ -18,7 +18,7 @@ implementation in this package.
 
 Parameterisation follows GPflow 2: positive parameters are softplus-transformed, the Gaussian likelihood variance has
 the 1e-6 floor, and ``trainable_variables`` are ordered kernel.lengthscales, kernel.variance, likelihood.variance,
-mean_function.c.
+mean_function.c -- preceded by kernel.alpha for ``RationalQuadratic`` (tf.Module visits attributes in sorted name order).
 """
 import types
 
@@ -158,6 +158,21 @@ class SquaredExponential(Stationary):
 RBF = SquaredExponential
 
 
+class RationalQuadratic(Stationary):
+    """``gpflow.kernels.RationalQuadratic``: ``variance * (1 + r2 / (2 alpha))^-alpha``, a scale mixture of squared
+    exponentials; ``alpha`` (positive, softplus) sets how heavy the tail is, alpha -> inf gives the SquaredExponential."""
+
+    def __init__(self, variance=1.0, lengthscales=1.0, alpha=1.0):
+        super().__init__(variance=variance, lengthscales=lengthscales)
+        self.alpha = Parameter(alpha, positive=True, name="kernel.alpha")
+        if self.alpha.size != 1:
+            raise ValueError("alpha must be a scalar")
+
+    @property
+    def parameters(self):
+        return (self.alpha, self.lengthscales, self.variance)
+
+
 class MeanFunction:
     parameters = ()
 
@@ -216,7 +231,7 @@ class GPR(GPModel):
 
     def __init__(self, data, kernel, mean_function=None, noise_variance=1.0, backend=None):
         if not isinstance(kernel, Stationary):
-            raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential")
+            raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic")
         self.kernel = kernel
         self.mean_function = Zero() if mean_function is None else mean_function
         if not isinstance(self.mean_function, (Zero, Constant)):
@@ -253,7 +268,7 @@ class GPR(GPModel):
     # -- parameters ---------------------------------------------------------------------------------------------------
     @property
     def _ordered_parameters(self):
-        params = [self.kernel.lengthscales, self.kernel.variance, self.likelihood.variance]
+        params = list(self.kernel.parameters) + [self.likelihood.variance]
         params.extend(self.mean_function.parameters)
         return params
 
@@ -275,7 +290,7 @@ class GPR(GPModel):
             pos += p.size
 
     def _theta(self):
-        """Constrained vector in packing order: lengthscale(s), kernel variance, noise variance, [mean c]."""
+        """Constrained vector in packing order: [alpha], lengthscale(s), kernel variance, noise variance, [mean c]."""
         return np.concatenate([np.asarray(p, dtype=np.float64).reshape(-1) for p in self._ordered_parameters])
 
     # -- objective ----------------------------------------------------------------------------------------------------
@@ -406,11 +421,12 @@ class Scipy:
 # gpflow.utilities look-alikes (used by save / load)
 # ---------------------------------------------------------------------------------------------------------------------
 def parameter_dict(model):
-    out = {
+    out = {".kernel.alpha": model.kernel.alpha} if isinstance(model.kernel, RationalQuadratic) else {}
+    out.update({
         ".kernel.lengthscales": model.kernel.lengthscales,
         ".kernel.variance": model.kernel.variance,
         ".likelihood.variance": model.likelihood.variance,
-    }
+    })
     if isinstance(model.mean_function, Constant):
         out[".mean_function.c"] = model.mean_function.c
     return out
@@ -438,7 +454,7 @@ def tabulate_module_summary(model):
 
 kernels = types.SimpleNamespace(
     Kernel=Kernel, Stationary=Stationary, Matern12=Matern12, Matern32=Matern32, Matern52=Matern52,
-    SquaredExponential=SquaredExponential, RBF=RBF,
+    SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic,
 )
 mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant)
 likelihoods = types.SimpleNamespace(Gaussian=Gaussian)
