@@ -236,11 +236,6 @@ int gpso_set_screen_mode(gpso_handle* h, int mode);
  * launches, out[8] refine windows, out[9] E_var, out[10] E_mean, out[11] 1 when the screening product kept all digit pairs (path 1); mode
  * 5: admissible distance below the best mean (path 4) */
 int gpso_screen_info(gpso_handle* h, double* out12);
-/* 3-digit screening product as CTA pairs (tcgen05.mma.cta_group::2, the B digits of a k-step split between the two shared
- * memories of a TPC; needs an even number of 128-row blocks) or as single CTAs (default: the pair form moves 17 % fewer
- * bytes into shared memory and reads 30 % fewer from it, but measured 5.48 vs 5.37 ms per window at N = 4096 -- the kernel is
- * bound by the accumulator hand-over, not by operand traffic); bit-identical results */
-int gpso_set_screen_pair(gpso_handle* h, int enabled);
 /* Pipe peaks of GPU `device`, measured now (~0.2 s): out4 = {int8 tensor TOP/s (tcgen05 kind::i8 issue rate), FP64 TFLOP/s
  * (DMMA.8x8x4 issue rate), L2 -> shared-memory bulk-copy GB/s, number of SMs}.  bench.py divides by these. */
 int gpso_probe_peaks(int device, double* out4);

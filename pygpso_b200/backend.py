@@ -124,7 +124,6 @@ def load_library():
         "gpso_set_l2_window": (i32, [H, i32]),
         "gpso_set_screen_mode": (i32, [H, i32]),
         "gpso_screen_info": (i32, [H, _c_double_p]),
-        "gpso_set_screen_pair": (i32, [H, i32]),
         "gpso_probe_peaks": (i32, [i32, _c_double_p]),
         "gpso_debug_screen_bound": (i32, [i32, dbl, dbl, _c_double_p, i32, i32, dbl, _c_double_p]),
         "gpso_debug_product_items": (i64, [i32, i32, i32, ctypes.POINTER(ctypes.c_int), i64, ctypes.POINTER(ctypes.c_int), i32,
@@ -152,7 +151,7 @@ EXPORTED_SYMBOLS = (
     "gpso_export_state_dev gpso_import_state_dev gpso_launch_count gpso_debug_fetch gpso_last_timing gpso_set_window "
     "gpso_set_profile gpso_last_windows gpso_set_predict_mode gpso_predict_info gpso_set_overlap "
     "gpso_set_factor_mode gpso_factor_info gpso_trim_pool gpso_debug_screen_windows gpso_debug_hybrid_plan gpso_debug_hybrid_items gpso_debug_factor_tasks gpso_debug_factor_tasks_cap gpso_debug_trace gpso_set_kinv_mode gpso_set_inverse_mode gpso_set_l2_window gpso_debug_product_items "
-    "gpso_set_screen_mode gpso_screen_info gpso_debug_screen_bound gpso_probe_peaks gpso_set_screen_pair"
+    "gpso_set_screen_mode gpso_screen_info gpso_debug_screen_bound gpso_probe_peaks"
 ).split()
 
 
@@ -398,10 +397,6 @@ class CudaSession:
         level first, 6 forced 2 digits with all digit pairs; results are bit-identical."""
         self.factorized = False
         _check(self._lib, self._lib.gpso_set_screen_mode(self._h, int(mode)), "gpso_set_screen_mode")
-
-    def set_screen_pair(self, enabled=True):
-        """3-digit screening product as CTA pairs (cta_group::2, default) or single CTAs; identical results."""
-        _check(self._lib, self._lib.gpso_set_screen_pair(self._h, int(bool(enabled))), "gpso_set_screen_pair")
 
     def screened_values(self, count):
         """Screened UCB (or mean, bound level) of the first ``count`` candidates of the last screened call (tests)."""

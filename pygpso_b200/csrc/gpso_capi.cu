@@ -13,6 +13,7 @@
 
 #include <algorithm>
 #include <array>
+#include <functional>
 #include <string>
 #include <map>
 #include <mutex>
@@ -219,7 +220,6 @@ struct gpso_handle {
     int chol_mode = 1;      // 1 = persistent dataflow kernel, 0 = one launch per step (reference schedule)
     // predict workspaces
     DevBuf KsT, part, blockbest, running, cand[2], leaves, omean, ovar, topk;
-    int topk_k = 0;         // records per window of the top-k pass in flight
     // joint posterior (kern_joint.cuh): scaled candidates, cross-covariance, mean, V^T, Sigma; for the samples the factor's
     // scratch (inverse diagonal blocks and their transposes, log-determinant, pivot status, scheduler state) and the padded
     // normals; host staging of candidates, normals and outputs.  Separate from the fit's buffers, which a joint call never touches.
@@ -247,7 +247,7 @@ struct gpso_handle {
     int hybrid_mode = 0;    // 0 = automatic (matrices of more than HYB_MIN_TILES tiles), 1 = off, 2 = always (leaves of 2 tiles: tests)
     int hybrid_nodes = 0;   // inner nodes of the last factorisation (0 = one persistent kernel)
     cudaStream_t aux_stream = nullptr;
-    cudaEvent_t ev_probe = nullptr;  // early verdict of a screening rung (run_screen_windows)
+    cudaEvent_t ev_probe = nullptr;  // early verdict of a screening rung (screen_pass)
     cudaEvent_t ev_start = nullptr, ev_xcov[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
     int overlap = 1;
     int predict_mode = 0;   // 0 = automatic, 1 = FP64 DMMA product, 2 = int8 tcgen05 product
@@ -261,8 +261,6 @@ struct gpso_handle {
     int screen_mode = 1;        // 0 off, 1 automatic (digits adapt to the survivor fraction), 2..4 forced digits
     int screen_S_cur = 0;       // rung of SCREEN_LADDER the automatic mode starts from
     int screen_built_S = 0;     // digits of the tiles in ozAs (0: stale)
-    int screen_pair = 0;        // CTA-pair (cta_group::2) form of the 3-digit screening product (gpso_set_screen_pair); measured no
-                                // faster than single CTAs (5.48 vs 5.37 ms per 174 080-candidate window at N = 4096): off by default
     bool screen_ready = false;  // fp32 copies and norms valid for the factor in force
     double alpha_l2 = 0.0, rho_max = 0.0, rho_l2sq = 0.0;
     double linv_frob2 = 0.0, linv_rowl2_max = 0.0;  // |L^-1|_F^2 (= tr K_y^-1) and the largest row norm of L^-1
@@ -270,9 +268,6 @@ struct gpso_handle {
     // [2] survivors, [3] E, [4] max |refined - screened| over the survivors, [5] best screened UCB, [6] screen windows,
     // [7] screening product ms, [8] refine windows, [9] E_var, [10] E_mean
     double scr_info[12] = {0};
-    const long long* rw_idx_map = nullptr;  // run_windows: global indices of the (gathered) candidates
-    bool rw_check = false;                  // run_windows: compare refined and screened UCB of every candidate
-    bool rw_check_mean = false;             // ... the stored value is the screened mean (bound-and-refine level 0)
     size_t scr_prod_marks = 0;
     // host copies of the hyper-parameters in force
     double ls_host[MAX_LS] = {0}, variance = 1.0, noise = 1.0, c0 = 0.0;
@@ -334,19 +329,38 @@ static int l2_setaside(gpso_handle* h, size_t bytes) {
     return 0;
 }
 
-template <int KID>
+// The covariance families, in one list: AllKernels::with runs f with a kernel id as a compile-time constant (gpso_create accepts
+// no other id), AllKernels::each runs it for every family and stops at the first error.
+template <int... KIDS>
+struct KernelIds {
+    template <class F>
+    static void with(int kid, F&& f) {
+        (void)((kid == KIDS ? (f(std::integral_constant<int, KIDS>()), true) : false) || ...);
+    }
+    template <class F>
+    static int each(F&& f) {
+        int rc = 0;
+        (void)(((rc = f(std::integral_constant<int, KIDS>())) == 0) && ...);
+        return rc;
+    }
+};
+using AllKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ>;
+
 static void launch_gram(gpso_handle* h, cudaStream_t st) {
     dim3 grid(h->Np / CT, h->Np / CT);
-    gram_kernel<KID><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->d, h->Np, h->variance, h->noise, h->K.as<double>(),
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        gram_kernel<kid><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->d, h->Np, h->variance, h->noise, h->K.as<double>(),
                                                h->rq_alpha);
+    });
 }
 
-template <int KID>
 static void launch_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long Mw_pad) {
     size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
-    crosscov_kernel<KID><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
-                                                                  h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                                  h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha);
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        crosscov_kernel<kid><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
+                                                                      h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
+                                                                      h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha);
+    });
 }
 
 template <int S>
@@ -355,17 +369,11 @@ static int oz_configure() {
     // full shared-memory carve-out for both kernels: the persistent product CTA (one per SM) must leave room for a
     // cross-covariance block of the next window on the same SM (they use different pipes and overlap)
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<S, OZ_TRMM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN12, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN32, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN52, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_SE, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_RQ, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN12, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN32, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_MATERN52, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_SE, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<KERNEL_RQ, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    return 0;
+    return AllKernels::each([](auto kid) -> int {
+        CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<kid, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<kid, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
+        return 0;
+    });
 }
 
 template <int S>
@@ -374,54 +382,32 @@ static int screen_configure() {
     CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<S, SCR_NT, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (S == 2) {
         CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<2, SCR_NT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ScrCfg<2, SCR_NT, true>::SMEM_BYTES));
-        CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<2, SCR_NT, true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, ScrCfg<2, SCR_NT, true, 4>::SMEM_BYTES));
         CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<2, SCR_NT, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<2, SCR_NT, true, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN12, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN32, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN52, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_SE, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_RQ, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN12, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN32, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN52, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_SE, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_RQ, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    return 0;
+    return AllKernels::each([](auto kid) -> int {
+        CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
+        CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        return 0;
+    });
 }
 
 static size_t screen_xcov_smem(int d) {
-    static const int pad_env = getenv("GPSO_SCR_XCOV_PAD") ? atoi(getenv("GPSO_SCR_XCOV_PAD")) : 0;  // co-residency experiments
-    return (size_t)(64 * d + 2 * d * OZ_XK + 2 * OZ_XK) * sizeof(float) + 8 * 64 * sizeof(double) + pad_env;
+    return (size_t)(64 * d + 2 * d * OZ_XK + 2 * OZ_XK) * sizeof(float) + 8 * 64 * sizeof(double);
 }
 
-template <int KID, int S>
+// S = 0: posterior mean only (bound pass)
+template <int S>
 static void launch_screen_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long ngroups, float bscale,
                                    uint8_t* B, double* wmean) {
-    crosscov_screen_kernel<KID, S, SCR_NT><<<(unsigned)ngroups, 256, screen_xcov_smem(h->d), st>>>(
-        Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs32.as<float>(), h->alpha32.as<float>(), h->N, h->Np, (float)h->variance, h->c0,
-        bscale, h->Np / 32, B, wmean, (float)h->rq_alpha);
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        crosscov_screen_kernel<kid, S, SCR_NT><<<(unsigned)ngroups, 256, screen_xcov_smem(h->d), st>>>(
+            Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs32.as<float>(), h->alpha32.as<float>(), h->N, h->Np, (float)h->variance,
+            h->c0, bscale, h->Np / 32, B, wmean, (float)h->rq_alpha);
+    });
 }
 
-template <int S>
-static void launch_screen_crosscov_s(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long ngroups, float bscale,
-                                     uint8_t* B, double* wmean) {
-    switch (h->kernel_id) {
-        case KERNEL_MATERN12: launch_screen_crosscov<KERNEL_MATERN12, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
-        case KERNEL_MATERN32: launch_screen_crosscov<KERNEL_MATERN32, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
-        case KERNEL_MATERN52: launch_screen_crosscov<KERNEL_MATERN52, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
-        case KERNEL_RQ: launch_screen_crosscov<KERNEL_RQ, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
-        default: launch_screen_crosscov<KERNEL_SE, S>(h, st, Xc, Mw, ngroups, bscale, B, wmean); break;
-    }
-}
-
-static bool screen_pair_enabled(const gpso_handle* h, int S) {
-    return h->screen_pair && S == ScrPairCfg::S && (h->nb % 2) == 0 && h->nsm >= 2;
-}
-
-template <int S, bool FULL, int KPSV = SCR_KPS>
-static void launch_screen_product_v(gpso_handle* h, cudaStream_t st, long long nct, long long ldp, double gscale, const uint8_t* B) {
+template <int S, bool FULL = false>
+static void launch_screen_product(gpso_handle* h, cudaStream_t st, long long nct, long long ldp, double gscale, const uint8_t* B) {
     ScrParams P;
     P.A = h->ozAs.as<uint8_t>();
     P.B = B;
@@ -432,30 +418,9 @@ static void launch_screen_product_v(gpso_handle* h, cudaStream_t st, long long n
     P.nks = h->Np / 32;
     P.nct = (int)nct;
     P.ldp = ldp;
-    // ring depth: the whole budget unless GPSO_SCR_STAGES asks for less (co-residency experiments)
-    static const int stages_env = getenv("GPSO_SCR_STAGES") ? atoi(getenv("GPSO_SCR_STAGES")) : 0;
-    using Cfg = ScrCfg<S, SCR_NT, FULL, KPSV>;
-    P.stages = (stages_env >= 2 && stages_env < Cfg::STAGES) ? stages_env : Cfg::STAGES;
-    static const int epi_env = getenv("GPSO_SCR_DEBUG_EPI") ? atoi(getenv("GPSO_SCR_DEBUG_EPI")) : 0;  // timing experiments only
-    P.debug_epi = epi_env;
-    if (!FULL && screen_pair_enabled(h, S)) {
-        // CTA pairs (cta_group::2): one cluster per TPC, each pair works on two adjacent row blocks of one candidate tile
-        P.stages = ScrPairCfg::STAGES;
-        const int nbp = h->nb / 2;
-        const long long punits = nct * ((nbp + 1) / 2);
-        const int clusters = (int)std::min<long long>(h->nsm / 2, punits);
-        ozaki_screen_pair_kernel<<<2 * clusters, OZ_THREADS, ScrPairCfg::SMEM_BYTES, st>>>(P);
-        return;
-    }
-    const size_t smem = (size_t)P.stages * Cfg::STAGE_BYTES + (Cfg::SMEM_BYTES - Cfg::RING_BYTES);
     const long long units = nct * ((h->nb + 1) / 2);
     const int grid = (int)std::min<long long>(h->nsm, units);
-    ozaki_screen_kernel<S, SCR_NT, FULL, KPSV><<<grid, OZ_THREADS, smem, st>>>(P);
-}
-
-template <int S>
-static void launch_screen_product(gpso_handle* h, cudaStream_t st, long long nct, long long ldp, double gscale, const uint8_t* B) {
-    launch_screen_product_v<S, false>(h, st, nct, ldp, gscale, B);
+    ozaki_screen_kernel<S, SCR_NT, FULL><<<grid, OZ_THREADS, ScrCfg<S, SCR_NT, FULL>::SMEM_BYTES, st>>>(P);
 }
 
 template <int S>
@@ -473,24 +438,14 @@ static void launch_screen_slices(gpso_handle* h, cudaStream_t st) {
 
 static size_t oz_xcov_smem(int d) { return (size_t)(OZ_NT * d + 2 * d * OZ_XK + 2 * OZ_XK + 8 * OZ_NT) * sizeof(double); }
 
-template <int KID, int S>
+template <int S>
 static void launch_oz_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long nct, double bscale,
                                uint8_t* B, double* wmean) {
-    crosscov_slices_kernel<KID, S><<<(unsigned)nct, 256, oz_xcov_smem(h->d), st>>>(
-        Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(), h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0, bscale,
-        h->Np / 32, B, wmean, h->rq_alpha);
-}
-
-template <int S>
-static void launch_oz_crosscov_s(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long nct, double bscale,
-                                 uint8_t* B, double* wmean) {
-    switch (h->kernel_id) {
-        case KERNEL_MATERN12: launch_oz_crosscov<KERNEL_MATERN12, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
-        case KERNEL_MATERN32: launch_oz_crosscov<KERNEL_MATERN32, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
-        case KERNEL_MATERN52: launch_oz_crosscov<KERNEL_MATERN52, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
-        case KERNEL_RQ: launch_oz_crosscov<KERNEL_RQ, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
-        default: launch_oz_crosscov<KERNEL_SE, S>(h, st, Xc, Mw, nct, bscale, B, wmean); break;
-    }
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        crosscov_slices_kernel<kid, S><<<(unsigned)nct, 256, oz_xcov_smem(h->d), st>>>(
+            Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(), h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
+            bscale, h->Np / 32, B, wmean, h->rq_alpha);
+    });
 }
 
 template <int S>
@@ -528,31 +483,23 @@ static void launch_oz_slices(gpso_handle* h, cudaStream_t st) {
         default: fn<8>(__VA_ARGS__); break;    \
     }
 
-template <int KID>
 static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride) {
-    if (!h->ard) {
-        lml_grad_kernel<KID, false><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
-                                                         h->d, h->Np, h->variance, 0, 1, h->gpart.as<double>(), stride, h->rq_alpha);
-        h->launches++;
-    } else {
-        for (int dim0 = 0; dim0 < h->d; dim0 += GRAD_DCH) {
-            int nd = std::min(GRAD_DCH, h->d - dim0);
-            lml_grad_kernel<KID, true><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(),
-                                                            h->N, h->d, h->Np, h->variance, dim0, nd, h->gpart.as<double>(),
-                                                            stride, h->rq_alpha);
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        if (!h->ard) {
+            lml_grad_kernel<kid, false><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
+                                                             h->d, h->Np, h->variance, 0, 1, h->gpart.as<double>(), stride, h->rq_alpha);
             h->launches++;
+        } else {
+            for (int dim0 = 0; dim0 < h->d; dim0 += GRAD_DCH) {
+                int nd = std::min(GRAD_DCH, h->d - dim0);
+                lml_grad_kernel<kid, true><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(),
+                                                                h->N, h->d, h->Np, h->variance, dim0, nd, h->gpart.as<double>(),
+                                                                stride, h->rq_alpha);
+                h->launches++;
+            }
         }
-    }
+    });
 }
-
-#define DISPATCH_KID(h, fn, ...)                                           \
-    switch ((h)->kernel_id) {                                              \
-        case KERNEL_MATERN12: fn<KERNEL_MATERN12>(__VA_ARGS__); break;     \
-        case KERNEL_MATERN32: fn<KERNEL_MATERN32>(__VA_ARGS__); break;     \
-        case KERNEL_MATERN52: fn<KERNEL_MATERN52>(__VA_ARGS__); break;     \
-        case KERNEL_RQ: fn<KERNEL_RQ>(__VA_ARGS__); break;                 \
-        default: fn<KERNEL_SE>(__VA_ARGS__); break;                        \
-    }
 
 // Function attributes (dynamic shared-memory limits, carve-out preferences) belong to the device's primary context: set once per
 // device and process, not per handle (the ~90 cudaFuncSetAttribute calls cost 0.3 s per gpso_create).
@@ -568,11 +515,6 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(dense_gemm_kernel<MODE_LAUUM_PART>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(predict_trmm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(joint_v_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN12>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN32>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_MATERN52>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_SE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_RQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(joint_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(diag_factor_inverse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(factor_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM_BYTES));
@@ -581,13 +523,11 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_KINV_S, OZ_LAUUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_KINV_S>::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_INV_S, OZ_GEMM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_INV_S>::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_HYB_S, OZ_GEMM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_HYB_S>::SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN12, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN32, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_MATERN52, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_SE, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<KERNEL_RQ, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
-    CU_TRY(cudaFuncSetAttribute(ozaki_screen_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ScrPairCfg::SMEM_BYTES));
-    CU_TRY(cudaFuncSetAttribute(ozaki_screen_pair_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    GP_TRY(AllKernels::each([](auto kid) -> int {
+        CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<kid>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+        CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
+        return 0;
+    }));
     GP_TRY(screen_configure<2>());
     GP_TRY(screen_configure<3>());
     GP_TRY(screen_configure<4>());
@@ -1267,7 +1207,7 @@ static int factor_pipeline(gpso_handle* h, cudaStream_t st, bool need_kinv) {
     scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(h->X.as<double>(), h->ls.as<double>(), h->n_ls(), h->N, h->d, Np,
                                                           h->Xs.as<double>());
     GP_TRY(check_launch(h, "scale_inputs"));
-    DISPATCH_KID(h, launch_gram, h, st);
+    launch_gram(h, st);
     GP_TRY(check_launch(h, "gram"));
 
     DenseParams P;
@@ -1424,8 +1364,7 @@ static int prepare_ozaki(gpso_handle* h, cudaStream_t st) {
     h->oz_est = 0.0;
     h->screen_ready = false;
     h->screen_built_S = 0;
-    static const int min_np = getenv("GPSO_OZ_MIN_NP") ? atoi(getenv("GPSO_OZ_MIN_NP")) : OZ_MIN_NP;  // tuning experiments only
-    bool want = h->predict_mode == 2 || (h->predict_mode == 0 && h->Np >= min_np);
+    bool want = h->predict_mode == 2 || (h->predict_mode == 0 && h->Np >= OZ_MIN_NP);
     if (!want || h->Np > OZ_MAX_NP) return 0;
     const int Np = h->Np;
     GP_TRY(h->rowscale.ensure((size_t)Np * sizeof(double)));
@@ -1465,8 +1404,7 @@ static int prepare_ozaki(gpso_handle* h, cudaStream_t st) {
         h->linv_frob2 += rl2[i];
         h->linv_rowl2_max = std::max(h->linv_rowl2_max, sqrt(rl2[i]));
     }
-    static const int scr_min_np = getenv("GPSO_SCREEN_MIN_NP") ? atoi(getenv("GPSO_SCREEN_MIN_NP")) : SCREEN_MIN_NP;
-    if (h->screen_mode != 0 && Np >= scr_min_np) {
+    if (h->screen_mode != 0 && Np >= SCREEN_MIN_NP) {
         GP_TRY(h->Xs32.ensure((size_t)h->d * Np * sizeof(float)));
         GP_TRY(h->alpha32.ensure((size_t)Np * sizeof(float)));
         screen_convert_kernel<<<(h->d * Np + 255) / 256, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->d, Np,
@@ -1501,15 +1439,13 @@ static int init_handle(gpso_handle* h, int device, int kernel_id, int ard, int m
     h->ard = ard ? 1 : 0;
     h->mean_id = mean_id;
     h->nsm = prop.multiProcessorCount;
-    if (getenv("GPSO_SCREEN_MODE")) h->screen_mode = std::min(std::max(atoi(getenv("GPSO_SCREEN_MODE")), 0), SCREEN_MODE_FULL2);  // tuning experiments
     h->l2_persist_max = (size_t)std::max(0, prop.persistingL2CacheMaxSize);
     h->l2_window_max = (size_t)std::max(0, prop.accessPolicyMaxWindowSize);
     // h->stream carries the tensor-core product kernels: highest priority, so that its persistent CTAs are placed before
     // the (default-priority) cross-covariance blocks of the next window when both become eligible at the same time
     int prio_least = 0, prio_greatest = 0;
     CU_TRY(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));
-    static const int prio_env = getenv("GPSO_PRODUCT_PRIO") ? atoi(getenv("GPSO_PRODUCT_PRIO")) : 1;  // 0: default priority (experiments)
-    CU_TRY(cudaStreamCreateWithPriority(&h->stream, cudaStreamNonBlocking, prio_env ? prio_greatest : prio_least));
+    CU_TRY(cudaStreamCreateWithPriority(&h->stream, cudaStreamNonBlocking, prio_greatest));
     CU_TRY(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
     CU_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
     CU_TRY(cudaEventCreateWithFlags(&h->ev_start, cudaEventDisableTiming));
@@ -1655,7 +1591,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     const int stride = 2 + nl + na;
     GP_TRY(h->gpart.ensure((size_t)nblk * stride * sizeof(double)));
     GP_TRY(h->gout.ensure((size_t)(stride + 4) * sizeof(double)));
-    DISPATCH_KID(h, launch_grad, h, st, nblk, stride);
+    launch_grad(h, st, nblk, stride);
     if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
     reduce_partials_kernel<<<stride, 256, 0, st>>>(h->gpart.as<double>(), nblk, stride, h->gout.as<double>());
     GP_TRY(check_launch(h, "reduce_partials"));
@@ -1813,46 +1749,44 @@ static void prof_collect(gpso_handle* h) {
 }
 
 // ---- the window pipeline ---------------------------------------------------------------------------------------------
-// Candidates are processed in windows.  Per window:  [H2D copy]  ->  cross-covariance (+ mean)  ->  variance product  ->
-// finalise (+ running arg-max).  With the int8 engine the cross-covariance of window w+1 (FP64 CUDA cores, stream
-// `aux`) overlaps the tensor-core product of window w (stream `st`): digit tiles and means are double-buffered, events
-// order the two streams.  Host-resident candidates are staged through two device buffers by a third (copy) stream.
-// mode 0: mean/var of every candidate are written out; mode 1: only the running arg-max record is kept.
-static int run_windows(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long M, int mode,
-                       double varsigma, double* mean_out, double* var_out) {
-    const bool oz = h->oz_S != 0;
+// Candidates are processed in windows.  Per window:  [H2D copy]  ->  cross-covariance (+ mean)  ->  product  ->  finalise.
+// With overlap the cross-covariance of window w+1 (stream `aux`) runs beside the product of window w (the handle's
+// high-priority stream): digit tiles and means are double-buffered, events order the two streams.  Host-resident candidates
+// are staged through two device buffers by a third (copy) stream.  The full-precision, screening and bound passes all run
+// through window_pipeline; each supplies its list of windows, whether it overlaps, and the work of one window.
+struct WindowSpan {
+    long long off, n;  // first candidate, candidates
+};
+
+static std::vector<WindowSpan> uniform_windows(long long M, long long W) {
+    std::vector<WindowSpan> wins;
+    for (long long off = 0; off < M; off += W) wins.push_back({off, std::min(W, M - off)});
+    return wins;
+}
+
+struct Window {
+    long long w, off, Mw;
+    const double* src;  // the window's candidates on the device
+    int b;              // digit-tile / mean buffer (0 without overlap)
+};
+
+// The work of one window.  xcov runs on the stream it is given, everything else on the product stream.  A pass without a
+// product stage (the bound pass) marks its cross-covariance only.  `after` runs once the window has released buffer b and may
+// stop the pass: the windows queued so far still complete and are joined.
+struct WindowStages {
+    std::function<int(const Window&, cudaStream_t)> xcov, product, finalise;
+    std::function<int(const Window&, cudaStream_t, bool*)> after;
+};
+
+// Queues the windows `wins` of the candidates (Xc_dev or Xc_host) behind the work already on `st`, the caller's stream, which
+// continues after the last of them.  W bounds the windows (staging buffer size).  *done: windows queued.
+static int window_pipeline(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long W,
+                           const std::vector<WindowSpan>& wins, bool overlap, const WindowStages& body, long long* done = nullptr) {
     const bool host = Xc_host != nullptr;
     const int d = h->d;
-    const long long W = window_size(h, M);
-    const long long nwin = (M + W - 1) / W;
-    // overlap needs the second set of buffers; a single window or the profiling mode (per-stage events) runs in order
-    const bool overlap = oz && h->overlap && !h->profile && nwin > 1;
-    const int nbuf = overlap ? 2 : 1;
-    GP_TRY(h->part.ensure((size_t)W * h->nb * sizeof(double)));
-    GP_TRY(h->blockbest.ensure((size_t)((W + 255) / 256) * sizeof(BestRec)));
-    for (int b = 0; b < nbuf; b++) {
-        GP_TRY(h->wmeanb[b].ensure((size_t)W * sizeof(double)));
-        if (oz) GP_TRY(h->ozBb[b].ensure((size_t)W * h->Np * h->oz_S));
-    }
-    if (!oz) GP_TRY(h->KsT.ensure((size_t)W * h->Np * sizeof(double)));
     if (host) {
-        size_t cbytes = (size_t)W * d * sizeof(double);
-        GP_TRY(h->cand[0].ensure(cbytes));
-        GP_TRY(h->cand[1].ensure(cbytes));
-        if (mode == 0) {
-            GP_TRY(h->omean.ensure((size_t)W * sizeof(double)));
-            GP_TRY(h->ovar.ensure((size_t)W * sizeof(double)));
-        }
-    }
-    const bool check = mode == 1 && h->rw_check && h->rw_idx_map != nullptr;
-    if (check) {  // refine pass of the screened arg-max: the finalised mean/var of the window are compared with the screened UCB
-        GP_TRY(h->omean.ensure((size_t)W * sizeof(double)));
-        GP_TRY(h->ovar.ensure((size_t)W * sizeof(double)));
-    }
-    if (mode == 2) {  // top-k: finalised mean/var of the window stay on the device, k records per window
-        GP_TRY(h->omean.ensure((size_t)W * sizeof(double)));
-        GP_TRY(h->ovar.ensure((size_t)W * sizeof(double)));
-        GP_TRY(h->topk.ensure((size_t)nwin * h->topk_k * sizeof(BestRec)));
+        GP_TRY(h->cand[0].ensure((size_t)W * d * sizeof(double)));
+        GP_TRY(h->cand[1].ensure((size_t)W * d * sizeof(double)));
     }
     cudaStream_t user_st = st;
     cudaStream_t xs = overlap ? h->aux_stream : st;  // stream of the cross-covariance kernels
@@ -1865,109 +1799,59 @@ static int run_windows(gpso_handle* h, cudaStream_t st, const double* Xc_dev, co
     }
     if (xs != st) CU_TRY(cudaStreamWaitEvent(xs, h->ev_start, 0));
     if (host) CU_TRY(cudaStreamWaitEvent(cs, h->ev_start, 0));
+    const bool marks = (bool)body.product;
     bool cand_busy[2] = {false, false}, buf_busy[2] = {false, false};
-
-    for (long long w = 0; w < nwin; w++) {
-        const int cb = (int)(w & 1);            // candidate staging buffer
-        const int b = overlap ? cb : 0;         // digit-tile / mean buffer
-        const long long off = w * W;
-        const long long Mw = std::min(W, M - off);
-        const long long Mw_pad = ((Mw + TB - 1) / TB) * TB;
+    long long w = 0;
+    for (bool stop = false; w < (long long)wins.size() && !stop; w++) {
+        const int cb = (int)(w & 1);  // candidate staging buffer
+        Window win = {w, wins[(size_t)w].off, wins[(size_t)w].n, nullptr, overlap ? cb : 0};
         h->last_windows++;
         // ---- 1. candidates of this window on the device
-        const double* src;
         if (host) {
             if (cand_busy[cb]) CU_TRY(cudaStreamWaitEvent(cs, h->ev_used[cb], 0));
-            CU_TRY(cudaMemcpyAsync(h->cand[cb].p, Xc_host + off * d, (size_t)Mw * d * sizeof(double), cudaMemcpyHostToDevice, cs));
+            CU_TRY(cudaMemcpyAsync(h->cand[cb].p, Xc_host + win.off * d, (size_t)win.Mw * d * sizeof(double), cudaMemcpyHostToDevice, cs));
             CU_TRY(cudaEventRecord(h->ev_copy[cb], cs));
             CU_TRY(cudaStreamWaitEvent(xs, h->ev_copy[cb], 0));
-            src = h->cand[cb].as<double>();
+            win.src = h->cand[cb].as<double>();
         } else {
-            src = Xc_dev + off * d;
+            win.src = Xc_dev + win.off * d;
         }
         // ---- 2. cross-covariance (+ posterior mean)
-        if (overlap && buf_busy[b]) CU_TRY(cudaStreamWaitEvent(xs, h->ev_free[b], 0));  // finalise(w-2) has read buffer b
+        if (overlap && buf_busy[win.b]) CU_TRY(cudaStreamWaitEvent(xs, h->ev_free[win.b], 0));  // window w-2 has released buffer b
         GP_TRY(prof_mark(h, xs));
         GP_TRY(trace_mark(h, xs, 1, w));
-        double gscale = 0.0;
-        long long nct = 0;
-        if (oz) {
-            const int S = h->oz_S;
-            nct = Mw_pad / OZ_NT;
-            const double beta = oz_beta(h);
-            const double bscale = ldexp(1.0, 8 * S - 2) / beta;
-            gscale = beta * ldexp(1.0, -2 * (8 * S - 2) + 8 * (S - 1));
-            DISPATCH_S(S, launch_oz_crosscov_s, h, xs, src, Mw, nct, bscale, h->ozBb[b].as<uint8_t>(), h->wmeanb[b].as<double>());
-            GP_TRY(check_launch(h, "crosscov_slices"));
-        } else {
-            DISPATCH_KID(h, launch_crosscov, h, xs, src, Mw, Mw_pad);
-            GP_TRY(check_launch(h, "crosscov"));
-        }
+        GP_TRY(body.xcov(win, xs));
         GP_TRY(trace_mark(h, xs, 2, w));
         if (host) {
             CU_TRY(cudaEventRecord(h->ev_used[cb], xs));
             cand_busy[cb] = true;
         }
         if (xs != st) {
-            CU_TRY(cudaEventRecord(h->ev_xcov[b], xs));
-            CU_TRY(cudaStreamWaitEvent(st, h->ev_xcov[b], 0));
+            CU_TRY(cudaEventRecord(h->ev_xcov[win.b], xs));
+            CU_TRY(cudaStreamWaitEvent(st, h->ev_xcov[win.b], 0));
         }
-        // ---- 3. variance product: part[I][c] = sum over the rows of block I of (L^-1 k*)^2
-        GP_TRY(prof_mark(h, st));
-        GP_TRY(prod_mark(h, st));
-        GP_TRY(trace_mark(h, st, 3, w));
-        if (oz) {
-            DISPATCH_S(h->oz_S, launch_oz_trmm, h, st, nct, Mw_pad, gscale, h->ozBb[b].as<uint8_t>());
-            GP_TRY(check_launch(h, "ozaki_trmm"));
-        } else {
-            PredictParams P;
-            P.Linv = h->Linv.as<double>();
-            P.KsT = h->KsT.as<double>();
-            P.part = h->part.as<double>();
-            P.Np = h->Np;
-            P.nb = h->nb;
-            P.nct = (int)(Mw_pad / TB);
-            P.counter = h->counter.as<int>();
-            CU_TRY(cudaMemsetAsync(h->counter.p, 0, sizeof(int), st));
-            int grid = std::min(h->nsm, P.nct * P.nb);
-            predict_trmm_kernel<<<grid, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
-            GP_TRY(check_launch(h, "predict_trmm"));
+        // ---- 3. product, 4. finalise
+        if (marks) {
+            GP_TRY(prof_mark(h, st));
+            GP_TRY(prod_mark(h, st));
+            GP_TRY(trace_mark(h, st, 3, w));
+            GP_TRY(body.product(win, st));
+            GP_TRY(prod_mark(h, st));
+            GP_TRY(trace_mark(h, st, 4, w));
+            GP_TRY(prof_mark(h, st));
         }
-        GP_TRY(prod_mark(h, st));
-        GP_TRY(trace_mark(h, st, 4, w));
-        GP_TRY(prof_mark(h, st));
-        // ---- 4. finalise: var, ucb, window arg-max merged into the running record
-        double* om = mode == 0 ? (host ? h->omean.as<double>() : mean_out + off) : (mode == 2 || check) ? h->omean.as<double>() : nullptr;
-        double* ov = mode == 0 ? (host ? h->ovar.as<double>() : var_out + off) : (mode == 2 || check) ? h->ovar.as<double>() : nullptr;
-        int fb = (int)((Mw + 255) / 256);
-        predict_finalize_kernel<<<fb, 256, 0, st>>>(h->part.as<double>(), h->wmeanb[b].as<double>(), h->nb, (int)Mw_pad, Mw, off,
-                                                    h->variance, h->noise, varsigma, mode == 2 ? 0 : mode, om, ov,
-                                                    h->blockbest.as<BestRec>(), mode == 1 ? h->rw_idx_map : nullptr);
-        GP_TRY(check_launch(h, "predict_finalize"));
-        if (check) {
-            screen_check_kernel<<<fb, 256, 0, st>>>(om, ov, Mw, h->rw_idx_map + off, varsigma, h->scr_ucb.as<double>(),
-                                                    h->scr_state.as<unsigned long long>(), h->rw_check_mean ? 1 : 0);
-            GP_TRY(check_launch(h, "screen_check"));
+        GP_TRY(body.finalise(win, st));
+        if (marks) {
+            GP_TRY(prof_mark(h, st));
+            GP_TRY(trace_mark(h, st, 5, w));
         }
-        if (mode == 2) {
-            topk_window_kernel<<<1, 1024, 0, st>>>(om, ov, Mw, off, varsigma, h->topk_k, h->topk.as<BestRec>() + w * h->topk_k);
-            GP_TRY(check_launch(h, "topk_window"));
-        }
-        if (mode == 1) {
-            best_merge_kernel<<<1, 256, 0, st>>>(h->blockbest.as<BestRec>(), fb, h->running.as<BestRec>(), w == 0 ? 1 : 0);
-            GP_TRY(check_launch(h, "best_merge"));
-        }
-        GP_TRY(prof_mark(h, st));
-        GP_TRY(trace_mark(h, st, 5, w));
         if (overlap) {
-            CU_TRY(cudaEventRecord(h->ev_free[b], st));
-            buf_busy[b] = true;
+            CU_TRY(cudaEventRecord(h->ev_free[win.b], st));
+            buf_busy[win.b] = true;
         }
-        if (host && mode == 0) {
-            CU_TRY(cudaMemcpyAsync(mean_out + off, h->omean.p, (size_t)Mw * sizeof(double), cudaMemcpyDeviceToHost, st));
-            CU_TRY(cudaMemcpyAsync(var_out + off, h->ovar.p, (size_t)Mw * sizeof(double), cudaMemcpyDeviceToHost, st));
-        }
+        if (body.after) GP_TRY(body.after(win, st, &stop));
     }
+    if (done) *done = w;
     if (st != user_st) {  // the caller's stream continues after the last product / finalise
         CU_TRY(cudaEventRecord(h->ev_start, st));
         CU_TRY(cudaStreamWaitEvent(user_st, h->ev_start, 0));
@@ -1975,15 +1859,125 @@ static int run_windows(gpso_handle* h, cudaStream_t st, const double* Xc_dev, co
     return 0;
 }
 
-static int predict_common_checks(gpso_handle* h, const void* a, long long M, const char* who) {
-    if (!h || !a) return fail(GPSO_E_BADARG, std::string(who) + ": null argument");
-    if (M <= 0) return fail(GPSO_E_BADARG, std::string(who) + ": M must be positive");
-    if (!h->factorized) return fail(GPSO_E_STATE, std::string(who) + ": call gpso_factorize first");
+// What the full-precision pass produces
+struct ScoreOutputs {
+    enum Kind { VALUES, ARGMAX, TOPK } kind;
+    double* mean = nullptr;              // VALUES: mean / var of every candidate, host or device memory like the candidates
+    double* var = nullptr;
+    const long long* idx_map = nullptr;  // ARGMAX, refine pass: global index of every (gathered) candidate; the refined UCB of
+    bool check_mean = false;             // each is compared with its screened UCB (check_mean: the screened value is the mean)
+    int k = 0;                           // TOPK: records per window
+};
+
+// The full-precision pass: the int8 tensor-core engine (oz_S digits) or the FP64 DMMA product
+static int full_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long M, double varsigma,
+                     const ScoreOutputs& out) {
+    const bool oz = h->oz_S != 0;
+    const bool host = Xc_host != nullptr;
+    const long long W = window_size(h, M);
+    const long long nwin = (M + W - 1) / W;
+    // overlap needs the second set of buffers; a single window or the profiling mode (per-stage events) runs in order
+    const bool overlap = oz && h->overlap && !h->profile && nwin > 1;
+    const int nbuf = overlap ? 2 : 1;
+    GP_TRY(h->part.ensure((size_t)W * h->nb * sizeof(double)));
+    GP_TRY(h->blockbest.ensure((size_t)((W + 255) / 256) * sizeof(BestRec)));
+    for (int b = 0; b < nbuf; b++) {
+        GP_TRY(h->wmeanb[b].ensure((size_t)W * sizeof(double)));
+        if (oz) GP_TRY(h->ozBb[b].ensure((size_t)W * h->Np * h->oz_S));
+    }
+    if (!oz) GP_TRY(h->KsT.ensure((size_t)W * h->Np * sizeof(double)));
+    const bool argmax = out.kind == ScoreOutputs::ARGMAX, topk = out.kind == ScoreOutputs::TOPK;
+    const bool check = argmax && out.idx_map != nullptr;
+    // the finalised mean / var of a window stay on the device: copied back to the host per window, read by the top-k pass
+    // or compared with the screened values
+    const bool staged = (out.kind == ScoreOutputs::VALUES && host) || topk || check;
+    if (staged) {
+        GP_TRY(h->omean.ensure((size_t)W * sizeof(double)));
+        GP_TRY(h->ovar.ensure((size_t)W * sizeof(double)));
+    }
+    if (topk) GP_TRY(h->topk.ensure((size_t)nwin * out.k * sizeof(BestRec)));
+    const int S = h->oz_S;
+    const double beta = oz ? oz_beta(h) : 0.0;
+    const double bscale = oz ? ldexp(1.0, 8 * S - 2) / beta : 0.0;
+    const double gscale = oz ? beta * ldexp(1.0, -2 * (8 * S - 2) + 8 * (S - 1)) : 0.0;
+    auto pad = [](long long Mw) { return ((Mw + TB - 1) / TB) * TB; };
+    WindowStages body;
+    body.xcov = [&](const Window& win, cudaStream_t xs) {
+        if (oz) {
+            DISPATCH_S(S, launch_oz_crosscov, h, xs, win.src, win.Mw, pad(win.Mw) / OZ_NT, bscale, h->ozBb[win.b].as<uint8_t>(),
+                       h->wmeanb[win.b].as<double>());
+            return check_launch(h, "crosscov_slices");
+        }
+        launch_crosscov(h, xs, win.src, win.Mw, pad(win.Mw));
+        return check_launch(h, "crosscov");
+    };
+    // part[I][c] = sum over the rows of block I of (L^-1 k*)^2
+    body.product = [&](const Window& win, cudaStream_t ps) {
+        const long long Mw_pad = pad(win.Mw);
+        if (oz) {
+            DISPATCH_S(S, launch_oz_trmm, h, ps, Mw_pad / OZ_NT, Mw_pad, gscale, h->ozBb[win.b].as<uint8_t>());
+            return check_launch(h, "ozaki_trmm");
+        }
+        PredictParams P;
+        P.Linv = h->Linv.as<double>();
+        P.KsT = h->KsT.as<double>();
+        P.part = h->part.as<double>();
+        P.Np = h->Np;
+        P.nb = h->nb;
+        P.nct = (int)(Mw_pad / TB);
+        P.counter = h->counter.as<int>();
+        CU_TRY(cudaMemsetAsync(h->counter.p, 0, sizeof(int), ps));
+        int grid = std::min(h->nsm, P.nct * P.nb);
+        predict_trmm_kernel<<<grid, GTHREADS, GEMM_SMEM_BYTES, ps>>>(P);
+        return check_launch(h, "predict_trmm");
+    };
+    // var, ucb, window arg-max merged into the running record / top-k records of the window / check of the survivors
+    body.finalise = [&](const Window& win, cudaStream_t ps) {
+        double* om = staged ? h->omean.as<double>() : out.mean ? out.mean + win.off : nullptr;
+        double* ov = staged ? h->ovar.as<double>() : out.var ? out.var + win.off : nullptr;
+        const int fb = (int)((win.Mw + 255) / 256);
+        predict_finalize_kernel<<<fb, 256, 0, ps>>>(h->part.as<double>(), h->wmeanb[win.b].as<double>(), h->nb, (int)pad(win.Mw), win.Mw,
+                                                    win.off, h->variance, h->noise, varsigma, argmax ? 1 : 0, om, ov,
+                                                    h->blockbest.as<BestRec>(), out.idx_map);
+        GP_TRY(check_launch(h, "predict_finalize"));
+        if (check) {
+            screen_check_kernel<<<fb, 256, 0, ps>>>(om, ov, win.Mw, out.idx_map + win.off, varsigma, h->scr_ucb.as<double>(),
+                                                    h->scr_state.as<unsigned long long>(), out.check_mean ? 1 : 0);
+            GP_TRY(check_launch(h, "screen_check"));
+        }
+        if (topk) {
+            topk_window_kernel<<<1, 1024, 0, ps>>>(om, ov, win.Mw, win.off, varsigma, out.k, h->topk.as<BestRec>() + win.w * out.k);
+            GP_TRY(check_launch(h, "topk_window"));
+        }
+        if (argmax) {
+            best_merge_kernel<<<1, 256, 0, ps>>>(h->blockbest.as<BestRec>(), fb, h->running.as<BestRec>(), win.w == 0 ? 1 : 0);
+            GP_TRY(check_launch(h, "best_merge"));
+        }
+        return 0;
+    };
+    if (out.kind == ScoreOutputs::VALUES && host)
+        body.after = [&](const Window& win, cudaStream_t ps, bool*) {
+            CU_TRY(cudaMemcpyAsync(out.mean + win.off, h->omean.p, (size_t)win.Mw * sizeof(double), cudaMemcpyDeviceToHost, ps));
+            CU_TRY(cudaMemcpyAsync(out.var + win.off, h->ovar.p, (size_t)win.Mw * sizeof(double), cudaMemcpyDeviceToHost, ps));
+            return 0;
+        };
+    return window_pipeline(h, st, Xc_dev, Xc_host, W, uniform_windows(M, W), overlap, body);
+}
+
+// per-call state of a scoring call: profiling and trace events and the window count start afresh
+static int begin_scoring(gpso_handle* h) {
     h->prof_used = 0;
     h->prod_used = 0;
     h->trace_used = 0;
     h->last_windows = 0;
     return set_device(h);
+}
+
+static int predict_common_checks(gpso_handle* h, const void* a, long long M, const char* who) {
+    if (!h || !a) return fail(GPSO_E_BADARG, std::string(who) + ": null argument");
+    if (M <= 0) return fail(GPSO_E_BADARG, std::string(who) + ": M must be positive");
+    if (!h->factorized) return fail(GPSO_E_STATE, std::string(who) + ": call gpso_factorize first");
+    return begin_scoring(h);
 }
 
 static int fetch_best(gpso_handle* h, cudaStream_t st, double* result_host) {
@@ -2035,7 +2029,7 @@ static void screen_error_model(const ScreenFit& f, int S, int full, double varsi
         est_var2 = unit * unit * f.rho_l2sq;           // second order: sum_i dv_i^2 (a bias; matters at 2 digits only)
     }
     // the fp32 covariance contract of kern_screen.cuh, for every kernel family and, for RationalQuadratic, every alpha.  The
-    // rest of the model (pick_slices' digit scale, the mean bound of bound_argmax, the int8 engines) relies only on
+    // rest of the model (pick_slices' digit scale, the mean bound of bound_pass, the int8 engines) relies only on
     // 0 <= k* <= variance, which RationalQuadratic satisfies too: no kernel-specific term anywhere else.
     const double eps_k32 = 2.0e-6 * f.variance;
     const double var_b = 2.0 * eps_k32 * sigma_f / sqrt(f.noise);
@@ -2077,8 +2071,7 @@ extern "C" int gpso_debug_screen_bound(int N, double variance, double noise, con
 
 static bool screen_applicable(const gpso_handle* h, long long M) {
     if (h->screen_mode == 0 || !h->screen_ready || h->oz_S == 0 || h->profile) return false;
-    static const int min_np = getenv("GPSO_SCREEN_MIN_NP") ? atoi(getenv("GPSO_SCREEN_MIN_NP")) : SCREEN_MIN_NP;  // tuning experiments
-    if (h->Np < min_np || M < SCREEN_MIN_M) return false;
+    if (h->Np < SCREEN_MIN_NP || M < SCREEN_MIN_M) return false;
     // the fp32 path needs the kernel variance and the lengthscales well inside the float range
     if (!(h->variance > 1e-30 && h->variance < 1e30)) return false;
     if (h->n_rq() && !(h->rq_alpha > 1e-30 && h->rq_alpha < 1e30)) return false;
@@ -2087,26 +2080,23 @@ static bool screen_applicable(const gpso_handle* h, long long M) {
     return true;
 }
 
-// The screening pass over all candidates: per window [H2D] -> fp32 cross-covariance digits (+ mean) on the side stream ->
-// low-digit tensor-core product -> screened UCB per candidate + running maximum.  Same stream / event choreography as
-// run_windows.  Leaves scr_ucb[0..M) and scr_state[0] (key of the maximum) on the device.
 // Window list of a screening pass over M candidates with windows of at most W (a multiple of 1024).  With the stream overlap
 // the cross-covariance of the FIRST window is the one stage nothing hides (1.6 ms of a 32 ms step when eight GPUs share the
 // candidates): the pipeline ramps up through a quarter and a half window; the rest is split evenly (no short tail launch).
-static void make_screen_windows(long long M, long long W, bool ramp, bool even, std::vector<std::pair<long long, long long>>& wins) {
+static void make_screen_windows(long long M, long long W, bool ramp, bool even, std::vector<WindowSpan>& wins) {
     wins.clear();
     long long off = 0;
     if (ramp && (M + W - 1) / W >= 3)
         for (long long part : {W / 4, W / 2}) {
             const long long r = part / 1024 * 1024;
             if (r >= 1024 && off + r < M) {
-                wins.emplace_back(off, r);
+                wins.push_back({off, r});
                 off += r;
             }
         }
     const long long rest = M - off, nrest = (rest + W - 1) / W;
     const long long each = (even && nrest > 0) ? std::min(W, ((rest + nrest - 1) / nrest + 1023) / 1024 * 1024) : W;
-    for (; off < M; off += each) wins.emplace_back(off, std::min(each, M - off));
+    for (; off < M; off += each) wins.push_back({off, std::min(each, M - off)});
 }
 
 extern "C" int64_t gpso_debug_screen_windows(int64_t M, int64_t W, int ramp, int even, int64_t* out, int64_t capacity) {
@@ -2114,35 +2104,33 @@ extern "C" int64_t gpso_debug_screen_windows(int64_t M, int64_t W, int ramp, int
         fail(GPSO_E_BADARG, "gpso_debug_screen_windows: need M > 0 and W a positive multiple of 1024");
         return -1;
     }
-    std::vector<std::pair<long long, long long>> wins;
+    std::vector<WindowSpan> wins;
     make_screen_windows(M, W, ramp != 0, even != 0, wins);
     if (out)
         for (size_t i = 0; i < wins.size() && (int64_t)(2 * i + 1) < capacity; i++) {
-            out[2 * i] = wins[i].first;
-            out[2 * i + 1] = wins[i].second;
+            out[2 * i] = wins[i].off;
+            out[2 * i + 1] = wins[i].n;
         }
     return (int64_t)wins.size();
 }
 
-static int run_screen_windows(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long M, int S, bool full,
-                              double varsigma, double two_e, bool* hopeless, cudaStream_t* product_stream_out) {
+// The screening pass over all candidates: per window [H2D] -> fp32 cross-covariance digits (+ mean) -> low-digit tensor-core
+// product -> screened UCB per candidate + running maximum.  Leaves scr_ucb[0..M) and scr_state[0] (key of the maximum) on the
+// device.
+static int screen_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long M, int S, bool full,
+                       double varsigma, double two_e, bool* hopeless) {
     *hopeless = false;
-    const bool host = Xc_host != nullptr;
-    const int d = h->d;
     const long long per_cand = (long long)h->Np * S;
     long long W = (WINDOW_BYTES / per_cand) / 1024 * 1024;
     if (h->window_override > 0) W = std::max<long long>(1024, h->window_override / 1024 * 1024);
     W = std::min(W, ((M + SCR_NT - 1) / SCR_NT) * SCR_NT);
     const long long nwin = (M + W - 1) / W;
-    // Side-stream overlap of the next window's cross-covariance: both kernels are power-bound, so running them side by side
-    // gains nothing measurable (profiles/r02c_screen_trace.json: 86.1 vs 88.4 ms per 2.1e6 candidates), and the CTA-pair
-    // product must not share its SMs with other blocks while its clusters are being placed (a co-resident cross-covariance
-    // kernel stalled it): with the pair kernel the windows run in order on one stream.
-    const bool overlap = h->overlap && nwin > 1 && !(!full && screen_pair_enabled(h, S));
+    // side-stream overlap of the next window's cross-covariance; both kernels are power-bound, so it gains little
+    // (profiles/r02c_screen_trace.json: 86.1 vs 88.4 ms per 2.1e6 candidates)
+    const bool overlap = h->overlap && nwin > 1;
     const int nbuf = overlap ? 2 : 1;
-    std::vector<std::pair<long long, long long>> wins;  // (first candidate, candidates)
+    std::vector<WindowSpan> wins;
     make_screen_windows(M, W, overlap && h->window_override == 0, h->window_override == 0, wins);
-    const long long nwin_total = (long long)wins.size();
     GP_TRY(h->part32.ensure((size_t)W * h->nb * sizeof(float)));
     GP_TRY(h->scr_ucb.ensure((size_t)M * sizeof(double)));
     GP_TRY(h->scr_state.ensure(4 * sizeof(unsigned long long)));
@@ -2150,15 +2138,10 @@ static int run_screen_windows(gpso_handle* h, cudaStream_t st, const double* Xc_
         GP_TRY(h->wmeanb[b].ensure((size_t)W * sizeof(double)));
         GP_TRY(h->ozBb[b].ensure((size_t)W * per_cand));
     }
-    if (host) {
-        GP_TRY(h->cand[0].ensure((size_t)W * d * sizeof(double)));
-        GP_TRY(h->cand[1].ensure((size_t)W * d * sizeof(double)));
-    }
     if (h->screen_built_S != S) {
+        // tiles above the block diagonal are neither built nor read: row block I of the product runs over k-steps
+        // [0, 4 (I + 1)) (OzItems<OZ_TRMM>), exactly the tiles linv_slices_kernel<S, false> writes
         GP_TRY(h->ozAs.ensure((size_t)h->Np * h->Np * S));
-        // tiles above the block diagonal stay zero: the CTA-pair kernel runs the shorter row block of a pair over the k-range
-        // of the longer one
-        CU_TRY(cudaMemsetAsync(h->ozAs.p, 0, (size_t)h->Np * h->Np * S, st));
         DISPATCH_SCREEN_S(S, launch_screen_slices, h, st);
         GP_TRY(check_launch(h, "screen_slices"));
         h->screen_built_S = S;
@@ -2166,111 +2149,65 @@ static int run_screen_windows(gpso_handle* h, cudaStream_t st, const double* Xc_
     CU_TRY(cudaMemsetAsync(h->scr_state.p, 0, 4 * sizeof(unsigned long long), st));
     // during the screening pass the persisting-L2 window of the product stream covers the low-digit tiles of L^-1
     GP_TRY(set_l2_window(h, h->ozAs.p, (size_t)h->Np * h->Np * S));
-    cudaStream_t user_st = st;
-    cudaStream_t xs = overlap ? h->aux_stream : st;
-    cudaStream_t cs = h->copy_stream;
-    CU_TRY(cudaEventRecord(h->ev_start, st));
-    if (overlap && st != h->stream) {
-        st = h->stream;
-        CU_TRY(cudaStreamWaitEvent(st, h->ev_start, 0));
-    }
-    if (xs != st) CU_TRY(cudaStreamWaitEvent(xs, h->ev_start, 0));
-    if (host) CU_TRY(cudaStreamWaitEvent(cs, h->ev_start, 0));
-    bool cand_busy[2] = {false, false}, buf_busy[2] = {false, false};
-    long long nwin_done = nwin_total, probe_rows = 0;
+    long long probe_rows = 0;
     unsigned long long* probe = reinterpret_cast<unsigned long long*>(h->host_rec + MAX_LS + 14);  // pinned, unused during the pass
     const double beta = oz_beta(h);
     const float bscale = (float)(ldexp(1.0, 8 * S - 2) / beta);
     // triangular product: levels t < S, the lowest kept level has weight 256^0; full product: levels t <= 2S-2
     const double gscale = full ? beta * ldexp(1.0, -2 * (8 * S - 2)) : beta * ldexp(1.0, -2 * (8 * S - 2) + 8 * (S - 1));
-    for (long long w = 0; w < nwin_total; w++) {
-        const int cb = (int)(w & 1);
-        const int b = overlap ? cb : 0;
-        const long long off = wins[(size_t)w].first;
-        const long long Mw = wins[(size_t)w].second;
-        const long long Mw_pad = ((Mw + SCR_NT - 1) / SCR_NT) * SCR_NT;
-        const double* src;
-        if (host) {
-            if (cand_busy[cb]) CU_TRY(cudaStreamWaitEvent(cs, h->ev_used[cb], 0));
-            CU_TRY(cudaMemcpyAsync(h->cand[cb].p, Xc_host + off * d, (size_t)Mw * d * sizeof(double), cudaMemcpyHostToDevice, cs));
-            CU_TRY(cudaEventRecord(h->ev_copy[cb], cs));
-            CU_TRY(cudaStreamWaitEvent(xs, h->ev_copy[cb], 0));
-            src = h->cand[cb].as<double>();
-        } else {
-            src = Xc_dev + off * d;
-        }
-        if (overlap && buf_busy[b]) CU_TRY(cudaStreamWaitEvent(xs, h->ev_free[b], 0));
-        GP_TRY(trace_mark(h, xs, 1, w));
-        DISPATCH_SCREEN_S(S, launch_screen_crosscov_s, h, xs, src, Mw, Mw_pad / 64, bscale, h->ozBb[b].as<uint8_t>(), h->wmeanb[b].as<double>());
-        GP_TRY(check_launch(h, "crosscov_screen"));
-        GP_TRY(trace_mark(h, xs, 2, w));
-        if (host) {
-            CU_TRY(cudaEventRecord(h->ev_used[cb], xs));
-            cand_busy[cb] = true;
-        }
-        if (xs != st) {
-            CU_TRY(cudaEventRecord(h->ev_xcov[b], xs));
-            CU_TRY(cudaStreamWaitEvent(st, h->ev_xcov[b], 0));
-        }
-        GP_TRY(prod_mark(h, st));
-        GP_TRY(trace_mark(h, st, 3, w));
+    auto pad = [](long long Mw) { return ((Mw + SCR_NT - 1) / SCR_NT) * SCR_NT; };
+    WindowStages body;
+    body.xcov = [&](const Window& win, cudaStream_t xs) {
+        DISPATCH_SCREEN_S(S, launch_screen_crosscov, h, xs, win.src, win.Mw, pad(win.Mw) / 64, bscale, h->ozBb[win.b].as<uint8_t>(),
+                          h->wmeanb[win.b].as<double>());
+        return check_launch(h, "crosscov_screen");
+    };
+    body.product = [&](const Window& win, cudaStream_t ps) {
+        const long long Mw_pad = pad(win.Mw);
         if (full) {
-            // four k-steps (64 KB of operands, one tcgen05.commit) per ring stage, three stages: 41.8 vs 43.4 ms per 2.1e6
-            // candidates against two k-steps x six stages (GPSO_SCR_KPS=2 for the A/B)
-            static const int kps_env = getenv("GPSO_SCR_KPS") ? atoi(getenv("GPSO_SCR_KPS")) : 4;
-            if (kps_env == 4) launch_screen_product_v<2, true, 4>(h, st, Mw_pad / SCR_NT, Mw_pad, gscale, h->ozBb[b].as<uint8_t>());
-            else launch_screen_product_v<2, true>(h, st, Mw_pad / SCR_NT, Mw_pad, gscale, h->ozBb[b].as<uint8_t>());
+            launch_screen_product<2, true>(h, ps, Mw_pad / SCR_NT, Mw_pad, gscale, h->ozBb[win.b].as<uint8_t>());
         } else {
-            DISPATCH_SCREEN_S(S, launch_screen_product, h, st, Mw_pad / SCR_NT, Mw_pad, gscale, h->ozBb[b].as<uint8_t>());
+            DISPATCH_SCREEN_S(S, launch_screen_product, h, ps, Mw_pad / SCR_NT, Mw_pad, gscale, h->ozBb[win.b].as<uint8_t>());
         }
-        GP_TRY(check_launch(h, "ozaki_screen"));
-        GP_TRY(trace_mark(h, st, 4, w));
-        GP_TRY(prod_mark(h, st));
-        screen_finalize_kernel<<<(unsigned)((Mw + 255) / 256), 256, 0, st>>>(h->part32.as<float>(), h->wmeanb[b].as<double>(), h->nb, Mw_pad, Mw,
-                                                                             off, h->variance, h->noise, varsigma, h->scr_ucb.as<double>(),
-                                                                             h->scr_state.as<unsigned long long>());
-        GP_TRY(check_launch(h, "screen_finalize"));
-        GP_TRY(trace_mark(h, st, 5, w));
-        if (overlap) {
-            CU_TRY(cudaEventRecord(h->ev_free[b], st));
-            buf_busy[b] = true;
-        }
-        h->last_windows++;
-        if (w == 0 && nwin_total >= 4) {
+        return check_launch(h, "ozaki_screen");
+    };
+    body.finalise = [&](const Window& win, cudaStream_t ps) {
+        screen_finalize_kernel<<<(unsigned)((win.Mw + 255) / 256), 256, 0, ps>>>(h->part32.as<float>(), h->wmeanb[win.b].as<double>(), h->nb,
+                                                                                 pad(win.Mw), win.Mw, win.off, h->variance, h->noise,
+                                                                                 varsigma, h->scr_ucb.as<double>(),
+                                                                                 h->scr_state.as<unsigned long long>());
+        return check_launch(h, "screen_finalize");
+    };
+    body.after = [&](const Window& win, cudaStream_t ps, bool* stop) {
+        if (win.w == 0 && wins.size() >= 4) {
             // early verdict on this variant: if more than 1/16 of the first window lies within 2E of the window's own best value
             // the screen cannot separate these candidates -- stop instead of paying for the other windows.  The count is
             // queued behind window 0 and read (pinned record) once window 1 has been queued, so the pipeline never drains.
             GP_TRY(h->surv_list.ensure(sizeof(long long)));
-            screen_select_kernel<<<(unsigned)((Mw + 255) / 256), 256, 0, st>>>(h->scr_ucb.as<double>(), Mw, two_e,
-                                                                              h->scr_state.as<unsigned long long>(),
-                                                                              h->surv_list.as<long long>(), 0u);
+            screen_select_kernel<<<(unsigned)((win.Mw + 255) / 256), 256, 0, ps>>>(h->scr_ucb.as<double>(), win.Mw, two_e,
+                                                                                   h->scr_state.as<unsigned long long>(),
+                                                                                   h->surv_list.as<long long>(), 0u);
             GP_TRY(check_launch(h, "screen_select"));
-            CU_TRY(cudaMemcpyAsync(probe, h->scr_state.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            CU_TRY(cudaMemsetAsync(h->scr_state.as<unsigned long long>() + 1, 0, sizeof(unsigned long long), st));
-            CU_TRY(cudaEventRecord(h->ev_probe, st));
-            probe_rows = Mw;
+            CU_TRY(cudaMemcpyAsync(probe, h->scr_state.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ps));
+            CU_TRY(cudaMemsetAsync(h->scr_state.as<unsigned long long>() + 1, 0, sizeof(unsigned long long), ps));
+            CU_TRY(cudaEventRecord(h->ev_probe, ps));
+            probe_rows = win.Mw;
         }
-        if (w == 1 && probe_rows > 0) {
+        if (win.w == 1 && probe_rows > 0) {
             CU_TRY(cudaEventSynchronize(h->ev_probe));
             if ((long long)probe[1] * 16 > probe_rows) {
                 *hopeless = true;
                 h->scr_info[2] = (double)probe[1] * ((double)M / (double)probe_rows);  // extrapolated survivor count, for the record
-                nwin_done = 2;
-                break;
+                *stop = true;
             }
         }
-    }
-    h->scr_info[6] = (double)nwin_done;
-    *product_stream_out = st;
-    GP_TRY(set_l2_window(h, h->ozA.p, (size_t)h->Np * h->Np * h->oz_S));  // back on the full-precision tiles (refine pass)
-    if (st != user_st) {
-        CU_TRY(cudaEventRecord(h->ev_start, st));
-        CU_TRY(cudaStreamWaitEvent(user_st, h->ev_start, 0));
-    }
-    return 0;
+        return 0;
+    };
+    long long done = 0;
+    GP_TRY(window_pipeline(h, st, Xc_dev, Xc_host, W, wins, overlap, body, &done));
+    h->scr_info[6] = (double)done;
+    return set_l2_window(h, h->ozA.p, (size_t)h->Np * h->Np * h->oz_S);  // back on the full-precision tiles (refine pass)
 }
-
-static int fetch_best(gpso_handle* h, cudaStream_t st, double* result_host);
 
 // ---- bound-and-refine, level 0 (screen mode 5) ---------------------------------------------------------------------------
 // UCB = mean + varsigma * var with sigma_n^2 <= var <= sigma_f^2 + sigma_n^2 for EVERY candidate (the posterior variance of
@@ -2278,55 +2215,30 @@ static int fetch_best(gpso_handle* h, cudaStream_t st, double* result_host);
 // |varsigma| sigma_f^2 below the best mean cannot be the arg-max whatever its variance.  Only the mean is evaluated for all
 // candidates (fp32 cross-covariance, error bound E_mean of screen_error_model); the survivors go straight to the
 // full-precision engine.  Exact like the digit screen, and much cheaper when the means spread wider than |varsigma| sigma_f^2;
-// when they do not (too many survivors) the caller continues with the digit screen over all candidates.
-static int run_bound_windows(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long M) {
-    const bool host = Xc_host != nullptr;
-    const int d = h->d;
+// when they do not (too many survivors) the caller continues with the digit screen over all candidates.  One stream.
+static int bound_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, long long M) {
     long long W = 1LL << 19;
     if (h->window_override > 0) W = std::max<long long>(1024, h->window_override / 1024 * 1024);
     W = std::min(W, ((M + SCR_NT - 1) / SCR_NT) * SCR_NT);
-    const long long nwin = (M + W - 1) / W;
     GP_TRY(h->scr_ucb.ensure((size_t)M * sizeof(double)));
     GP_TRY(h->scr_state.ensure(4 * sizeof(unsigned long long)));
     GP_TRY(h->wmeanb[0].ensure((size_t)W * sizeof(double)));
-    if (host) {
-        GP_TRY(h->cand[0].ensure((size_t)W * d * sizeof(double)));
-        GP_TRY(h->cand[1].ensure((size_t)W * d * sizeof(double)));
-    }
     CU_TRY(cudaMemsetAsync(h->scr_state.p, 0, 4 * sizeof(unsigned long long), st));
-    cudaStream_t cs = h->copy_stream;
-    CU_TRY(cudaEventRecord(h->ev_start, st));
-    if (host) CU_TRY(cudaStreamWaitEvent(cs, h->ev_start, 0));
-    bool cand_busy[2] = {false, false};
-    for (long long w = 0; w < nwin; w++) {
-        const int cb = (int)(w & 1);
-        const long long off = w * W;
-        const long long Mw = std::min(W, M - off);
-        const long long Mw_pad = ((Mw + SCR_NT - 1) / SCR_NT) * SCR_NT;
-        const double* src;
-        if (host) {
-            if (cand_busy[cb]) CU_TRY(cudaStreamWaitEvent(cs, h->ev_used[cb], 0));
-            CU_TRY(cudaMemcpyAsync(h->cand[cb].p, Xc_host + off * d, (size_t)Mw * d * sizeof(double), cudaMemcpyHostToDevice, cs));
-            CU_TRY(cudaEventRecord(h->ev_copy[cb], cs));
-            CU_TRY(cudaStreamWaitEvent(st, h->ev_copy[cb], 0));
-            src = h->cand[cb].as<double>();
-        } else {
-            src = Xc_dev + off * d;
-        }
-        GP_TRY(trace_mark(h, st, 1, w));
-        launch_screen_crosscov_s<0>(h, st, src, Mw, Mw_pad / 64, 0.0f, nullptr, h->wmeanb[0].as<double>());
-        GP_TRY(check_launch(h, "crosscov_mean"));
-        GP_TRY(trace_mark(h, st, 2, w));
-        if (host) {
-            CU_TRY(cudaEventRecord(h->ev_used[cb], st));
-            cand_busy[cb] = true;
-        }
-        bound_finalize_kernel<<<(unsigned)((Mw + 255) / 256), 256, 0, st>>>(h->wmeanb[0].as<double>(), Mw, off, h->scr_ucb.as<double>(),
-                                                                            h->scr_state.as<unsigned long long>());
-        GP_TRY(check_launch(h, "bound_finalize"));
-        h->last_windows++;
-    }
-    h->scr_info[6] = (double)nwin;
+    WindowStages body;
+    body.xcov = [&](const Window& win, cudaStream_t xs) {
+        launch_screen_crosscov<0>(h, xs, win.src, win.Mw, ((win.Mw + SCR_NT - 1) / SCR_NT) * SCR_NT / 64, 0.0f, nullptr,
+                                  h->wmeanb[0].as<double>());
+        return check_launch(h, "crosscov_mean");
+    };
+    body.finalise = [&](const Window& win, cudaStream_t ps) {
+        bound_finalize_kernel<<<(unsigned)((win.Mw + 255) / 256), 256, 0, ps>>>(h->wmeanb[0].as<double>(), win.Mw, win.off,
+                                                                                h->scr_ucb.as<double>(),
+                                                                                h->scr_state.as<unsigned long long>());
+        return check_launch(h, "bound_finalize");
+    };
+    long long done = 0;
+    GP_TRY(window_pipeline(h, st, Xc_dev, Xc_host, W, uniform_windows(M, W), false, body, &done));
+    h->scr_info[6] = (double)done;
     return 0;
 }
 
@@ -2370,14 +2282,10 @@ static int refine_survivors(gpso_handle* h, cudaStream_t st, const double* Xc_de
         GP_TRY(check_launch(h, "gather_rows"));
         rdev = h->surv_X.as<double>();
     }
-    h->rw_idx_map = h->surv_list.as<long long>();
-    h->rw_check = true;
-    h->rw_check_mean = mean_only;
-    int rc = run_windows(h, st, rdev, rhost, count, 1, varsigma, nullptr, nullptr);
-    h->rw_idx_map = nullptr;
-    h->rw_check = false;
-    h->rw_check_mean = false;
-    GP_TRY(rc);
+    ScoreOutputs out = {ScoreOutputs::ARGMAX};
+    out.idx_map = h->surv_list.as<long long>();
+    out.check_mean = mean_only;
+    GP_TRY(full_pass(h, st, rdev, rhost, count, varsigma, out));
     unsigned long long dbits = 0;
     CU_TRY(cudaMemcpyAsync(&dbits, h->scr_state.as<unsigned long long>() + 2, sizeof dbits, cudaMemcpyDeviceToHost, st));
     GP_TRY(fetch_best(h, st, result_host));  // synchronises st
@@ -2407,7 +2315,7 @@ static int score_argmax(gpso_handle* h, cudaStream_t st, const double* Xc_dev, c
         if (h->screen_mode == SCREEN_MODE_BOUND) {
             // level 0: posterior mean of every candidate, variance bounded by the prior
             screen_error_bound(h, SCREEN_S_MAX, false, varsigma, &E, &e_var, &e_mean);
-            GP_TRY(run_bound_windows(h, st, Xc_dev, Xc_host, M));
+            GP_TRY(bound_pass(h, st, Xc_dev, Xc_host, M));
             const double width = fabs(varsigma) * h->variance * (1.0 + 2.0e-6);  // |varsigma| (v_max - v_min) with rounding slack
             h->scr_info[1] = 0.0;
             h->scr_info[3] = e_mean;
@@ -2444,10 +2352,9 @@ static int score_argmax(gpso_handle* h, cudaStream_t st, const double* Xc_dev, c
             const int S = v.S;
             screen_error_bound(h, S, v.full, varsigma, &E, &e_var, &e_mean);
             if (automatic && !(e_var <= 1.0 * h->variance)) continue;  // a looser bound than the prior variance separates nothing
-            cudaStream_t pst = st;
             bool hopeless = false;
             h->prod_used = 0;
-            GP_TRY(run_screen_windows(h, st, Xc_dev, Xc_host, M, S, v.full, varsigma, 2.0 * E, &hopeless, &pst));
+            GP_TRY(screen_pass(h, st, Xc_dev, Xc_host, M, S, v.full, varsigma, 2.0 * E, &hopeless));
             h->scr_prod_marks = h->prod_used;
             h->scr_info[1] = S;
             h->scr_info[3] = E;
@@ -2474,15 +2381,34 @@ static int score_argmax(gpso_handle* h, cudaStream_t st, const double* Xc_dev, c
             }
         }
     }
-    GP_TRY(run_windows(h, st, Xc_dev, Xc_host, M, 1, varsigma, nullptr, nullptr));
+    GP_TRY(full_pass(h, st, Xc_dev, Xc_host, M, varsigma, {ScoreOutputs::ARGMAX}));
     return fetch_best(h, st, result_host);
+}
+
+// Device time of a scoring call in last_ms[0]: `work` is queued on st between ev_t0 and ev_t1, `finish` waits for ev_t1 (after
+// queueing the copies of the results behind it, where there are any).
+template <class Work, class Finish>
+static int timed_call(gpso_handle* h, cudaStream_t st, Work&& work, Finish&& finish) {
+    CU_TRY(cudaEventRecord(h->ev_t0, st));
+    GP_TRY(work());
+    CU_TRY(cudaEventRecord(h->ev_t1, st));
+    GP_TRY(finish());
+    float ms = 0;
+    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
+    h->last_ms[0] = ms;
+    return 0;
+}
+
+static int wait_t1(gpso_handle* h) {
+    CU_TRY(cudaEventSynchronize(h->ev_t1));
+    return 0;
 }
 
 extern "C" int gpso_predict_y_dev(gpso_handle* h, const double* Xc_dev, int64_t M, double* mean_dev, double* var_dev,
                                   void* stream) {
     GP_TRY(predict_common_checks(h, Xc_dev, M, "gpso_predict_y_dev"));
     if (!mean_dev || !var_dev) return fail(GPSO_E_BADARG, "gpso_predict_y_dev: null output");
-    return run_windows(h, (cudaStream_t)stream, Xc_dev, nullptr, M, 0, 0.0, mean_dev, var_dev);
+    return full_pass(h, (cudaStream_t)stream, Xc_dev, nullptr, M, 0.0, {ScoreOutputs::VALUES, mean_dev, var_dev});
 }
 
 extern "C" int gpso_ucb_argmax_dev(gpso_handle* h, const double* Xc_dev, int64_t M, double varsigma, double* result_host,
@@ -2490,41 +2416,27 @@ extern "C" int gpso_ucb_argmax_dev(gpso_handle* h, const double* Xc_dev, int64_t
     GP_TRY(predict_common_checks(h, Xc_dev, M, "gpso_ucb_argmax_dev"));
     if (!result_host) return fail(GPSO_E_BADARG, "gpso_ucb_argmax_dev: null output");
     cudaStream_t st = (cudaStream_t)stream;
-    CU_TRY(cudaEventRecord(h->ev_t0, st));
-    GP_TRY(score_argmax(h, st, Xc_dev, nullptr, M, varsigma, result_host));
-    CU_TRY(cudaEventRecord(h->ev_t1, st));
-    CU_TRY(cudaEventSynchronize(h->ev_t1));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
-    h->last_ms[0] = ms;
-    return 0;
+    return timed_call(h, st, [&] { return score_argmax(h, st, Xc_dev, nullptr, M, varsigma, result_host); }, [&] { return wait_t1(h); });
 }
 
 extern "C" int gpso_predict_y_host(gpso_handle* h, const double* Xc_host, int64_t M, double* mean_host, double* var_host) {
     GP_TRY(predict_common_checks(h, Xc_host, M, "gpso_predict_y_host"));
     if (!mean_host || !var_host) return fail(GPSO_E_BADARG, "gpso_predict_y_host: null output");
-    CU_TRY(cudaEventRecord(h->ev_t0, h->stream));
-    GP_TRY(run_windows(h, h->stream, nullptr, Xc_host, M, 0, 0.0, mean_host, var_host));
-    CU_TRY(cudaEventRecord(h->ev_t1, h->stream));
-    CU_TRY(cudaStreamSynchronize(h->stream));
-    prof_collect(h);
-    float ms = 0;
-    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
-    h->last_ms[0] = ms;
-    return 0;
+    cudaStream_t st = h->stream;
+    return timed_call(
+        h, st, [&] { return full_pass(h, st, nullptr, Xc_host, M, 0.0, {ScoreOutputs::VALUES, mean_host, var_host}); },
+        [&] {
+            CU_TRY(cudaStreamSynchronize(st));
+            prof_collect(h);
+            return 0;
+        });
 }
 
 extern "C" int gpso_ucb_argmax_host(gpso_handle* h, const double* Xc_host, int64_t M, double varsigma, double* result_host) {
     GP_TRY(predict_common_checks(h, Xc_host, M, "gpso_ucb_argmax_host"));
     if (!result_host) return fail(GPSO_E_BADARG, "gpso_ucb_argmax_host: null output");
-    CU_TRY(cudaEventRecord(h->ev_t0, h->stream));
-    GP_TRY(score_argmax(h, h->stream, nullptr, Xc_host, M, varsigma, result_host));
-    CU_TRY(cudaEventRecord(h->ev_t1, h->stream));
-    CU_TRY(cudaEventSynchronize(h->ev_t1));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
-    h->last_ms[0] = ms;
-    return 0;
+    cudaStream_t st = h->stream;
+    return timed_call(h, st, [&] { return score_argmax(h, st, nullptr, Xc_host, M, varsigma, result_host); }, [&] { return wait_t1(h); });
 }
 
 // Top-k variant of the fused scoring call: the k candidates with the highest UCB in arg-max order (first NaN, larger UCB,
@@ -2532,18 +2444,18 @@ extern "C" int gpso_ucb_argmax_host(gpso_handle* h, const double* Xc_host, int64
 static int topk_common(gpso_handle* h, cudaStream_t st, const double* Xc_dev, const double* Xc_host, int64_t M, double varsigma, int k,
                        double* result_host, int* found) {
     if (k < 1 || k > TOPK_MAX) return fail(GPSO_E_BADARG, "gpso_ucb_topk: k must be in 1..64");
-    h->topk_k = k;
-    CU_TRY(cudaEventRecord(h->ev_t0, st));
-    GP_TRY(run_windows(h, st, Xc_dev, Xc_host, M, 2, varsigma, nullptr, nullptr));
-    CU_TRY(cudaEventRecord(h->ev_t1, st));
-    const size_t nrec = (size_t)h->last_windows * k;
-    std::vector<BestRec> rec(nrec);
-    CU_TRY(cudaMemcpyAsync(rec.data(), h->topk.p, nrec * sizeof(BestRec), cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
-    prof_collect(h);
-    float ms = 0;
-    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
-    h->last_ms[0] = ms;
+    ScoreOutputs out = {ScoreOutputs::TOPK};
+    out.k = k;
+    std::vector<BestRec> rec;
+    GP_TRY(timed_call(
+        h, st, [&] { return full_pass(h, st, Xc_dev, Xc_host, M, varsigma, out); },
+        [&] {
+            rec.resize((size_t)h->last_windows * k);
+            CU_TRY(cudaMemcpyAsync(rec.data(), h->topk.p, rec.size() * sizeof(BestRec), cudaMemcpyDeviceToHost, st));
+            CU_TRY(cudaStreamSynchronize(st));
+            prof_collect(h);
+            return 0;
+        }));
     std::vector<BestRec> live;
     for (const BestRec& r : rec)
         if (r.idx != 0x7fffffffffffffffLL) live.push_back(r);
@@ -2592,20 +2504,22 @@ static int joint_ready(gpso_handle* h, const char* who) {
     return set_device(h);
 }
 
-template <int KID>
 static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, int M, int Mp) {
     size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
-    crosscov_kernel<KID><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
-                                                              h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                              h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha);
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        crosscov_kernel<kid><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
+                                                                  h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
+                                                                  h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha);
+    });
 }
 
-template <int KID>
 static void launch_joint_syrk(gpso_handle* h, cudaStream_t st, int M, int Mp, double jitter) {
     const int mb = Mp / TB;
-    joint_syrk_kernel<KID><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp, h->Np,
-                                                                               h->d, h->variance, jitter, h->jSigma.as<double>(),
-                                                                               h->rq_alpha);
+    AllKernels::with(h->kernel_id, [&](auto kid) {
+        joint_syrk_kernel<kid><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp,
+                                                                                   h->Np, h->d, h->variance, jitter,
+                                                                                   h->jSigma.as<double>(), h->rq_alpha);
+    });
 }
 
 // scaled candidates -> cross-covariance + mean -> V^T = (L^-1 K*)^T -> lower triangle of K** - V^T V (+ jitter I) in jSigma
@@ -2619,7 +2533,7 @@ static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M,
     GP_TRY(h->jcounter.ensure(sizeof(int)));
     scale_inputs_kernel<<<(Mp + 255) / 256, 256, 0, st>>>(Xc, h->ls.as<double>(), h->n_ls(), M, h->d, Mp, h->jXcs.as<double>());
     GP_TRY(check_launch(h, "scale_inputs"));
-    DISPATCH_KID(h, launch_joint_crosscov, h, st, Xc, M, Mp);
+    launch_joint_crosscov(h, st, Xc, M, Mp);
     GP_TRY(check_launch(h, "crosscov"));
     JointVParams P;
     P.Linv = h->Linv.as<double>();
@@ -2632,7 +2546,7 @@ static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M,
     CU_TRY(cudaMemsetAsync(h->jcounter.p, 0, sizeof(int), st));
     joint_v_kernel<<<std::min(h->nsm > 0 ? h->nsm : 148, P.nct * P.nb), GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
     GP_TRY(check_launch(h, "joint_v"));
-    DISPATCH_KID(h, launch_joint_syrk, h, st, M, Mp, jitter);
+    launch_joint_syrk(h, st, M, Mp, jitter);
     return check_launch(h, "joint_syrk");
 }
 
@@ -2824,12 +2738,8 @@ extern "C" int gpso_grow_ucb_argmax_range(gpso_handle* h, const double* bounds_h
                                           int64_t row1, double* result_host) {
     if (!h || !bounds_host || !result_host) return fail(GPSO_E_BADARG, "gpso_grow_ucb_argmax: null argument");
     if (!h->factorized) return fail(GPSO_E_STATE, "gpso_grow_ucb_argmax: call gpso_factorize first");
-    h->prof_used = 0;
-    h->prod_used = 0;
-    h->trace_used = 0;
-    h->last_windows = 0;
+    GP_TRY(begin_scoring(h));
     if (d != h->d) return fail(GPSO_E_BADARG, "gpso_grow_ucb_argmax: dimension differs from the training data");
-    GP_TRY(set_device(h));
     const long long total = gpso_grow_count(depth);
     if (total <= 0) return fail(GPSO_E_BADARG, "gpso_grow_ucb_argmax: bad depth");
     if (row0 < 0 || row1 > total || row0 >= row1) return fail(GPSO_E_BADARG, "gpso_grow_ucb_argmax: empty or out-of-range row range");
@@ -2841,16 +2751,16 @@ extern "C" int gpso_grow_ucb_argmax_range(gpso_handle* h, const double* bounds_h
     for (int j = 0; j < d; j++)
         if (!(bounds_host[2 * j + 1] > bounds_host[2 * j])) return fail(GPSO_E_BADARG, "gpso_grow_ucb_argmax: need hi > lo per dimension");
     if (depth < 1 || depth > 20) return fail(GPSO_E_BADARG, "gpso_grow_ucb_argmax: depth must be in 1..20");
-    CU_TRY(cudaEventRecord(h->ev_t0, st));
-    CU_TRY(cudaMemcpyAsync(bdev, bounds_host, sizeof(double) * 2 * d, cudaMemcpyHostToDevice, st));
-    grow_leaves_kernel<<<(unsigned)((rows + 127) / 128), LEAF_THREADS, leaf_smem_bytes(d), st>>>(bdev, d, depth, rows, h->leaves.as<double>(), row0);
-    GP_TRY(check_launch(h, "grow_leaves"));
-    GP_TRY(score_argmax(h, st, h->leaves.as<double>(), nullptr, rows, varsigma, result_host));
-    CU_TRY(cudaEventRecord(h->ev_t1, st));
-    CU_TRY(cudaEventSynchronize(h->ev_t1));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
-    h->last_ms[0] = ms;
+    GP_TRY(timed_call(
+        h, st,
+        [&] {
+            CU_TRY(cudaMemcpyAsync(bdev, bounds_host, sizeof(double) * 2 * d, cudaMemcpyHostToDevice, st));
+            grow_leaves_kernel<<<(unsigned)((rows + 127) / 128), LEAF_THREADS, leaf_smem_bytes(d), st>>>(bdev, d, depth, rows,
+                                                                                                         h->leaves.as<double>(), row0);
+            GP_TRY(check_launch(h, "grow_leaves"));
+            return score_argmax(h, st, h->leaves.as<double>(), nullptr, rows, varsigma, result_host);
+        },
+        [&] { return wait_t1(h); }));
     result_host[0] += (double)row0;
     return 0;
 }
@@ -3109,12 +3019,6 @@ extern "C" int gpso_set_screen_mode(gpso_handle* h, int mode) {
     h->screen_S_cur = 0;
     if (h->nb > 0) g_screen_hint[std::min(h->nb, 64)] = ScreenHint();  // an explicit call restarts the ladder for this matrix size
     h->factorized = false;  // the fp32 copies are prepared by the next gpso_factorize
-    return 0;
-}
-
-extern "C" int gpso_set_screen_pair(gpso_handle* h, int enabled) {
-    if (!h) return fail(GPSO_E_BADARG, "gpso_set_screen_pair: null handle");
-    h->screen_pair = enabled != 0;
     return 0;
 }
 

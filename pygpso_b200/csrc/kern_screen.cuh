@@ -2,7 +2,7 @@
 // possibly be the arg-max; the few survivors are then re-scored by the full-precision engine (kern_ozaki.cuh, S = 5..8
 // digits), whose record is what the call returns.  The returned (index, mean, var, ucb) is therefore bit-identical to the
 // unscreened path as long as the true winner survives, which the error bound E below guarantees with a wide margin and the
-// caller verifies on the survivors (gpso_capi.cu: screened_argmax; on any doubt it falls back to the full pass).
+// caller verifies on the survivors (gpso_capi.cu: score_argmax; on any doubt it falls back to the full pass).
 //
 // Why it pays: the full-precision product kernel is bound by L2 -> SM operand traffic, not by the tensor pipe (105.9 GB per
 // 87 040-candidate window at N = 4096, S = 6 = 8.97 ms at the 11.8 TB/s the L2 delivers; profiles/r01s4_ncu_summary.md).
@@ -25,21 +25,19 @@
 namespace gpso {
 
 constexpr int SCR_NT = 128;  // candidates per tile of the screening product
-#ifndef SCR_KPS
-#define SCR_KPS 2
-#endif
 
 // FULL: all S^2 digit pairs are kept (levels 0 .. 2S-2): the product of the S-digit operands is then exact and the only error
 // left is the operand rounding -- at S = 2 that is 4 pairs instead of the 6 of the triangular 3-digit product, with 16 KB
 // instead of 24 KB of operands per k-step.  (The triangular 2-digit product drops the pair (1,1), which is as large as the result.)
-template <int S, int NT, bool FULL = false, int KPSV = SCR_KPS>
+template <int S, int NT, bool FULL = false>
 struct ScrCfg {
     static constexpr int A_BYTES = S * OZ_A_SLICE;
     static constexpr int B_SLICE = NT * 32;
     static constexpr int B_BYTES = S * B_SLICE;
     // k-steps (of 32) per ring stage: one bulk copy of A and one of B per stage (consecutive k-steps are contiguous in both
-    // digit buffers) and ONE tcgen05.commit per stage -- every row block has a multiple of 4 k-steps
-    static constexpr int KPS = KPSV;
+    // digit buffers) and ONE tcgen05.commit per stage -- every row block has a multiple of 4 k-steps.  The 2-digit full product
+    // takes four (64 KB of operands per stage, three stages): 41.8 vs 43.4 ms per 2.1e6 candidates against two k-steps x six stages
+    static constexpr int KPS = FULL ? 4 : 2;
     static constexpr int STAGE_BYTES = KPS * (A_BYTES + B_BYTES);
     // the ring is what hides the L2 latency: bytes in flight / latency is the operand bandwidth this CTA can draw (24 KB
     // chunks, 8 in flight reach 20 TB/s chip-wide, profiles/r01_i8_tcgen05_probe.txt).  192 KB leave room for one
@@ -62,8 +60,6 @@ struct ScrParams {
     double gscale;
     int nb, nks, nct;
     long long ldp;
-    int stages;              // ring depth in use (<= ScrCfg::STAGES; the launch passes the matching dynamic shared memory)
-    int debug_epi;           // timing experiments only: 1 = hand the accumulators back without reading them (results are garbage)
 };
 
 // ---- FP32 covariance (screening only) -----------------------------------------------------------------------------------
@@ -225,7 +221,7 @@ __global__ void __launch_bounds__(256) screen_convert_kernel(const double* __res
 }
 
 // S = 0: posterior mean only (no digit tiles are formed or written): the first level of the bound-and-refine arg-max, which
-// needs nothing but the mean of every candidate (gpso_capi.cu: bound_argmax).
+// needs nothing but the mean of every candidate (gpso_capi.cu: bound_pass).
 // One block = 64 candidates x all training points (super-steps of 128 training points), the register tiling of
 // crosscov_slices_kernel in FP32: thread = 2 candidates (lane, lane + 32) x 16 consecutive training points (warp w owns
 // points 16 w .. 16 w + 15 of the super-step).  The digit tiles are written in the NT-candidate layout of the screening
@@ -367,23 +363,21 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
 // ---- the screening product ------------------------------------------------------------------------------------------------
 // Same roles as ozaki_kernel: warp 0 producer (cp.async.bulk + mbarrier tx), warp 1 single-thread tcgen05.mma issuer, warps
 // 2..9 epilogue.  Work unit = candidate tile x pair of row blocks (I, nb-1-I) via OzItems<OZ_TRMM> (OzParams-compatible view).
-template <int S, int NT, bool FULL, int KPSV = SCR_KPS>
+template <int S, int NT, bool FULL>
 __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_screen_kernel(ScrParams P) {
-    using Cfg = ScrCfg<S, NT, FULL, KPSV>;
+    using Cfg = ScrCfg<S, NT, FULL>;
     constexpr int LEVELS = Cfg::LEVELS;
     constexpr int STAGES = Cfg::STAGES;
     constexpr int NBUF = Cfg::NBUF;
     extern __shared__ __align__(1024) uint8_t scr_smem_raw[];
     uint8_t* ring = scr_smem_raw;
-    const int nstages = P.stages;  // ring depth in use; barriers and scratch follow the ring
-    const size_t ring_bytes = (size_t)nstages * Cfg::STAGE_BYTES;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(scr_smem_raw + ring_bytes);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(scr_smem_raw + Cfg::RING_BYTES);
     uint64_t* full = bars;                      // [STAGES]
     uint64_t* empty = bars + STAGES;            // [STAGES]
     uint64_t* tmem_full = bars + 2 * STAGES;    // [2]
     uint64_t* tmem_empty = tmem_full + 2;       // [2]
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
-    float* red = reinterpret_cast<float*>(scr_smem_raw + ring_bytes + 1024);  // [4][NT]
+    float* red = reinterpret_cast<float*>(scr_smem_raw + Cfg::RING_BYTES + 1024);  // [4][NT]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
@@ -429,7 +423,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_screen_kernel(ScrParams P
                     oz_mbar_expect_tx(&full[st], Cfg::STAGE_BYTES);
                     oz_bulk_g2s_hint(dst, a + (size_t)ks * Cfg::A_BYTES, Cfg::KPS * Cfg::A_BYTES, &full[st], keep);
                     oz_bulk_g2s(dst + Cfg::KPS * Cfg::A_BYTES, b + (size_t)ks * Cfg::B_BYTES, Cfg::KPS * Cfg::B_BYTES, &full[st]);
-                    if (++st == nstages) {
+                    if (++st == STAGES) {
                         st = 0;
                         ph ^= 1;
                     }
@@ -483,7 +477,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_screen_kernel(ScrParams P
                         }
                     }
                     oz_commit(&empty[st]);
-                    if (++st == nstages) {
+                    if (++st == STAGES) {
                         st = 0;
                         ph ^= 1;
                     }
@@ -511,13 +505,6 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_screen_kernel(ScrParams P
             oz_fence_after();
             acc_ph[buf] ^= 1;
             const uint32_t tacc = tbase + ((uint32_t)(lg * 32) << 16) + (uint32_t)(buf * Cfg::ACC_COLS + hsel * (NT / 2));
-            if (P.debug_epi == 1) {
-                oz_fence_before();
-                __syncwarp();
-                if (lane == 0) oz_mbar_arrive(&tmem_empty[buf]);
-                buf = (buf + 1 == NBUF) ? 0 : buf + 1;
-                continue;
-            }
             float tot[NCH];
             // software-pipelined drain: the TMEM loads of chunk cc+1 are in flight while chunk cc is reduced, so the issuer
             // (which waits for the hand-over when there is only one accumulator buffer) gets the columns back after the read
@@ -575,286 +562,6 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_screen_kernel(ScrParams P
     oz_fence_before();
     __syncthreads();
     if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(OZ_TMEM_COLS));
-}
-
-// ---- CTA-pair version of the 3-digit screening product (tcgen05.mma.cta_group::2, M = 256) ------------------------------------
-// Two CTAs of a cluster (the two SMs of a TPC) work on ONE 128-candidate tile and TWO adjacent row blocks (CTA r: block 2 bp + r)
-// with a common k-range (the shorter block multiplies zero tiles for four more k-steps: the A buffer is cleared before its
-// digits are built).  Each MMA covers both row blocks; its B operand is SPLIT between the two shared memories, so every CTA
-// loads and reads only part of the B digits of a k-step:
-//      m1  A_0 x [B_0 | B_1]  N = 256   levels 0,1     CTA0 holds B_0, CTA1 holds B_1                (region Y, 4 KB)
-//      m2  A_0 x  B_2         N = 128   level  2       CTA r holds candidates 64 r .. 64 r + 63 of B_2 (region Z, 2 KB)
-//      m3  A_1 x [B_0 | B_1]  N = 256   levels 1,2     region Y again
-//      m4  A_2 x  B_0         N = 128   level  2       CTA r holds candidates 64 r .. 64 r + 63 of B_0 (region X, 2 KB)
-// Per CTA and k-step: 20 KB loaded instead of 24 KB, 28 KB of operand reads by the tensor core instead of 40 KB.
-// Synchronisation: the leader CTA (rank 0) issues; stage release and accumulator hand-over are tcgen05.commit multicasts to
-// both CTAs; CTA1 forwards "my stage is loaded" and "my epilogue has drained the accumulators" to barriers in the leader's
-// shared memory (mapa + mbarrier.arrive.release.cluster).
-struct ScrPairCfg {
-    static constexpr int S = 3, NT = 128;
-    static constexpr int A_BYTES = S * OZ_A_SLICE;
-    static constexpr int Y_BYTES = 4096, X_BYTES = 2048, Z_BYTES = 2048;
-    static constexpr int STAGE_BYTES = A_BYTES + Y_BYTES + X_BYTES + Z_BYTES;
-    static constexpr int STAGES = 9;
-    static constexpr int RING_BYTES = STAGES * STAGE_BYTES;
-    static constexpr int SMEM_BYTES = RING_BYTES + 1024 + 4 * NT * (int)sizeof(float);
-};
-
-__device__ __forceinline__ uint32_t oz_cluster_rank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void oz_cluster_sync() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void oz_mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\tmapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.shared::cluster.b64 _, [ra];\n\t}\n" ::"r"(oz_smem(bar)),
-        "r"(rank)
-        : "memory");
-}
-// wait on a barrier whose arrivals come from the other CTA of the pair.  Plain (cta-scope) acquire like every other wait of
-// these kernels: what the barrier orders is read by the tensor core through the async proxy (tcgen05.fence::after_thread_sync
-// follows), not by this thread; a cluster-scope acquire made ptxas emit an L1 invalidation per wait and cost 2.3x in kernel time.
-__device__ __forceinline__ void oz_mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\tOZC_WAIT:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
-        "@P1 bra OZC_DONE;\n\tbra OZC_WAIT;\n\tOZC_DONE:\n\t}\n" ::"r"(oz_smem(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void oz_commit_pair(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(oz_smem(bar)),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
-__device__ __forceinline__ void oz_mma_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// instruction descriptor of the pair MMA: D = S32, A = B = signed int8, K-major, M = 256, N = n
-__device__ __forceinline__ uint32_t oz_idesc_pair(int n) {
-    return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-}
-
-// work items of a CTA pair: (candidate tile, pair of block-pairs (nbp-1-j, j)); block-pair bp = row blocks 2 bp, 2 bp + 1
-struct ScrPairItems {
-    int nbp, npp, nct;
-    long long u;
-    int it;
-    unsigned stride;
-    __device__ __forceinline__ ScrPairItems(int nb, int nct_) : nbp(nb >> 1), npp(((nb >> 1) + 1) >> 1), nct(nct_), u(blockIdx.x >> 1), it(0),
-                                                                 stride(gridDim.x >> 1) {}
-    __device__ __forceinline__ bool next(int& bp, long long& ct, int& n) {
-        if (u >= (long long)nct * npp) return false;
-        ct = u / npp;
-        const int j = (int)(u - ct * npp);
-        const int items = (nbp - 1 - j != j) ? 2 : 1;
-        bp = it == 0 ? nbp - 1 - j : j;
-        n = 4 * (2 * bp + 2);
-        if (++it == items) {
-            it = 0;
-            u += stride;
-        }
-        return true;
-    }
-};
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(OZ_THREADS, 1) ozaki_screen_pair_kernel(ScrParams P) {
-    using Cfg = ScrPairCfg;
-    constexpr int S = Cfg::S, NT = Cfg::NT, STAGES = Cfg::STAGES;
-    extern __shared__ __align__(1024) uint8_t scr_smem_raw[];
-    uint8_t* ring = scr_smem_raw;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(scr_smem_raw + Cfg::RING_BYTES);
-    uint64_t* full = bars;                         // [STAGES] this CTA's stage is loaded (tx bytes)
-    uint64_t* peer_full = bars + STAGES;           // [STAGES] leader only: CTA1's stage is loaded
-    uint64_t* empty = bars + 2 * STAGES;           // [STAGES] the MMAs reading the stage are done (multicast commit)
-    uint64_t* tmem_full = bars + 3 * STAGES;       // accumulators complete (multicast commit)
-    uint64_t* tmem_empty = tmem_full + 1;          // leader only: own epilogue has drained (8 warps)
-    uint64_t* peer_tmem_empty = tmem_full + 2;     // leader only: CTA1's epilogue has drained (8 warps)
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 3);
-    float* red = reinterpret_cast<float*>(scr_smem_raw + Cfg::RING_BYTES + 1024);  // [4][NT]
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = oz_cluster_rank();
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < STAGES; i++) {
-            oz_mbar_init(&full[i], 1);
-            oz_mbar_init(&peer_full[i], 1);
-            oz_mbar_init(&empty[i], 1);
-        }
-        oz_mbar_init(tmem_full, 1);
-        oz_mbar_init(tmem_empty, 8);
-        oz_mbar_init(peer_tmem_empty, 8);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(oz_smem(tmem_slot)), "r"(OZ_TMEM_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
-    }
-    oz_fence_before();
-    __syncthreads();
-    oz_cluster_sync();
-    oz_fence_after();
-    const uint32_t tbase = *tmem_slot;
-    const int nks = P.nks;
-
-    if (warp == 0) {
-        // ================= producer (both CTAs) =================
-        if (lane == 0) {
-            int st = 0;
-            uint32_t ph = 0;
-            const uint64_t keep = oz_policy_evict_last();
-            ScrPairItems items(P.nb, P.nct);
-            int bp, n;
-            long long ct;
-            while (items.next(bp, ct, n)) {
-                const int I = 2 * bp + (int)rank;
-                const uint8_t* a = P.A + ((size_t)I * nks) * Cfg::A_BYTES;
-                const uint8_t* b = P.B + ((size_t)ct * nks) * (S * 4096);
-                for (int ks = 0; ks < n; ks++) {
-                    oz_mbar_wait(&empty[st], ph ^ 1);
-                    uint8_t* dst = ring + (size_t)st * Cfg::STAGE_BYTES;
-                    const uint8_t* bk = b + (size_t)ks * (S * 4096);
-                    oz_mbar_expect_tx(&full[st], Cfg::STAGE_BYTES);
-                    oz_bulk_g2s_hint(dst, a + (size_t)ks * Cfg::A_BYTES, Cfg::A_BYTES, &full[st], keep);
-                    oz_bulk_g2s(dst + Cfg::A_BYTES, bk + rank * 4096, Cfg::Y_BYTES, &full[st]);                                // B_rank
-                    oz_bulk_g2s(dst + Cfg::A_BYTES + Cfg::Y_BYTES, bk + rank * 2048, Cfg::X_BYTES, &full[st]);                 // half of B_0
-                    oz_bulk_g2s(dst + Cfg::A_BYTES + Cfg::Y_BYTES + Cfg::X_BYTES, bk + 2 * 4096 + rank * 2048, Cfg::Z_BYTES, &full[st]);  // half of B_2
-                    if (++st == STAGES) {
-                        st = 0;
-                        ph ^= 1;
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            int st = 0;
-            uint32_t ph = 0, acc_ph = 0;
-            ScrPairItems items(P.nb, P.nct);
-            int bp, n;
-            long long ct;
-            if (rank == 0) {
-                // ================= MMA issuer (leader) =================
-                const uint32_t ring_addr = oz_smem(ring);
-                while (items.next(bp, ct, n)) {
-                    oz_mbar_wait(tmem_empty, acc_ph ^ 1);
-                    oz_mbar_wait_cluster(peer_tmem_empty, acc_ph ^ 1);
-                    oz_fence_after();
-                    for (int ks = 0; ks < n; ks++) {
-                        oz_mbar_wait(&full[st], ph);
-                        oz_mbar_wait_cluster(&peer_full[st], ph);
-                        oz_fence_after();
-                        const uint32_t sa = ring_addr + (uint32_t)st * Cfg::STAGE_BYTES;
-                        const uint32_t sy = sa + Cfg::A_BYTES, sx = sy + Cfg::Y_BYTES, sz = sx + Cfg::X_BYTES;
-                        const uint32_t acc = ks > 0 ? 1u : 0u;
-                        oz_mma_pair(tbase + 0 * NT, oz_desc(sa + 0 * OZ_A_SLICE), oz_desc(sy), oz_idesc_pair(256), acc);  // levels 0,1
-                        oz_mma_pair(tbase + 2 * NT, oz_desc(sa + 0 * OZ_A_SLICE), oz_desc(sz), oz_idesc_pair(128), acc);  // level 2
-                        oz_mma_pair(tbase + 1 * NT, oz_desc(sa + 1 * OZ_A_SLICE), oz_desc(sy), oz_idesc_pair(256), 1u);   // levels 1,2
-                        oz_mma_pair(tbase + 2 * NT, oz_desc(sa + 2 * OZ_A_SLICE), oz_desc(sx), oz_idesc_pair(128), 1u);   // level 2
-                        oz_commit_pair(&empty[st]);
-                        if (++st == STAGES) {
-                            st = 0;
-                            ph ^= 1;
-                        }
-                    }
-                    oz_commit_pair(tmem_full);
-                    acc_ph ^= 1;
-                }
-            } else {
-                // ================= forwarder (CTA1): my stage is loaded -> leader =================
-                while (items.next(bp, ct, n)) {
-                    for (int ks = 0; ks < n; ks++) {
-                        oz_mbar_wait(&full[st], ph);
-                        oz_mbar_arrive_remote(&peer_full[st], 0);
-                        if (++st == STAGES) {
-                            st = 0;
-                            ph ^= 1;
-                        }
-                    }
-                }
-            }
-        }
-    } else {
-        // ================= epilogue (both CTAs: own 128 rows) =================
-        const int lg = warp & 3;
-        const int hsel = (warp - 2) >> 2;
-        const int et = threadIdx.x - 64;
-        constexpr int NCH = NT / 16;
-        uint32_t acc_ph = 0;
-        ScrPairItems items(P.nb, P.nct);
-        int bp, n;
-        long long ct;
-        while (items.next(bp, ct, n)) {
-            const int I = 2 * bp + (int)rank;
-            const int row = I * 128 + lg * 32 + lane;
-            const float rs = (float)(P.rowscale[row] * P.gscale);
-            oz_mbar_wait(tmem_full, acc_ph);
-            oz_fence_after();
-            acc_ph ^= 1;
-            const uint32_t tacc = tbase + ((uint32_t)(lg * 32) << 16) + (uint32_t)(hsel * (NT / 2));
-            float tot[NCH];
-#pragma unroll
-            for (int cc = 0; cc < NCH; cc++) {
-                uint32_t r[S][8];
-#pragma unroll
-                for (int t = 0; t < S; t++) oz_tmem_ld8(tacc + (uint32_t)(t * NT + cc * 8), r[t]);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (cc == NCH - 1) {
-                    oz_fence_before();
-                    __syncwarp();
-                    if (lane == 0) {
-                        if (rank == 0) oz_mbar_arrive(tmem_empty);
-                        else oz_mbar_arrive_remote(peer_tmem_empty, 0);
-                    }
-                }
-                float v[8];
-#pragma unroll
-                for (int i = 0; i < 8; i++) {
-                    float w = (float)(int32_t)r[0][i];
-#pragma unroll
-                    for (int t = 1; t < S; t++) w = fmaf(w, 256.0f, (float)(int32_t)r[t][i]);
-                    w *= rs;
-                    v[i] = w * w;
-                }
-#pragma unroll
-                for (int o = 16, nn = 4; o >= 4; o >>= 1, nn >>= 1) {
-                    const bool up = (lane & o) != 0;
-#pragma unroll
-                    for (int i = 0; i < nn; i++) {
-                        const float send = up ? v[i] : v[i + nn];
-                        const float keepv = up ? v[i + nn] : v[i];
-                        v[i] = keepv + __shfl_xor_sync(0xffffffffu, send, o);
-                    }
-                }
-                const float t2 = v[0] + __shfl_xor_sync(0xffffffffu, v[0], 2);
-                tot[cc] = t2 + __shfl_xor_sync(0xffffffffu, t2, 1);
-            }
-            const int idx = ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1);
-            asm volatile("bar.sync 1, 256;" ::: "memory");
-            if ((lane & 3) == 0) {
-#pragma unroll
-                for (int cc = 0; cc < NCH; cc++) red[lg * NT + hsel * (NT / 2) + cc * 8 + idx] = tot[cc];
-            }
-            asm volatile("bar.sync 1, 256;" ::: "memory");
-            if (et < NT) {
-                const float s = (red[et] + red[NT + et]) + (red[2 * NT + et] + red[3 * NT + et]);
-                P.part[(size_t)I * P.ldp + (size_t)ct * NT + et] = s;
-            }
-        }
-    }
-    oz_fence_before();
-    __syncthreads();
-    oz_cluster_sync();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(OZ_TMEM_COLS));
 }
 
 // ---- order-preserving key of a double for atomicMax on 64-bit words ---------------------------------------------------------

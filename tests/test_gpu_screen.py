@@ -233,29 +233,3 @@ def test_c3_shape_screened_vs_full(cuda):
     s.close()
     assert dm[0] == ref[0]
     assert abs(dm[3] - ref[3]) <= 1e-8 * max(abs(ref[3]), 1.0)
-
-
-@pytest.mark.timeout(120)
-@pytest.mark.parametrize("N,d,M", [(1024, 4, 70_000), (2000, 6, 90_000)])
-def test_cta_pair_product_equals_single_cta_product(cuda, N, d, M):
-    """The cta_group::2 form of the 3-digit screening product (two row blocks per MMA, B digits split between the two shared
-    memories of a TPC) must reproduce the single-CTA kernel's screened values bit for bit: same integers, same fp32 epilogue."""
-    X, y = synthetic(N, d, seed=N + 1)
-    h = go.Hyper(0.25 * np.sqrt(d), 1.0, 1e-3, 0.05)
-    Xc = np.random.default_rng(M).random((M, d))
-    s = open_session(cuda, "Matern52", X, y)
-    s.set_screen_mode(3)
-    s.factorize(theta_of(h))
-    out = {}
-    for pair in (False, True):
-        s.set_screen_pair(pair)
-        rec = s.ucb_argmax(Xc, VARSIGMA)
-        info = s.screen_info()
-        assert info["path"] == "screened" and info["digits"] == 3, info
-        out[pair] = (rec, s.screened_values(M))
-    s.set_screen_mode(0)
-    s.factorize(theta_of(h))
-    ref = s.ucb_argmax(Xc, VARSIGMA)
-    s.close()
-    assert same_record(out[False][0], ref) and same_record(out[True][0], ref)
-    assert np.array_equal(out[False][1], out[True][1])

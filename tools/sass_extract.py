@@ -15,8 +15,8 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "pygpso_b200", "libgpso_b200.so")
 KERNELS = {
-    "ozaki_screen_kernel_S2_all_pairs": "19ozaki_screen_kernelILi2ELi128ELb1ELi4EE",
-    "ozaki_screen_kernel_S3_NT128": "19ozaki_screen_kernelILi3ELi128ELb0ELi2EE",
+    "ozaki_screen_kernel_S2_all_pairs": "19ozaki_screen_kernelILi2ELi128ELb1EE",
+    "ozaki_screen_kernel_S3_NT128": "19ozaki_screen_kernelILi3ELi128ELb0EE",
     "ozaki_kernel_S6_TRMM": "12ozaki_kernelILi6ELi0EE",
     "ozaki_kernel_S7_LAUUM": "12ozaki_kernelILi7ELi1EE",
     "ozaki_kernel_S8_GEMM": "12ozaki_kernelILi8ELi2EE",
