@@ -20,6 +20,9 @@
  *         [ lengthscale(s) (1, or d when ard) , kernel variance , likelihood (noise) variance , mean constant (if any) ]
  *     GPSO_KERNEL_RQ puts its shape parameter alpha first (tf.Module lists kernel.alpha before kernel.lengthscales):
  *         [ alpha , lengthscale(s) , kernel variance , likelihood (noise) variance , mean constant (if any) ]
+ *     GPSO_MEAN_LINEAR (m(x) = x . A + b) packs d + 1 mean entries in the place of the constant, A before b ('A' < 'b'):
+ *         [ (alpha) , lengthscale(s) , kernel variance , likelihood (noise) variance , A[0..d-1] , b ]
+ *     d is the input dimension of gpso_set_data, so the count is known from then on (as for ARD lengthscales).
  *     `u`     = unconstrained (softplus pre-image; noise variance has the 1e-6 floor of gpflow.likelihoods.Gaussian),
  *     `theta` = constrained values.
  */
@@ -46,8 +49,8 @@ enum {
 /* gpflow.kernels.* accepted by GPRSurrogate(gp_kernel=...), gp_surrogate.py:393-402, default Matern52 (:424) */
 enum { GPSO_KERNEL_MATERN12 = 0, GPSO_KERNEL_MATERN32 = 1, GPSO_KERNEL_MATERN52 = 2, GPSO_KERNEL_SE = 3, GPSO_KERNEL_RQ = 4 };
 /* GPSO_KERNEL_RQ = gpflow.kernels.RationalQuadratic: variance * (1 + r2 / (2 alpha))^-alpha, alpha > 0 (softplus) */
-/* gpflow.mean_functions.*: None/Zero or Constant (:167, :427) */
-enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1 };
+/* gpflow.mean_functions.*: None/Zero or Constant (:167, :427), or Linear (m(x) = x . A + b, A[d,1] and b unconstrained) */
+enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1, GPSO_MEAN_LINEAR = 2 };
 
 /* ---- library ------------------------------------------------------------------------------------------------- */
 int gpso_version(void);                 /* ABI version, currently 1 */
@@ -125,7 +128,9 @@ int gpso_grow_ucb_argmax_range(gpso_handle* h, const double* bounds_host, int d,
 
 /* ---- multi-GPU: share one fit with the ranks that score candidate shards -------------------------------------- */
 /* The fitted state (theta, scaled training inputs, alpha, L^-1) is exposed as ONE contiguous device buffer so the host
- * side can broadcast it with a single NCCL call (torch.distributed.broadcast) and import it on the other ranks. */
+ * side can broadcast it with a single NCCL call (torch.distributed.broadcast) and import it on the other ranks.
+ * GPSO_MEAN_LINEAR handles append A (d doubles) after L^-1, so their state is 8 d bytes longer; a state is only imported into
+ * a handle that has a linear mean exactly when the exporting handle had one (GPSO_E_BADARG otherwise). */
 int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes);   /* size for a given problem shape */
 int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t bytes, void* stream);
 int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream);

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libgpso_b200.so")
 SOURCES = ["gpso_capi.cu"]
-HEADERS = ["common.cuh", "gemm_core.cuh", "kern_cov.cuh", "kern_dense.cuh", "kern_leaves.cuh", "kern_ozaki.cuh", "kern_predict.cuh", "kern_joint.cuh", "kern_screen.cuh", "kern_probe.cuh"]
+HEADERS = ["common.cuh", "gemm_core.cuh", "kern_cov.cuh", "kern_dense.cuh", "kern_leaves.cuh", "kern_ozaki.cuh", "kern_predict.cuh", "kern_joint.cuh", "kern_screen.cuh", "kern_probe.cuh", "kern_mean.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -189,9 +189,11 @@ class CudaSession:
         self.device = device
         self.kernel = kernel
         self.ard = n_lengthscales > 1
+        # has_mean is the mean id of the C ABI: 0 / False none, 1 / True constant, 2 linear (m(x) = x . A + b)
+        self.mean_id = int(has_mean)
         self.has_mean = bool(has_mean)
         handle = ctypes.c_void_p()
-        _check(lib, lib.gpso_create(device, KERNEL_IDS[kernel], int(self.ard), int(self.has_mean), ctypes.byref(handle)),
+        _check(lib, lib.gpso_create(device, KERNEL_IDS[kernel], int(self.ard), self.mean_id, ctypes.byref(handle)),
                "gpso_create")
         self._h = handle
         self.N = self.d = 0

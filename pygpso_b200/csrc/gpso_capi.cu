@@ -29,6 +29,7 @@
 #include "kern_joint.cuh"
 #include "kern_screen.cuh"
 #include "kern_probe.cuh"
+#include "kern_mean.cuh"
 
 using namespace gpso;
 
@@ -212,6 +213,7 @@ struct gpso_handle {
     bool used_pending[2] = {false, false};
     // data + fitted state
     DevBuf X, y, Xs, ls, alpha;
+    DevBuf meanA;  // GPSO_MEAN_LINEAR: A (d doubles)
     DevBuf K, Linv, LinvT, T, Kinv;
     DevBuf resid, a, logdet, scalars, gpart, gout, info, counter;
     // persistent Cholesky scheduler: task queue (rebuilt when nb changes) and its state [next, err, cnt[nb*nb]]
@@ -270,7 +272,8 @@ struct gpso_handle {
     double scr_info[12] = {0};
     size_t scr_prod_marks = 0;
     // host copies of the hyper-parameters in force
-    double ls_host[MAX_LS] = {0}, variance = 1.0, noise = 1.0, c0 = 0.0;
+    double ls_host[MAX_LS] = {0}, variance = 1.0, noise = 1.0, c0 = 0.0;  // c0: the mean constant, or b of the linear mean
+    double A_host[MAX_LS] = {0};  // GPSO_MEAN_LINEAR: A, also in meanA on the device
     double rq_alpha = 1.0;  // RationalQuadratic shape (KERNEL_RQ only; the other kernels never read it)
     bool have_data = false, factorized = false;
     double factor_nlml = 0.0;
@@ -294,7 +297,9 @@ struct gpso_handle {
     std::vector<double> trace_out;
     int n_ls() const { return ard ? d : 1; }
     int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
-    int n_params() const { return n_rq() + n_ls() + 2 + (mean_id == GPSO_MEAN_CONSTANT ? 1 : 0); }
+    bool linear() const { return mean_id == GPSO_MEAN_LINEAR; }
+    int n_mean() const { return mean_id == GPSO_MEAN_CONSTANT ? 1 : (linear() ? d + 1 : 0); }  // A (d entries) before b
+    int n_params() const { return n_rq() + n_ls() + 2 + n_mean(); }
 };
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -554,6 +559,7 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     GP_TRY(h->y.ensure((size_t)Np * sizeof(double)));
     GP_TRY(h->Xs.ensure((size_t)d * Np * sizeof(double)));
     GP_TRY(h->ls.ensure(MAX_LS * sizeof(double)));
+    if (h->linear()) GP_TRY(h->meanA.ensure(MAX_LS * sizeof(double)));
     GP_TRY(h->alpha.ensure((size_t)Np * sizeof(double)));
     GP_TRY(h->resid.ensure((size_t)Np * sizeof(double)));
     GP_TRY(h->a.ensure((size_t)Np * sizeof(double)));
@@ -583,6 +589,14 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
 static int upload_lengthscales(gpso_handle* h, cudaStream_t st) {
     CU_TRY(cudaMemcpyAsync(h->ls.p, h->ls_host, sizeof(double) * h->n_ls(), cudaMemcpyHostToDevice, st));
     return 0;
+}
+
+// Linear mean: out[0..rows) += sgn * (x_i . A) for the rows x_i of X, one launch on st, the stream that produces out (the
+// constant b is already in out as c0).  Nothing for the other mean functions.
+static int add_linear_offset(gpso_handle* h, cudaStream_t st, const double* X, long long rows, double sgn, double* out) {
+    if (!h->linear()) return 0;
+    linear_offset_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(X, rows, h->d, h->meanA.as<double>(), sgn, out);
+    return check_launch(h, "linear_offset");
 }
 
 // Task list of the persistent factorisation kernel (kern_dense.cuh): topological, with look-ahead.  Cholesky in blocks of
@@ -1203,6 +1217,7 @@ static int factor_pipeline(gpso_handle* h, cudaStream_t st, bool need_kinv) {
     const int Np = h->Np, nb = h->nb;
     GP_TRY(l2_setaside(h, 0));  // the whole L2 for the tile traffic of the factorisation (see set_l2_window)
     GP_TRY(upload_lengthscales(h, st));
+    if (h->linear()) CU_TRY(cudaMemcpyAsync(h->meanA.p, h->A_host, sizeof(double) * h->d, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemsetAsync(h->info.p, 0, sizeof(int), st));
     scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(h->X.as<double>(), h->ls.as<double>(), h->n_ls(), h->N, h->d, Np,
                                                           h->Xs.as<double>());
@@ -1302,6 +1317,7 @@ static int factor_pipeline(gpso_handle* h, cudaStream_t st, bool need_kinv) {
     }
     residual_kernel<<<(Np + 255) / 256, 256, 0, st>>>(h->y.as<double>(), h->c0, h->N, Np, h->resid.as<double>());
     GP_TRY(check_launch(h, "residual"));
+    GP_TRY(add_linear_offset(h, st, h->X.as<double>(), h->N, -1.0, h->resid.as<double>()));  // (y - b) - x . A
     tri_matvec_kernel<true><<<(Np + 7) / 8, 256, 0, st>>>(P.Linv, h->resid.as<double>(), Np, h->a.as<double>());
     GP_TRY(check_launch(h, "trimv_lower"));
     tri_matvec_kernel<false><<<(Np + 7) / 8, 256, 0, st>>>(P.LinvT, h->a.as<double>(), Np, h->alpha.as<double>());
@@ -1458,7 +1474,8 @@ static int init_handle(gpso_handle* h, int device, int kernel_id, int ard, int m
     }
     CU_TRY(cudaEventCreate(&h->ev_t0));
     CU_TRY(cudaEventCreate(&h->ev_t1));
-    CU_TRY(cudaHostAlloc((void**)&h->host_rec, (MAX_LS + 16) * sizeof(double), cudaHostAllocDefault));
+    // room for the gradient record of gpso_neg_lml_grad: 4 + partial sums (up to MAX_LS + 3) + the linear mean's A (MAX_LS)
+    CU_TRY(cudaHostAlloc((void**)&h->host_rec, (2 * MAX_LS + 16) * sizeof(double), cudaHostAllocDefault));
     GP_TRY(configure_kernels_once(device));
     return 0;
 }
@@ -1469,7 +1486,7 @@ extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso
     if (!out) return fail(GPSO_E_BADARG, "gpso_create: out is null");
     *out = nullptr;
     if (kernel_id < 0 || kernel_id > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
-    if (mean_id != GPSO_MEAN_ZERO && mean_id != GPSO_MEAN_CONSTANT) return fail(GPSO_E_BADARG, "gpso_create: unknown mean id");
+    if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create: unknown mean id");
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) return fail(GPSO_E_NOGPU, "gpso_create: no CUDA device available");
     if (device < 0 || device >= n) return fail(GPSO_E_BADARG, "gpso_create: device index out of range");
@@ -1561,7 +1578,13 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
     h->noise = theta[nl + 1];
     if (!(h->variance > 0.0 || (allow_zero && h->variance == 0.0)) || !(h->noise > 0.0))
         return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
-    h->c0 = (h->mean_id == GPSO_MEAN_CONSTANT) ? theta[nl + 2] : 0.0;
+    const double* m = theta + nl + 2;  // the mean function's entries
+    if (h->linear()) {
+        for (int k = 0; k < h->d; k++) h->A_host[k] = m[k];
+        h->c0 = m[h->d];
+    } else {
+        h->c0 = (h->mean_id == GPSO_MEAN_CONSTANT) ? m[0] : 0.0;
+    }
     return 0;
 }
 
@@ -1578,7 +1601,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     for (int i = 0; i < nl; i++) theta[na + i] = softplus(u[i]);
     theta[na + nl] = softplus(u[nl]);
     theta[na + nl + 1] = NOISE_FLOOR + softplus(u[nl + 1]);
-    if (h->mean_id == GPSO_MEAN_CONSTANT) theta[na + nl + 2] = u[nl + 2];
+    for (int i = 0; i < h->n_mean(); i++) theta[na + nl + 2 + i] = u[nl + 2 + i];  // unconstrained
     // softplus(u) underflows to exactly 0 for u < -745 and L-BFGS-B line searches do probe such points: like GPflow, evaluate
     // them (kernel variance 0 -> K_y = noise * I; lengthscale 0 -> NaN objective) instead of rejecting the call
     GP_TRY(load_theta(h, theta.data(), p, "gpso_neg_lml_grad", true));
@@ -1589,18 +1612,23 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     const int nb64 = h->Np / CT;
     const int nblk = nb64 * (nb64 + 1) / 2;
     const int stride = 2 + nl + na;
+    const int nA = h->linear() ? h->d : 0;  // X^T alpha follows the reduced partial sums in gout
     GP_TRY(h->gpart.ensure((size_t)nblk * stride * sizeof(double)));
-    GP_TRY(h->gout.ensure((size_t)(stride + 4) * sizeof(double)));
+    GP_TRY(h->gout.ensure((size_t)(stride + 4 + nA) * sizeof(double)));
     launch_grad(h, st, nblk, stride);
     if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
     reduce_partials_kernel<<<stride, 256, 0, st>>>(h->gpart.as<double>(), nblk, stride, h->gout.as<double>());
     GP_TRY(check_launch(h, "reduce_partials"));
+    if (nA) {
+        linear_grad_kernel<<<nA, 256, 0, st>>>(h->X.as<double>(), h->alpha.as<double>(), h->N, h->d, h->gout.as<double>() + stride);
+        GP_TRY(check_launch(h, "linear_grad"));
+    }
     CU_TRY(cudaEventRecord(h->ev_t1, st));
-    // one pinned record [scalars(3) | info | gradient partial sums(stride)]: three truly asynchronous copies, one wait
+    // one pinned record [scalars(3) | info | gradient partial sums(stride) | X^T alpha(nA)]: three truly asynchronous copies, one wait
     double* rec = h->host_rec;
     CU_TRY(cudaMemcpyAsync(rec, h->scalars.p, 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(rec + 3, h->info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(rec + 4, h->gout.p, sizeof(double) * stride, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(rec + 4, h->gout.p, sizeof(double) * (stride + nA), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     const double* sc = rec;
     const double* g = rec + 4;
@@ -1624,6 +1652,10 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     grad_host[nl] = h->variance > 0.0 ? -(0.5 * g[0] / h->variance) * sigmoid(u[nl]) : 0.0;
     grad_host[nl + 1] = -(0.5 * g[1]) * sigmoid(u[nl + 1]);
     if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[nl + 2] = -sc[2];
+    if (nA) {  // d(-LML)/dA = -X^T alpha, d(-LML)/db = -sum(alpha)
+        for (int k = 0; k < nA; k++) grad_host[nl + 2 + k] = -g[stride + k];
+        grad_host[nl + 2 + nA] = -sc[2];
+    }
     // alpha (slot stride - 1 of the partial sums); alpha == 0 only when softplus underflowed: the entry is 0, as for the variance
     if (na) grad_host[-1] = h->rq_alpha > 0.0 ? -(0.5 * g[stride - 1]) * sigmoid(u[-1]) : 0.0;
     return 0;
@@ -1906,10 +1938,12 @@ static int full_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, cons
         if (oz) {
             DISPATCH_S(S, launch_oz_crosscov, h, xs, win.src, win.Mw, pad(win.Mw) / OZ_NT, bscale, h->ozBb[win.b].as<uint8_t>(),
                        h->wmeanb[win.b].as<double>());
-            return check_launch(h, "crosscov_slices");
+            GP_TRY(check_launch(h, "crosscov_slices"));
+        } else {
+            launch_crosscov(h, xs, win.src, win.Mw, pad(win.Mw));
+            GP_TRY(check_launch(h, "crosscov"));
         }
-        launch_crosscov(h, xs, win.src, win.Mw, pad(win.Mw));
-        return check_launch(h, "crosscov");
+        return add_linear_offset(h, xs, win.src, win.Mw, 1.0, h->wmeanb[win.b].as<double>());
     };
     // part[I][c] = sum over the rows of block I of (L^-1 k*)^2
     body.product = [&](const Window& win, cudaStream_t ps) {
@@ -2160,7 +2194,8 @@ static int screen_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, co
     body.xcov = [&](const Window& win, cudaStream_t xs) {
         DISPATCH_SCREEN_S(S, launch_screen_crosscov, h, xs, win.src, win.Mw, pad(win.Mw) / 64, bscale, h->ozBb[win.b].as<uint8_t>(),
                           h->wmeanb[win.b].as<double>());
-        return check_launch(h, "crosscov_screen");
+        GP_TRY(check_launch(h, "crosscov_screen"));
+        return add_linear_offset(h, xs, win.src, win.Mw, 1.0, h->wmeanb[win.b].as<double>());  // the refine pass adds the same
     };
     body.product = [&](const Window& win, cudaStream_t ps) {
         const long long Mw_pad = pad(win.Mw);
@@ -2228,7 +2263,8 @@ static int bound_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, con
     body.xcov = [&](const Window& win, cudaStream_t xs) {
         launch_screen_crosscov<0>(h, xs, win.src, win.Mw, ((win.Mw + SCR_NT - 1) / SCR_NT) * SCR_NT / 64, 0.0f, nullptr,
                                   h->wmeanb[0].as<double>());
-        return check_launch(h, "crosscov_mean");
+        GP_TRY(check_launch(h, "crosscov_mean"));
+        return add_linear_offset(h, xs, win.src, win.Mw, 1.0, h->wmeanb[0].as<double>());
     };
     body.finalise = [&](const Window& win, cudaStream_t ps) {
         bound_finalize_kernel<<<(unsigned)((win.Mw + 255) / 256), 256, 0, ps>>>(h->wmeanb[0].as<double>(), win.Mw, win.off,
@@ -2535,6 +2571,7 @@ static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M,
     GP_TRY(check_launch(h, "scale_inputs"));
     launch_joint_crosscov(h, st, Xc, M, Mp);
     GP_TRY(check_launch(h, "crosscov"));
+    GP_TRY(add_linear_offset(h, st, Xc, M, 1.0, h->jmean.as<double>()));
     JointVParams P;
     P.Linv = h->Linv.as<double>();
     P.KsT = h->jKsT.as<double>();
@@ -2771,16 +2808,16 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// multi-GPU state exchange: [ header (128 doubles) | Xs (d*Np) | alpha (Np) | Linv (Np*Np) ]
-// header: N, d, kernel variance, noise variance, mean constant, -LML, kernel id, ard, RationalQuadratic alpha (0 for the
-// other kernels), lengthscales from slot 16
+// multi-GPU state exchange: [ header (128 doubles) | Xs (d*Np) | alpha (Np) | Linv (Np*Np) | A (d, linear mean only) ]
+// header: N, d, kernel variance, noise variance, mean constant (b of the linear mean), -LML, kernel id, ard, RationalQuadratic
+// alpha (0 for the other kernels), mean id, lengthscales from slot 16.  A does not fit beside 64 lengthscales in the header.
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int STATE_HEADER = 128;
 
 extern "C" int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes) {
     if (!h || !bytes || N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_state_bytes: bad argument");
     long long Np = ((N + TB - 1) / TB) * TB;
-    *bytes = (int64_t)sizeof(double) * (STATE_HEADER + (long long)d * Np + Np + Np * Np);
+    *bytes = (int64_t)sizeof(double) * (STATE_HEADER + (long long)d * Np + Np + Np * Np + (h->linear() ? d : 0));
     return 0;
 }
 
@@ -2802,6 +2839,7 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     hdr[6] = h->kernel_id;
     hdr[7] = h->ard;
     if (h->n_rq()) hdr[8] = h->rq_alpha;
+    hdr[9] = h->mean_id;
     for (int i = 0; i < h->n_ls(); i++) hdr[16 + i] = h->ls_host[i];
     double* dst = (double*)dst_dev;
     CU_TRY(cudaStreamSynchronize(h->stream));
@@ -2810,6 +2848,8 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER, h->Xs.p, sizeof(double) * h->d * Np, cudaMemcpyDeviceToDevice, st));
     CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + h->d * Np, h->alpha.p, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));
     CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + h->d * Np + Np, h->Linv.p, sizeof(double) * Np * Np, cudaMemcpyDeviceToDevice, st));
+    if (h->linear())
+        CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + h->d * Np + Np + Np * Np, h->meanA.p, sizeof(double) * h->d, cudaMemcpyDeviceToDevice, st));
     CU_TRY(cudaStreamSynchronize(st));
     return 0;
 }
@@ -2830,6 +2870,8 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     CU_TRY(cudaStreamSynchronize(st));
     if ((int)hdr[0] != N || (int)hdr[1] != d) return fail(GPSO_E_BADARG, "gpso_import_state_dev: header shape mismatch");
     if ((int)hdr[6] != h->kernel_id || (int)hdr[7] != h->ard) return fail(GPSO_E_BADARG, "gpso_import_state_dev: kernel mismatch");
+    if (((int)hdr[9] == GPSO_MEAN_LINEAR) != h->linear())
+        return fail(GPSO_E_BADARG, "gpso_import_state_dev: linear mean function on one side only");
     h->variance = hdr[2];
     h->noise = hdr[3];
     h->c0 = hdr[4];
@@ -2840,6 +2882,10 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     CU_TRY(cudaMemcpyAsync(h->Xs.p, src + STATE_HEADER, sizeof(double) * d * Np, cudaMemcpyDeviceToDevice, st));
     CU_TRY(cudaMemcpyAsync(h->alpha.p, src + STATE_HEADER + d * Np, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));
     CU_TRY(cudaMemcpyAsync(h->Linv.p, src + STATE_HEADER + d * Np + Np, sizeof(double) * Np * Np, cudaMemcpyDeviceToDevice, st));
+    if (h->linear()) {
+        CU_TRY(cudaMemcpyAsync(h->meanA.p, src + STATE_HEADER + d * Np + Np + Np * Np, sizeof(double) * d, cudaMemcpyDeviceToDevice, st));
+        CU_TRY(cudaMemcpyAsync(h->A_host, h->meanA.p, sizeof(double) * d, cudaMemcpyDeviceToHost, st));
+    }
     GP_TRY(upload_lengthscales(h, st));
     CU_TRY(cudaStreamSynchronize(st));
     GP_TRY(prepare_ozaki(h, st));  // the digit tiles are rebuilt locally from the imported L^-1 (bit-identical on every rank)

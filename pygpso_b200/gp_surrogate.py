@@ -286,7 +286,7 @@ class GPSurrogate:
     ):
         """
         :param gp_kernel: covariance function (``pygpso_b200.gpmodel.kernels.*``)
-        :param gp_meanf: mean function (``gpmodel.mean_functions.Constant`` / ``Zero``) or None
+        :param gp_meanf: mean function (``gpmodel.mean_functions.Constant`` / ``Linear`` / ``Zero``) or None
         :param optimiser: object with ``minimize(closure, variables)``; default ``gpmodel.optimizers.Scipy()``
         :param varsigma: UCB multiplier, ``ucb = mean + varsigma * var``
         :param points: initial list of :class:`GPPoint`
@@ -624,7 +624,12 @@ class GPRSurrogate(GPSurrogate):
         gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
         assert hasattr(gpmodel.mean_functions, info["gpr_meanf"])
         meanf_cls = getattr(gpmodel.mean_functions, info["gpr_meanf"])
-        gp_meanf = meanf_cls(np.zeros(info["gpr_meanf_shape"])) if meanf_cls is gpmodel.Constant else meanf_cls()
+        if meanf_cls is gpmodel.Constant:
+            gp_meanf = meanf_cls(np.zeros(info["gpr_meanf_shape"]))
+        elif meanf_cls is gpmodel.Linear:  # gpr_meanf_shape is the shape of A, [d, 1]; multiple_assign restores A and b below
+            gp_meanf = meanf_cls(np.zeros(info["gpr_meanf_shape"]), np.zeros(1))
+        else:
+            gp_meanf = meanf_cls()
         optimiser = cls._deserialse_optimiser(info["optimiser"])
 
         model = gpmodel.GPR(

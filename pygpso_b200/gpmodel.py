@@ -8,7 +8,7 @@ and ``gpflow.models.GPR`` (gpso/gp_surrogate.py:138,165-169,397,424-429,463-473,
     optimiser.minimize(model.training_loss, model.trainable_variables)     :500-503
     model.predict_y(Xnew) -> (mean[M,1], var[M,1]) with ``.numpy()``      :298,325; plotting.py:351-356
     model.predict_f(Xnew, full_cov=True), model.predict_f_samples(Xnew, S)   (joint posterior, user code)
-    model.kernel.lengthscales / .variance, model.likelihood.variance, model.mean_function.c   (summaries, save)
+    model.kernel.lengthscales / .variance, model.likelihood.variance, model.mean_function.c (.A, .b)   (summaries, save)
     gpflow.utilities.parameter_dict / multiple_assign / freeze            :462-473,514-519
 
 so exactly that surface is provided here under the same names (``kernels``, ``mean_functions``, ``likelihoods``,
@@ -18,7 +18,8 @@ implementation in this package.
 
 Parameterisation follows GPflow 2: positive parameters are softplus-transformed, the Gaussian likelihood variance has
 the 1e-6 floor, and ``trainable_variables`` are ordered kernel.lengthscales, kernel.variance, likelihood.variance,
-mean_function.c -- preceded by kernel.alpha for ``RationalQuadratic`` (tf.Module visits attributes in sorted name order).
+mean_function.c (or mean_function.A, mean_function.b for ``Linear``) -- preceded by kernel.alpha for ``RationalQuadratic``
+(tf.Module visits attributes in sorted name order).
 """
 import types
 
@@ -193,6 +194,30 @@ class Constant(MeanFunction):
         return (self.c,)
 
 
+class Linear(MeanFunction):
+    """``gpflow.mean_functions.Linear``: ``m(X) = X @ A + b`` with ``A[d,1]`` and ``b[1]``, both unconstrained.  GPflow's
+    default ``A = ones((1, 1))`` fits one input dimension only; ``GPR`` checks ``A`` against the inputs when data is set."""
+
+    def __init__(self, A=None, b=None):
+        A = np.ones((1, 1)) if A is None else A
+        b = np.zeros(1) if b is None else b
+        self.A = Parameter(A, positive=False, name="mean_function.A")
+        self.b = Parameter(b, positive=False, name="mean_function.b")
+        if len(self.A.shape) != 2 or self.A.shape[1] != 1:
+            raise ValueError(f"A must have shape [d, 1] (a single output), got {tuple(self.A.shape)}")
+        if self.b.size != 1:
+            raise ValueError("b must be a scalar (pyGPSO scores are one-dimensional)")
+
+    @property
+    def parameters(self):
+        return (self.A, self.b)
+
+
+# mean id of the C ABI (GPSO_MEAN_*) passed to open_session: False / True for Zero / Constant, 2 for Linear
+def _mean_id(mean_function):
+    return 2 if isinstance(mean_function, Linear) else isinstance(mean_function, Constant)
+
+
 class Gaussian:
     def __init__(self, variance=1.0):
         self.variance = Parameter(variance, positive=True, lower=NOISE_VARIANCE_FLOOR, name="likelihood.variance")
@@ -234,14 +259,14 @@ class GPR(GPModel):
             raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic")
         self.kernel = kernel
         self.mean_function = Zero() if mean_function is None else mean_function
-        if not isinstance(self.mean_function, (Zero, Constant)):
-            raise TypeError("mean_function must be Zero or Constant")
+        if not isinstance(self.mean_function, (Zero, Constant, Linear)):
+            raise TypeError("mean_function must be Zero, Constant or Linear")
         self.likelihood = Gaussian(noise_variance)
         self._backend = backend if backend is not None else _backend.default_backend()
         self._session = self._backend.open_session(
             kernel=type(kernel).__name__,
             n_lengthscales=self.kernel.lengthscales.size,
-            has_mean=isinstance(self.mean_function, Constant),
+            has_mean=_mean_id(self.mean_function),
         )
         self._factor_key = None
         self.n_loss_evaluations = 0
@@ -261,6 +286,9 @@ class GPR(GPModel):
             raise ValueError(f"data must be (X[N,d], Y[N,1]); got {x.shape}, {y.shape}")
         if self.kernel.lengthscales.size not in (1, x.shape[1]):
             raise ValueError("ARD lengthscales must have one entry per input dimension")
+        if isinstance(self.mean_function, Linear) and self.mean_function.A.shape[0] != x.shape[1]:
+            raise ValueError(f"Linear mean function: A must have shape [{x.shape[1]}, 1] for {x.shape[1]}-dimensional inputs, "
+                             f"got {list(self.mean_function.A.shape)}")
         self._data = (x, y)
         self._session.set_data(x, y)
         self._factor_key = None
@@ -290,7 +318,7 @@ class GPR(GPModel):
             pos += p.size
 
     def _theta(self):
-        """Constrained vector in packing order: [alpha], lengthscale(s), kernel variance, noise variance, [mean c]."""
+        """Constrained vector in packing order: [alpha], lengthscale(s), kernel variance, noise variance, [mean c | A, b]."""
         return np.concatenate([np.asarray(p, dtype=np.float64).reshape(-1) for p in self._ordered_parameters])
 
     # -- objective ----------------------------------------------------------------------------------------------------
@@ -429,6 +457,9 @@ def parameter_dict(model):
     })
     if isinstance(model.mean_function, Constant):
         out[".mean_function.c"] = model.mean_function.c
+    elif isinstance(model.mean_function, Linear):
+        out[".mean_function.A"] = model.mean_function.A
+        out[".mean_function.b"] = model.mean_function.b
     return out
 
 
@@ -456,7 +487,7 @@ kernels = types.SimpleNamespace(
     Kernel=Kernel, Stationary=Stationary, Matern12=Matern12, Matern32=Matern32, Matern52=Matern52,
     SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic,
 )
-mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant)
+mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant, Linear=Linear)
 likelihoods = types.SimpleNamespace(Gaussian=Gaussian)
 optimizers = types.SimpleNamespace(Scipy=Scipy)
 models = types.SimpleNamespace(GPModel=GPModel, GPR=GPR)
