@@ -139,7 +139,9 @@ int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, in
 /* kernel launches issued by this handle since creation (our own kernels only; memcpy/memset not counted) */
 int64_t gpso_launch_count(gpso_handle* h);
 /* copy device-side intermediates to the host for parity tests: which = 1 L (N*N, lower), 2 L^-1 (N*N, lower),
- * 3 alpha (N), 4 K_y^-1 (N*N, lower; valid after gpso_neg_lml_grad) */
+ * 3 alpha (N), 4 K_y^-1 (N*N, lower; valid after gpso_neg_lml_grad), 5 the screened value (UCB, or the mean for the
+ * mean-bound level) of the first `count` candidates of the last fused arg-max call: GPSO_E_STATE when that call's last
+ * screening level did not write all of them (an unscreened call, or the early stop after its first windows) */
 int gpso_debug_fetch(gpso_handle* h, int which, double* out_host, int64_t count);
 /* elapsed device time in ms of the last gpso_ucb_argmax_* / gpso_predict_y_* / gpso_neg_lml_grad call (CUDA events on
  * the launching stream): out[0]=total; with gpso_set_profile(h,1) also the per-stage sums over all windows:

@@ -264,6 +264,7 @@ struct gpso_handle {
     int screen_S_cur = 0;       // rung of SCREEN_LADDER the automatic mode starts from
     int screen_built_S = 0;     // digits of the tiles in ozAs (0: stale)
     bool screen_ready = false;  // fp32 copies and norms valid for the factor in force
+    long long scr_rows = 0;     // scr_ucb[0, scr_rows) holds the values the last screening level of the last fused call wrote
     double alpha_l2 = 0.0, rho_max = 0.0, rho_l2sq = 0.0;
     double linv_frob2 = 0.0, linv_rowl2_max = 0.0;  // |L^-1|_F^2 (= tr K_y^-1) and the largest row norm of L^-1
     // last call: [0] path (0 unscreened, 1 screened, 2 fallback: too many survivors, 3 fallback: check failed), [1] digits,
@@ -2239,8 +2240,10 @@ static int screen_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, co
         return 0;
     };
     long long done = 0;
+    h->scr_rows = 0;
     GP_TRY(window_pipeline(h, st, Xc_dev, Xc_host, W, wins, overlap, body, &done));
     h->scr_info[6] = (double)done;
+    for (long long w = 0; w < done; w++) h->scr_rows += wins[(size_t)w].n;  // after the early stop: the windows that ran
     return set_l2_window(h, h->ozA.p, (size_t)h->Np * h->Np * h->oz_S);  // back on the full-precision tiles (refine pass)
 }
 
@@ -2273,8 +2276,10 @@ static int bound_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, con
         return check_launch(h, "bound_finalize");
     };
     long long done = 0;
+    h->scr_rows = 0;
     GP_TRY(window_pipeline(h, st, Xc_dev, Xc_host, W, uniform_windows(M, W), false, body, &done));
     h->scr_info[6] = (double)done;
+    h->scr_rows = std::min(M, done * W);
     return 0;
 }
 
@@ -2343,6 +2348,7 @@ static int score_argmax(gpso_handle* h, cudaStream_t st, const double* Xc_dev, c
                         double* result_host) {
     for (int i = 0; i < 12; i++) h->scr_info[i] = 0.0;
     h->scr_prod_marks = 0;
+    h->scr_rows = 0;
     // the screen keeps one double per candidate: when that does not fit beside the caller's data the call runs unscreened
     const bool room = screen_applicable(h, M) && h->scr_ucb.ensure((size_t)M * sizeof(double)) == 0;
     if (room) {
@@ -2906,7 +2912,10 @@ extern "C" int gpso_debug_fetch(gpso_handle* h, int which, double* out_host, int
     CU_TRY(cudaStreamSynchronize(h->stream));
     const int N = h->N, Np = h->Np;
     if (which == 5) {  // screened value (UCB, or mean for the bound level) of the first `count` candidates of the last screened call
-        if (!h->scr_ucb.p || (size_t)count * sizeof(double) > h->scr_ucb.cap) return fail(GPSO_E_BADARG, "gpso_debug_fetch: no screened values");
+        // scr_ucb outlives the call that wrote it: refuse rows the last fused call did not screen (unscreened call, early stop)
+        if (count < 0 || count > h->scr_rows)
+            return fail(GPSO_E_STATE, "gpso_debug_fetch: the last fused call screened " + std::to_string(h->scr_rows) + " candidates, not " +
+                                          std::to_string(count));
         CU_TRY(cudaMemcpy(out_host, h->scr_ucb.p, sizeof(double) * (size_t)count, cudaMemcpyDeviceToHost));
         return 0;
     }
