@@ -73,10 +73,7 @@ constexpr int OZ_INV_S = 8;                    // digits per operand of the int8
 // run on the SMs the chain-bound factorisation leaves idle); the int8 engine takes the levels above.  Measured per LML+grad
 // evaluation: N = 300 0.40 -> 0.31 ms, 600 0.54 -> 0.47, 1024 0.73 -> 0.68 (cap 8 = everything in the kernel up to 1024 rows);
 // at 4096 rows the FP64 merges start to get in the chain's way (cap 4 / 8 / 16: 3.23 / 3.26 / 3.41 ms).
-static inline int oz_inv_dmma_cap(int n_tiles) {
-    static const int cap_env = getenv("GPSO_INV_DMMA_CAP") ? atoi(getenv("GPSO_INV_DMMA_CAP")) : 0;  // tuning experiments only
-    return cap_env > 0 ? cap_env : (n_tiles >= 24 ? 4 : 8);
-}
+static inline int oz_inv_dmma_cap(int n_tiles) { return n_tiles >= 24 ? 4 : 8; }
 constexpr int OZ_HYB_S = 7;                    // digits per operand of the hybrid factorisation's panel and Schur products: 54-bit fixed point per
                                                // row, the rounding of an fp64 product of the same operands (the K_y^-1 product uses the same)
 constexpr int OZ_INV_MIN_NP = 512;             // automatic mode; measured down to N = 512 (0.498 -> 0.474 ms there, 2.05 -> 1.75 ms at 2048)
@@ -125,8 +122,7 @@ struct DevPool {
         return p;
     }
     bool give(int dev, void* p, size_t bytes) {
-        static const bool enabled = !(getenv("GPSO_POOL") && atoi(getenv("GPSO_POOL")) == 0);  // A/B measurements only
-        if (!enabled || dev < 0 || dev >= POOL_MAX_DEV) return false;
+        if (dev < 0 || dev >= POOL_MAX_DEV) return false;
         std::lock_guard<std::mutex> lock(mu);
         if (cached[dev] + bytes > POOL_MAX_CACHED) return false;
         blocks[dev].emplace(bytes, p);
@@ -216,10 +212,7 @@ struct gpso_handle {
     DevBuf meanA;  // GPSO_MEAN_LINEAR: A (d doubles)
     DevBuf K, Linv, LinvT, T, Kinv;
     DevBuf resid, a, logdet, scalars, gpart, gout, info, counter;
-    // persistent Cholesky scheduler: task queue (rebuilt when nb changes) and its state [next, err, cnt[nb*nb]]
-    DevBuf chol_tasks, chol_state;
-    int chol_tasks_nb = 0, chol_ntasks = 0, chol_ncounters = 0, chol_W = 4;
-    int chol_mode = 1;      // 1 = persistent dataflow kernel, 0 = one launch per step (reference schedule)
+    DevBuf chol_state;      // state [next, err, counters] of the fit's persistent factorisation kernel (task lists: factor_plans)
     // predict workspaces
     DevBuf KsT, part, blockbest, running, cand[2], leaves, omean, ovar, topk;
     // joint posterior (kern_joint.cuh): scaled candidates, cross-covariance, mean, V^T, Sigma; for the samples the factor's
@@ -238,15 +231,17 @@ struct gpso_handle {
     DevBuf ozL, ozLT, ozLI, ozXT, rsL, rsLT, rsLI, rsXT;
     struct InvLevel { int s; size_t xt_off; int xt_rounds; size_t y_off; int y_rounds; };
     int inverse_mode = 0;   // 0 = automatic (int8 from OZ_INV_MIN_NP), 1 = FP64 DMMA tile tasks, 2 = int8 tcgen05
-    int chol_tasks_cap = -1;     // levels s < cap of the inverse recursion are in the cached task list
-    // hybrid factorisation (hybrid_node): task lists / item tables per sub-matrix size, built on first use
+    // persistent and hybrid factorisation (hybrid_node): task lists / item tables per sub-matrix size, built on first use
     struct FactorPlan { DevBuf tasks; int ntasks = 0, ncounters = 0; };
     struct InvPlan { DevBuf items; std::vector<InvLevel> levels; };
     struct ItemList { DevBuf items; int rounds = 0; };
     std::map<int, FactorPlan> factor_plans;    // key 2048 n + levels of the inverse done by the kernel (cap)
     std::map<int, InvPlan> inv_plans;          // key n
     std::map<long long, ItemList> hyb_items;   // key (kind, split, n)
-    int hybrid_mode = 0;    // 0 = automatic (matrices of more than HYB_MIN_TILES tiles), 1 = off, 2 = always (leaves of 2 tiles: tests)
+    // gpso_set_factor_mode: 0 = one launch per step (reference schedule), 1 = persistent kernel, hybrid above HYB_LEAF_TILES
+    // tiles (automatic), 2 = one persistent kernel for the whole matrix, 3 = hybrid with leaves of 2 tiles (tests); the hybrid
+    // needs the int8 inverse engine in force, without it modes 1 and 3 are mode 2
+    int factor_mode = 1;
     int hybrid_nodes = 0;   // inner nodes of the last factorisation (0 = one persistent kernel)
     cudaStream_t aux_stream = nullptr;
     cudaEvent_t ev_probe = nullptr;  // early verdict of a screening rung (screen_pass)
@@ -319,6 +314,18 @@ static int check_launch(gpso_handle* h, const char* what) {
         return fail(GPSO_E_CUDA, b);
     }
     h->launches++;
+    return 0;
+}
+
+// Pivot status of a factorisation (LAPACK info: the 1-based row of the first non-positive pivot, < 0 when the tile scheduler
+// gave up waiting) -> return code and message; `what` names the factorised matrix.
+static int pivot_status(int info, const char* what) {
+    if (info < 0) return fail(GPSO_E_CUDA, "Cholesky tile scheduler timed out waiting for a dependency");
+    if (info > 0) {
+        char b[128];
+        snprintf(b, sizeof b, "%s is not positive definite (pivot %d)", what, info);
+        return fail(info, b);
+    }
     return 0;
 }
 
@@ -626,12 +633,11 @@ struct FactorTask {
 }  // namespace
 
 static int make_factor_tasks(int nb, int nsm, std::vector<int>& flat, int& ntasks, int& ncounters_out, int inv_cap = 1 << 30) {
-    // panels per block of the two-level blocking; GPSO_CHOL_W overrides it for scheduling experiments (tools/factor_sim.py)
-    static const int w_env = getenv("GPSO_CHOL_W") ? atoi(getenv("GPSO_CHOL_W")) : 0;
-    // up to 47 panels (the leaves of the hybrid factorisation, every matrix up to N = 4096) the factorisation is bound by its
-    // chains of dependent tile tasks, not by the DMMA pipe: unblocked updates (W = 1) keep the off-diagonal chain PANEL -> UPDATE
-    // -> PANEL at 56 us per step (W = 2: 63 us); measured 3.28 vs 3.40 ms per LML+grad evaluation at N = 4096, 1.38 vs 1.52 at 2048
-    const int W = w_env > 0 ? w_env : (nb >= 48 ? 4 : 1);
+    // panels per block of the two-level blocking.  Up to 47 panels (the leaves of the hybrid factorisation, every matrix up to
+    // N = 4096) the factorisation is bound by its chains of dependent tile tasks, not by the DMMA pipe: unblocked updates (W = 1)
+    // keep the off-diagonal chain PANEL -> UPDATE -> PANEL at 56 us per step (W = 2: 63 us); measured 3.28 vs 3.40 ms per LML+grad
+    // evaluation at N = 4096, 1.38 vs 1.52 at 2048
+    const int W = nb >= 48 ? 4 : 1;
     if (nb < 1 || nb > 255) return fail(GPSO_E_BADARG, "matrix too large for the tile scheduler (more than 255 panels)");
     const int LV = 8;  // levels of the inverse recursion: s = 1 .. 128
     auto T = [nb](int i, int j) { return i * nb + j; };          // tile counters
@@ -645,9 +651,8 @@ static int make_factor_tasks(int nb, int nsm, std::vector<int>& flat, int& ntask
     auto ops = [W](int j) { return chol_ops(j, W); };
     auto fin = [W](int j) { return chol_ops(j, W) + 1; };
     // "tile (i, j) is final": its own counter, or for the strip-solved tile below the diagonal the strip counter
-    static const bool split = !(getenv("GPSO_PANEL_STRIPS") && atoi(getenv("GPSO_PANEL_STRIPS")) == 0);  // A/B only
-    auto FINC = [&](int i, int j) { return (split && i == j + 1) ? STRIP(j) : T(i, j); };
-    auto FINV = [&](int i, int j) { return (split && i == j + 1) ? PANEL_STRIPS : fin(j); };
+    auto FINC = [&](int i, int j) { return i == j + 1 ? STRIP(j) : T(i, j); };
+    auto FINV = [&](int i, int j) { return i == j + 1 ? PANEL_STRIPS : fin(j); };
 
     const double t_wide_us = 17.0 * W + 12.0;  // tile time of a wide update (DMMA at peak + tile write-back)
     const double pops_per_us = nsm / t_wide_us;
@@ -719,8 +724,8 @@ static int make_factor_tasks(int nb, int nsm, std::vector<int>& flat, int& ntask
             // the first diagonal tile of a block still lacks the wide update of the previous block: all but the last panel of
             // it were applied by an ordinary task while the chain was busy with that panel (PRE, queued below), so that every
             // DIAG fuses exactly one panel (10 us on the chain instead of 10 W)
-            const bool pre_done = split && W >= 2 && p > 0 && p % W == 0;
-            const int nprev = p == 0 ? 0 : ((p % W != 0 || pre_done) ? 1 : W);
+            const bool pre_done = W >= 2 && p > 0 && p % W == 0;
+            const int nprev = p > 0 ? 1 : 0;
             FactorTask dg(CT_DIAG, p, p, p, nprev, 0);
             if (p > 0) dg.dep(T(p, p), ops(p) - 1).dep(FINC(p, p - 1), FINV(p, p - 1));
             if (pre_done) dg.dep(PRE(p), 1);
@@ -740,16 +745,13 @@ static int make_factor_tasks(int nb, int nsm, std::vector<int>& flat, int& ntask
             auto panel_task = [&](int i) {
                 return FactorTask(CT_PANEL, p, i, p, 0, 0).dep(T(p, p), fin(p)).dep(T(i, p), ops(p)).done(T(i, p), fin(p));
             };
-            int first_late = p + 1;
-            if (split && p + 1 < nb) {
+            if (p + 1 < nb)
                 for (int k = 0; k < PANEL_STRIPS; k++)
                     q.push_back(FactorTask(CT_PANEL, p, p + 1, p, k + 1, 0).dep(T(p, p), fin(p)).dep(T(p + 1, p), ops(p)).done(STRIP(p), 0));
-                if (p + 2 < nb) q.push_back(panel_task(p + 2));
-                first_late = p + 3;
-            }
+            if (p + 2 < nb) q.push_back(panel_task(p + 2));
             cover((p > p0 ? 42.0 : 30.0 + 10.0 * nprev) - narrow * 30.0 / nsm);
-            for (int i = first_late; i < nb; i++) q.push_back(panel_task(i));
-            if (split && W >= 2 && p == p1 - 2 && p1 - p0 == W && p1 < nb)
+            for (int i = p + 3; i < nb; i++) q.push_back(panel_task(i));
+            if (W >= 2 && p == p1 - 2 && p1 - p0 == W && p1 < nb)
                 q.push_back(FactorTask(CT_UPD, p0, p1, p1, W - 1, 0).dep(T(p1, p), fin(p)).dep(T(p1, p1), b).done(PRE(p1), 1));
             {
                 FactorTask tr(CT_TRANSPOSE, p, p, p, 0, 0);
@@ -791,19 +793,32 @@ static int get_factor_plan(gpso_handle* h, int n, int inv_cap, gpso_handle::Fact
     return 0;
 }
 
-static int build_factor_tasks(gpso_handle* h, int inv_cap) {
-    if (h->chol_tasks_nb == h->nb && h->chol_tasks_cap == inv_cap) return 0;
-    std::vector<int> flat;
-    int ntasks = 0, ncounters = 0;
-    GP_TRY(make_factor_tasks(h->nb, h->nsm > 0 ? h->nsm : 148, flat, ntasks, ncounters, inv_cap));
-    h->chol_tasks_cap = inv_cap;
-    GP_TRY(h->chol_tasks.ensure(flat.size() * sizeof(int)));
-    GP_TRY(h->chol_state.ensure((size_t)(2 + ncounters) * sizeof(int)));
-    CU_TRY(cudaMemcpy(h->chol_tasks.p, flat.data(), flat.size() * sizeof(int), cudaMemcpyHostToDevice));
-    h->chol_tasks_nb = h->nb;
-    h->chol_ntasks = ntasks;
-    h->chol_ncounters = ncounters;
-    return 0;
+// Operands of the dense kernels for the n-tile diagonal block that starts at tile t0 of matrices with row pitch Np (T may be
+// null: only the FP64 inverse recursion uses it).
+static DenseParams dense_block(double* K, double* Linv, double* LinvT, double* T, int Np, int t0, int n) {
+    const size_t off = (size_t)t0 * TB * Np + (size_t)t0 * TB;
+    DenseParams P{};
+    P.K = K + off;
+    P.Linv = Linv + off;
+    P.LinvT = LinvT + off;
+    P.T = T ? T + off : nullptr;
+    P.Np = Np;
+    P.nb = n;
+    P.pivot_off = t0 * TB;
+    return P;
+}
+
+// One launch of the persistent factorisation kernel over the task list of `plan` (rows >= N of the block are padding);
+// `state` is its scheduler state, cleared here.
+static int launch_factor(gpso_handle* h, cudaStream_t st, const DenseParams& P, int N, const gpso_handle::FactorPlan* plan,
+                         DevBuf& state, double* logdet, int* info) {
+    const size_t bytes = (size_t)(2 + plan->ncounters) * sizeof(int);
+    GP_TRY(state.ensure(bytes));
+    CU_TRY(cudaMemsetAsync(state.p, 0, bytes, st));
+    const int grid = std::min(plan->ntasks, h->nsm > 0 ? h->nsm : 148);
+    factor_persistent_kernel<<<grid, GTHREADS, DIAG_SMEM_BYTES, st>>>(P, N, plan->tasks.as<int>(), plan->ntasks, state.as<int>(), logdet,
+                                                                       info);
+    return check_launch(h, "factor_persistent");
 }
 
 // Host-only introspection (no GPU needed): the task list for a matrix of nb panels on nsm SMs, TASK_WORDS ints per task.
@@ -823,29 +838,41 @@ extern "C" int gpso_debug_factor_tasks_cap(int nb, int nsm, int inv_cap, int* ou
     return 0;
 }
 
-// K_y^-1 = L^-T L^-1 on the int8 tensor cores (kern_ozaki.cuh, OZ_LAUUM).  The tiles (row block I, 64-wide column tile
-// ct <= 2I+1) cost nks - 4I k-steps each (the contraction runs over k >= i only); they are dealt to the nsm persistent CTAs
-// longest-first, each to the CTA with the least work so far, and stored as a [rounds][nsm] table the kernel walks by rounds.
-static void make_lauum_items(int nb, int G, std::vector<int>& flat, int& rounds_out) {
-    const int nks = nb * 4;
+// Deal tiles (row block, 64-row tile of B, first k-step, k-steps) to G persistent CTAs, longest first, each to the CTA with the
+// least work so far; appended to `all` as a [rounds][G][4] table (-1 = none).
+static void deal_items(std::vector<std::array<int, 4>>& items, int G, std::vector<int>& all, size_t& off, int& rounds) {
+    std::stable_sort(items.begin(), items.end(), [](const std::array<int, 4>& a, const std::array<int, 4>& b) { return a[3] > b[3]; });
     std::vector<std::vector<int>> per(G);
     std::vector<long long> load(G, 0);
-    for (int I = 0; I < nb; I++) {  // I ascending = cost descending
-        const long long cost = (nks - 4 * I) + 6;
-        for (int ct = 0; ct <= 2 * I + 1; ct++) {
-            int best = 0;
-            for (int g = 1; g < G; g++)
-                if (load[g] < load[best]) best = g;
-            per[best].push_back((I << 16) | ct);
-            load[best] += cost;
-        }
+    for (size_t i = 0; i < items.size(); i++) {
+        int best = 0;
+        for (int g = 1; g < G; g++)
+            if (load[g] < load[best]) best = g;
+        per[best].push_back((int)i);
+        load[best] += items[i][3] + 6;
     }
-    size_t rounds = 0;
-    for (int g = 0; g < G; g++) rounds = std::max(rounds, per[g].size());
-    flat.assign(rounds * G, -1);
+    size_t r = 0;
+    for (int g = 0; g < G; g++) r = std::max(r, per[g].size());
+    off = all.size();
+    rounds = (int)r;
+    all.resize(off + r * G * 4, -1);
     for (int g = 0; g < G; g++)
-        for (size_t r = 0; r < per[g].size(); r++) flat[r * G + g] = per[g][r];
-    rounds_out = (int)rounds;
+        for (size_t k = 0; k < per[g].size(); k++)
+            for (int c = 0; c < 4; c++) all[off + (k * G + g) * 4 + c] = items[per[g][k]][c];
+}
+
+// K_y^-1 = L^-T L^-1 on the int8 tensor cores (kern_ozaki.cuh, OZ_LAUUM).  The tiles (row block I, 64-wide column tile
+// ct <= 2I+1) cost nks - 4I k-steps each (the contraction runs over k >= i only); they are dealt as above and stored as a
+// [rounds][nsm] table of I << 16 | ct (-1 = none) the kernel walks by rounds.
+static void make_lauum_items(int nb, int G, std::vector<int>& flat, int& rounds) {
+    std::vector<std::array<int, 4>> items;
+    for (int I = 0; I < nb; I++)
+        for (int ct = 0; ct <= 2 * I + 1; ct++) items.push_back({I, ct, 0, 4 * (nb - I)});
+    std::vector<int> all;
+    size_t off = 0;
+    deal_items(items, G, all, off, rounds);
+    flat.resize(all.size() / 4);
+    for (size_t k = 0; k < flat.size(); k++) flat[k] = all[4 * k] < 0 ? -1 : (all[4 * k] << 16 | all[4 * k + 1]);
 }
 
 static int build_lauum_items(gpso_handle* h) {
@@ -900,29 +927,6 @@ static int kinv_int8(gpso_handle* h, cudaStream_t st) {
 namespace {
 struct InvLevelInfo { int s; size_t xt_off; int xt_rounds; size_t y_off; int y_rounds; };
 }
-// Deal tiles (row block, 64-row tile of B, first k-step, k-steps) to G persistent CTAs, longest first, each to the CTA with the
-// least work so far; appended to `all` as a [rounds][G][4] table (-1 = none).
-static void deal_items(std::vector<std::array<int, 4>>& items, int G, std::vector<int>& all, size_t& off, int& rounds) {
-    std::stable_sort(items.begin(), items.end(), [](const std::array<int, 4>& a, const std::array<int, 4>& b) { return a[3] > b[3]; });
-    std::vector<std::vector<int>> per(G);
-    std::vector<long long> load(G, 0);
-    for (size_t i = 0; i < items.size(); i++) {
-        int best = 0;
-        for (int g = 1; g < G; g++)
-            if (load[g] < load[best]) best = g;
-        per[best].push_back((int)i);
-        load[best] += items[i][3] + 6;
-    }
-    size_t r = 0;
-    for (int g = 0; g < G; g++) r = std::max(r, per[g].size());
-    off = all.size();
-    rounds = (int)r;
-    all.resize(off + r * G * 4, -1);
-    for (int g = 0; g < G; g++)
-        for (size_t k = 0; k < per[g].size(); k++)
-            for (int c = 0; c < 4; c++) all[off + (k * G + g) * 4 + c] = items[per[g][k]][c];
-}
-
 static void make_inverse_items(int nb, int G, std::vector<int>& all, std::vector<InvLevelInfo>& levels) {
     all.clear();
     levels.clear();
@@ -974,10 +978,12 @@ static int ensure_inverse_buffers(gpso_handle* h) {
     return 0;
 }
 
+// S digits per operand of the products below: OZ_INV_S for the inverse factor, OZ_HYB_S for the panel solve and Schur
+// complement of the hybrid factorisation.
 // Digits of the rows of the n-tile sub-matrix whose first element is M (row pitch Np), over the k-range `kind` selects.
 template <int S>
-static int oz_range_digits_t(gpso_handle* h, cudaStream_t st, const double* M, int n, int kind, int s, DevBuf& scales, DevBuf& out,
-                             const char* what) {
+static int oz_range_digits(gpso_handle* h, cudaStream_t st, const double* M, int n, int kind, int s, DevBuf& scales, DevBuf& out,
+                           const char* what) {
     const int Np = h->Np, nks = Np / 32;
     range_rowscale_kernel<<<n * 16, 256, 0, st>>>(M, Np, kind, s, n, scales.as<double>());
     GP_TRY(check_launch(h, what));
@@ -987,9 +993,9 @@ static int oz_range_digits_t(gpso_handle* h, cudaStream_t st, const double* M, i
 
 // out[i][j] (+)= sign * sum_k A[i][k] B[j][k] over the tiles and k-ranges of an item table, on the int8 tensor cores
 template <int S>
-static int oz_range_product_t(gpso_handle* h, cudaStream_t st, const DevBuf& A, const DevBuf& rsA, const DevBuf& B, const DevBuf& rsB,
-                              const int* items, int rounds, int n, double* out, double* out_t, double sign, bool accumulate,
-                              const char* what) {
+static int oz_range_product(gpso_handle* h, cudaStream_t st, const DevBuf& A, const DevBuf& rsA, const DevBuf& B, const DevBuf& rsB,
+                            const int* items, int rounds, int n, double* out, double* out_t, double sign, bool accumulate,
+                            const char* what) {
     OzParams P;
     P.A = A.as<uint8_t>();
     P.B = B.as<uint8_t>();
@@ -1012,19 +1018,6 @@ static int oz_range_product_t(gpso_handle* h, cudaStream_t st, const DevBuf& A, 
     return check_launch(h, what);
 }
 
-// digits = OZ_INV_S (8: inverse-factor products) or OZ_HYB_S (7: panel solve and Schur complement of the hybrid factorisation)
-static int oz_range_digits(gpso_handle* h, cudaStream_t st, const double* M, int n, int kind, int s, DevBuf& scales, DevBuf& out,
-                           const char* what, int digits = OZ_INV_S) {
-    return digits == 7 ? oz_range_digits_t<7>(h, st, M, n, kind, s, scales, out, what)
-                       : oz_range_digits_t<OZ_INV_S>(h, st, M, n, kind, s, scales, out, what);
-}
-static int oz_range_product(gpso_handle* h, cudaStream_t st, const DevBuf& A, const DevBuf& rsA, const DevBuf& B, const DevBuf& rsB,
-                            const int* items, int rounds, int n, double* out, double* out_t, double sign, bool accumulate,
-                            const char* what, int digits = OZ_INV_S) {
-    return digits == 7 ? oz_range_product_t<7>(h, st, A, rsA, B, rsB, items, rounds, n, out, out_t, sign, accumulate, what)
-                       : oz_range_product_t<OZ_INV_S>(h, st, A, rsA, B, rsB, items, rounds, n, out, out_t, sign, accumulate, what);
-}
-
 // Levels s_lo <= s < s_hi of the recursive-doubling inverse of the n-tile diagonal block that starts at tile t0 (the whole
 // matrix: t0 = 0, n = nb, all levels).  A single level (the merge of a hybrid node) only needs the L21 rows of the factor.
 static int inverse_int8(gpso_handle* h, cudaStream_t st, int t0, int n, int s_lo, int s_hi) {
@@ -1038,16 +1031,16 @@ static int inverse_int8(gpso_handle* h, cudaStream_t st, int t0, int n, int s_lo
     double* LinvT = h->LinvT.as<double>() + off;
     double* T = h->T.as<double>() + off;
     const bool single = s_hi <= 2 * s_lo;
-    GP_TRY(oz_range_digits(h, st, L, n, single ? OZR_PANEL : OZR_L, single ? s_lo : 1, h->rsL, h->ozL, "digits_L"));
+    GP_TRY(oz_range_digits<OZ_INV_S>(h, st, L, n, single ? OZR_PANEL : OZR_L, single ? s_lo : 1, h->rsL, h->ozL, "digits_L"));
     for (const gpso_handle::InvLevel& lv : plan->levels) {
         if (lv.xt_rounds == 0 || lv.s < s_lo || lv.s >= s_hi) continue;
-        GP_TRY(oz_range_digits(h, st, LinvT, n, OZR_LINVT, lv.s, h->rsLT, h->ozLT, "digits_LinvT"));
-        GP_TRY(oz_range_product(h, st, h->ozLT, h->rsLT, h->ozL, h->rsL, plan->items.as<int>() + lv.xt_off, lv.xt_rounds, n, T, nullptr,
-                                1.0, false, "inverse_xt"));
-        GP_TRY(oz_range_digits(h, st, T, n, OZR_XT, lv.s, h->rsXT, h->ozXT, "digits_XT"));
-        GP_TRY(oz_range_digits(h, st, Linv, n, OZR_LINV, lv.s, h->rsLI, h->ozLI, "digits_Linv"));
-        GP_TRY(oz_range_product(h, st, h->ozLI, h->rsLI, h->ozXT, h->rsXT, plan->items.as<int>() + lv.y_off, lv.y_rounds, n, Linv, LinvT,
-                                -1.0, false, "inverse_y"));
+        GP_TRY(oz_range_digits<OZ_INV_S>(h, st, LinvT, n, OZR_LINVT, lv.s, h->rsLT, h->ozLT, "digits_LinvT"));
+        GP_TRY(oz_range_product<OZ_INV_S>(h, st, h->ozLT, h->rsLT, h->ozL, h->rsL, plan->items.as<int>() + lv.xt_off, lv.xt_rounds, n, T,
+                                          nullptr, 1.0, false, "inverse_xt"));
+        GP_TRY(oz_range_digits<OZ_INV_S>(h, st, T, n, OZR_XT, lv.s, h->rsXT, h->ozXT, "digits_XT"));
+        GP_TRY(oz_range_digits<OZ_INV_S>(h, st, Linv, n, OZR_LINV, lv.s, h->rsLI, h->ozLI, "digits_Linv"));
+        GP_TRY(oz_range_product<OZ_INV_S>(h, st, h->ozLI, h->rsLI, h->ozXT, h->rsXT, plan->items.as<int>() + lv.y_off, lv.y_rounds, n, Linv,
+                                          LinvT, -1.0, false, "inverse_y"));
     }
     return 0;
 }
@@ -1057,17 +1050,16 @@ static int inverse_int8(gpso_handle* h, cudaStream_t st, int t0, int n, int s_lo
 // the FP64 DMMA pipe above (0.55 of its peak at N = 8192).  The exact-integer products that already build L^-1 run at ~2.5x
 // the FP64 peak in fp64-equivalent work, so a node of n tiles is split after s = the largest power of two below n:
 //      [A11      ]      L11, L11^-1            the node's first half, recursively
-//      [A21  A22 ]      L21 = A21 L11^-T       one int8 product (8 digits per operand, 62-bit fixed point per row)
+//      [A21  A22 ]      L21 = A21 L11^-T       one int8 product (OZ_HYB_S = 7 digits per operand, 54-bit fixed point per row)
 //                       A22 -= L21 L21^T       one int8 product, accumulated into the lower tiles of A22
 //                       L22, L22^-1            the second half, recursively
 //                       L21^-1 = -L22^-1 L21 L11^-1     the level-s merge of the recursive-doubling inverse (work the whole-matrix
 //                                                      inverse did anyway)
 // Leaves (<= HYB_LEAF_TILES tiles) are factorised by the persistent FP64 kernel on the sub-matrix in place; that kernel is
 // bound by its chain of 128-tile steps (~70 us each), so smaller leaves do not shorten it, they only add product launches.
+// Without the hybrid the whole matrix is one leaf.
 constexpr int HYB_LEAF_TILES = 32;  // 4096 rows: measured 11.8 ms per LML+grad evaluation at N = 8192 against 13.5 with leaves of 2048 and 14.1
                                     // with one kernel; at N = 4096 one kernel (3.43 ms) beats two leaves of 2048 (3.89 ms)
-
-static int get_factor_plan(gpso_handle* h, int n, int inv_cap, gpso_handle::FactorPlan** out);
 
 // Tile table of one hybrid product for a node of n tiles split after s.  kind 0: L21 tile (I, J), I >= s > J, contraction over
 // the tiles [0, J] of row block J of L11^-1;  kind 1: Schur tile (I, J), s <= J <= I, contraction over the s tiles of L21.
@@ -1140,48 +1132,32 @@ extern "C" int64_t gpso_debug_hybrid_items(int kind, int s, int n, int nsm, int*
     return (int64_t)all.size();
 }
 
-static int hybrid_leaf(gpso_handle* h, cudaStream_t st, int t0, int n) {
+// Cholesky factor and inverse of the n-tile diagonal block at tile t0, in place, by the persistent FP64 kernel.  inv8: the int8
+// engine is in force for the inverse factor; it then takes the levels from oz_inv_dmma_cap up, the kernel the levels below.
+static int hybrid_leaf(gpso_handle* h, cudaStream_t st, int t0, int n, bool inv8) {
     const int Np = h->Np;
-    const size_t off = (size_t)t0 * 128 * Np + (size_t)t0 * 128;
-    DenseParams P;
-    P.K = h->K.as<double>() + off;
-    P.Linv = h->Linv.as<double>() + off;
-    P.LinvT = h->LinvT.as<double>() + off;
-    P.T = h->T.as<double>() + off;
-    P.Kinv = nullptr;
-    P.Np = Np;
-    P.nb = n;
-    P.p = 0;
-    P.s = 0;
-    P.pivot_off = t0 * 128;
-    const int Nsub = h->N - t0 * 128;
+    if (n > 1) GP_TRY(h->T.ensure((size_t)Np * Np * sizeof(double), true));
+    const DenseParams P = dense_block(h->K.as<double>(), h->Linv.as<double>(), h->LinvT.as<double>(), h->T.as<double>(), Np, t0, n);
+    const int Nsub = h->N - t0 * TB;
+    double* logdet = h->logdet.as<double>() + t0;
     if (n == 1) {
-        diag_factor_inverse_kernel<<<1, DIAG_THREADS, DIAG_SMEM_BYTES, st>>>(P.K, P.Linv, Np, 0, Nsub, h->logdet.as<double>() + t0,
-                                                                             h->info.as<int>(), P.pivot_off);
+        diag_factor_inverse_kernel<<<1, DIAG_THREADS, DIAG_SMEM_BYTES, st>>>(P.K, P.Linv, Np, 0, Nsub, logdet, h->info.as<int>(), P.pivot_off);
         GP_TRY(check_launch(h, "diag_factor_inverse"));
         diag_transpose_kernel<<<1, 256, DIAG_TRANSPOSE_SMEM, st>>>(P.Linv, P.LinvT, Np);
         return check_launch(h, "diag_transpose");
     }
-    const int inv_cap = oz_inv_dmma_cap(n);
-    const bool inv8 = n * 128 >= OZ_INV_MIN_NP && inv_cap < n;
+    const int cap = inv8 ? oz_inv_dmma_cap(n) : (1 << 30);
     gpso_handle::FactorPlan* plan = nullptr;
-    GP_TRY(get_factor_plan(h, n, inv8 ? inv_cap : (1 << 30), &plan));
-    GP_TRY(h->chol_state.ensure((size_t)(2 + plan->ncounters) * sizeof(int)));
-    int* state = h->chol_state.as<int>();
-    CU_TRY(cudaMemsetAsync(state, 0, (size_t)(2 + plan->ncounters) * sizeof(int), st));
-    const int grid = std::min(plan->ntasks, h->nsm > 0 ? h->nsm : 148);
-    factor_persistent_kernel<<<grid, GTHREADS, DIAG_SMEM_BYTES, st>>>(P, Nsub, plan->tasks.as<int>(), plan->ntasks, state,
-                                                                       h->logdet.as<double>() + t0, h->info.as<int>());
-    GP_TRY(check_launch(h, "factor_persistent"));
-    if (inv8) GP_TRY(inverse_int8(h, st, t0, n, inv_cap, n));
+    GP_TRY(get_factor_plan(h, n, cap, &plan));
+    GP_TRY(launch_factor(h, st, P, Nsub, plan, h->chol_state, logdet, h->info.as<int>()));
+    if (cap < n) GP_TRY(inverse_int8(h, st, t0, n, cap, n));
     return 0;
 }
 
-static int hybrid_node(gpso_handle* h, cudaStream_t st, int t0_root, int n_root, int leaf) {
+static int hybrid_node(gpso_handle* h, cudaStream_t st, int t0_root, int n_root, int leaf, bool inv8) {
     std::vector<std::array<int, 4>> ops;
     plan_hybrid(t0_root, n_root, leaf, ops);
     const int Np = h->Np;
-    static const int hyb_s = (getenv("GPSO_HYB_S") && atoi(getenv("GPSO_HYB_S")) == 8) ? 8 : OZ_HYB_S;  // A/B measurements only
     for (const std::array<int, 4>& op : ops) {
         const int t0 = op[1], n = op[2], s = op[3];
         const size_t off = (size_t)t0 * 128 * Np + (size_t)t0 * 128;
@@ -1189,25 +1165,65 @@ static int hybrid_node(gpso_handle* h, cudaStream_t st, int t0_root, int n_root,
         gpso_handle::ItemList* items = nullptr;
         switch (op[0]) {
             case HYB_LEAF:
-                GP_TRY(hybrid_leaf(h, st, t0, n));
+                GP_TRY(hybrid_leaf(h, st, t0, n, inv8));
                 break;
             case HYB_PANEL:  // L21 = A21 L11^-T
                 h->hybrid_nodes++;
-                GP_TRY(oz_range_digits(h, st, A, n, OZR_PANEL, s, h->rsL, h->ozL, "digits_A21", hyb_s));
-                GP_TRY(oz_range_digits(h, st, h->Linv.as<double>() + off, n, OZR_LOWER, s, h->rsLI, h->ozLI, "digits_Linv11", hyb_s));
+                GP_TRY(ensure_inverse_buffers(h));  // the products of a node use the digit buffers of the int8 inverse
+                GP_TRY(oz_range_digits<OZ_HYB_S>(h, st, A, n, OZR_PANEL, s, h->rsL, h->ozL, "digits_A21"));
+                GP_TRY(oz_range_digits<OZ_HYB_S>(h, st, h->Linv.as<double>() + off, n, OZR_LOWER, s, h->rsLI, h->ozLI, "digits_Linv11"));
                 GP_TRY(get_hybrid_items(h, 0, s, n, &items));
-                GP_TRY(oz_range_product(h, st, h->ozL, h->rsL, h->ozLI, h->rsLI, items->items.as<int>(), items->rounds, n, A, nullptr, 1.0,
-                                        false, "hybrid_panel", hyb_s));
+                GP_TRY(oz_range_product<OZ_HYB_S>(h, st, h->ozL, h->rsL, h->ozLI, h->rsLI, items->items.as<int>(), items->rounds, n, A, nullptr,
+                                                  1.0, false, "hybrid_panel"));
                 break;
             case HYB_SCHUR:  // A22 -= L21 L21^T (lower tiles)
-                GP_TRY(oz_range_digits(h, st, A, n, OZR_PANEL, s, h->rsL, h->ozL, "digits_L21", hyb_s));
+                GP_TRY(oz_range_digits<OZ_HYB_S>(h, st, A, n, OZR_PANEL, s, h->rsL, h->ozL, "digits_L21"));
                 GP_TRY(get_hybrid_items(h, 1, s, n, &items));
-                GP_TRY(oz_range_product(h, st, h->ozL, h->rsL, h->ozL, h->rsL, items->items.as<int>(), items->rounds, n, A, nullptr, -1.0,
-                                        true, "hybrid_schur", hyb_s));
+                GP_TRY(oz_range_product<OZ_HYB_S>(h, st, h->ozL, h->rsL, h->ozL, h->rsL, items->items.as<int>(), items->rounds, n, A, nullptr,
+                                                  -1.0, true, "hybrid_schur"));
                 break;
             default:         // L21^-1 = -L22^-1 L21 L11^-1: the level-s merge of the recursive-doubling inverse
                 GP_TRY(inverse_int8(h, st, t0, n, s, 2 * s));
                 break;
+        }
+    }
+    return 0;
+}
+
+// The reference schedule (gpso_set_factor_mode 0): one launch per step of the blocked Cholesky, then the inverse factor by
+// recursive doubling, level by level.
+static int factor_stepwise(gpso_handle* h, cudaStream_t st, bool inv8) {
+    const int Np = h->Np, nb = h->nb;
+    DenseParams P = dense_block(h->K.as<double>(), h->Linv.as<double>(), h->LinvT.as<double>(), nullptr, Np, 0, nb);
+    for (int p = 0; p < nb; p++) {
+        diag_factor_inverse_kernel<<<1, DIAG_THREADS, DIAG_SMEM_BYTES, st>>>(P.K, P.Linv, Np, p, h->N, h->logdet.as<double>(),
+                                                                             h->info.as<int>());
+        GP_TRY(check_launch(h, "diag_factor_inverse"));
+        int nt = nb - 1 - p;
+        if (nt > 0) {
+            P.p = p;
+            dense_gemm_kernel<MODE_CHOL_PANEL><<<nt, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
+            GP_TRY(check_launch(h, "chol_panel"));
+            dense_gemm_kernel<MODE_CHOL_TRAIL><<<nt*(nt + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
+            GP_TRY(check_launch(h, "chol_trailing"));
+        }
+    }
+    diag_transpose_kernel<<<nb, 256, DIAG_TRANSPOSE_SMEM, st>>>(P.Linv, P.LinvT, Np);
+    GP_TRY(check_launch(h, "diag_transpose"));
+    if (inv8) {
+        GP_TRY(inverse_int8(h, st, 0, nb, 1, nb));
+    } else if (nb > 1) {
+        GP_TRY(h->T.ensure((size_t)Np * Np * sizeof(double), true));
+        P.T = h->T.as<double>();
+        for (int s = 1; s < nb; s *= 2) {
+            int cnt = 0;
+            for (int q = 0; 2 * q * s < nb; q++) cnt += s * trtri_pair_vtiles(nb, s, q);
+            if (cnt == 0) continue;
+            P.s = s;
+            dense_gemm_kernel<MODE_TRTRI_XT><<<cnt, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
+            GP_TRY(check_launch(h, "trtri_xt"));
+            dense_gemm_kernel<MODE_TRTRI_Y><<<cnt, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
+            GP_TRY(check_launch(h, "trtri_y"));
         }
     }
     return 0;
@@ -1226,81 +1242,23 @@ static int factor_pipeline(gpso_handle* h, cudaStream_t st, bool need_kinv) {
     launch_gram(h, st);
     GP_TRY(check_launch(h, "gram"));
 
-    DenseParams P;
-    P.K = h->K.as<double>();
-    P.Linv = h->Linv.as<double>();
-    P.LinvT = h->LinvT.as<double>();
-    P.T = nullptr;
-    P.Kinv = nullptr;
-    P.Np = Np;
-    P.nb = nb;
-    P.p = 0;
-    P.s = 0;
-    static const int inv_min_np = getenv("GPSO_INV_MIN_NP") ? atoi(getenv("GPSO_INV_MIN_NP")) : OZ_INV_MIN_NP;     // tuning experiments only
-    static const int kinv_min_np = getenv("GPSO_KINV_MIN_NP") ? atoi(getenv("GPSO_KINV_MIN_NP")) : OZ_KINV_MIN_NP;
-    const bool inv8 = nb > 1 && Np <= OZ_MAX_NP && (h->inverse_mode == 2 || (h->inverse_mode == 0 && Np >= inv_min_np));
-    static const int hyb_leaf_env = getenv("GPSO_HYB_LEAF") ? atoi(getenv("GPSO_HYB_LEAF")) : 0;  // tuning experiments only
-    const int hyb_leaf = h->hybrid_mode == 2 ? 2 : (hyb_leaf_env > 0 ? hyb_leaf_env : HYB_LEAF_TILES);
+    const bool inv8 = nb > 1 && Np <= OZ_MAX_NP && (h->inverse_mode == 2 || (h->inverse_mode == 0 && Np >= OZ_INV_MIN_NP));
     h->hybrid_nodes = 0;
-    if (h->chol_mode == 1 && inv8 && h->hybrid_mode != 1 && nb > hyb_leaf) {
-        GP_TRY(ensure_inverse_buffers(h));
-        GP_TRY(hybrid_node(h, st, 0, nb, hyb_leaf));
-    } else if (h->chol_mode == 1 && nb > 1) {
-        // one persistent launch: blocked Cholesky + L^-1 (diagonal blocks, their transposes and -- unless the int8 engine
-        // takes it over below -- the recursive doubling)
-        const int inv_cap = inv8 ? oz_inv_dmma_cap(nb) : (1 << 30);
-        GP_TRY(build_factor_tasks(h, inv_cap));
-        GP_TRY(h->T.ensure((size_t)Np * Np * sizeof(double), true));
-        P.T = h->T.as<double>();
-        int* state = h->chol_state.as<int>();
-        CU_TRY(cudaMemsetAsync(state, 0, (size_t)(2 + h->chol_ncounters) * sizeof(int), st));
-        const int grid = std::min(h->chol_ntasks, h->nsm > 0 ? h->nsm : 148);
-        factor_persistent_kernel<<<grid, GTHREADS, DIAG_SMEM_BYTES, st>>>(P, h->N, h->chol_tasks.as<int>(), h->chol_ntasks, state,
-                                                                           h->logdet.as<double>(), h->info.as<int>());
-        GP_TRY(check_launch(h, "factor_persistent"));
-        if (inv8 && inv_cap < nb) GP_TRY(inverse_int8(h, st, 0, nb, inv_cap, nb));
+    if (h->factor_mode == 0) {
+        GP_TRY(factor_stepwise(h, st, inv8));
     } else {
-        for (int p = 0; p < nb; p++) {
-            diag_factor_inverse_kernel<<<1, DIAG_THREADS, DIAG_SMEM_BYTES, st>>>(P.K, P.Linv, Np, p, h->N, h->logdet.as<double>(),
-                                                                                 h->info.as<int>());
-            GP_TRY(check_launch(h, "diag_factor_inverse"));
-            int nt = nb - 1 - p;
-            if (nt > 0) {
-                P.p = p;
-                dense_gemm_kernel<MODE_CHOL_PANEL><<<nt, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
-                GP_TRY(check_launch(h, "chol_panel"));
-                dense_gemm_kernel<MODE_CHOL_TRAIL><<<nt*(nt + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
-                GP_TRY(check_launch(h, "chol_trailing"));
-            }
-        }
-        diag_transpose_kernel<<<nb, 256, DIAG_TRANSPOSE_SMEM, st>>>(P.Linv, P.LinvT, Np);
-        GP_TRY(check_launch(h, "diag_transpose"));
-        if (inv8) {
-            GP_TRY(inverse_int8(h, st, 0, nb, 1, nb));
-        } else if (nb > 1) {
-            GP_TRY(h->T.ensure((size_t)Np * Np * sizeof(double), true));
-            P.T = h->T.as<double>();
-            for (int s = 1; s < nb; s *= 2) {
-                int cnt = 0;
-                for (int q = 0; 2 * q * s < nb; q++) cnt += s * trtri_pair_vtiles(nb, s, q);
-                if (cnt == 0) continue;
-                P.s = s;
-                dense_gemm_kernel<MODE_TRTRI_XT><<<cnt, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
-                GP_TRY(check_launch(h, "trtri_xt"));
-                dense_gemm_kernel<MODE_TRTRI_Y><<<cnt, GTHREADS, GEMM_SMEM_BYTES, st>>>(P);
-                GP_TRY(check_launch(h, "trtri_y"));
-            }
-        }
+        const bool hybrid = inv8 && h->factor_mode != 2;
+        GP_TRY(hybrid_node(h, st, 0, nb, hybrid ? (h->factor_mode == 3 ? 2 : HYB_LEAF_TILES) : nb, inv8));
     }
+    DenseParams P = dense_block(h->K.as<double>(), h->Linv.as<double>(), h->LinvT.as<double>(), nullptr, Np, 0, nb);
     if (need_kinv) {
         GP_TRY(h->Kinv.ensure((size_t)Np * Np * sizeof(double), true));
         P.Kinv = h->Kinv.as<double>();
-        const bool int8 = Np <= OZ_MAX_NP && (h->kinv_mode == 2 || (h->kinv_mode == 0 && Np >= kinv_min_np));
+        const bool int8 = Np <= OZ_MAX_NP && (h->kinv_mode == 2 || (h->kinv_mode == 0 && Np >= OZ_KINV_MIN_NP));
         if (int8) {
             GP_TRY(kinv_int8(h, st));
         } else {
-            static const bool split = !(getenv("GPSO_LAUUM_SPLIT") && atoi(getenv("GPSO_LAUUM_SPLIT")) == 0);  // A/B only
-            if (split && nb >= 2 && nb <= 4) {
+            if (nb >= 2 && nb <= 4) {
                 // every 128-wide k-chunk of every tile on its own SM, then a fixed-order sum (kern_dense.cuh: lauum_reduce_kernel)
                 int chunks = 0;
                 for (int i = 0; i < nb; i++) chunks += (i + 1) * (nb - i);
@@ -1338,16 +1296,15 @@ static double nlml_from_scalars(const gpso_handle* h, const double* sc) {
 // L^-1, beta = scale of k*), hence  |d(sum V^2)| <~ 6 * sigma_f * beta * 2^(-8S) * sqrt(N) * max_i rho_i.  The parity
 // tolerance of the posterior variance is 1e-8 * kernel variance; S is the smallest digit count whose estimate is below
 // OZ_TARGET of it.
-static int pick_slices(const gpso_handle* h, double rho_max, double beta, double* est_out) {
+static double slices_error(const gpso_handle* h, double rho_max, double beta, int S) {  // the estimate / tolerance at S digits
     const double sigma_f = sqrt(h->variance);
     const double tol = 1.0e-8 * h->variance;
-    for (int S = 5; S <= 8; S++) {
-        double est = 6.0 * sigma_f * beta * ldexp(1.0, -8 * S) * sqrt((double)h->N) * rho_max / tol;
-        if (est <= OZ_TARGET || S == 8) {
-            *est_out = est;
-            return S;
-        }
-    }
+    return 6.0 * sigma_f * beta * ldexp(1.0, -8 * S) * sqrt((double)h->N) * rho_max / tol;
+}
+
+static int pick_slices(const gpso_handle* h, double rho_max, double beta) {
+    for (int S = 5; S < 8; S++)
+        if (slices_error(h, rho_max, beta, S) <= OZ_TARGET) return S;
     return 8;
 }
 
@@ -1397,13 +1354,8 @@ static int prepare_ozaki(gpso_handle* h, cudaStream_t st) {
     double rho_max = 0.0;
     for (int i = 0; i < h->N; i++) rho_max = std::max(rho_max, rs[i]);
     if (!(rho_max > 0.0) || !std::isfinite(rho_max)) return 0;  // degenerate factor: stay on the FP64 path
-    double est = 0.0;
-    int S = h->oz_force_slices ? h->oz_force_slices : pick_slices(h, rho_max, oz_beta(h), &est);
-    if (h->oz_force_slices) {
-        double e2 = 0.0;
-        pick_slices(h, rho_max, oz_beta(h), &e2);
-        est = 6.0 * sqrt(h->variance) * oz_beta(h) * ldexp(1.0, -8 * S) * sqrt((double)h->N) * rho_max / (1.0e-8 * h->variance);
-    }
+    const int S = h->oz_force_slices ? h->oz_force_slices : pick_slices(h, rho_max, oz_beta(h));
+    const double est = slices_error(h, rho_max, oz_beta(h), S);
     GP_TRY(h->ozA.ensure((size_t)Np * Np * S));
     DISPATCH_S(S, launch_oz_slices, h, st);
     GP_TRY(check_launch(h, "linv_slices"));
@@ -1639,13 +1591,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
     h->last_ms[0] = ms;
     h->last_ms[1] = h->last_ms[2] = h->last_ms[3] = 0;
-    if (info < 0) return fail(GPSO_E_CUDA, "Cholesky tile scheduler timed out waiting for a dependency");
-    if (info > 0) {
-        char b[128];
-        snprintf(b, sizeof b, "Gram matrix is not positive definite (pivot %d)", info);
-        fail(info, b);
-        return info;
-    }
+    GP_TRY(pivot_status(info, "Gram matrix"));
     *f_host = nlml_from_scalars(h, sc);
     // dLML/dtheta = 0.5 * sum W * dK/dtheta ; chain through softplus: dtheta/du = sigmoid(u)
     for (int i = 0; i < nl; i++) grad_host[i] = -(0.5 * g[2 + i] / h->ls_host[i]) * sigmoid(u[i]);
@@ -1675,13 +1621,7 @@ extern "C" int gpso_factorize(gpso_handle* h, const double* theta_host, int p) {
     CU_TRY(cudaMemcpyAsync(sc, h->scalars.p, sizeof sc, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(&info, h->info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
-    if (info < 0) return fail(GPSO_E_CUDA, "Cholesky tile scheduler timed out waiting for a dependency");
-    if (info > 0) {
-        char b[128];
-        snprintf(b, sizeof b, "Gram matrix is not positive definite (pivot %d)", info);
-        fail(info, b);
-        return info;
-    }
+    GP_TRY(pivot_status(info, "Gram matrix"));
     h->factor_nlml = nlml_from_scalars(h, sc);
     GP_TRY(prepare_ozaki(h, st));
     h->factorized = true;
@@ -2621,27 +2561,13 @@ static int joint_samples(gpso_handle* h, cudaStream_t st, const double* Xc, int 
     GP_TRY(h->jLinvT.ensure(mat));
     GP_TRY(h->jlogdet.ensure((size_t)mb * sizeof(double)));
     GP_TRY(h->jinfo.ensure(sizeof(int)));
-    GP_TRY(h->jstate.ensure((size_t)(2 + plan->ncounters) * sizeof(int)));
     GP_TRY(h->jZ.ensure((size_t)Sp * Mp * sizeof(double)));
     // the panel solves read whole diagonal blocks of the inverse, whose zero sub-blocks above the diagonal the diagonal task
     // never writes: cleared on every call (Mp^2 doubles, ~1 % of the factorisation's time at any size)
     CU_TRY(cudaMemsetAsync(h->jLinv.p, 0, mat, st));
-    CU_TRY(cudaMemsetAsync(h->jstate.p, 0, (size_t)(2 + plan->ncounters) * sizeof(int), st));
     CU_TRY(cudaMemsetAsync(h->jinfo.p, 0, sizeof(int), st));
-    DenseParams P;
-    P.K = h->jSigma.as<double>();
-    P.Linv = h->jLinv.as<double>();
-    P.LinvT = h->jLinvT.as<double>();
-    P.T = nullptr;
-    P.Kinv = nullptr;
-    P.Np = Mp;
-    P.nb = mb;
-    P.p = 0;
-    P.s = 0;
-    const int grid = std::min(plan->ntasks, h->nsm > 0 ? h->nsm : 148);
-    factor_persistent_kernel<<<grid, GTHREADS, DIAG_SMEM_BYTES, st>>>(P, M, plan->tasks.as<int>(), plan->ntasks, h->jstate.as<int>(),
-                                                                       h->jlogdet.as<double>(), h->jinfo.as<int>());
-    GP_TRY(check_launch(h, "factor_persistent"));
+    const DenseParams P = dense_block(h->jSigma.as<double>(), h->jLinv.as<double>(), h->jLinvT.as<double>(), nullptr, Mp, 0, mb);
+    GP_TRY(launch_factor(h, st, P, M, plan, h->jstate, h->jlogdet.as<double>(), h->jinfo.as<int>()));
     joint_tril_kernel<<<mb, 256, 0, st>>>(h->jSigma.as<double>(), Mp);
     GP_TRY(check_launch(h, "joint_tril"));
     const long long nz = (long long)Sp * Mp;
@@ -2657,14 +2583,7 @@ static int joint_pivot_status(gpso_handle* h, cudaStream_t st) {
     int info = 0;
     CU_TRY(cudaMemcpyAsync(&info, h->jinfo.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
-    if (info < 0) return fail(GPSO_E_CUDA, "Cholesky tile scheduler timed out waiting for a dependency");
-    if (info > 0) {
-        char b[128];
-        snprintf(b, sizeof b, "posterior covariance + jitter is not positive definite (pivot %d)", info);
-        fail(info, b);
-        return info;
-    }
-    return 0;
+    return pivot_status(info, "posterior covariance + jitter");
 }
 
 static int joint_sample_checks(gpso_handle* h, const void* xc, long long M, int S, double jitter, const void* z, const void* out,
@@ -2973,8 +2892,7 @@ extern "C" int gpso_set_overlap(gpso_handle* h, int enabled) {
 
 extern "C" int gpso_set_factor_mode(gpso_handle* h, int mode) {
     if (!h || mode < 0 || mode > 3) return fail(GPSO_E_BADARG, "gpso_set_factor_mode: bad argument");
-    h->chol_mode = mode == 0 ? 0 : 1;
-    h->hybrid_mode = mode == 2 ? 1 : (mode == 3 ? 2 : 0);
+    h->factor_mode = mode;
     return 0;
 }
 
@@ -2994,7 +2912,7 @@ extern "C" int gpso_trim_pool(int device, int64_t* cached_bytes_before) {
 
 extern "C" int gpso_factor_info(gpso_handle* h, int* out2) {
     if (!h || !out2) return fail(GPSO_E_BADARG, "gpso_factor_info: null argument");
-    out2[0] = h->chol_mode == 0 ? 0 : (h->hybrid_nodes > 0 ? 2 : 1);
+    out2[0] = h->factor_mode == 0 ? 0 : (h->hybrid_nodes > 0 ? 2 : 1);
     out2[1] = h->hybrid_nodes;
     return 0;
 }

@@ -204,7 +204,7 @@ def test_inverse_engines_agree(cuda, N, d, noise, persistent):
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("N,d", [(129, 2), (300, 3), (1100, 5), (2100, 6)])
 def test_factor_schedules_agree(cuda, N, d):
-    """Persistent dataflow kernel (blocks of 2 panels below 48 panels, fused diagonal update) against the step-by-step
+    """Persistent dataflow kernel (unblocked updates below 48 panels, fused diagonal update) against the step-by-step
     launches: same factor up to summation order, same LML / gradient well inside the parity tolerances, both against the
     oracle."""
     X, y = synthetic(N, d, seed=3)

@@ -4,15 +4,13 @@ Discrete-event replay of the persistent factorisation kernel's task queue (no GP
 order, each waits for the counters its task names, runs for the task's duration and signals.  Task durations are the
 measured ones (DESIGN.md 3.3, profiles/r01s3_ncu_summary.md): DIAG 35 us + 10 us per fused update panel, PANEL 25 us (8 us per row strip of the tile below the diagonal block),
 narrow update 31 us, wide update 17 W + 12 us, TRANSPOSE 5 us.  Prints the makespan, the critical chain
-(sum over panels of DIAG + PANEL) and the work bound (sum of durations / workers), for the library's own queue and for
-other panels-per-block W (GPSO_CHOL_W is read when the library builds a queue, so each W runs in a subprocess).
+(sum over panels of DIAG + PANEL) and the work bound (sum of durations / workers) of the library's own queue.
 
     python tools/factor_sim.py [nb ...]        e.g.  python tools/factor_sim.py 32 64
 """
 import ctypes
 import heapq
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -89,22 +87,11 @@ def simulate(nb, nsm=148, with_inverse=False):
 
 
 def main():
-    if len(sys.argv) > 1 and sys.argv[1] == "--one":
-        r = simulate(int(sys.argv[2]))
-        print(f"{r['makespan_us']:.0f} {r['work_bound_us']:.0f} {r['chain_us']:.0f} {r['idle_waiting_us_per_worker']:.0f} {r['tasks']}")
-        return
-    sizes = [int(a) for a in sys.argv[1:]] or [32, 64]
-    for nb in sizes:
-        print(f"nb = {nb} (N = {nb * 128}): makespan / work bound / DIAG+PANEL chain / mean wait per worker [us], tasks")
-        for W in (0, 2, 3, 4, 6, 8):
-            env = dict(os.environ)
-            if W:
-                env["GPSO_CHOL_W"] = str(W)
-            else:
-                env.pop("GPSO_CHOL_W", None)
-            out = subprocess.run([sys.executable, __file__, "--one", str(nb)], env=env, capture_output=True, text=True)
-            label = f"W = {W}" if W else "library default"
-            print(f"  {label:16s} {out.stdout.strip() or out.stderr.strip()[-200:]}")
+    for nb in [int(a) for a in sys.argv[1:]] or [32, 64]:
+        r = simulate(nb)
+        print(f"nb = {nb} (N = {nb * 128}): makespan {r['makespan_us']:.0f} us, work bound {r['work_bound_us']:.0f} us, "
+              f"DIAG+PANEL chain {r['chain_us']:.0f} us, mean wait per worker {r['idle_waiting_us_per_worker']:.0f} us, "
+              f"{r['tasks']} tasks")
 
 
 if __name__ == "__main__":
