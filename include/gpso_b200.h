@@ -22,6 +22,9 @@
  *         [ alpha , lengthscale(s) , kernel variance , likelihood (noise) variance , mean constant (if any) ]
  *     GPSO_MEAN_LINEAR (m(x) = x . A + b) packs d + 1 mean entries in the place of the constant, A before b ('A' < 'b'):
  *         [ (alpha) , lengthscale(s) , kernel variance , likelihood (noise) variance , A[0..d-1] , b ]
+ *     GPSO_KERNEL_SUM (gpflow.kernels.Sum, k = sum_c k_c) packs each component's block in component order, then the noise
+ *     and the mean entries:
+ *         [ c0: (alpha) , lengthscale(s) , variance ; c1: ... ; ... ; likelihood (noise) variance , mean entries ]
  *     d is the input dimension of gpso_set_data, so the count is known from then on (as for ARD lengthscales).
  *     `u`     = unconstrained (softplus pre-image; noise variance has the 1e-6 floor of gpflow.likelihoods.Gaussian),
  *     `theta` = constrained values.
@@ -49,6 +52,11 @@ enum {
 /* gpflow.kernels.* accepted by GPRSurrogate(gp_kernel=...), gp_surrogate.py:393-402, default Matern52 (:424) */
 enum { GPSO_KERNEL_MATERN12 = 0, GPSO_KERNEL_MATERN32 = 1, GPSO_KERNEL_MATERN52 = 2, GPSO_KERNEL_SE = 3, GPSO_KERNEL_RQ = 4 };
 /* GPSO_KERNEL_RQ = gpflow.kernels.RationalQuadratic: variance * (1 + r2 / (2 alpha))^-alpha, alpha > 0 (softplus) */
+/* GPSO_KERNEL_SUM = gpflow.kernels.Sum of 1..GPSO_MAX_SUM components, each one of the five ids above with its own variance,
+ * lengthscale(s) and alpha; created with gpso_create_sum (gpso_create refuses it: it has no components).  Components times
+ * the input dimension d may not exceed 64.  The prior variance k(x, x) is var_tot = sum_c variance_c. */
+enum { GPSO_KERNEL_SUM = 5 };
+#define GPSO_MAX_SUM 4
 /* gpflow.mean_functions.*: None/Zero or Constant (:167, :427), or Linear (m(x) = x . A + b, A[d,1] and b unconstrained) */
 enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1, GPSO_MEAN_LINEAR = 2 };
 
@@ -59,6 +67,8 @@ int gpso_device_count(void);            /* number of CUDA devices, or GPSO_E_* *
 
 /* ---- life cycle: replaces gpflow.models.GPR(...) construction, gp_surrogate.py:490-495 ----------------------- */
 int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** out);
+/* A sum kernel of n components (1..GPSO_MAX_SUM): kernel_ids[n] in GPSO_KERNEL_MATERN12..GPSO_KERNEL_RQ, ard[n] in {0, 1}. */
+int gpso_create_sum(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out);
 int gpso_destroy(gpso_handle* h);
 
 /* model.data = (x, y), gp_surrogate.py:498.  X_host[N,d], y_host[N] are copied to the device. */
@@ -130,7 +140,10 @@ int gpso_grow_ucb_argmax_range(gpso_handle* h, const double* bounds_host, int d,
 /* The fitted state (theta, scaled training inputs, alpha, L^-1) is exposed as ONE contiguous device buffer so the host
  * side can broadcast it with a single NCCL call (torch.distributed.broadcast) and import it on the other ranks.
  * GPSO_MEAN_LINEAR handles append A (d doubles) after L^-1, so their state is 8 d bytes longer; a state is only imported into
- * a handle that has a linear mean exactly when the exporting handle had one (GPSO_E_BADARG otherwise). */
+ * a handle that has a linear mean exactly when the exporting handle had one (GPSO_E_BADARG otherwise).
+ * GPSO_KERNEL_SUM handles carry the C scaled copies of the inputs (C d Np doubles in the place of d Np) and append a component
+ * block after L^-1 (and A): [C, then per component: family, lengthscale count, variance, alpha, lengthscales].  A state is
+ * only imported into a sum handle with the same component count, families and ARD flags (GPSO_E_BADARG otherwise). */
 int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes);   /* size for a given problem shape */
 int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t bytes, void* stream);
 int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream);

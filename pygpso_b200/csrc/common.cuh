@@ -373,6 +373,43 @@ __device__ __forceinline__ void cov_and_radial(double r2, double var, double alp
     }
 }
 
+// ---- sum kernel (gpflow.kernels.Sum) -----------------------------------------------------------------------------------
+// k = sum_c k_c in component order, each component one of the five families above with its own variance, alpha and
+// lengthscales.  Component c reads its own scaled inputs Xs_c = X / ls_c, stored at Xs + c * d * Np ([C][d][Np]), and its
+// lengthscales expanded to d entries at ls + c * d.  The table travels by value as the last kernel argument (constant bank):
+// every thread reads the same family, so the switch below never diverges.
+constexpr int KERNEL_SUM = 5;
+constexpr int MAX_SUM = 4;
+struct SumTable {
+    int n;                 // components, 1..MAX_SUM (0 in the launches of the other kernels, which never read the table)
+    int fam[MAX_SUM];      // KERNEL_MATERN12 .. KERNEL_RQ
+    double var[MAX_SUM];   // component variances
+    double alpha[MAX_SUM]; // RationalQuadratic shape (read for KERNEL_RQ components only)
+};
+
+__device__ __forceinline__ double sum_term(const SumTable& t, int c, double r2) {
+    const double v = t.var[c], a = t.alpha[c];
+    switch (t.fam[c]) {
+        case KERNEL_MATERN12: return cov_from_r2<KERNEL_MATERN12>(r2, v, a);
+        case KERNEL_MATERN32: return cov_from_r2<KERNEL_MATERN32>(r2, v, a);
+        case KERNEL_MATERN52: return cov_from_r2<KERNEL_MATERN52>(r2, v, a);
+        case KERNEL_SE: return cov_from_r2<KERNEL_SE>(r2, v, a);
+        default: return cov_from_r2<KERNEL_RQ>(r2, v, a);
+    }
+}
+
+template <int W>
+__device__ __forceinline__ void sum_term_v(const SumTable& t, int c, const double (&r2)[W], double (&k)[W]) {
+    const double v = t.var[c], a = t.alpha[c];
+    switch (t.fam[c]) {
+        case KERNEL_MATERN12: cov_from_r2_v<KERNEL_MATERN12, W>(r2, v, a, k); break;
+        case KERNEL_MATERN32: cov_from_r2_v<KERNEL_MATERN32, W>(r2, v, a, k); break;
+        case KERNEL_MATERN52: cov_from_r2_v<KERNEL_MATERN52, W>(r2, v, a, k); break;
+        case KERNEL_SE: cov_from_r2_v<KERNEL_SE, W>(r2, v, a, k); break;
+        default: cov_from_r2_v<KERNEL_RQ, W>(r2, v, a, k); break;
+    }
+}
+
 // ---- deterministic block reductions -----------------------------------------------------------------------------
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

@@ -271,6 +271,11 @@ struct gpso_handle {
     double ls_host[MAX_LS] = {0}, variance = 1.0, noise = 1.0, c0 = 0.0;  // c0: the mean constant, or b of the linear mean
     double A_host[MAX_LS] = {0};  // GPSO_MEAN_LINEAR: A, also in meanA on the device
     double rq_alpha = 1.0;  // RationalQuadratic shape (KERNEL_RQ only; the other kernels never read it)
+    // KERNEL_SUM (gpso_create_sum): the component table the covariance kernels take (families, variances, alphas; n = 0 for the
+    // other kernels) and the ARD flag of each component.  `variance` then holds the prior variance var_tot = sum_c var_c, the fp64
+    // sum in component order, and ls_host the lengthscales of every component expanded to d entries ([C][d], as on the device).
+    SumTable sum = {};
+    int sum_ard[MAX_SUM] = {0};
     bool have_data = false, factorized = false;
     double factor_nlml = 0.0;
     double* host_rec = nullptr;  // pinned: results of an evaluation come back in one record without staging copies
@@ -291,11 +296,21 @@ struct gpso_handle {
     std::vector<int> trace_tags;
     size_t trace_used = 0;
     std::vector<double> trace_out;
-    int n_ls() const { return ard ? d : 1; }
+    bool is_sum() const { return kernel_id == KERNEL_SUM; }
+    int dx() const { return is_sum() ? sum.n * d : d; }  // rows of the scaled inputs Xs: [C][d] for a sum
+    int n_ls() const { return is_sum() ? dx() : (ard ? d : 1); }
     int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
+    int comp_ls(int c) const { return sum_ard[c] ? d : 1; }      // packed lengthscales of sum component c
+    int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + 1; }  // [alpha], lengthscale(s), variance
+    int n_kernel_params() const {
+        if (!is_sum()) return n_rq() + n_ls() + 1;
+        int n = 0;
+        for (int c = 0; c < sum.n; c++) n += comp_params(c);
+        return n;
+    }
     bool linear() const { return mean_id == GPSO_MEAN_LINEAR; }
     int n_mean() const { return mean_id == GPSO_MEAN_CONSTANT ? 1 : (linear() ? d + 1 : 0); }  // A (d entries) before b
-    int n_params() const { return n_rq() + n_ls() + 2 + n_mean(); }
+    int n_params() const { return n_kernel_params() + 1 + n_mean(); }
 };
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -357,22 +372,26 @@ struct KernelIds {
         return rc;
     }
 };
+static_assert(GPSO_KERNEL_SUM == KERNEL_SUM && GPSO_MAX_SUM == MAX_SUM, "sum kernel constants of the C ABI");
 using AllKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ>;
+// The covariance kernels also have a KERNEL_SUM instantiation; the gradient runs the families' own kernel per component.
+using CovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM>;
 
 static void launch_gram(gpso_handle* h, cudaStream_t st) {
     dim3 grid(h->Np / CT, h->Np / CT);
-    AllKernels::with(h->kernel_id, [&](auto kid) {
+    CovKernels::with(h->kernel_id, [&](auto kid) {
         gram_kernel<kid><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->d, h->Np, h->variance, h->noise, h->K.as<double>(),
-                                               h->rq_alpha);
+                                               h->rq_alpha, h->sum);
     });
 }
 
 static void launch_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long Mw_pad) {
-    size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
-    AllKernels::with(h->kernel_id, [&](auto kid) {
+    size_t sm = (size_t)(XG * h->dx() + 8 * XG) * sizeof(double);
+    CovKernels::with(h->kernel_id, [&](auto kid) {
         crosscov_kernel<kid><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
                                                                       h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                                      h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha);
+                                                                      h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha,
+                                                                      h->sum);
     });
 }
 
@@ -382,7 +401,7 @@ static int oz_configure() {
     // full shared-memory carve-out for both kernels: the persistent product CTA (one per SM) must leave room for a
     // cross-covariance block of the next window on the same SM (they use different pipes and overlap)
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<S, OZ_TRMM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    return AllKernels::each([](auto kid) -> int {
+    return CovKernels::each([](auto kid) -> int {
         CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<kid, S>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         CU_TRY(cudaFuncSetAttribute(crosscov_slices_kernel<kid, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
         return 0;
@@ -397,7 +416,7 @@ static int screen_configure() {
         CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<2, SCR_NT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ScrCfg<2, SCR_NT, true>::SMEM_BYTES));
         CU_TRY(cudaFuncSetAttribute(ozaki_screen_kernel<2, SCR_NT, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
-    return AllKernels::each([](auto kid) -> int {
+    return CovKernels::each([](auto kid) -> int {
         CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, S, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
         CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, S, SCR_NT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         return 0;
@@ -412,10 +431,10 @@ static size_t screen_xcov_smem(int d) {
 template <int S>
 static void launch_screen_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long ngroups, float bscale,
                                    uint8_t* B, double* wmean) {
-    AllKernels::with(h->kernel_id, [&](auto kid) {
-        crosscov_screen_kernel<kid, S, SCR_NT><<<(unsigned)ngroups, 256, screen_xcov_smem(h->d), st>>>(
+    CovKernels::with(h->kernel_id, [&](auto kid) {
+        crosscov_screen_kernel<kid, S, SCR_NT><<<(unsigned)ngroups, 256, screen_xcov_smem(h->dx()), st>>>(
             Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs32.as<float>(), h->alpha32.as<float>(), h->N, h->Np, (float)h->variance,
-            h->c0, bscale, h->Np / 32, B, wmean, (float)h->rq_alpha);
+            h->c0, bscale, h->Np / 32, B, wmean, (float)h->rq_alpha, h->sum);
     });
 }
 
@@ -454,10 +473,10 @@ static size_t oz_xcov_smem(int d) { return (size_t)(OZ_NT * d + 2 * d * OZ_XK + 
 template <int S>
 static void launch_oz_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long nct, double bscale,
                                uint8_t* B, double* wmean) {
-    AllKernels::with(h->kernel_id, [&](auto kid) {
-        crosscov_slices_kernel<kid, S><<<(unsigned)nct, 256, oz_xcov_smem(h->d), st>>>(
+    CovKernels::with(h->kernel_id, [&](auto kid) {
+        crosscov_slices_kernel<kid, S><<<(unsigned)nct, 256, oz_xcov_smem(h->dx()), st>>>(
             Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(), h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-            bscale, h->Np / 32, B, wmean, h->rq_alpha);
+            bscale, h->Np / 32, B, wmean, h->rq_alpha, h->sum);
     });
 }
 
@@ -496,18 +515,21 @@ static void launch_oz_slices(gpso_handle* h, cudaStream_t st) {
         default: fn<8>(__VA_ARGS__); break;    \
     }
 
-static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride) {
-    AllKernels::with(h->kernel_id, [&](auto kid) {
-        if (!h->ard) {
-            lml_grad_kernel<kid, false><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
-                                                             h->d, h->Np, h->variance, 0, 1, h->gpart.as<double>(), stride, h->rq_alpha);
+// The partial sums of one covariance family (a sum kernel calls this once per component, with the component's own scaled
+// inputs, variance and alpha, into its own block of partial sums).
+static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride, int kernel_id, int ard, const double* Xs, double var,
+                        double rq_alpha, double* part) {
+    AllKernels::with(kernel_id, [&](auto kid) {
+        if (!ard) {
+            lml_grad_kernel<kid, false><<<nblk, 256, 0, st>>>(Xs, h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
+                                                             h->d, h->Np, var, 0, 1, part, stride, rq_alpha);
             h->launches++;
         } else {
             for (int dim0 = 0; dim0 < h->d; dim0 += GRAD_DCH) {
                 int nd = std::min(GRAD_DCH, h->d - dim0);
-                lml_grad_kernel<kid, true><<<nblk, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(),
-                                                                h->N, h->d, h->Np, h->variance, dim0, nd, h->gpart.as<double>(),
-                                                                stride, h->rq_alpha);
+                lml_grad_kernel<kid, true><<<nblk, 256, 0, st>>>(Xs, h->alpha.as<double>(), h->Kinv.as<double>(),
+                                                                h->N, h->d, h->Np, var, dim0, nd, part,
+                                                                stride, rq_alpha);
                 h->launches++;
             }
         }
@@ -536,7 +558,7 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_KINV_S, OZ_LAUUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_KINV_S>::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_INV_S, OZ_GEMM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_INV_S>::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_HYB_S, OZ_GEMM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_HYB_S>::SMEM_BYTES));
-    GP_TRY(AllKernels::each([](auto kid) -> int {
+    GP_TRY(CovKernels::each([](auto kid) -> int {
         CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<kid>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
         CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
         return 0;
@@ -565,7 +587,7 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     size_t mat = (size_t)Np * Np * sizeof(double);
     GP_TRY(h->X.ensure((size_t)N * d * sizeof(double)));
     GP_TRY(h->y.ensure((size_t)Np * sizeof(double)));
-    GP_TRY(h->Xs.ensure((size_t)d * Np * sizeof(double)));
+    GP_TRY(h->Xs.ensure((size_t)(h->is_sum() ? h->sum.n : 1) * d * Np * sizeof(double)));
     GP_TRY(h->ls.ensure(MAX_LS * sizeof(double)));
     if (h->linear()) GP_TRY(h->meanA.ensure(MAX_LS * sizeof(double)));
     GP_TRY(h->alpha.ensure((size_t)Np * sizeof(double)));
@@ -591,6 +613,20 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     h->d = d;
     h->Np = Np;
     h->nb = Np / TB;
+    return 0;
+}
+
+// Xs[dim][Np] = X / ls; a sum: Xs_c = X / ls_c at Xs + c d Np, the division of the bare kernel (ls_c expanded to d entries)
+static int scale_inputs(gpso_handle* h, cudaStream_t st, const double* X, int rows, int Np, double* Xs) {
+    if (!h->is_sum()) {
+        scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>(), h->n_ls(), rows, h->d, Np, Xs);
+        return check_launch(h, "scale_inputs");
+    }
+    for (int c = 0; c < h->sum.n; c++) {
+        scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>() + (size_t)c * h->d, h->d, rows, h->d, Np,
+                                                              Xs + (size_t)c * h->d * Np);
+        GP_TRY(check_launch(h, "scale_inputs"));
+    }
     return 0;
 }
 
@@ -1236,9 +1272,7 @@ static int factor_pipeline(gpso_handle* h, cudaStream_t st, bool need_kinv) {
     GP_TRY(upload_lengthscales(h, st));
     if (h->linear()) CU_TRY(cudaMemcpyAsync(h->meanA.p, h->A_host, sizeof(double) * h->d, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemsetAsync(h->info.p, 0, sizeof(int), st));
-    scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(h->X.as<double>(), h->ls.as<double>(), h->n_ls(), h->N, h->d, Np,
-                                                          h->Xs.as<double>());
-    GP_TRY(check_launch(h, "scale_inputs"));
+    GP_TRY(scale_inputs(h, st, h->X.as<double>(), h->N, Np, h->Xs.as<double>()));
     launch_gram(h, st);
     GP_TRY(check_launch(h, "gram"));
 
@@ -1374,9 +1408,9 @@ static int prepare_ozaki(gpso_handle* h, cudaStream_t st) {
         h->linv_rowl2_max = std::max(h->linv_rowl2_max, sqrt(rl2[i]));
     }
     if (h->screen_mode != 0 && Np >= SCREEN_MIN_NP) {
-        GP_TRY(h->Xs32.ensure((size_t)h->d * Np * sizeof(float)));
+        GP_TRY(h->Xs32.ensure((size_t)h->dx() * Np * sizeof(float)));
         GP_TRY(h->alpha32.ensure((size_t)Np * sizeof(float)));
-        screen_convert_kernel<<<(h->d * Np + 255) / 256, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->d, Np,
+        screen_convert_kernel<<<(h->dx() * Np + 255) / 256, 256, 0, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->dx(), Np,
                                                                        h->Xs32.as<float>(), h->alpha32.as<float>());
         GP_TRY(check_launch(h, "screen_convert"));
         std::vector<double> al(Np);
@@ -1427,19 +1461,45 @@ static int init_handle(gpso_handle* h, int device, int kernel_id, int ard, int m
     }
     CU_TRY(cudaEventCreate(&h->ev_t0));
     CU_TRY(cudaEventCreate(&h->ev_t1));
-    // room for the gradient record of gpso_neg_lml_grad: 4 + partial sums (up to MAX_LS + 3) + the linear mean's A (MAX_LS)
-    CU_TRY(cudaHostAlloc((void**)&h->host_rec, (2 * MAX_LS + 16) * sizeof(double), cudaHostAllocDefault));
+    // room for the gradient record of gpso_neg_lml_grad: 4 + partial sums (up to MAX_LS + 3, a sum kernel's components up to
+    // MAX_LS + 3 MAX_SUM together) + the linear mean's A (MAX_LS)
+    CU_TRY(cudaHostAlloc((void**)&h->host_rec, (2 * MAX_LS + 16 + 3 * MAX_SUM) * sizeof(double), cudaHostAllocDefault));
     GP_TRY(configure_kernels_once(device));
     return 0;
 }
 
 extern "C" int gpso_destroy(gpso_handle* h);
 
+static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out);
+
 extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** out) {
     if (!out) return fail(GPSO_E_BADARG, "gpso_create: out is null");
     *out = nullptr;
+    // GPSO_KERNEL_SUM has components: gpso_create_sum
     if (kernel_id < 0 || kernel_id > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
     if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create: unknown mean id");
+    return create_handle(device, kernel_id, ard, mean_id, SumTable{}, nullptr, out);
+}
+
+extern "C" int gpso_create_sum(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out) {
+    if (!out) return fail(GPSO_E_BADARG, "gpso_create_sum: out is null");
+    *out = nullptr;
+    if (n < 1 || n > MAX_SUM) return fail(GPSO_E_BADARG, "gpso_create_sum: the number of components must be in 1..4");
+    if (!kernel_ids || !ard) return fail(GPSO_E_BADARG, "gpso_create_sum: null argument");
+    if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create_sum: unknown mean id");
+    SumTable sum = {};
+    sum.n = n;
+    for (int c = 0; c < n; c++) {
+        if (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create_sum: unknown component kernel id");
+        if (ard[c] != 0 && ard[c] != 1) return fail(GPSO_E_BADARG, "gpso_create_sum: ard flags must be 0 or 1");
+        sum.fam[c] = kernel_ids[c];
+        sum.var[c] = 1.0;
+        sum.alpha[c] = 1.0;
+    }
+    return create_handle(device, KERNEL_SUM, 0, mean_id, sum, ard, out);
+}
+
+static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) return fail(GPSO_E_NOGPU, "gpso_create: no CUDA device available");
     if (device < 0 || device >= n) return fail(GPSO_E_BADARG, "gpso_create: device index out of range");
@@ -1453,6 +1513,8 @@ extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso
     }
     CU_TRY(cudaSetDevice(device));
     gpso_handle* h = new gpso_handle();
+    h->sum = sum;
+    for (int c = 0; c < sum.n; c++) h->sum_ard[c] = sum_ard[c];
     int rc = init_handle(h, device, kernel_id, ard, mean_id, prop);
     if (rc != 0) {
         gpso_destroy(h);  // releases whatever was created before the failure (null streams / events are skipped)
@@ -1497,6 +1559,8 @@ extern "C" int gpso_set_data(gpso_handle* h, const double* X_host, const double*
     if (!h || !X_host || !y_host) return fail(GPSO_E_BADARG, "gpso_set_data: null argument");
     if (N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_set_data: N and d must be positive");
     if (d > MAX_LS) return fail(GPSO_E_BADARG, "gpso_set_data: input dimension above the supported maximum (64)");
+    if (h->is_sum() && h->sum.n * d > MAX_LS)
+        return fail(GPSO_E_BADARG, "gpso_set_data: a sum kernel supports components x input dimension up to 64");
     GP_TRY(set_device(h));
     CU_TRY(cudaStreamSynchronize(h->stream));
     GP_TRY(ensure_shape(h, N, d));
@@ -1509,11 +1573,44 @@ extern "C" int gpso_set_data(gpso_handle* h, const double* X_host, const double*
     return 0;
 }
 
+static void load_mean(gpso_handle* h, const double* m) {  // the mean function's entries of the packed vector
+    if (h->linear()) {
+        for (int k = 0; k < h->d; k++) h->A_host[k] = m[k];
+        h->c0 = m[h->d];
+    } else {
+        h->c0 = (h->mean_id == GPSO_MEAN_CONSTANT) ? m[0] : 0.0;
+    }
+}
+
 static int load_theta(gpso_handle* h, const double* theta, int p, const char* who, bool allow_zero = false) {
     if (p != h->n_params()) {
         char b[256];
         snprintf(b, sizeof b, "%s: expected %d hyper-parameters, got %d", who, h->n_params(), p);
         return fail(GPSO_E_BADARG, b);
+    }
+    auto positive = [&](double v) { return v > 0.0 || (allow_zero && v == 0.0); };
+    if (h->is_sum()) {
+        // per component [alpha], lengthscale(s), variance; the prior variance is their variances' fp64 sum in component order
+        double var_tot = 0.0;
+        for (int c = 0; c < h->sum.n; c++) {
+            if (h->sum.fam[c] == KERNEL_RQ) {
+                if (!positive(theta[0])) return fail(GPSO_E_BADARG, std::string(who) + ": alpha must be positive");
+                h->sum.alpha[c] = *theta++;
+            }
+            const int nl = h->comp_ls(c);
+            for (int i = 0; i < nl; i++)
+                if (!positive(theta[i])) return fail(GPSO_E_BADARG, std::string(who) + ": lengthscale must be positive");
+            for (int k = 0; k < h->d; k++) h->ls_host[c * h->d + k] = theta[nl > 1 ? k : 0];
+            if (!positive(theta[nl])) return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
+            h->sum.var[c] = theta[nl];
+            var_tot = (c == 0) ? theta[nl] : var_tot + theta[nl];
+            theta += nl + 1;
+        }
+        h->variance = var_tot;
+        h->noise = theta[0];
+        if (!(h->noise > 0.0)) return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
+        load_mean(h, theta + 1);
+        return 0;
     }
     if (h->n_rq()) {
         if (!(theta[0] > 0.0) && !(allow_zero && theta[0] == 0.0))
@@ -1531,12 +1628,80 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
     h->noise = theta[nl + 1];
     if (!(h->variance > 0.0 || (allow_zero && h->variance == 0.0)) || !(h->noise > 0.0))
         return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
-    const double* m = theta + nl + 2;  // the mean function's entries
-    if (h->linear()) {
-        for (int k = 0; k < h->d; k++) h->A_host[k] = m[k];
-        h->c0 = m[h->d];
-    } else {
-        h->c0 = (h->mean_id == GPSO_MEAN_CONSTANT) ? m[0] : 0.0;
+    load_mean(h, theta + nl + 2);
+    return 0;
+}
+
+// Sum kernel: the gradient of a sum with respect to one component's parameters is that component's own gradient, so the
+// family's lml_grad_kernel runs once per component (its scaled inputs Xs_c, variance and alpha) into the component's own block
+// of partial sums, and each block is chained through the component's sigmoids.  The noise and mean entries are taken once.
+static int neg_lml_grad_sum(gpso_handle* h, const double* u, int p, double* f_host, double* grad_host) {
+    const int K = h->n_kernel_params();
+    std::vector<double> theta(p);
+    for (int i = 0; i < K; i++) theta[i] = softplus(u[i]);
+    theta[K] = NOISE_FLOOR + softplus(u[K]);
+    for (int i = 0; i < h->n_mean(); i++) theta[K + 1 + i] = u[K + 1 + i];
+    GP_TRY(load_theta(h, theta.data(), p, "gpso_neg_lml_grad", true));
+    h->factorized = false;
+    cudaStream_t st = h->stream;
+    CU_TRY(cudaEventRecord(h->ev_t0, st));
+    GP_TRY(factor_pipeline(h, st, true));
+    const int nb64 = h->Np / CT;
+    const int nblk = nb64 * (nb64 + 1) / 2;
+    int stride[MAX_SUM], off[MAX_SUM + 1] = {0};
+    for (int c = 0; c < h->sum.n; c++) {
+        stride[c] = 2 + h->comp_ls(c) + (h->sum.fam[c] == KERNEL_RQ);
+        off[c + 1] = off[c] + stride[c];
+    }
+    const int total = off[h->sum.n];
+    const int nA = h->linear() ? h->d : 0;
+    GP_TRY(h->gpart.ensure((size_t)nblk * total * sizeof(double)));
+    GP_TRY(h->gout.ensure((size_t)(total + 4 + nA) * sizeof(double)));
+    for (int c = 0; c < h->sum.n; c++) {
+        double* part = h->gpart.as<double>() + (size_t)nblk * off[c];
+        launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], h->Xs.as<double>() + (size_t)c * h->d * h->Np,
+                    h->sum.var[c], h->sum.alpha[c], part);
+        if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
+        reduce_partials_kernel<<<stride[c], 256, 0, st>>>(part, nblk, stride[c], h->gout.as<double>() + off[c]);
+        GP_TRY(check_launch(h, "reduce_partials"));
+    }
+    if (nA) {
+        linear_grad_kernel<<<nA, 256, 0, st>>>(h->X.as<double>(), h->alpha.as<double>(), h->N, h->d, h->gout.as<double>() + total);
+        GP_TRY(check_launch(h, "linear_grad"));
+    }
+    CU_TRY(cudaEventRecord(h->ev_t1, st));
+    double* rec = h->host_rec;
+    CU_TRY(cudaMemcpyAsync(rec, h->scalars.p, 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(rec + 3, h->info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(rec + 4, h->gout.p, sizeof(double) * (total + nA), cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    const double* sc = rec;
+    int info = 0;
+    memcpy(&info, rec + 3, sizeof(int));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, h->ev_t0, h->ev_t1);
+    h->last_ms[0] = ms;
+    h->last_ms[1] = h->last_ms[2] = h->last_ms[3] = 0;
+    GP_TRY(pivot_status(info, "Gram matrix"));
+    *f_host = nlml_from_scalars(h, sc);
+    int pos = 0;
+    for (int c = 0; c < h->sum.n; c++) {
+        const double* g = rec + 4 + off[c];
+        if (h->sum.fam[c] == KERNEL_RQ) {  // alpha == 0 only when softplus underflowed: the entry is 0, as for the variance
+            grad_host[pos] = h->sum.alpha[c] > 0.0 ? -(0.5 * g[stride[c] - 1]) * sigmoid(u[pos]) : 0.0;
+            pos++;
+        }
+        const int nl = h->comp_ls(c);
+        for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[2 + i] / h->ls_host[c * h->d + i]) * sigmoid(u[pos + i]);
+        pos += nl;
+        grad_host[pos] = h->sum.var[c] > 0.0 ? -(0.5 * g[0] / h->sum.var[c]) * sigmoid(u[pos]) : 0.0;
+        pos++;
+    }
+    grad_host[pos] = -(0.5 * rec[4 + 1]) * sigmoid(u[pos]);  // sum_i W_ii, taken from the first component's block
+    if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[pos + 1] = -sc[2];
+    if (nA) {
+        for (int k = 0; k < nA; k++) grad_host[pos + 1 + k] = -rec[4 + total + k];
+        grad_host[pos + 1 + nA] = -sc[2];
     }
     return 0;
 }
@@ -1546,6 +1711,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     if (!h->have_data) return fail(GPSO_E_STATE, "gpso_neg_lml_grad: call gpso_set_data first");
     if (p != h->n_params()) return fail(GPSO_E_BADARG, "gpso_neg_lml_grad: wrong number of hyper-parameters");
     GP_TRY(set_device(h));
+    if (h->is_sum()) return neg_lml_grad_sum(h, u, p, f_host, grad_host);
     const int nl = h->n_ls(), na = h->n_rq();
     std::vector<double> theta(p);
     for (int i = 0; i < na; i++) theta[i] = softplus(u[i]);  // alpha: positive, no floor
@@ -1568,7 +1734,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     const int nA = h->linear() ? h->d : 0;  // X^T alpha follows the reduced partial sums in gout
     GP_TRY(h->gpart.ensure((size_t)nblk * stride * sizeof(double)));
     GP_TRY(h->gout.ensure((size_t)(stride + 4 + nA) * sizeof(double)));
-    launch_grad(h, st, nblk, stride);
+    launch_grad(h, st, nblk, stride, h->kernel_id, h->ard, h->Xs.as<double>(), h->variance, h->rq_alpha, h->gpart.as<double>());
     if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
     reduce_partials_kernel<<<stride, 256, 0, st>>>(h->gpart.as<double>(), nblk, stride, h->gout.as<double>());
     GP_TRY(check_launch(h, "reduce_partials"));
@@ -2050,6 +2216,8 @@ static bool screen_applicable(const gpso_handle* h, long long M) {
     // the fp32 path needs the kernel variance and the lengthscales well inside the float range
     if (!(h->variance > 1e-30 && h->variance < 1e30)) return false;
     if (h->n_rq() && !(h->rq_alpha > 1e-30 && h->rq_alpha < 1e30)) return false;
+    for (int c = 0; c < h->sum.n; c++)
+        if (h->sum.fam[c] == KERNEL_RQ && !(h->sum.alpha[c] > 1e-30 && h->sum.alpha[c] < 1e30)) return false;
     for (int i = 0; i < h->n_ls(); i++)
         if (!(h->ls_host[i] > 1e-30 && h->ls_host[i] < 1e30)) return false;
     return true;
@@ -2487,34 +2655,33 @@ static int joint_ready(gpso_handle* h, const char* who) {
 }
 
 static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, int M, int Mp) {
-    size_t sm = (size_t)(XG * h->d + 8 * XG) * sizeof(double);
-    AllKernels::with(h->kernel_id, [&](auto kid) {
+    size_t sm = (size_t)(XG * h->dx() + 8 * XG) * sizeof(double);
+    CovKernels::with(h->kernel_id, [&](auto kid) {
         crosscov_kernel<kid><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
                                                                   h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                                  h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha);
+                                                                  h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha, h->sum);
     });
 }
 
 static void launch_joint_syrk(gpso_handle* h, cudaStream_t st, int M, int Mp, double jitter) {
     const int mb = Mp / TB;
-    AllKernels::with(h->kernel_id, [&](auto kid) {
+    CovKernels::with(h->kernel_id, [&](auto kid) {
         joint_syrk_kernel<kid><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp,
                                                                                    h->Np, h->d, h->variance, jitter,
-                                                                                   h->jSigma.as<double>(), h->rq_alpha);
+                                                                                   h->jSigma.as<double>(), h->rq_alpha, h->sum);
     });
 }
 
 // scaled candidates -> cross-covariance + mean -> V^T = (L^-1 K*)^T -> lower triangle of K** - V^T V (+ jitter I) in jSigma
 static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M, double jitter) {
     const int Mp = (M + TB - 1) / TB * TB, Np = h->Np;
-    GP_TRY(h->jXcs.ensure((size_t)h->d * Mp * sizeof(double)));
+    GP_TRY(h->jXcs.ensure((size_t)h->dx() * Mp * sizeof(double)));
     GP_TRY(h->jKsT.ensure((size_t)Mp * Np * sizeof(double)));
     GP_TRY(h->jmean.ensure((size_t)Mp * sizeof(double)));
     GP_TRY(h->jVT.ensure((size_t)Mp * Np * sizeof(double)));
     GP_TRY(h->jSigma.ensure((size_t)Mp * Mp * sizeof(double)));
     GP_TRY(h->jcounter.ensure(sizeof(int)));
-    scale_inputs_kernel<<<(Mp + 255) / 256, 256, 0, st>>>(Xc, h->ls.as<double>(), h->n_ls(), M, h->d, Mp, h->jXcs.as<double>());
-    GP_TRY(check_launch(h, "scale_inputs"));
+    GP_TRY(scale_inputs(h, st, Xc, M, Mp, h->jXcs.as<double>()));
     launch_joint_crosscov(h, st, Xc, M, Mp);
     GP_TRY(check_launch(h, "crosscov"));
     GP_TRY(add_linear_offset(h, st, Xc, M, 1.0, h->jmean.as<double>()));
@@ -2733,16 +2900,28 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// multi-GPU state exchange: [ header (128 doubles) | Xs (d*Np) | alpha (Np) | Linv (Np*Np) | A (d, linear mean only) ]
+// multi-GPU state exchange: [ header (128 doubles) | Xs (d*Np) | alpha (Np) | Linv (Np*Np) | A (d, linear mean only)
+//                              | component block (sum only) ]
 // header: N, d, kernel variance, noise variance, mean constant (b of the linear mean), -LML, kernel id, ard, RationalQuadratic
 // alpha (0 for the other kernels), mean id, lengthscales from slot 16.  A does not fit beside 64 lengthscales in the header.
+// A sum kernel: slot 2 is the prior variance var_tot, Xs holds the C scaled copies (C*d*Np), the header's lengthscales are the
+// components' expanded to d entries each, and the component block is [C, then per component: family, lengthscale count,
+// variance, alpha, lengthscales].
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int STATE_HEADER = 128;
+
+static long long sum_block_size(const gpso_handle* h, int d) {
+    if (!h->is_sum()) return 0;
+    long long n = 1;
+    for (int c = 0; c < h->sum.n; c++) n += 4 + (h->sum_ard[c] ? d : 1);
+    return n;
+}
 
 extern "C" int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes) {
     if (!h || !bytes || N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_state_bytes: bad argument");
     long long Np = ((N + TB - 1) / TB) * TB;
-    *bytes = (int64_t)sizeof(double) * (STATE_HEADER + (long long)d * Np + Np + Np * Np + (h->linear() ? d : 0));
+    const long long dx = (long long)(h->is_sum() ? h->sum.n : 1) * d;
+    *bytes = (int64_t)sizeof(double) * (STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? d : 0) + sum_block_size(h, d));
     return 0;
 }
 
@@ -2770,18 +2949,31 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     CU_TRY(cudaStreamSynchronize(h->stream));
     CU_TRY(cudaMemcpyAsync(dst, hdr, sizeof hdr, cudaMemcpyHostToDevice, st));
     size_t Np = h->Np;
-    CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER, h->Xs.p, sizeof(double) * h->d * Np, cudaMemcpyDeviceToDevice, st));
-    CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + h->d * Np, h->alpha.p, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));
-    CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + h->d * Np + Np, h->Linv.p, sizeof(double) * Np * Np, cudaMemcpyDeviceToDevice, st));
+    const size_t dx = h->dx();
+    CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER, h->Xs.p, sizeof(double) * dx * Np, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np, h->alpha.p, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np, h->Linv.p, sizeof(double) * Np * Np, cudaMemcpyDeviceToDevice, st));
     if (h->linear())
-        CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + h->d * Np + Np + Np * Np, h->meanA.p, sizeof(double) * h->d, cudaMemcpyDeviceToDevice, st));
+        CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np + Np * Np, h->meanA.p, sizeof(double) * h->d, cudaMemcpyDeviceToDevice, st));
+    std::vector<double> blk;
+    if (h->is_sum()) {
+        blk.push_back(h->sum.n);
+        for (int c = 0; c < h->sum.n; c++) {
+            const int nl = h->comp_ls(c);
+            blk.insert(blk.end(), {(double)h->sum.fam[c], (double)nl, h->sum.var[c], h->sum.alpha[c]});
+            for (int i = 0; i < nl; i++) blk.push_back(h->ls_host[c * h->d + i]);
+        }
+        CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? h->d : 0), blk.data(),
+                               sizeof(double) * blk.size(), cudaMemcpyHostToDevice, st));
+    }
     CU_TRY(cudaStreamSynchronize(st));
     return 0;
 }
 
 extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream) {
     if (!h || !src_dev) return fail(GPSO_E_BADARG, "gpso_import_state_dev: null argument");
-    if (N <= 0 || d <= 0 || d > MAX_LS) return fail(GPSO_E_BADARG, "gpso_import_state_dev: bad shape");
+    if (N <= 0 || d <= 0 || d > MAX_LS || (h && h->is_sum() && h->sum.n * d > MAX_LS))
+        return fail(GPSO_E_BADARG, "gpso_import_state_dev: bad shape");
     GP_TRY(set_device(h));
     int64_t need = 0;
     gpso_state_bytes(h, N, d, &need);
@@ -2797,6 +2989,22 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     if ((int)hdr[6] != h->kernel_id || (int)hdr[7] != h->ard) return fail(GPSO_E_BADARG, "gpso_import_state_dev: kernel mismatch");
     if (((int)hdr[9] == GPSO_MEAN_LINEAR) != h->linear())
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: linear mean function on one side only");
+    const size_t dx = h->dx();
+    std::vector<double> blk(sum_block_size(h, d));
+    if (h->is_sum()) {
+        // the component block: the same count, families and lengthscale counts (ARD flags) as this handle's, or no import
+        CU_TRY(cudaMemcpyAsync(blk.data(), src + STATE_HEADER + dx * h->Np + h->Np + (size_t)h->Np * h->Np + (h->linear() ? d : 0),
+                               sizeof(double) * blk.size(), cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
+        bool same = (int)blk[0] == h->sum.n;
+        for (int c = 0, q = 1; same && c < h->sum.n; q += 4 + h->comp_ls(c), c++)
+            same = (int)blk[q] == h->sum.fam[c] && (int)blk[q + 1] == h->comp_ls(c);
+        if (!same) return fail(GPSO_E_BADARG, "gpso_import_state_dev: sum kernel component mismatch");
+        for (int c = 0, q = 1; c < h->sum.n; q += 4 + h->comp_ls(c), c++) {
+            h->sum.var[c] = blk[q + 2];
+            h->sum.alpha[c] = blk[q + 3];
+        }
+    }
     h->variance = hdr[2];
     h->noise = hdr[3];
     h->c0 = hdr[4];
@@ -2804,11 +3012,11 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     if (h->n_rq()) h->rq_alpha = hdr[8];
     for (int i = 0; i < h->n_ls(); i++) h->ls_host[i] = hdr[16 + i];
     size_t Np = h->Np;
-    CU_TRY(cudaMemcpyAsync(h->Xs.p, src + STATE_HEADER, sizeof(double) * d * Np, cudaMemcpyDeviceToDevice, st));
-    CU_TRY(cudaMemcpyAsync(h->alpha.p, src + STATE_HEADER + d * Np, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));
-    CU_TRY(cudaMemcpyAsync(h->Linv.p, src + STATE_HEADER + d * Np + Np, sizeof(double) * Np * Np, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->Xs.p, src + STATE_HEADER, sizeof(double) * dx * Np, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->alpha.p, src + STATE_HEADER + dx * Np, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->Linv.p, src + STATE_HEADER + dx * Np + Np, sizeof(double) * Np * Np, cudaMemcpyDeviceToDevice, st));
     if (h->linear()) {
-        CU_TRY(cudaMemcpyAsync(h->meanA.p, src + STATE_HEADER + d * Np + Np + Np * Np, sizeof(double) * d, cudaMemcpyDeviceToDevice, st));
+        CU_TRY(cudaMemcpyAsync(h->meanA.p, src + STATE_HEADER + dx * Np + Np + Np * Np, sizeof(double) * d, cudaMemcpyDeviceToDevice, st));
         CU_TRY(cudaMemcpyAsync(h->A_host, h->meanA.p, sizeof(double) * d, cudaMemcpyDeviceToHost, st));
     }
     GP_TRY(upload_lengthscales(h, st));

@@ -23,12 +23,54 @@ constexpr int CDCH = 32;  // dimensions staged in shared memory per pass
 
 template <int KID>
 __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs, int N, int d, int Np, double var,
-                                                   double noise, double* __restrict__ K, double rq_alpha) {
+                                                   double noise, double* __restrict__ K, double rq_alpha, SumTable sum) {
     const int bj = blockIdx.x, bi = blockIdx.y;
     if (bj > bi) return;
     __shared__ double sXi[CDCH][CT];
     const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
     const int j = bj * CT + tx;
+    if constexpr (KID == KERNEL_SUM) {
+        // the loop below once per component (its own scaled inputs), the component values added in order
+        double kv[16];
+        for (int c = 0; c < sum.n; c++) {
+            const double* Xc = Xs + (size_t)c * d * Np;
+            double r2[16];
+#pragma unroll
+            for (int r = 0; r < 16; r++) r2[r] = 0.0;
+            for (int d0 = 0; d0 < d; d0 += CDCH) {
+                int dc = min(CDCH, d - d0);
+                __syncthreads();
+                for (int e = threadIdx.x; e < dc * CT; e += 256) sXi[e / CT][e % CT] = Xc[(size_t)(d0 + e / CT) * Np + bi * CT + e % CT];
+                __syncthreads();
+                for (int dd = 0; dd < dc; dd++) {
+                    double xj = Xc[(size_t)(d0 + dd) * Np + j];
+#pragma unroll
+                    for (int r = 0; r < 16; r++) {
+                        double df = sXi[dd][ty + 4 * r] - xj;
+                        r2[r] = fma(df, df, r2[r]);
+                    }
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < 16; r++) {
+                const double t = sum_term(sum, c, r2[r]);
+                kv[r] = (c == 0) ? t : kv[r] + t;
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 16; r++) {
+            int i = bi * CT + ty + 4 * r;
+            double v;
+            if (i < N && j < N) {
+                v = kv[r];
+                if (i == j) v += noise;
+            } else {
+                v = (i == j) ? 1.0 : 0.0;
+            }
+            K[(size_t)i * Np + j] = v;
+        }
+        return;
+    }
     double r2[16];
 #pragma unroll
     for (int r = 0; r < 16; r++) r2[r] = 0.0;
@@ -73,38 +115,82 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
                                                        const double* __restrict__ ls, int n_ls,
                                                        const double* __restrict__ Xs, const double* __restrict__ alpha,
                                                        int N, int Np, double var, double c0, double* __restrict__ KsT,
-                                                       double* __restrict__ mean, double rq_alpha) {
-    extern __shared__ double sm[];  // [XG][d] scaled candidate coords, then [8 warps][XG] reduction scratch
+                                                       double* __restrict__ mean, double rq_alpha, SumTable sum) {
+    extern __shared__ double sm[];  // [XG][d] scaled candidate coords (sum: [C][XG][d]), then [8 warps][XG] reduction scratch
     double* sC = sm;
-    double* sR = sm + XG * d;
+    const int nsc = (KID == KERNEL_SUM) ? sum.n : 1;  // scaled copies of the candidates
+    double* sR = sm + nsc * XG * d;
     const long long cbase = (long long)blockIdx.x * XG;
-    for (int e = threadIdx.x; e < XG * d; e += 256) {
-        long long c = cbase + e / d;
-        int dim = e % d;
-        sC[e] = (c < Mw) ? Xc[c * d + dim] / ls[n_ls > 1 ? dim : 0] : 0.0;
+    if constexpr (KID == KERNEL_SUM) {
+        // component q divides by its own lengthscales (expanded to d entries at ls + q d): the bare kernel's division
+        for (int e = threadIdx.x; e < nsc * XG * d; e += 256) {
+            const int q = e / (XG * d), f = e - q * XG * d;
+            long long c = cbase + f / d;
+            int dim = f % d;
+            sC[e] = (c < Mw) ? Xc[c * d + dim] / ls[q * d + dim] : 0.0;
+        }
+    } else {
+        for (int e = threadIdx.x; e < XG * d; e += 256) {
+            long long c = cbase + e / d;
+            int dim = e % d;
+            sC[e] = (c < Mw) ? Xc[c * d + dim] / ls[n_ls > 1 ? dim : 0] : 0.0;
+        }
     }
     __syncthreads();
     double macc[XG];
 #pragma unroll
     for (int c = 0; c < XG; c++) macc[c] = 0.0;
-    for (int j = threadIdx.x; j < Np; j += 256) {
-        double r2[XG];
+    if constexpr (KID == KERNEL_SUM) {
+        for (int j = threadIdx.x; j < Np; j += 256) {
+            double kv[XG];
+            for (int q = 0; q < sum.n; q++) {
+                const double* Xq = Xs + (size_t)q * d * Np;
+                const double* sq = sC + q * XG * d;
+                double r2[XG];
 #pragma unroll
-        for (int c = 0; c < XG; c++) r2[c] = 0.0;
-        for (int dim = 0; dim < d; dim++) {
-            double xj = Xs[(size_t)dim * Np + j];
+                for (int c = 0; c < XG; c++) r2[c] = 0.0;
+                for (int dim = 0; dim < d; dim++) {
+                    double xj = Xq[(size_t)dim * Np + j];
+#pragma unroll
+                    for (int c = 0; c < XG; c++) {
+                        double df = xj - sq[c * d + dim];
+                        r2[c] = fma(df, df, r2[c]);
+                    }
+                }
+#pragma unroll
+                for (int c = 0; c < XG; c++) {
+                    const double t = sum_term(sum, q, r2[c]);
+                    kv[c] = (q == 0) ? t : kv[c] + t;
+                }
+            }
+            double a = alpha[j];
 #pragma unroll
             for (int c = 0; c < XG; c++) {
-                double df = xj - sC[c * d + dim];
-                r2[c] = fma(df, df, r2[c]);
+                double k = (j < N && cbase + c < Mw) ? kv[c] : 0.0;
+                KsT[(size_t)(cbase + c) * Np + j] = k;
+                macc[c] = fma(k, a, macc[c]);
             }
         }
-        double a = alpha[j];  // zero for j >= N
+    } else {
+        for (int j = threadIdx.x; j < Np; j += 256) {
+            double r2[XG];
 #pragma unroll
-        for (int c = 0; c < XG; c++) {
-            double k = (j < N && cbase + c < Mw) ? cov_from_r2<KID>(r2[c], var, rq_alpha) : 0.0;
-            KsT[(size_t)(cbase + c) * Np + j] = k;
-            macc[c] = fma(k, a, macc[c]);
+            for (int c = 0; c < XG; c++) r2[c] = 0.0;
+            for (int dim = 0; dim < d; dim++) {
+                double xj = Xs[(size_t)dim * Np + j];
+#pragma unroll
+                for (int c = 0; c < XG; c++) {
+                    double df = xj - sC[c * d + dim];
+                    r2[c] = fma(df, df, r2[c]);
+                }
+            }
+            double a = alpha[j];  // zero for j >= N
+#pragma unroll
+            for (int c = 0; c < XG; c++) {
+                double k = (j < N && cbase + c < Mw) ? cov_from_r2<KID>(r2[c], var, rq_alpha) : 0.0;
+                KsT[(size_t)(cbase + c) * Np + j] = k;
+                macc[c] = fma(k, a, macc[c]);
+            }
         }
     }
 #pragma unroll

@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_v_kernel(JointVParams P) {
 template <int KID>
 __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* __restrict__ VT, const double* __restrict__ Xcs, int M,
                                                                  int Mp, int Np, int d, double var, double jitter,
-                                                                 double* __restrict__ Sigma, double rq_alpha) {
+                                                                 double* __restrict__ Sigma, double rq_alpha, SumTable sum) {
     extern __shared__ double smem[];
     int a, b;
     tri_index(blockIdx.x, a, b);
@@ -109,6 +109,21 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* _
             v = (gi == gj) ? 1.0 : 0.0;
         } else if (gj > gi) {
             v = 0.0;
+        } else if constexpr (KID == KERNEL_SUM) {
+            // Xcs[C][d][Mp]: component q's scaled candidates at Xcs + q d Mp; the diagonal starts from exactly sum_q var_q
+            double k = 0.0;
+            for (int q = 0; q < sum.n; q++) {
+                const double* Xq = Xcs + (size_t)q * d * Mp;
+                double r2 = 0.0;
+                for (int dim = 0; dim < d; dim++) {
+                    const double df = Xq[(size_t)dim * Mp + gi] - Xq[(size_t)dim * Mp + gj];
+                    r2 = fma(df, df, r2);
+                }
+                const double t = sum_term(sum, q, r2);
+                k = (q == 0) ? t : k + t;
+            }
+            v = k - smem[r * JST + c];
+            if (gi == gj) v += jitter;
         } else {
             double r2 = 0.0;
             for (int dim = 0; dim < d; dim++) {

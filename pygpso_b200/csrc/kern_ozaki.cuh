@@ -379,20 +379,31 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                                                               const double* __restrict__ ls, int n_ls,
                                                               const double* __restrict__ Xs, const double* __restrict__ alpha, int N,
                                                               int Np, double var, double c0, double bscale, int nks,
-                                                              uint8_t* __restrict__ B, double* __restrict__ mean, double rq_alpha) {
+                                                              uint8_t* __restrict__ B, double* __restrict__ mean, double rq_alpha,
+                                                              SumTable sum) {
+    // sum: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs and in shared memory alike
+    const int dx = (KID == KERNEL_SUM) ? sum.n * d : d;
     extern __shared__ double sm[];
-    double* sC = sm;                      // [d][64]       scaled candidate coordinates, dimension-major
-    double* sX = sC + d * OZ_NT;          // [2][d][128]   scaled training coordinates of the current / next super-step
-    double* sAl = sX + 2 * d * OZ_XK;     // [2][128]
+    double* sC = sm;                      // [dx][64]      scaled candidate coordinates, dimension-major
+    double* sX = sC + dx * OZ_NT;         // [2][dx][128]  scaled training coordinates of the current / next super-step
+    double* sAl = sX + 2 * dx * OZ_XK;    // [2][128]
     double* sR = sAl + 2 * OZ_XK;         // [8][64]       per-warp partial means
     const int tid = threadIdx.x, cl = tid & 31, kg = tid >> 5;
     const long long ct = blockIdx.x;
-    for (int e = tid; e < OZ_NT * d; e += 256) {
-        int cc = e / d, dim = e - cc * d;
-        long long cg = ct * OZ_NT + cc;
-        sC[dim * OZ_NT + cc] = (cg < Mw) ? Xc[cg * d + dim] / ls[n_ls > 1 ? dim : 0] : 0.0;
+    if constexpr (KID == KERNEL_SUM) {
+        for (int e = tid; e < OZ_NT * dx; e += 256) {
+            int cc = e / dx, qd = e - cc * dx, dim = qd % d;  // qd = q d + dim: component q divides by its own lengthscales
+            long long cg = ct * OZ_NT + cc;
+            sC[qd * OZ_NT + cc] = (cg < Mw) ? Xc[cg * d + dim] / ls[qd] : 0.0;
+        }
+    } else {
+        for (int e = tid; e < OZ_NT * d; e += 256) {
+            int cc = e / d, dim = e - cc * d;
+            long long cg = ct * OZ_NT + cc;
+            sC[dim * OZ_NT + cc] = (cg < Mw) ? Xc[cg * d + dim] / ls[n_ls > 1 ? dim : 0] : 0.0;
+        }
     }
-    for (int e = tid; e < d * OZ_XK; e += 256) sX[e] = Xs[(size_t)(e >> 7) * Np + (e & 127)];
+    for (int e = tid; e < dx * OZ_XK; e += 256) sX[e] = Xs[(size_t)(e >> 7) * Np + (e & 127)];
     if (tid < OZ_XK) sAl[tid] = alpha[tid];
     const bool cvalid[2] = {ct * OZ_NT + cl < Mw, ct * OZ_NT + cl + 32 < Mw};
     double macc[2] = {0.0, 0.0};
@@ -404,15 +415,68 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
         if (ss + 1 < nss) {
             // next slab of training coordinates / alpha: asynchronous 16-byte copies (LDGSTS), no registers and no
             // scoreboard stall in front of the FP64 work (13 % of the issue stalls when these were plain loads)
-            double* nx = sX + (b ^ 1) * d * OZ_XK;
-            for (int e = tid; e < d * (OZ_XK / 2); e += 256) {
+            double* nx = sX + (b ^ 1) * dx * OZ_XK;
+            for (int e = tid; e < dx * (OZ_XK / 2); e += 256) {
                 const int dim = e >> 6, pr = (e & 63) * 2;
                 cp_async16(nx + dim * OZ_XK + pr, Xs + (size_t)dim * Np + (ss + 1) * OZ_XK + pr);
             }
             if (tid < OZ_XK / 2) cp_async16(sAl + (b ^ 1) * OZ_XK + tid * 2, alpha + (ss + 1) * OZ_XK + tid * 2);
             cp_async_commit();
         }
-        const double* x = sX + b * d * OZ_XK + kg * 16;
+        const double* x = sX + b * dx * OZ_XK + kg * 16;
+        if constexpr (KID == KERNEL_SUM) {
+            // one candidate at a time (the component loop needs a second register tile): per component the distance loop
+            // and covariance of the bare kernel, the component values added in order
+            const int j0 = ss * OZ_XK + kg * 16;
+            const int ks = ss * 4 + (kg >> 1), half = kg & 1;
+            const double* al = sAl + b * OZ_XK + kg * 16;
+#pragma unroll
+            for (int a = 0; a < 2; a++) {
+                double kv[16];
+                for (int q = 0; q < sum.n; q++) {
+                    double r2[16];
+#pragma unroll
+                    for (int i = 0; i < 16; i++) r2[i] = 0.0;
+                    for (int dim = q * d; dim < (q + 1) * d; dim++) {
+                        const double xa = sC[dim * OZ_NT + cl + 32 * a];
+                        const double2* xr = reinterpret_cast<const double2*>(x + dim * OZ_XK);
+#pragma unroll
+                        for (int i = 0; i < 8; i++) {
+                            const double2 xv = xr[i];
+                            double df = xv.x - xa;
+                            r2[2 * i] = fma(df, df, r2[2 * i]);
+                            df = xv.y - xa;
+                            r2[2 * i + 1] = fma(df, df, r2[2 * i + 1]);
+                        }
+                    }
+#pragma unroll
+                    for (int g = 0; g < 16; g += XW) {
+                        double rr[XW], kk[XW];
+#pragma unroll
+                        for (int i = 0; i < XW; i++) rr[i] = r2[g + i];
+                        sum_term_v<XW>(sum, q, rr, kk);
+#pragma unroll
+                        for (int i = 0; i < XW; i++) kv[g + i] = (q == 0) ? kk[i] : kv[g + i] + kk[i];
+                    }
+                }
+                uint32_t out[S][4];
+#pragma unroll
+                for (int p = 0; p < S; p++) out[p][0] = out[p][1] = out[p][2] = out[p][3] = 0u;
+#pragma unroll
+                for (int g = 0; g < 16; g++) {
+                    const double k = (cvalid[a] && j0 + g < N) ? kv[g] : 0.0;
+                    macc[a] = fma(k, al[g], macc[a]);
+                    unsigned long long z = oz_digits<S>(k, bscale);
+#pragma unroll
+                    for (int p = 0; p < S; p++) out[p][g >> 2] = oz_put(out[p][g >> 2], z, S - 1 - p, g & 3);
+                }
+                const int c = cl + 32 * a;
+                uint8_t* dst = B + ((size_t)ct * nks + ks) * S * OZ_B_SLICE + (c >> 3) * 256 + half * 128 + (c & 7) * 16;
+#pragma unroll
+                for (int p = 0; p < S; p++) *reinterpret_cast<uint4*>(dst + (size_t)p * OZ_B_SLICE) = make_uint4(out[p][0], out[p][1], out[p][2], out[p][3]);
+            }
+            continue;
+        }
         double r2[2][16];
 #pragma unroll
         for (int i = 0; i < 16; i++) r2[0][i] = r2[1][i] = 0.0;

@@ -231,28 +231,44 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                                                                  const double* __restrict__ ls, int n_ls,
                                                                  const float* __restrict__ Xs32, const float* __restrict__ alpha32,
                                                                  int N, int Np, float var, double c0, float bscale, int nks,
-                                                                 uint8_t* __restrict__ B, double* __restrict__ mean, float rq_alpha) {
+                                                                 uint8_t* __restrict__ B, double* __restrict__ mean, float rq_alpha,
+                                                                 SumTable sum) {
+    // sum: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs32 and in shared memory alike
+    const int dx = (KID == KERNEL_SUM) ? sum.n * d : d;
     extern __shared__ __align__(16) float smf[];
-    float* sC = smf;                       // [d][64]
-    float* sX = sC + d * 64;               // [2][d][128]
-    float* sAl = sX + 2 * d * OZ_XK;       // [2][128]
+    float* sC = smf;                       // [dx][64]
+    float* sX = sC + dx * 64;              // [2][dx][128]
+    float* sAl = sX + 2 * dx * OZ_XK;      // [2][128]
     double* sR = reinterpret_cast<double*>(sAl + 2 * OZ_XK);  // [8][64]
     __shared__ int sBad[64];
     const int tid = threadIdx.x, cl = tid & 31, kg = tid >> 5;
     const long long blk = blockIdx.x;      // 64-candidate group
     if (tid < 64) sBad[tid] = 0;
     __syncthreads();
-    for (int e = tid; e < 64 * d; e += 256) {
-        const int cc = e / d, dim = e - cc * d;
-        const long long cg = blk * 64 + cc;
-        double x = 0.0;
-        if (cg < Mw) {
-            x = Xc[cg * d + dim] / ls[n_ls > 1 ? dim : 0];
-            if (!(fabs(x) <= 1.0e15)) sBad[cc] = 1;  // NaN, inf or beyond the fp32-safe range (benign race: all write 1)
+    if constexpr (KID == KERNEL_SUM) {
+        for (int e = tid; e < 64 * dx; e += 256) {
+            const int cc = e / dx, qd = e - cc * dx, dim = qd % d;  // qd = q d + dim: component q's own lengthscales
+            const long long cg = blk * 64 + cc;
+            double x = 0.0;
+            if (cg < Mw) {
+                x = Xc[cg * d + dim] / ls[qd];
+                if (!(fabs(x) <= 1.0e15)) sBad[cc] = 1;
+            }
+            sC[qd * 64 + cc] = (float)x;
         }
-        sC[dim * 64 + cc] = (float)x;
+    } else {
+        for (int e = tid; e < 64 * d; e += 256) {
+            const int cc = e / d, dim = e - cc * d;
+            const long long cg = blk * 64 + cc;
+            double x = 0.0;
+            if (cg < Mw) {
+                x = Xc[cg * d + dim] / ls[n_ls > 1 ? dim : 0];
+                if (!(fabs(x) <= 1.0e15)) sBad[cc] = 1;  // NaN, inf or beyond the fp32-safe range (benign race: all write 1)
+            }
+            sC[dim * 64 + cc] = (float)x;
+        }
     }
-    for (int e = tid; e < d * (OZ_XK / 4); e += 256) {
+    for (int e = tid; e < dx * (OZ_XK / 4); e += 256) {
         const int dim = e >> 5, q4 = (e & 31) * 4;
         cp_async16(sX + dim * OZ_XK + q4, Xs32 + (size_t)dim * Np + q4);
     }
@@ -269,30 +285,66 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
         __syncthreads();
         const int b = ss & 1;
         if (ss + 1 < nss) {
-            float* nx = sX + (b ^ 1) * d * OZ_XK;
-            for (int e = tid; e < d * (OZ_XK / 4); e += 256) {
+            float* nx = sX + (b ^ 1) * dx * OZ_XK;
+            for (int e = tid; e < dx * (OZ_XK / 4); e += 256) {
                 const int dim = e >> 5, q4 = (e & 31) * 4;
                 cp_async16(nx + dim * OZ_XK + q4, Xs32 + (size_t)dim * Np + (ss + 1) * OZ_XK + q4);
             }
             if (tid < OZ_XK / 4) cp_async16(sAl + (b ^ 1) * OZ_XK + tid * 4, alpha32 + (ss + 1) * OZ_XK + tid * 4);
             cp_async_commit();
         }
-        const float* x = sX + b * d * OZ_XK + kg * 16;
+        const float* x = sX + b * dx * OZ_XK + kg * 16;
         // squared distances of this thread's two candidates (low / high half) to its 16 training points
         f32x2_t r2[16];
 #pragma unroll
         for (int i = 0; i < 16; i++) r2[i] = 0ULL;
-        for (int dim = 0; dim < d; dim++) {
-            const f32x2_t xc = f2_pack(sC[dim * 64 + cl], sC[dim * 64 + cl + 32]);
-            const float4* xr = reinterpret_cast<const float4*>(x + dim * OZ_XK);
+        f32x2_t kv[16];  // sum: the covariance, component values added in order in fp32
+        if constexpr (KID == KERNEL_SUM) {
+            for (int q = 0; q < sum.n; q++) {
+                f32x2_t rq[16];
 #pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const float4 xv = xr[i];
-                f32x2_t df;
-                df = f2_sub(f2_pack(xv.x, xv.x), xc); r2[4 * i] = f2_fma(df, df, r2[4 * i]);
-                df = f2_sub(f2_pack(xv.y, xv.y), xc); r2[4 * i + 1] = f2_fma(df, df, r2[4 * i + 1]);
-                df = f2_sub(f2_pack(xv.z, xv.z), xc); r2[4 * i + 2] = f2_fma(df, df, r2[4 * i + 2]);
-                df = f2_sub(f2_pack(xv.w, xv.w), xc); r2[4 * i + 3] = f2_fma(df, df, r2[4 * i + 3]);
+                for (int i = 0; i < 16; i++) rq[i] = 0ULL;
+                for (int dim = q * d; dim < (q + 1) * d; dim++) {
+                    const f32x2_t xc = f2_pack(sC[dim * 64 + cl], sC[dim * 64 + cl + 32]);
+                    const float4* xr = reinterpret_cast<const float4*>(x + dim * OZ_XK);
+#pragma unroll
+                    for (int i = 0; i < 4; i++) {
+                        const float4 xv = xr[i];
+                        f32x2_t df;
+                        df = f2_sub(f2_pack(xv.x, xv.x), xc); rq[4 * i] = f2_fma(df, df, rq[4 * i]);
+                        df = f2_sub(f2_pack(xv.y, xv.y), xc); rq[4 * i + 1] = f2_fma(df, df, rq[4 * i + 1]);
+                        df = f2_sub(f2_pack(xv.z, xv.z), xc); rq[4 * i + 2] = f2_fma(df, df, rq[4 * i + 2]);
+                        df = f2_sub(f2_pack(xv.w, xv.w), xc); rq[4 * i + 3] = f2_fma(df, df, rq[4 * i + 3]);
+                    }
+                }
+                const float v = (float)sum.var[q], al = (float)sum.alpha[q];
+                const int fam = sum.fam[q];
+#pragma unroll
+                for (int g = 0; g < 16; g++) {
+                    f32x2_t t;
+                    switch (fam) {
+                        case KERNEL_MATERN12: t = cov32x2_from_r2<KERNEL_MATERN12>(rq[g], v, al); break;
+                        case KERNEL_MATERN32: t = cov32x2_from_r2<KERNEL_MATERN32>(rq[g], v, al); break;
+                        case KERNEL_MATERN52: t = cov32x2_from_r2<KERNEL_MATERN52>(rq[g], v, al); break;
+                        case KERNEL_SE: t = cov32x2_from_r2<KERNEL_SE>(rq[g], v, al); break;
+                        default: t = cov32x2_from_r2<KERNEL_RQ>(rq[g], v, al); break;
+                    }
+                    kv[g] = (q == 0) ? t : f2_add(kv[g], t);
+                }
+            }
+        } else {
+            for (int dim = 0; dim < d; dim++) {
+                const f32x2_t xc = f2_pack(sC[dim * 64 + cl], sC[dim * 64 + cl + 32]);
+                const float4* xr = reinterpret_cast<const float4*>(x + dim * OZ_XK);
+#pragma unroll
+                for (int i = 0; i < 4; i++) {
+                    const float4 xv = xr[i];
+                    f32x2_t df;
+                    df = f2_sub(f2_pack(xv.x, xv.x), xc); r2[4 * i] = f2_fma(df, df, r2[4 * i]);
+                    df = f2_sub(f2_pack(xv.y, xv.y), xc); r2[4 * i + 1] = f2_fma(df, df, r2[4 * i + 1]);
+                    df = f2_sub(f2_pack(xv.z, xv.z), xc); r2[4 * i + 2] = f2_fma(df, df, r2[4 * i + 2]);
+                    df = f2_sub(f2_pack(xv.w, xv.w), xc); r2[4 * i + 3] = f2_fma(df, df, r2[4 * i + 3]);
+                }
             }
         }
         const int j0 = ss * OZ_XK + kg * 16;
@@ -310,7 +362,9 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
         const bool tail = j0 + 16 > N;
 #pragma unroll
         for (int g = 0; g < 16; g++) {
-            f32x2_t k2 = cov32x2_from_r2<KID>(r2[g], var, rq_alpha);
+            f32x2_t k2;
+            if constexpr (KID == KERNEL_SUM) k2 = kv[g];
+            else k2 = cov32x2_from_r2<KID>(r2[g], var, rq_alpha);
             float k0, k1;
             f2_unpack(k2, k0, k1);
             k0 = cvalid[0] ? k0 : 0.0f;

@@ -600,15 +600,18 @@ class GPRSurrogate(GPSurrogate):
         with open(os.path.join(folder, self.GPR_FILE), "wb") as handle:
             dill.dump(params, handle)
         meanf = model.mean_function
+        is_sum = isinstance(model.kernel, gpmodel.Sum)
         save_info = {
             "gpr_kernel": model.kernel.__class__.__name__,
-            "gpr_kernel_shape": model.kernel.lengthscales.shape.as_list(),
+            "gpr_kernel_shape": [] if is_sum else model.kernel.lengthscales.shape.as_list(),
             "gpr_meanf": meanf.__class__.__name__,
             "gpr_meanf_shape": meanf.parameters[0].shape.as_list() if meanf.parameters else [],
             "gp_varsigma": self.gp_varsigma,
             "gp_likelihood": self.gp_lik_sigma,
             "optimiser": self._serialise_optimiser(),
         }
+        if is_sum:  # component families and lengthscale shapes, in component order
+            save_info["gpr_kernel_components"] = [[k.__class__.__name__, k.lengthscales.shape.as_list()] for k in model.kernel.kernels]
         with open(os.path.join(folder, self.GPR_INFO), "w") as handle:
             handle.write(json.dumps(save_info))
 
@@ -621,7 +624,11 @@ class GPRSurrogate(GPSurrogate):
 
         info = load_json(os.path.join(folder, cls.GPR_INFO))
         assert hasattr(gpmodel.kernels, info["gpr_kernel"])
-        gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
+        if info["gpr_kernel"] == "Sum":  # multiple_assign restores every component's parameters below
+            gp_kernel = gpmodel.Sum([getattr(gpmodel.kernels, name)(lengthscales=np.ones(shape))
+                                     for name, shape in info["gpr_kernel_components"]])
+        else:
+            gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
         assert hasattr(gpmodel.mean_functions, info["gpr_meanf"])
         meanf_cls = getattr(gpmodel.mean_functions, info["gpr_meanf"])
         if meanf_cls is gpmodel.Constant:

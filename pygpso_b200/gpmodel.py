@@ -19,7 +19,8 @@ implementation in this package.
 Parameterisation follows GPflow 2: positive parameters are softplus-transformed, the Gaussian likelihood variance has
 the 1e-6 floor, and ``trainable_variables`` are ordered kernel.lengthscales, kernel.variance, likelihood.variance,
 mean_function.c (or mean_function.A, mean_function.b for ``Linear``) -- preceded by kernel.alpha for ``RationalQuadratic``
-(tf.Module visits attributes in sorted name order).
+(tf.Module visits attributes in sorted name order).  A ``Sum`` kernel lists its components' parameters in component order,
+each component's in that same sorted order.
 """
 import types
 
@@ -120,8 +121,12 @@ class Parameter:
 # ---------------------------------------------------------------------------------------------------------------------
 # kernels / mean functions / likelihood
 # ---------------------------------------------------------------------------------------------------------------------
+MAX_SUM = 4  # GPSO_MAX_SUM: components of a Sum kernel
+
+
 class Kernel:
-    pass
+    def __add__(self, other):
+        return Sum([self, other])
 
 
 class Stationary(Kernel):
@@ -157,6 +162,30 @@ class SquaredExponential(Stationary):
 
 
 RBF = SquaredExponential
+
+
+class Sum(Kernel):
+    """``gpflow.kernels.Sum``: ``k(x, x') = sum_c k_c(x, x')`` over 1..4 stationary components, each with its own variance,
+    lengthscale(s) and (RationalQuadratic) alpha.  Nested sums are flattened as GPflow's ``Combination`` does, so ``(a + b) + c``
+    and ``a + (b + c)`` are the same three-component sum.  The same kernel object twice would share its parameters in GPflow
+    (tf.Module deduplicates variables); that is refused rather than silently duplicated."""
+
+    def __init__(self, kernels, name=None):
+        flat = []
+        for k in kernels:
+            if not isinstance(k, Kernel):
+                raise TypeError("can only combine Kernel instances")
+            flat.extend(k.kernels if isinstance(k, Sum) else [k])
+        if any(flat[i] is flat[j] for i in range(len(flat)) for j in range(i)):
+            raise ValueError("a kernel object appears twice in the sum: GPflow would share its parameters between the terms, "
+                             "which this model does not support; use two separate kernel objects")
+        if not 1 <= len(flat) <= MAX_SUM:
+            raise ValueError(f"a Sum kernel takes 1..{MAX_SUM} components, got {len(flat)}")
+        self.kernels = flat
+
+    @property
+    def parameters(self):
+        return tuple(p for k in self.kernels for p in k.parameters)
 
 
 class RationalQuadratic(Stationary):
@@ -255,19 +284,27 @@ class GPR(GPModel):
     """
 
     def __init__(self, data, kernel, mean_function=None, noise_variance=1.0, backend=None):
-        if not isinstance(kernel, Stationary):
-            raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic")
+        parts = kernel.kernels if isinstance(kernel, Sum) else [kernel]
+        if not all(isinstance(k, Stationary) for k in parts):
+            raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic, "
+                            "or a Sum of them")
         self.kernel = kernel
         self.mean_function = Zero() if mean_function is None else mean_function
         if not isinstance(self.mean_function, (Zero, Constant, Linear)):
             raise TypeError("mean_function must be Zero, Constant or Linear")
         self.likelihood = Gaussian(noise_variance)
         self._backend = backend if backend is not None else _backend.default_backend()
-        self._session = self._backend.open_session(
-            kernel=type(kernel).__name__,
-            n_lengthscales=self.kernel.lengthscales.size,
-            has_mean=_mean_id(self.mean_function),
-        )
+        if isinstance(kernel, Sum):
+            self._session = self._backend.open_session(
+                kernel="Sum", n_lengthscales=0, has_mean=_mean_id(self.mean_function),
+                components=[(type(k).__name__, k.lengthscales.size) for k in parts],
+            )
+        else:
+            self._session = self._backend.open_session(
+                kernel=type(kernel).__name__,
+                n_lengthscales=self.kernel.lengthscales.size,
+                has_mean=_mean_id(self.mean_function),
+            )
         self._factor_key = None
         self.n_loss_evaluations = 0
         self.data = data
@@ -284,8 +321,9 @@ class GPR(GPModel):
         y = np.ascontiguousarray(y, dtype=np.float64)
         if x.ndim != 2 or y.ndim != 2 or y.shape != (x.shape[0], 1):
             raise ValueError(f"data must be (X[N,d], Y[N,1]); got {x.shape}, {y.shape}")
-        if self.kernel.lengthscales.size not in (1, x.shape[1]):
-            raise ValueError("ARD lengthscales must have one entry per input dimension")
+        for k in self.kernel.kernels if isinstance(self.kernel, Sum) else [self.kernel]:
+            if k.lengthscales.size not in (1, x.shape[1]):
+                raise ValueError("ARD lengthscales must have one entry per input dimension")
         if isinstance(self.mean_function, Linear) and self.mean_function.A.shape[0] != x.shape[1]:
             raise ValueError(f"Linear mean function: A must have shape [{x.shape[1]}, 1] for {x.shape[1]}-dimensional inputs, "
                              f"got {list(self.mean_function.A.shape)}")
@@ -448,13 +486,20 @@ class Scipy:
 # ---------------------------------------------------------------------------------------------------------------------
 # gpflow.utilities look-alikes (used by save / load)
 # ---------------------------------------------------------------------------------------------------------------------
+def _kernel_leaves(prefix, kernel):
+    out = {f"{prefix}.alpha": kernel.alpha} if isinstance(kernel, RationalQuadratic) else {}
+    out.update({f"{prefix}.lengthscales": kernel.lengthscales, f"{prefix}.variance": kernel.variance})
+    return out
+
+
 def parameter_dict(model):
-    out = {".kernel.alpha": model.kernel.alpha} if isinstance(model.kernel, RationalQuadratic) else {}
-    out.update({
-        ".kernel.lengthscales": model.kernel.lengthscales,
-        ".kernel.variance": model.kernel.variance,
-        ".likelihood.variance": model.likelihood.variance,
-    })
+    if isinstance(model.kernel, Sum):  # GPflow's leaf paths: .kernel.kernels[i].<name>
+        out = {}
+        for i, k in enumerate(model.kernel.kernels):
+            out.update(_kernel_leaves(f".kernel.kernels[{i}]", k))
+    else:
+        out = _kernel_leaves(".kernel", model.kernel)
+    out[".likelihood.variance"] = model.likelihood.variance
     if isinstance(model.mean_function, Constant):
         out[".mean_function.c"] = model.mean_function.c
     elif isinstance(model.mean_function, Linear):
@@ -485,7 +530,7 @@ def tabulate_module_summary(model):
 
 kernels = types.SimpleNamespace(
     Kernel=Kernel, Stationary=Stationary, Matern12=Matern12, Matern32=Matern32, Matern52=Matern52,
-    SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic,
+    SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic, Sum=Sum,
 )
 mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant, Linear=Linear)
 likelihoods = types.SimpleNamespace(Gaussian=Gaussian)
