@@ -25,6 +25,7 @@
  *     GPSO_KERNEL_SUM (gpflow.kernels.Sum, k = sum_c k_c) packs each component's block in component order, then the noise
  *     and the mean entries:
  *         [ c0: (alpha) , lengthscale(s) , variance ; c1: ... ; ... ; likelihood (noise) variance , mean entries ]
+ *     GPSO_KERNEL_PRODUCT (gpflow.kernels.Product, k = prod_c k_c) packs its factors the same way.
  *     d is the input dimension of gpso_set_data, so the count is known from then on (as for ARD lengthscales).
  *     `u`     = unconstrained (softplus pre-image; noise variance has the 1e-6 floor of gpflow.likelihoods.Gaussian),
  *     `theta` = constrained values.
@@ -57,6 +58,10 @@ enum { GPSO_KERNEL_MATERN12 = 0, GPSO_KERNEL_MATERN32 = 1, GPSO_KERNEL_MATERN52 
  * the input dimension d may not exceed 64.  The prior variance k(x, x) is var_tot = sum_c variance_c. */
 enum { GPSO_KERNEL_SUM = 5 };
 #define GPSO_MAX_SUM 4
+/* GPSO_KERNEL_PRODUCT = gpflow.kernels.Product of 1..GPSO_MAX_SUM factors, each one of the five ids above with its own variance,
+ * lengthscale(s) and alpha; created with gpso_create_product (gpso_create refuses it).  Factors times the input dimension d
+ * may not exceed 64.  The prior variance k(x, x) is var_prod = prod_c variance_c (fp64, factor order). */
+enum { GPSO_KERNEL_PRODUCT = 6 };
 /* gpflow.mean_functions.*: None/Zero or Constant (:167, :427), or Linear (m(x) = x . A + b, A[d,1] and b unconstrained) */
 enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1, GPSO_MEAN_LINEAR = 2 };
 
@@ -69,6 +74,8 @@ int gpso_device_count(void);            /* number of CUDA devices, or GPSO_E_* *
 int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** out);
 /* A sum kernel of n components (1..GPSO_MAX_SUM): kernel_ids[n] in GPSO_KERNEL_MATERN12..GPSO_KERNEL_RQ, ard[n] in {0, 1}. */
 int gpso_create_sum(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out);
+/* A product kernel of n factors, with the arguments and checks of gpso_create_sum. */
+int gpso_create_product(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out);
 int gpso_destroy(gpso_handle* h);
 
 /* model.data = (x, y), gp_surrogate.py:498.  X_host[N,d], y_host[N] are copied to the device. */
@@ -143,7 +150,9 @@ int gpso_grow_ucb_argmax_range(gpso_handle* h, const double* bounds_host, int d,
  * a handle that has a linear mean exactly when the exporting handle had one (GPSO_E_BADARG otherwise).
  * GPSO_KERNEL_SUM handles carry the C scaled copies of the inputs (C d Np doubles in the place of d Np) and append a component
  * block after L^-1 (and A): [C, then per component: family, lengthscale count, variance, alpha, lengthscales].  A state is
- * only imported into a sum handle with the same component count, families and ARD flags (GPSO_E_BADARG otherwise). */
+ * only imported into a sum handle with the same component count, families and ARD flags (GPSO_E_BADARG otherwise).
+ * GPSO_KERNEL_PRODUCT handles do the same, with var_prod in the header's variance slot and the factor variances in the block;
+ * a product state is only imported into a product handle with the same factors, and a sum state into a sum handle. */
 int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes);   /* size for a given problem shape */
 int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t bytes, void* stream);
 int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream);

@@ -79,6 +79,7 @@ def load_library():
         "gpso_device_count": (i32, []),
         "gpso_create": (i32, [i32, i32, i32, i32, ctypes.POINTER(H)]),
         "gpso_create_sum": (i32, [i32, i32, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(H)]),
+        "gpso_create_product": (i32, [i32, i32, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(H)]),
         "gpso_destroy": (i32, [H]),
         "gpso_set_data": (i32, [H, _c_double_p, _c_double_p, i32, i32]),
         "gpso_neg_lml_grad": (i32, [H, _c_double_p, i32, _c_double_p, _c_double_p]),
@@ -144,7 +145,7 @@ def load_library():
 
 
 EXPORTED_SYMBOLS = (
-    "gpso_version gpso_last_error gpso_device_count gpso_create gpso_create_sum gpso_destroy gpso_set_data gpso_neg_lml_grad "
+    "gpso_version gpso_last_error gpso_device_count gpso_create gpso_create_sum gpso_create_product gpso_destroy gpso_set_data gpso_neg_lml_grad "
     "gpso_factorize gpso_factor_lml gpso_predict_y_host gpso_predict_y_dev gpso_ucb_argmax_host gpso_ucb_argmax_dev "
     "gpso_ucb_topk_host gpso_ucb_topk_dev "
     "gpso_predict_f_cov_host gpso_predict_f_cov_dev gpso_predict_f_samples_host gpso_predict_f_samples_dev "
@@ -184,7 +185,8 @@ class CudaSession:
     """One gpso_handle."""
 
     def __init__(self, lib, device, kernel, n_lengthscales, has_mean, components=None):
-        """``components``: for ``kernel="Sum"`` the list ``[(family, n_lengthscales), ...]`` of the sum's components."""
+        """``components``: for ``kernel="Sum"`` (``"Product"``) the list ``[(family, n_lengthscales), ...]`` of the sum's
+        components (the product's factors)."""
         self._lib = lib
         self.device = device
         self.kernel = kernel
@@ -192,18 +194,19 @@ class CudaSession:
         self.mean_id = int(has_mean)
         self.has_mean = bool(has_mean)
         handle = ctypes.c_void_p()
-        if kernel == "Sum":
+        if kernel in ("Sum", "Product"):
             if not components or any(fam not in KERNEL_IDS for fam, _ in components):
-                raise ValueError(f"a Sum session needs components from {sorted(KERNEL_IDS)}, got {components!r}")
+                raise ValueError(f"a {kernel} session needs components from {sorted(KERNEL_IDS)}, got {components!r}")
             self.components = [(fam, int(nl)) for fam, nl in components]
             self.ard = False
             n = len(self.components)
             ids = (ctypes.c_int * n)(*[KERNEL_IDS[fam] for fam, _ in self.components])
             ards = (ctypes.c_int * n)(*[int(nl > 1) for _, nl in self.components])
-            _check(lib, lib.gpso_create_sum(device, n, ids, ards, self.mean_id, ctypes.byref(handle)), "gpso_create_sum")
+            create = "gpso_create_sum" if kernel == "Sum" else "gpso_create_product"
+            _check(lib, getattr(lib, create)(device, n, ids, ards, self.mean_id, ctypes.byref(handle)), create)
         else:
             if kernel not in KERNEL_IDS:
-                raise ValueError(f"unsupported kernel {kernel!r}; choose from {sorted(KERNEL_IDS)} or Sum")
+                raise ValueError(f"unsupported kernel {kernel!r}; choose from {sorted(KERNEL_IDS)}, Sum or Product")
             self.ard = n_lengthscales > 1
             _check(lib, lib.gpso_create(device, KERNEL_IDS[kernel], int(self.ard), self.mean_id, ctypes.byref(handle)),
                    "gpso_create")

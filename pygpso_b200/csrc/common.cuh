@@ -383,7 +383,7 @@ constexpr int MAX_SUM = 4;
 struct SumTable {
     int n;                 // components, 1..MAX_SUM (0 in the launches of the other kernels, which never read the table)
     int fam[MAX_SUM];      // KERNEL_MATERN12 .. KERNEL_RQ
-    double var[MAX_SUM];   // component variances
+    double var[MAX_SUM];   // component variances (a product: {var_prod, 1, 1, 1})
     double alpha[MAX_SUM]; // RationalQuadratic shape (read for KERNEL_RQ components only)
 };
 
@@ -398,6 +398,16 @@ __device__ __forceinline__ double sum_term(const SumTable& t, int c, double r2) 
     }
 }
 
+// ---- product kernel (gpflow.kernels.Product) ---------------------------------------------------------------------------
+// k = prod_c k_c in factor order, with the sum kernel's layout and table.  The table's variances are {var_prod, 1, 1, 1}
+// (var_prod = prod_c var_c, fp64 in factor order): k = cov(r2_0; var_prod) * prod_{c>=1} cov(r2_c; 1), so k(x, x) is exactly
+// var_prod, small factor variances cannot underflow in fp32, and a one-factor product is its bare kernel's operations.
+constexpr int KERNEL_PRODUCT = 6;
+__host__ __device__ constexpr bool composite_kernel(int kid) { return kid == KERNEL_SUM || kid == KERNEL_PRODUCT; }
+// the running combination of the component values: added for a sum, multiplied for a product
+template <int KID>
+__device__ __forceinline__ double combine(double acc, double t) { return KID == KERNEL_PRODUCT ? acc * t : acc + t; }
+
 template <int W>
 __device__ __forceinline__ void sum_term_v(const SumTable& t, int c, const double (&r2)[W], double (&k)[W]) {
     const double v = t.var[c], a = t.alpha[c];
@@ -407,6 +417,19 @@ __device__ __forceinline__ void sum_term_v(const SumTable& t, int c, const doubl
         case KERNEL_MATERN52: cov_from_r2_v<KERNEL_MATERN52, W>(r2, v, a, k); break;
         case KERNEL_SE: cov_from_r2_v<KERNEL_SE, W>(r2, v, a, k); break;
         default: cov_from_r2_v<KERNEL_RQ, W>(r2, v, a, k); break;
+    }
+}
+
+// cov_and_radial of factor c's family (the product gradient), warp-uniform like sum_term
+__device__ __forceinline__ void sum_term_radial(const SumTable& t, int c, double r2, double& k, double& g, double& ka) {
+    const double v = t.var[c], a = t.alpha[c];
+    ka = 0.0;
+    switch (t.fam[c]) {
+        case KERNEL_MATERN12: cov_and_radial<KERNEL_MATERN12>(r2, v, a, k, g, ka); break;
+        case KERNEL_MATERN32: cov_and_radial<KERNEL_MATERN32>(r2, v, a, k, g, ka); break;
+        case KERNEL_MATERN52: cov_and_radial<KERNEL_MATERN52>(r2, v, a, k, g, ka); break;
+        case KERNEL_SE: cov_and_radial<KERNEL_SE>(r2, v, a, k, g, ka); break;
+        default: cov_and_radial<KERNEL_RQ>(r2, v, a, k, g, ka); break;
     }
 }
 

@@ -276,6 +276,9 @@ struct gpso_handle {
     // sum in component order, and ls_host the lengthscales of every component expanded to d entries ([C][d], as on the device).
     SumTable sum = {};
     int sum_ard[MAX_SUM] = {0};
+    // KERNEL_PRODUCT (gpso_create_product) shares that table and ARD flags.  `variance` holds var_prod = prod_c var_c (fp64,
+    // factor order), the table's variances are {var_prod, 1, 1, 1}, and prod_var keeps the factor variances themselves.
+    double prod_var[MAX_SUM] = {0};
     bool have_data = false, factorized = false;
     double factor_nlml = 0.0;
     double* host_rec = nullptr;  // pinned: results of an evaluation come back in one record without staging copies
@@ -297,13 +300,16 @@ struct gpso_handle {
     size_t trace_used = 0;
     std::vector<double> trace_out;
     bool is_sum() const { return kernel_id == KERNEL_SUM; }
-    int dx() const { return is_sum() ? sum.n * d : d; }  // rows of the scaled inputs Xs: [C][d] for a sum
-    int n_ls() const { return is_sum() ? dx() : (ard ? d : 1); }
+    bool is_product() const { return kernel_id == KERNEL_PRODUCT; }
+    bool composite() const { return composite_kernel(kernel_id); }  // a sum or a product: the component table is in force
+    int dx() const { return composite() ? sum.n * d : d; }  // rows of the scaled inputs Xs: [C][d] for a sum or a product
+    int n_ls() const { return composite() ? dx() : (ard ? d : 1); }
+    double comp_var(int c) const { return is_product() ? prod_var[c] : sum.var[c]; }  // component c's own variance
     int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
     int comp_ls(int c) const { return sum_ard[c] ? d : 1; }      // packed lengthscales of sum component c
     int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + 1; }  // [alpha], lengthscale(s), variance
     int n_kernel_params() const {
-        if (!is_sum()) return n_rq() + n_ls() + 1;
+        if (!composite()) return n_rq() + n_ls() + 1;
         int n = 0;
         for (int c = 0; c < sum.n; c++) n += comp_params(c);
         return n;
@@ -372,10 +378,12 @@ struct KernelIds {
         return rc;
     }
 };
-static_assert(GPSO_KERNEL_SUM == KERNEL_SUM && GPSO_MAX_SUM == MAX_SUM, "sum kernel constants of the C ABI");
+static_assert(GPSO_KERNEL_SUM == KERNEL_SUM && GPSO_KERNEL_PRODUCT == KERNEL_PRODUCT && GPSO_MAX_SUM == MAX_SUM,
+              "sum and product kernel constants of the C ABI");
 using AllKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ>;
-// The covariance kernels also have a KERNEL_SUM instantiation; the gradient runs the families' own kernel per component.
-using CovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM>;
+// The covariance kernels also have KERNEL_SUM and KERNEL_PRODUCT instantiations; the gradient of a sum runs the families' own
+// kernel per component, a product's runs lml_grad_product_kernel.
+using CovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM, KERNEL_PRODUCT>;
 
 static void launch_gram(gpso_handle* h, cudaStream_t st) {
     dim3 grid(h->Np / CT, h->Np / CT);
@@ -558,6 +566,9 @@ static int configure_kernels() {
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_KINV_S, OZ_LAUUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_KINV_S>::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_INV_S, OZ_GEMM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_INV_S>::SMEM_BYTES));
     CU_TRY(cudaFuncSetAttribute(ozaki_kernel<OZ_HYB_S, OZ_GEMM>, cudaFuncAttributeMaxDynamicSharedMemorySize, OzCfg<OZ_HYB_S>::SMEM_BYTES));
+    // up to 64 scaled coordinate rows of the tile's rows and columns, and four ARD factors' pair weights
+    CU_TRY(cudaFuncSetAttribute(lml_grad_product_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (2 * MAX_LS * CT + MAX_SUM * CT * CT) * (int)sizeof(double)));
     GP_TRY(CovKernels::each([](auto kid) -> int {
         CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<kid>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
         CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
@@ -587,7 +598,7 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     size_t mat = (size_t)Np * Np * sizeof(double);
     GP_TRY(h->X.ensure((size_t)N * d * sizeof(double)));
     GP_TRY(h->y.ensure((size_t)Np * sizeof(double)));
-    GP_TRY(h->Xs.ensure((size_t)(h->is_sum() ? h->sum.n : 1) * d * Np * sizeof(double)));
+    GP_TRY(h->Xs.ensure((size_t)(h->composite() ? h->sum.n : 1) * d * Np * sizeof(double)));
     GP_TRY(h->ls.ensure(MAX_LS * sizeof(double)));
     if (h->linear()) GP_TRY(h->meanA.ensure(MAX_LS * sizeof(double)));
     GP_TRY(h->alpha.ensure((size_t)Np * sizeof(double)));
@@ -618,7 +629,7 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
 
 // Xs[dim][Np] = X / ls; a sum: Xs_c = X / ls_c at Xs + c d Np, the division of the bare kernel (ls_c expanded to d entries)
 static int scale_inputs(gpso_handle* h, cudaStream_t st, const double* X, int rows, int Np, double* Xs) {
-    if (!h->is_sum()) {
+    if (!h->composite()) {
         scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>(), h->n_ls(), rows, h->d, Np, Xs);
         return check_launch(h, "scale_inputs");
     }
@@ -1475,28 +1486,43 @@ static int create_handle(int device, int kernel_id, int ard, int mean_id, const 
 extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** out) {
     if (!out) return fail(GPSO_E_BADARG, "gpso_create: out is null");
     *out = nullptr;
-    // GPSO_KERNEL_SUM has components: gpso_create_sum
+    // GPSO_KERNEL_SUM and GPSO_KERNEL_PRODUCT have components: gpso_create_sum, gpso_create_product
     if (kernel_id < 0 || kernel_id > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
     if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create: unknown mean id");
     return create_handle(device, kernel_id, ard, mean_id, SumTable{}, nullptr, out);
 }
 
-extern "C" int gpso_create_sum(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out) {
-    if (!out) return fail(GPSO_E_BADARG, "gpso_create_sum: out is null");
+// The arguments of gpso_create_sum and gpso_create_product: n components (1..MAX_SUM) of the five families, ARD flags 0 / 1.
+static int component_table(const char* who, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out,
+                           SumTable& tab) {
+    const std::string w(who);
+    if (!out) return fail(GPSO_E_BADARG, w + ": out is null");
     *out = nullptr;
-    if (n < 1 || n > MAX_SUM) return fail(GPSO_E_BADARG, "gpso_create_sum: the number of components must be in 1..4");
-    if (!kernel_ids || !ard) return fail(GPSO_E_BADARG, "gpso_create_sum: null argument");
-    if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create_sum: unknown mean id");
-    SumTable sum = {};
-    sum.n = n;
+    if (n < 1 || n > MAX_SUM) return fail(GPSO_E_BADARG, w + ": the number of components must be in 1..4");
+    if (!kernel_ids || !ard) return fail(GPSO_E_BADARG, w + ": null argument");
+    if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, w + ": unknown mean id");
+    tab = {};
+    tab.n = n;
     for (int c = 0; c < n; c++) {
-        if (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create_sum: unknown component kernel id");
-        if (ard[c] != 0 && ard[c] != 1) return fail(GPSO_E_BADARG, "gpso_create_sum: ard flags must be 0 or 1");
-        sum.fam[c] = kernel_ids[c];
-        sum.var[c] = 1.0;
-        sum.alpha[c] = 1.0;
+        if (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ) return fail(GPSO_E_BADARG, w + ": unknown component kernel id");
+        if (ard[c] != 0 && ard[c] != 1) return fail(GPSO_E_BADARG, w + ": ard flags must be 0 or 1");
+        tab.fam[c] = kernel_ids[c];
+        tab.var[c] = 1.0;
+        tab.alpha[c] = 1.0;
     }
+    return 0;
+}
+
+extern "C" int gpso_create_sum(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out) {
+    SumTable sum;
+    GP_TRY(component_table("gpso_create_sum", n, kernel_ids, ard, mean_id, out, sum));
     return create_handle(device, KERNEL_SUM, 0, mean_id, sum, ard, out);
+}
+
+extern "C" int gpso_create_product(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out) {
+    SumTable tab;
+    GP_TRY(component_table("gpso_create_product", n, kernel_ids, ard, mean_id, out, tab));
+    return create_handle(device, KERNEL_PRODUCT, 0, mean_id, tab, ard, out);
 }
 
 static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out) {
@@ -1514,7 +1540,10 @@ static int create_handle(int device, int kernel_id, int ard, int mean_id, const 
     CU_TRY(cudaSetDevice(device));
     gpso_handle* h = new gpso_handle();
     h->sum = sum;
-    for (int c = 0; c < sum.n; c++) h->sum_ard[c] = sum_ard[c];
+    for (int c = 0; c < sum.n; c++) {
+        h->sum_ard[c] = sum_ard[c];
+        h->prod_var[c] = sum.var[c];
+    }
     int rc = init_handle(h, device, kernel_id, ard, mean_id, prop);
     if (rc != 0) {
         gpso_destroy(h);  // releases whatever was created before the failure (null streams / events are skipped)
@@ -1559,8 +1588,9 @@ extern "C" int gpso_set_data(gpso_handle* h, const double* X_host, const double*
     if (!h || !X_host || !y_host) return fail(GPSO_E_BADARG, "gpso_set_data: null argument");
     if (N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_set_data: N and d must be positive");
     if (d > MAX_LS) return fail(GPSO_E_BADARG, "gpso_set_data: input dimension above the supported maximum (64)");
-    if (h->is_sum() && h->sum.n * d > MAX_LS)
-        return fail(GPSO_E_BADARG, "gpso_set_data: a sum kernel supports components x input dimension up to 64");
+    if (h->composite() && h->sum.n * d > MAX_LS)
+        return fail(GPSO_E_BADARG, h->is_sum() ? "gpso_set_data: a sum kernel supports components x input dimension up to 64"
+                                               : "gpso_set_data: a product kernel supports factors x input dimension up to 64");
     GP_TRY(set_device(h));
     CU_TRY(cudaStreamSynchronize(h->stream));
     GP_TRY(ensure_shape(h, N, d));
@@ -1589,8 +1619,9 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
         return fail(GPSO_E_BADARG, b);
     }
     auto positive = [&](double v) { return v > 0.0 || (allow_zero && v == 0.0); };
-    if (h->is_sum()) {
-        // per component [alpha], lengthscale(s), variance; the prior variance is their variances' fp64 sum in component order
+    if (h->composite()) {
+        // per component [alpha], lengthscale(s), variance; the prior variance is their variances' fp64 sum (a product: product)
+        // in component order
         double var_tot = 0.0;
         for (int c = 0; c < h->sum.n; c++) {
             if (h->sum.fam[c] == KERNEL_RQ) {
@@ -1602,11 +1633,18 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
                 if (!positive(theta[i])) return fail(GPSO_E_BADARG, std::string(who) + ": lengthscale must be positive");
             for (int k = 0; k < h->d; k++) h->ls_host[c * h->d + k] = theta[nl > 1 ? k : 0];
             if (!positive(theta[nl])) return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
-            h->sum.var[c] = theta[nl];
-            var_tot = (c == 0) ? theta[nl] : var_tot + theta[nl];
+            if (h->is_product()) {
+                h->prod_var[c] = theta[nl];
+                var_tot = (c == 0) ? theta[nl] : var_tot * theta[nl];
+            } else {
+                h->sum.var[c] = theta[nl];
+                var_tot = (c == 0) ? theta[nl] : var_tot + theta[nl];
+            }
             theta += nl + 1;
         }
         h->variance = var_tot;
+        if (h->is_product())  // the table: var_prod on the first factor, unit variance on the others
+            for (int c = 0; c < h->sum.n; c++) h->sum.var[c] = (c == 0) ? var_tot : 1.0;
         h->noise = theta[0];
         if (!(h->noise > 0.0)) return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
         load_mean(h, theta + 1);
@@ -1634,8 +1672,11 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
 
 // Sum kernel: the gradient of a sum with respect to one component's parameters is that component's own gradient, so the
 // family's lml_grad_kernel runs once per component (its scaled inputs Xs_c, variance and alpha) into the component's own block
-// of partial sums, and each block is chained through the component's sigmoids.  The noise and mean entries are taken once.
-static int neg_lml_grad_sum(gpso_handle* h, const double* u, int p, double* f_host, double* grad_host) {
+// of partial sums, and each block is chained through the component's sigmoids.
+// Product kernel: dK/dtheta_c = P_-c dk_c/dtheta_c, all factors' entries from one lml_grad_product_kernel launch and one
+// reduction, whatever the ARD flags: [s_K, sum_i W_ii, then per factor its lengthscale entries and (RationalQuadratic) alpha];
+// d/d var_c = s_K / var_c for every factor.  The noise and mean entries are taken once.
+static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double* f_host, double* grad_host) {
     const int K = h->n_kernel_params();
     std::vector<double> theta(p);
     for (int i = 0; i < K; i++) theta[i] = softplus(u[i]);
@@ -1648,22 +1689,42 @@ static int neg_lml_grad_sum(gpso_handle* h, const double* u, int p, double* f_ho
     GP_TRY(factor_pipeline(h, st, true));
     const int nb64 = h->Np / CT;
     const int nblk = nb64 * (nb64 + 1) / 2;
-    int stride[MAX_SUM], off[MAX_SUM + 1] = {0};
+    // where component c's entries sit in the reduced partial sums: its variance entry (s_K), lengthscales and alpha
+    int ik[MAX_SUM], il[MAX_SUM], ia[MAX_SUM], stride[MAX_SUM], off[MAX_SUM + 1] = {0};
+    if (h->is_product()) off[0] = 2;
     for (int c = 0; c < h->sum.n; c++) {
-        stride[c] = 2 + h->comp_ls(c) + (h->sum.fam[c] == KERNEL_RQ);
+        const int nls = h->comp_ls(c), rq = h->sum.fam[c] == KERNEL_RQ;
+        stride[c] = (h->is_product() ? 0 : 2) + nls + rq;
+        ik[c] = h->is_product() ? 0 : off[c];
+        il[c] = h->is_product() ? off[c] : off[c] + 2;
+        ia[c] = il[c] + nls;
         off[c + 1] = off[c] + stride[c];
     }
     const int total = off[h->sum.n];
     const int nA = h->linear() ? h->d : 0;
     GP_TRY(h->gpart.ensure((size_t)nblk * total * sizeof(double)));
     GP_TRY(h->gout.ensure((size_t)(total + 4 + nA) * sizeof(double)));
-    for (int c = 0; c < h->sum.n; c++) {
-        double* part = h->gpart.as<double>() + (size_t)nblk * off[c];
-        launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], h->Xs.as<double>() + (size_t)c * h->d * h->Np,
-                    h->sum.var[c], h->sum.alpha[c], part);
-        if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
-        reduce_partials_kernel<<<stride[c], 256, 0, st>>>(part, nblk, stride[c], h->gout.as<double>() + off[c]);
+    if (h->is_product()) {
+        int ard_mask = 0, nard = 0;
+        for (int c = 0; c < h->sum.n; c++) {
+            ard_mask |= h->sum_ard[c] << c;
+            nard += h->sum_ard[c];
+        }
+        const size_t smem = ((size_t)2 * h->dx() * CT + (size_t)nard * CT * CT) * sizeof(double);
+        lml_grad_product_kernel<<<nblk, 256, smem, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N, h->d,
+                                                         h->Np, ard_mask, h->gpart.as<double>(), total, h->sum);
+        GP_TRY(check_launch(h, "lml_grad_product"));
+        reduce_partials_kernel<<<total, 256, 0, st>>>(h->gpart.as<double>(), nblk, total, h->gout.as<double>());
         GP_TRY(check_launch(h, "reduce_partials"));
+    } else {
+        for (int c = 0; c < h->sum.n; c++) {
+            double* part = h->gpart.as<double>() + (size_t)nblk * off[c];
+            launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], h->Xs.as<double>() + (size_t)c * h->d * h->Np,
+                        h->sum.var[c], h->sum.alpha[c], part);
+            if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
+            reduce_partials_kernel<<<stride[c], 256, 0, st>>>(part, nblk, stride[c], h->gout.as<double>() + off[c]);
+            GP_TRY(check_launch(h, "reduce_partials"));
+        }
     }
     if (nA) {
         linear_grad_kernel<<<nA, 256, 0, st>>>(h->X.as<double>(), h->alpha.as<double>(), h->N, h->d, h->gout.as<double>() + total);
@@ -1684,20 +1745,21 @@ static int neg_lml_grad_sum(gpso_handle* h, const double* u, int p, double* f_ho
     h->last_ms[1] = h->last_ms[2] = h->last_ms[3] = 0;
     GP_TRY(pivot_status(info, "Gram matrix"));
     *f_host = nlml_from_scalars(h, sc);
+    const double* g = rec + 4;
     int pos = 0;
     for (int c = 0; c < h->sum.n; c++) {
-        const double* g = rec + 4 + off[c];
         if (h->sum.fam[c] == KERNEL_RQ) {  // alpha == 0 only when softplus underflowed: the entry is 0, as for the variance
-            grad_host[pos] = h->sum.alpha[c] > 0.0 ? -(0.5 * g[stride[c] - 1]) * sigmoid(u[pos]) : 0.0;
+            grad_host[pos] = h->sum.alpha[c] > 0.0 ? -(0.5 * g[ia[c]]) * sigmoid(u[pos]) : 0.0;
             pos++;
         }
         const int nl = h->comp_ls(c);
-        for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[2 + i] / h->ls_host[c * h->d + i]) * sigmoid(u[pos + i]);
+        for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[il[c] + i] / h->ls_host[c * h->d + i]) * sigmoid(u[pos + i]);
         pos += nl;
-        grad_host[pos] = h->sum.var[c] > 0.0 ? -(0.5 * g[0] / h->sum.var[c]) * sigmoid(u[pos]) : 0.0;
+        const double var_c = h->comp_var(c);
+        grad_host[pos] = var_c > 0.0 ? -(0.5 * g[ik[c]] / var_c) * sigmoid(u[pos]) : 0.0;
         pos++;
     }
-    grad_host[pos] = -(0.5 * rec[4 + 1]) * sigmoid(u[pos]);  // sum_i W_ii, taken from the first component's block
+    grad_host[pos] = -(0.5 * g[1]) * sigmoid(u[pos]);  // sum_i W_ii, taken from the first component's block
     if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[pos + 1] = -sc[2];
     if (nA) {
         for (int k = 0; k < nA; k++) grad_host[pos + 1 + k] = -rec[4 + total + k];
@@ -1711,7 +1773,7 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     if (!h->have_data) return fail(GPSO_E_STATE, "gpso_neg_lml_grad: call gpso_set_data first");
     if (p != h->n_params()) return fail(GPSO_E_BADARG, "gpso_neg_lml_grad: wrong number of hyper-parameters");
     GP_TRY(set_device(h));
-    if (h->is_sum()) return neg_lml_grad_sum(h, u, p, f_host, grad_host);
+    if (h->composite()) return neg_lml_grad_composite(h, u, p, f_host, grad_host);
     const int nl = h->n_ls(), na = h->n_rq();
     std::vector<double> theta(p);
     for (int i = 0; i < na; i++) theta[i] = softplus(u[i]);  // alpha: positive, no floor
@@ -2901,17 +2963,18 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 
 // ---------------------------------------------------------------------------------------------------------------------
 // multi-GPU state exchange: [ header (128 doubles) | Xs (d*Np) | alpha (Np) | Linv (Np*Np) | A (d, linear mean only)
-//                              | component block (sum only) ]
+//                              | component block (sum and product only) ]
 // header: N, d, kernel variance, noise variance, mean constant (b of the linear mean), -LML, kernel id, ard, RationalQuadratic
 // alpha (0 for the other kernels), mean id, lengthscales from slot 16.  A does not fit beside 64 lengthscales in the header.
 // A sum kernel: slot 2 is the prior variance var_tot, Xs holds the C scaled copies (C*d*Np), the header's lengthscales are the
 // components' expanded to d entries each, and the component block is [C, then per component: family, lengthscale count,
-// variance, alpha, lengthscales].
+// variance, alpha, lengthscales].  A product kernel: the same, with slot 2 the prior variance var_prod and the factor variances
+// in the component block.
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int STATE_HEADER = 128;
 
 static long long sum_block_size(const gpso_handle* h, int d) {
-    if (!h->is_sum()) return 0;
+    if (!h->composite()) return 0;
     long long n = 1;
     for (int c = 0; c < h->sum.n; c++) n += 4 + (h->sum_ard[c] ? d : 1);
     return n;
@@ -2920,7 +2983,7 @@ static long long sum_block_size(const gpso_handle* h, int d) {
 extern "C" int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes) {
     if (!h || !bytes || N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_state_bytes: bad argument");
     long long Np = ((N + TB - 1) / TB) * TB;
-    const long long dx = (long long)(h->is_sum() ? h->sum.n : 1) * d;
+    const long long dx = (long long)(h->composite() ? h->sum.n : 1) * d;
     *bytes = (int64_t)sizeof(double) * (STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? d : 0) + sum_block_size(h, d));
     return 0;
 }
@@ -2956,11 +3019,11 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     if (h->linear())
         CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np + Np * Np, h->meanA.p, sizeof(double) * h->d, cudaMemcpyDeviceToDevice, st));
     std::vector<double> blk;
-    if (h->is_sum()) {
+    if (h->composite()) {
         blk.push_back(h->sum.n);
         for (int c = 0; c < h->sum.n; c++) {
             const int nl = h->comp_ls(c);
-            blk.insert(blk.end(), {(double)h->sum.fam[c], (double)nl, h->sum.var[c], h->sum.alpha[c]});
+            blk.insert(blk.end(), {(double)h->sum.fam[c], (double)nl, h->comp_var(c), h->sum.alpha[c]});
             for (int i = 0; i < nl; i++) blk.push_back(h->ls_host[c * h->d + i]);
         }
         CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? h->d : 0), blk.data(),
@@ -2972,7 +3035,7 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
 
 extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream) {
     if (!h || !src_dev) return fail(GPSO_E_BADARG, "gpso_import_state_dev: null argument");
-    if (N <= 0 || d <= 0 || d > MAX_LS || (h && h->is_sum() && h->sum.n * d > MAX_LS))
+    if (N <= 0 || d <= 0 || d > MAX_LS || (h && h->composite() && h->sum.n * d > MAX_LS))
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: bad shape");
     GP_TRY(set_device(h));
     int64_t need = 0;
@@ -2991,7 +3054,7 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: linear mean function on one side only");
     const size_t dx = h->dx();
     std::vector<double> blk(sum_block_size(h, d));
-    if (h->is_sum()) {
+    if (h->composite()) {
         // the component block: the same count, families and lengthscale counts (ARD flags) as this handle's, or no import
         CU_TRY(cudaMemcpyAsync(blk.data(), src + STATE_HEADER + dx * h->Np + h->Np + (size_t)h->Np * h->Np + (h->linear() ? d : 0),
                                sizeof(double) * blk.size(), cudaMemcpyDeviceToHost, st));
@@ -2999,13 +3062,20 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
         bool same = (int)blk[0] == h->sum.n;
         for (int c = 0, q = 1; same && c < h->sum.n; q += 4 + h->comp_ls(c), c++)
             same = (int)blk[q] == h->sum.fam[c] && (int)blk[q + 1] == h->comp_ls(c);
-        if (!same) return fail(GPSO_E_BADARG, "gpso_import_state_dev: sum kernel component mismatch");
+        if (!same)
+            return fail(GPSO_E_BADARG, h->is_sum() ? "gpso_import_state_dev: sum kernel component mismatch"
+                                                   : "gpso_import_state_dev: product kernel component mismatch");
         for (int c = 0, q = 1; c < h->sum.n; q += 4 + h->comp_ls(c), c++) {
-            h->sum.var[c] = blk[q + 2];
+            if (h->is_product())  // the table's variances are {var_prod, 1, 1, 1}, var_prod from slot 2
+                h->prod_var[c] = blk[q + 2];
+            else
+                h->sum.var[c] = blk[q + 2];
             h->sum.alpha[c] = blk[q + 3];
         }
     }
     h->variance = hdr[2];
+    if (h->is_product())
+        for (int c = 0; c < h->sum.n; c++) h->sum.var[c] = (c == 0) ? h->variance : 1.0;
     h->noise = hdr[3];
     h->c0 = hdr[4];
     h->factor_nlml = hdr[5];

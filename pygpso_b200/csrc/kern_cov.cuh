@@ -29,8 +29,8 @@ __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs
     __shared__ double sXi[CDCH][CT];
     const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
     const int j = bj * CT + tx;
-    if constexpr (KID == KERNEL_SUM) {
-        // the loop below once per component (its own scaled inputs), the component values added in order
+    if constexpr (composite_kernel(KID)) {
+        // the loop below once per component (its own scaled inputs), the component values added (multiplied) in order
         double kv[16];
         for (int c = 0; c < sum.n; c++) {
             const double* Xc = Xs + (size_t)c * d * Np;
@@ -54,7 +54,7 @@ __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs
 #pragma unroll
             for (int r = 0; r < 16; r++) {
                 const double t = sum_term(sum, c, r2[r]);
-                kv[r] = (c == 0) ? t : kv[r] + t;
+                kv[r] = (c == 0) ? t : combine<KID>(kv[r], t);
             }
         }
 #pragma unroll
@@ -118,10 +118,10 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
                                                        double* __restrict__ mean, double rq_alpha, SumTable sum) {
     extern __shared__ double sm[];  // [XG][d] scaled candidate coords (sum: [C][XG][d]), then [8 warps][XG] reduction scratch
     double* sC = sm;
-    const int nsc = (KID == KERNEL_SUM) ? sum.n : 1;  // scaled copies of the candidates
+    const int nsc = composite_kernel(KID) ? sum.n : 1;  // scaled copies of the candidates
     double* sR = sm + nsc * XG * d;
     const long long cbase = (long long)blockIdx.x * XG;
-    if constexpr (KID == KERNEL_SUM) {
+    if constexpr (composite_kernel(KID)) {
         // component q divides by its own lengthscales (expanded to d entries at ls + q d): the bare kernel's division
         for (int e = threadIdx.x; e < nsc * XG * d; e += 256) {
             const int q = e / (XG * d), f = e - q * XG * d;
@@ -140,7 +140,7 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
     double macc[XG];
 #pragma unroll
     for (int c = 0; c < XG; c++) macc[c] = 0.0;
-    if constexpr (KID == KERNEL_SUM) {
+    if constexpr (composite_kernel(KID)) {
         for (int j = threadIdx.x; j < Np; j += 256) {
             double kv[XG];
             for (int q = 0; q < sum.n; q++) {
@@ -160,7 +160,7 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
 #pragma unroll
                 for (int c = 0; c < XG; c++) {
                     const double t = sum_term(sum, q, r2[c]);
-                    kv[c] = (q == 0) ? t : kv[c] + t;
+                    kv[c] = (q == 0) ? t : combine<KID>(kv[c], t);
                 }
             }
             double a = alpha[j];
@@ -300,6 +300,136 @@ __global__ void __launch_bounds__(256) lml_grad_kernel(const double* __restrict_
     for (int q = 0; q < (ARD ? GRAD_DCH : 1); q++) {
         v = block_sum<256>(s_l[q], sRed);
         if (threadIdx.x == 0 && q < ndim) part[(size_t)blk * part_stride + 2 + dim0 + q] = v;
+    }
+}
+
+// ---- LML gradient of a product kernel (k = prod_c k_c) -----------------------------------------------------------
+// dK/dtheta_c = P_-c dk_c/dtheta_c with P_-c = prod_{j != c} k_j formed per pair from prefix and suffix products (never as
+// K / k_c: k_c can be 0).  One launch for every entry: one block per lower 64x64 tile, the tile's scaled coordinates of all C
+// factors (rows bi and columns bj, [C d][64] each) in shared memory, each pair's factor values formed once.  Partial sums:
+//   part[blk][0] = sum W*K                                  (-> d/d var_c = s_K / var_c for every factor)
+//   part[blk][1] = sum_i W_ii                               (-> d/d noise)
+//   then per factor c in order, at off_c (off_0 = 2):
+//   part[blk][off_c + q] = sum W*P_-c*g_c*(xs_i - xs_j)_q^2  (ARD: q < d)   or   sum W*P_-c*g_c*r2_c  (scalar lengthscale)
+//   part[blk][off_c + n_ls_c] = sum W*P_-c*dk_c/dalpha      (RationalQuadratic factors only)
+// Scalar entries reduce from registers.  An ARD factor's per-pair weight W*P_-c*g_c goes to shared memory ([64][64] per ARD
+// factor), and a second pass gives warp w the dimensions e = w, w + 8, ... of all ARD factors, each summed over the tile's
+// 4096 pairs in a fixed order: the distance work is at most twice the product's, whatever d.
+__global__ void __launch_bounds__(256) lml_grad_product_kernel(const double* __restrict__ Xs, const double* __restrict__ alpha,
+                                                               const double* __restrict__ Kinv, int N, int d, int Np, int ard_mask,
+                                                               double* __restrict__ part, int part_stride, SumTable tab) {
+    int blk = blockIdx.x;
+    int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
+    while ((bi + 1) * (bi + 2) / 2 <= blk) bi++;
+    while (bi * (bi + 1) / 2 > blk) bi--;
+    int bj = blk - bi * (bi + 1) / 2;
+    const int n = tab.n, dx = n * d;
+    extern __shared__ double smg[];
+    double* sXi = smg;                // [dx][64] scaled coordinates of the tile's rows
+    double* sXj = smg + dx * CT;      // [dx][64] ... and of its columns
+    double* sW = sXj + dx * CT;       // [ARD factors][64 * 64] per-pair weights W P_-c g_c
+    __shared__ double sRed[8];
+    for (int e = threadIdx.x; e < dx * CT; e += 256) {
+        const size_t row = (size_t)(e / CT) * Np;
+        sXi[e] = Xs[row + bi * CT + e % CT];
+        sXj[e] = Xs[row + bj * CT + e % CT];
+    }
+    __syncthreads();
+    const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
+    const int j = bj * CT + tx;
+    const double aj = alpha[j];
+    const double wsym = (bi == bj) ? 1.0 : 2.0;
+    double s_k = 0.0, s_tr = 0.0, s_l[MAX_SUM], s_a[MAX_SUM];
+#pragma unroll
+    for (int c = 0; c < MAX_SUM; c++) s_l[c] = s_a[c] = 0.0;
+#pragma unroll 1
+    for (int r = 0; r < 16; r++) {
+        const int il = ty + 4 * r, i = bi * CT + il;
+        const bool valid = i < N && j < N;
+        // diagonal tiles: the tile holds both triangles of a symmetric quantity, take every element once
+        double W = 0.0;
+        if (valid) W = fma(alpha[i], aj, -((j <= i) ? Kinv[(size_t)i * Np + j] : Kinv[(size_t)j * Np + i])) * wsym;
+        double r2[MAX_SUM], k[MAX_SUM], g[MAX_SUM], ka[MAX_SUM];
+#pragma unroll
+        for (int c = 0; c < MAX_SUM; c++) {
+            r2[c] = 0.0;
+            k[c] = 1.0;  // absent factors: the products below stay those of the n present ones
+            g[c] = ka[c] = 0.0;
+            if (c < n) {
+                for (int q = c * d; q < (c + 1) * d; q++) {
+                    const double df = sXi[q * CT + il] - sXj[q * CT + tx];
+                    r2[c] = fma(df, df, r2[c]);
+                }
+                sum_term_radial(tab, c, r2[c], k[c], g[c], ka[c]);
+            }
+        }
+        double pre[MAX_SUM], suf[MAX_SUM];
+        pre[0] = 1.0;
+#pragma unroll
+        for (int c = 1; c < MAX_SUM; c++) pre[c] = pre[c - 1] * k[c - 1];
+        suf[MAX_SUM - 1] = 1.0;
+#pragma unroll
+        for (int c = MAX_SUM - 2; c >= 0; c--) suf[c] = suf[c + 1] * k[c + 1];
+        if (valid) {
+            s_k = fma(W, pre[MAX_SUM - 1] * k[MAX_SUM - 1], s_k);
+            if (i == j) s_tr += W;
+        }
+        int slot = 0;
+#pragma unroll
+        for (int c = 0; c < MAX_SUM; c++) {
+            if (c < n) {
+                const double pw = W * (pre[c] * suf[c]);
+                if (ard_mask >> c & 1) {
+                    sW[slot * CT * CT + il * CT + tx] = valid ? pw * g[c] : 0.0;
+                    slot++;
+                } else if (valid) {
+                    s_l[c] = fma(pw * g[c], fmax(r2[c], 0.0), s_l[c]);
+                }
+                if (valid && tab.fam[c] == KERNEL_RQ) s_a[c] = fma(pw, ka[c], s_a[c]);
+            }
+        }
+    }
+    double v = block_sum<256>(s_k, sRed);
+    if (threadIdx.x == 0) part[(size_t)blk * part_stride + 0] = v;
+    v = block_sum<256>(s_tr, sRed);
+    if (threadIdx.x == 0) part[(size_t)blk * part_stride + 1] = v;
+    int off = 2;
+#pragma unroll
+    for (int c = 0; c < MAX_SUM; c++) {
+        if (c >= n) break;
+        const bool ard = ard_mask >> c & 1, rq = tab.fam[c] == KERNEL_RQ;
+        if (!ard) {
+            v = block_sum<256>(s_l[c], sRed);
+            if (threadIdx.x == 0) part[(size_t)blk * part_stride + off] = v;
+        }
+        const int nl = ard ? d : 1;
+        if (rq) {
+            v = block_sum<256>(s_a[c], sRed);
+            if (threadIdx.x == 0) part[(size_t)blk * part_stride + off + nl] = v;
+        }
+        off += nl + rq;
+    }
+    if (ard_mask == 0) return;
+    __syncthreads();  // the weights of every pair are in sW
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int c = 0, slot = 0, o = 2; c < n; c++) {
+        const bool ard = ard_mask >> c & 1;
+        if (ard) {
+            const double* ws = sW + slot * CT * CT;
+            for (int q = w; q < d; q += 8) {
+                const double* xi = sXi + (c * d + q) * CT;
+                const double* xj = sXj + (c * d + q) * CT;
+                double acc = 0.0;
+                for (int p = lane; p < CT * CT; p += 32) {
+                    const double df = xi[p >> 6] - xj[p & 63];
+                    acc = fma(ws[p], df * df, acc);
+                }
+                acc = warp_sum(acc);
+                if (lane == 0) part[(size_t)blk * part_stride + o + q] = acc;
+            }
+            slot++;
+        }
+        o += (ard ? d : 1) + (tab.fam[c] == KERNEL_RQ);
     }
 }
 

@@ -109,8 +109,9 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* _
             v = (gi == gj) ? 1.0 : 0.0;
         } else if (gj > gi) {
             v = 0.0;
-        } else if constexpr (KID == KERNEL_SUM) {
-            // Xcs[C][d][Mp]: component q's scaled candidates at Xcs + q d Mp; the diagonal starts from exactly sum_q var_q
+        } else if constexpr (composite_kernel(KID)) {
+            // Xcs[C][d][Mp]: component q's scaled candidates at Xcs + q d Mp; the diagonal starts from exactly
+            // sum_q var_q (a product: var_prod, its unit factors being exactly 1 at r = 0)
             double k = 0.0;
             for (int q = 0; q < sum.n; q++) {
                 const double* Xq = Xcs + (size_t)q * d * Mp;
@@ -120,7 +121,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* _
                     r2 = fma(df, df, r2);
                 }
                 const double t = sum_term(sum, q, r2);
-                k = (q == 0) ? t : k + t;
+                k = (q == 0) ? t : combine<KID>(k, t);
             }
             v = k - smem[r * JST + c];
             if (gi == gj) v += jitter;

@@ -381,8 +381,8 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                                                               int Np, double var, double c0, double bscale, int nks,
                                                               uint8_t* __restrict__ B, double* __restrict__ mean, double rq_alpha,
                                                               SumTable sum) {
-    // sum: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs and in shared memory alike
-    const int dx = (KID == KERNEL_SUM) ? sum.n * d : d;
+    // sum / product: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs and in shared memory alike
+    const int dx = composite_kernel(KID) ? sum.n * d : d;
     extern __shared__ double sm[];
     double* sC = sm;                      // [dx][64]      scaled candidate coordinates, dimension-major
     double* sX = sC + dx * OZ_NT;         // [2][dx][128]  scaled training coordinates of the current / next super-step
@@ -390,7 +390,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
     double* sR = sAl + 2 * OZ_XK;         // [8][64]       per-warp partial means
     const int tid = threadIdx.x, cl = tid & 31, kg = tid >> 5;
     const long long ct = blockIdx.x;
-    if constexpr (KID == KERNEL_SUM) {
+    if constexpr (composite_kernel(KID)) {
         for (int e = tid; e < OZ_NT * dx; e += 256) {
             int cc = e / dx, qd = e - cc * dx, dim = qd % d;  // qd = q d + dim: component q divides by its own lengthscales
             long long cg = ct * OZ_NT + cc;
@@ -424,9 +424,9 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
             cp_async_commit();
         }
         const double* x = sX + b * dx * OZ_XK + kg * 16;
-        if constexpr (KID == KERNEL_SUM) {
+        if constexpr (composite_kernel(KID)) {
             // one candidate at a time (the component loop needs a second register tile): per component the distance loop
-            // and covariance of the bare kernel, the component values added in order
+            // and covariance of the bare kernel, the component values added (multiplied) in order
             const int j0 = ss * OZ_XK + kg * 16;
             const int ks = ss * 4 + (kg >> 1), half = kg & 1;
             const double* al = sAl + b * OZ_XK + kg * 16;
@@ -456,7 +456,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                         for (int i = 0; i < XW; i++) rr[i] = r2[g + i];
                         sum_term_v<XW>(sum, q, rr, kk);
 #pragma unroll
-                        for (int i = 0; i < XW; i++) kv[g + i] = (q == 0) ? kk[i] : kv[g + i] + kk[i];
+                        for (int i = 0; i < XW; i++) kv[g + i] = (q == 0) ? kk[i] : combine<KID>(kv[g + i], kk[i]);
                     }
                 }
                 uint32_t out[S][4];

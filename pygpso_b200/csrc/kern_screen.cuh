@@ -233,8 +233,8 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                                                                  int N, int Np, float var, double c0, float bscale, int nks,
                                                                  uint8_t* __restrict__ B, double* __restrict__ mean, float rq_alpha,
                                                                  SumTable sum) {
-    // sum: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs32 and in shared memory alike
-    const int dx = (KID == KERNEL_SUM) ? sum.n * d : d;
+    // sum / product: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs32 and in shared memory alike
+    const int dx = composite_kernel(KID) ? sum.n * d : d;
     extern __shared__ __align__(16) float smf[];
     float* sC = smf;                       // [dx][64]
     float* sX = sC + dx * 64;              // [2][dx][128]
@@ -245,7 +245,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
     const long long blk = blockIdx.x;      // 64-candidate group
     if (tid < 64) sBad[tid] = 0;
     __syncthreads();
-    if constexpr (KID == KERNEL_SUM) {
+    if constexpr (composite_kernel(KID)) {
         for (int e = tid; e < 64 * dx; e += 256) {
             const int cc = e / dx, qd = e - cc * dx, dim = qd % d;  // qd = q d + dim: component q's own lengthscales
             const long long cg = blk * 64 + cc;
@@ -298,8 +298,8 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
         f32x2_t r2[16];
 #pragma unroll
         for (int i = 0; i < 16; i++) r2[i] = 0ULL;
-        f32x2_t kv[16];  // sum: the covariance, component values added in order in fp32
-        if constexpr (KID == KERNEL_SUM) {
+        f32x2_t kv[16];  // sum / product: the covariance, component values added (multiplied) in order in fp32
+        if constexpr (composite_kernel(KID)) {
             for (int q = 0; q < sum.n; q++) {
                 f32x2_t rq[16];
 #pragma unroll
@@ -329,7 +329,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                         case KERNEL_SE: t = cov32x2_from_r2<KERNEL_SE>(rq[g], v, al); break;
                         default: t = cov32x2_from_r2<KERNEL_RQ>(rq[g], v, al); break;
                     }
-                    kv[g] = (q == 0) ? t : f2_add(kv[g], t);
+                    kv[g] = (q == 0) ? t : (KID == KERNEL_PRODUCT ? f2_mul(kv[g], t) : f2_add(kv[g], t));
                 }
             }
         } else {
@@ -363,7 +363,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
 #pragma unroll
         for (int g = 0; g < 16; g++) {
             f32x2_t k2;
-            if constexpr (KID == KERNEL_SUM) k2 = kv[g];
+            if constexpr (composite_kernel(KID)) k2 = kv[g];
             else k2 = cov32x2_from_r2<KID>(r2[g], var, rq_alpha);
             float k0, k1;
             f2_unpack(k2, k0, k1);

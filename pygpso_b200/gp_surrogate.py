@@ -600,7 +600,7 @@ class GPRSurrogate(GPSurrogate):
         with open(os.path.join(folder, self.GPR_FILE), "wb") as handle:
             dill.dump(params, handle)
         meanf = model.mean_function
-        is_sum = isinstance(model.kernel, gpmodel.Sum)
+        is_sum = isinstance(model.kernel, gpmodel.Combination)  # a Sum or a Product
         save_info = {
             "gpr_kernel": model.kernel.__class__.__name__,
             "gpr_kernel_shape": [] if is_sum else model.kernel.lengthscales.shape.as_list(),
@@ -610,7 +610,7 @@ class GPRSurrogate(GPSurrogate):
             "gp_likelihood": self.gp_lik_sigma,
             "optimiser": self._serialise_optimiser(),
         }
-        if is_sum:  # component families and lengthscale shapes, in component order
+        if is_sum:  # component (factor) families and lengthscale shapes, in order
             save_info["gpr_kernel_components"] = [[k.__class__.__name__, k.lengthscales.shape.as_list()] for k in model.kernel.kernels]
         with open(os.path.join(folder, self.GPR_INFO), "w") as handle:
             handle.write(json.dumps(save_info))
@@ -624,9 +624,9 @@ class GPRSurrogate(GPSurrogate):
 
         info = load_json(os.path.join(folder, cls.GPR_INFO))
         assert hasattr(gpmodel.kernels, info["gpr_kernel"])
-        if info["gpr_kernel"] == "Sum":  # multiple_assign restores every component's parameters below
-            gp_kernel = gpmodel.Sum([getattr(gpmodel.kernels, name)(lengthscales=np.ones(shape))
-                                     for name, shape in info["gpr_kernel_components"]])
+        if info["gpr_kernel"] in ("Sum", "Product"):  # multiple_assign restores every component's parameters below
+            gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])([getattr(gpmodel.kernels, name)(lengthscales=np.ones(shape))
+                                                                     for name, shape in info["gpr_kernel_components"]])
         else:
             gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
         assert hasattr(gpmodel.mean_functions, info["gpr_meanf"])

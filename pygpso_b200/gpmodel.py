@@ -19,8 +19,8 @@ implementation in this package.
 Parameterisation follows GPflow 2: positive parameters are softplus-transformed, the Gaussian likelihood variance has
 the 1e-6 floor, and ``trainable_variables`` are ordered kernel.lengthscales, kernel.variance, likelihood.variance,
 mean_function.c (or mean_function.A, mean_function.b for ``Linear``) -- preceded by kernel.alpha for ``RationalQuadratic``
-(tf.Module visits attributes in sorted name order).  A ``Sum`` kernel lists its components' parameters in component order,
-each component's in that same sorted order.
+(tf.Module visits attributes in sorted name order).  A ``Sum`` (``Product``) kernel lists its components' (factors')
+parameters in component order, each component's in that same sorted order.
 """
 import types
 
@@ -121,12 +121,15 @@ class Parameter:
 # ---------------------------------------------------------------------------------------------------------------------
 # kernels / mean functions / likelihood
 # ---------------------------------------------------------------------------------------------------------------------
-MAX_SUM = 4  # GPSO_MAX_SUM: components of a Sum kernel
+MAX_SUM = 4  # GPSO_MAX_SUM: components of a Sum kernel, factors of a Product kernel
 
 
 class Kernel:
     def __add__(self, other):
         return Sum([self, other])
+
+    def __mul__(self, other):
+        return Product([self, other])
 
 
 class Stationary(Kernel):
@@ -164,28 +167,44 @@ class SquaredExponential(Stationary):
 RBF = SquaredExponential
 
 
-class Sum(Kernel):
-    """``gpflow.kernels.Sum``: ``k(x, x') = sum_c k_c(x, x')`` over 1..4 stationary components, each with its own variance,
-    lengthscale(s) and (RationalQuadratic) alpha.  Nested sums are flattened as GPflow's ``Combination`` does, so ``(a + b) + c``
-    and ``a + (b + c)`` are the same three-component sum.  The same kernel object twice would share its parameters in GPflow
-    (tf.Module deduplicates variables); that is refused rather than silently duplicated."""
+class Combination(Kernel):
+    """GPflow's ``Combination``: 1..4 kernels combined in order.  Nested combinations of the same kind are flattened, so
+    ``(a + b) + c`` and ``a + (b + c)`` are the same three-component sum (and likewise for products).  The same kernel object
+    twice would share its parameters in GPflow (tf.Module deduplicates variables); that is refused rather than silently
+    duplicated."""
+
+    _what = "combination"  # the noun of the error messages: "sum" / "product"
 
     def __init__(self, kernels, name=None):
         flat = []
         for k in kernels:
             if not isinstance(k, Kernel):
                 raise TypeError("can only combine Kernel instances")
-            flat.extend(k.kernels if isinstance(k, Sum) else [k])
+            flat.extend(k.kernels if type(k) is type(self) else [k])
         if any(flat[i] is flat[j] for i in range(len(flat)) for j in range(i)):
-            raise ValueError("a kernel object appears twice in the sum: GPflow would share its parameters between the terms, "
-                             "which this model does not support; use two separate kernel objects")
+            raise ValueError(f"a kernel object appears twice in the {self._what}: GPflow would share its parameters between the "
+                             "terms, which this model does not support; use two separate kernel objects")
         if not 1 <= len(flat) <= MAX_SUM:
-            raise ValueError(f"a Sum kernel takes 1..{MAX_SUM} components, got {len(flat)}")
+            raise ValueError(f"a {type(self).__name__} kernel takes 1..{MAX_SUM} components, got {len(flat)}")
         self.kernels = flat
 
     @property
     def parameters(self):
         return tuple(p for k in self.kernels for p in k.parameters)
+
+
+class Sum(Combination):
+    """``gpflow.kernels.Sum``: ``k(x, x') = sum_c k_c(x, x')`` over 1..4 stationary components, each with its own variance,
+    lengthscale(s) and (RationalQuadratic) alpha."""
+
+    _what = "sum"
+
+
+class Product(Combination):
+    """``gpflow.kernels.Product``: ``k(x, x') = prod_c k_c(x, x')`` over 1..4 stationary factors, each with its own variance,
+    lengthscale(s) and (RationalQuadratic) alpha.  The prior variance k(x, x) is the product of the factor variances."""
+
+    _what = "product"
 
 
 class RationalQuadratic(Stationary):
@@ -284,7 +303,10 @@ class GPR(GPModel):
     """
 
     def __init__(self, data, kernel, mean_function=None, noise_variance=1.0, backend=None):
-        parts = kernel.kernels if isinstance(kernel, Sum) else [kernel]
+        parts = kernel.kernels if isinstance(kernel, Combination) else [kernel]
+        if isinstance(kernel, Combination) and any(isinstance(k, Combination) for k in parts):
+            raise TypeError("sums of products and products of sums are not supported: the components of a Sum and the factors "
+                            "of a Product must be Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic")
         if not all(isinstance(k, Stationary) for k in parts):
             raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic, "
                             "or a Sum of them")
@@ -294,9 +316,9 @@ class GPR(GPModel):
             raise TypeError("mean_function must be Zero, Constant or Linear")
         self.likelihood = Gaussian(noise_variance)
         self._backend = backend if backend is not None else _backend.default_backend()
-        if isinstance(kernel, Sum):
+        if isinstance(kernel, Combination):
             self._session = self._backend.open_session(
-                kernel="Sum", n_lengthscales=0, has_mean=_mean_id(self.mean_function),
+                kernel=type(kernel).__name__, n_lengthscales=0, has_mean=_mean_id(self.mean_function),
                 components=[(type(k).__name__, k.lengthscales.size) for k in parts],
             )
         else:
@@ -321,7 +343,7 @@ class GPR(GPModel):
         y = np.ascontiguousarray(y, dtype=np.float64)
         if x.ndim != 2 or y.ndim != 2 or y.shape != (x.shape[0], 1):
             raise ValueError(f"data must be (X[N,d], Y[N,1]); got {x.shape}, {y.shape}")
-        for k in self.kernel.kernels if isinstance(self.kernel, Sum) else [self.kernel]:
+        for k in self.kernel.kernels if isinstance(self.kernel, Combination) else [self.kernel]:
             if k.lengthscales.size not in (1, x.shape[1]):
                 raise ValueError("ARD lengthscales must have one entry per input dimension")
         if isinstance(self.mean_function, Linear) and self.mean_function.A.shape[0] != x.shape[1]:
@@ -493,7 +515,7 @@ def _kernel_leaves(prefix, kernel):
 
 
 def parameter_dict(model):
-    if isinstance(model.kernel, Sum):  # GPflow's leaf paths: .kernel.kernels[i].<name>
+    if isinstance(model.kernel, Combination):  # GPflow's leaf paths: .kernel.kernels[i].<name>
         out = {}
         for i, k in enumerate(model.kernel.kernels):
             out.update(_kernel_leaves(f".kernel.kernels[{i}]", k))
@@ -531,6 +553,7 @@ def tabulate_module_summary(model):
 kernels = types.SimpleNamespace(
     Kernel=Kernel, Stationary=Stationary, Matern12=Matern12, Matern32=Matern32, Matern52=Matern52,
     SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic, Sum=Sum,
+    Product=Product,
 )
 mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant, Linear=Linear)
 likelihoods = types.SimpleNamespace(Gaussian=Gaussian)
