@@ -26,6 +26,9 @@
  *     and the mean entries:
  *         [ c0: (alpha) , lengthscale(s) , variance ; c1: ... ; ... ; likelihood (noise) variance , mean entries ]
  *     GPSO_KERNEL_PRODUCT (gpflow.kernels.Product, k = prod_c k_c) packs its factors the same way.
+ *     GPSO_KERNEL_PERIODIC (gpflow.kernels.Periodic(base, period)) packs its base kernel's block, then the period(s) ('base_kernel'
+ *     < 'period' in tf.Module's sorted names):
+ *         [ (alpha) , lengthscale(s) , kernel variance , period(s) (1, or d when period_ard) , likelihood (noise) variance , mean entries ]
  *     d is the input dimension of gpso_set_data, so the count is known from then on (as for ARD lengthscales).
  *     `u`     = unconstrained (softplus pre-image; noise variance has the 1e-6 floor of gpflow.likelihoods.Gaussian),
  *     `theta` = constrained values.
@@ -62,6 +65,11 @@ enum { GPSO_KERNEL_SUM = 5 };
  * lengthscale(s) and alpha; created with gpso_create_product (gpso_create refuses it).  Factors times the input dimension d
  * may not exceed 64.  The prior variance k(x, x) is var_prod = prod_c variance_c (fp64, factor order). */
 enum { GPSO_KERNEL_PRODUCT = 6 };
+/* GPSO_KERNEL_PERIODIC = gpflow.kernels.Periodic(base_kernel, period) with a GPSO_KERNEL_SE or GPSO_KERNEL_RQ base: k = base.K_r2(r2),
+ * r2 = sum_j sin^2(pi (x_j - x'_j) / p_j) / l_j^2, evaluated as the base kernel on 2 d embedded rows (cos and sin of 2 pi x_j / p_j,
+ * over 2 l_j).  Created with gpso_create_periodic (gpso_create refuses it); the input dimension d may not exceed 32.  The prior
+ * variance k(x, x) is the base variance. */
+enum { GPSO_KERNEL_PERIODIC = 7 };
 /* gpflow.mean_functions.*: None/Zero or Constant (:167, :427), or Linear (m(x) = x . A + b, A[d,1] and b unconstrained) */
 enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1, GPSO_MEAN_LINEAR = 2 };
 
@@ -76,6 +84,17 @@ int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** o
 int gpso_create_sum(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out);
 /* A product kernel of n factors, with the arguments and checks of gpso_create_sum. */
 int gpso_create_product(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out);
+/* A periodic kernel: base_id GPSO_KERNEL_SE or GPSO_KERNEL_RQ, ard = one base lengthscale per dimension, period_ard = one period
+ * per dimension (flags 0 or 1). */
+int gpso_create_periodic(int device, int base_id, int ard, int period_ard, int mean_id, gpso_handle** out);
+/* A sum (kind GPSO_KERNEL_SUM) or product (GPSO_KERNEL_PRODUCT) whose components may be periodic: kernel_ids[c] is one of the five
+ * families, or GPSO_KERNEL_PERIODIC with the base base_ids[c] (GPSO_KERNEL_SE or GPSO_KERNEL_RQ) and the period ARD flag
+ * period_ard[c]; ard[c] is the lengthscale ARD flag (of the base for a periodic component).  A periodic component packs its block
+ * as a bare periodic kernel does ([ (alpha), lengthscale(s), variance, period(s) ]) and counts 2 d rows: the rows of all components
+ * (d each, 2 d for a periodic one) may not exceed 64.  Validated like gpso_create_sum / gpso_create_product, which keep refusing the
+ * periodic id. */
+int gpso_create_combination(int device, int kind, int n, const int* kernel_ids, const int* ard, const int* base_ids,
+                            const int* period_ard, int mean_id, gpso_handle** out);
 int gpso_destroy(gpso_handle* h);
 
 /* model.data = (x, y), gp_surrogate.py:498.  X_host[N,d], y_host[N] are copied to the device. */
@@ -152,7 +171,12 @@ int gpso_grow_ucb_argmax_range(gpso_handle* h, const double* bounds_host, int d,
  * block after L^-1 (and A): [C, then per component: family, lengthscale count, variance, alpha, lengthscales].  A state is
  * only imported into a sum handle with the same component count, families and ARD flags (GPSO_E_BADARG otherwise).
  * GPSO_KERNEL_PRODUCT handles do the same, with var_prod in the header's variance slot and the factor variances in the block;
- * a product state is only imported into a product handle with the same factors, and a sum state into a sum handle. */
+ * a product state is only imported into a product handle with the same factors, and a sum state into a sum handle.
+ * GPSO_KERNEL_PERIODIC handles carry the 2 d embedded rows of the inputs (2 d Np doubles in the place of d Np) and the period(s)
+ * in the header; a periodic state is only imported into a periodic handle with the same base and ARD flags, and a periodic state
+ * never into a handle of its base family or the other way round.  A sum / product with periodic components (gpso_create_combination)
+ * carries each component's rows (2 d embedded rows for a periodic one) and, in the component block, family + 16 for a periodic
+ * component (its base's id) followed after its lengthscales by its period count and period(s). */
 int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes);   /* size for a given problem shape */
 int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t bytes, void* stream);
 int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream);

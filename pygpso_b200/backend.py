@@ -13,6 +13,7 @@ import os
 import numpy as np
 
 KERNEL_IDS = {"Matern12": 0, "Matern32": 1, "Matern52": 2, "SquaredExponential": 3, "RationalQuadratic": 4}
+KERNEL_PERIODIC = 7  # GPSO_KERNEL_PERIODIC
 _LIB_NAME = "libgpso_b200.so"
 _ABI_VERSION = 1
 
@@ -80,6 +81,9 @@ def load_library():
         "gpso_create": (i32, [i32, i32, i32, i32, ctypes.POINTER(H)]),
         "gpso_create_sum": (i32, [i32, i32, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(H)]),
         "gpso_create_product": (i32, [i32, i32, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(H)]),
+        "gpso_create_periodic": (i32, [i32, i32, i32, i32, i32, ctypes.POINTER(H)]),
+        "gpso_create_combination": (i32, [i32, i32, i32, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int),
+                                          ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(H)]),
         "gpso_destroy": (i32, [H]),
         "gpso_set_data": (i32, [H, _c_double_p, _c_double_p, i32, i32]),
         "gpso_neg_lml_grad": (i32, [H, _c_double_p, i32, _c_double_p, _c_double_p]),
@@ -145,7 +149,7 @@ def load_library():
 
 
 EXPORTED_SYMBOLS = (
-    "gpso_version gpso_last_error gpso_device_count gpso_create gpso_create_sum gpso_create_product gpso_destroy gpso_set_data gpso_neg_lml_grad "
+    "gpso_version gpso_last_error gpso_device_count gpso_create gpso_create_sum gpso_create_product gpso_create_periodic gpso_create_combination gpso_destroy gpso_set_data gpso_neg_lml_grad "
     "gpso_factorize gpso_factor_lml gpso_predict_y_host gpso_predict_y_dev gpso_ucb_argmax_host gpso_ucb_argmax_dev "
     "gpso_ucb_topk_host gpso_ucb_topk_dev "
     "gpso_predict_f_cov_host gpso_predict_f_cov_dev gpso_predict_f_samples_host gpso_predict_f_samples_dev "
@@ -186,7 +190,9 @@ class CudaSession:
 
     def __init__(self, lib, device, kernel, n_lengthscales, has_mean, components=None):
         """``components``: for ``kernel="Sum"`` (``"Product"``) the list ``[(family, n_lengthscales), ...]`` of the sum's
-        components (the product's factors)."""
+        components (the product's factors), ``("Periodic", n_lengthscales, base family, n_periods)`` for a periodic one; for
+        ``kernel="Periodic"`` the one entry ``[(base family, n_periods)]``, the base
+        being SquaredExponential or RationalQuadratic with ``n_lengthscales`` lengthscales."""
         self._lib = lib
         self.device = device
         self.kernel = kernel
@@ -195,15 +201,34 @@ class CudaSession:
         self.has_mean = bool(has_mean)
         handle = ctypes.c_void_p()
         if kernel in ("Sum", "Product"):
-            if not components or any(fam not in KERNEL_IDS for fam, _ in components):
-                raise ValueError(f"a {kernel} session needs components from {sorted(KERNEL_IDS)}, got {components!r}")
-            self.components = [(fam, int(nl)) for fam, nl in components]
+            def known(c):
+                return c[0] in KERNEL_IDS or (c[0] == "Periodic" and len(c) == 4 and c[2] in ("SquaredExponential", "RationalQuadratic"))
+            if not components or not all(known(c) for c in components):
+                raise ValueError(f"a {kernel} session needs components from {sorted(KERNEL_IDS)} or periodic ones, got {components!r}")
+            self.components = [tuple(c) for c in components]
             self.ard = False
             n = len(self.components)
-            ids = (ctypes.c_int * n)(*[KERNEL_IDS[fam] for fam, _ in self.components])
-            ards = (ctypes.c_int * n)(*[int(nl > 1) for _, nl in self.components])
-            create = "gpso_create_sum" if kernel == "Sum" else "gpso_create_product"
-            _check(lib, getattr(lib, create)(device, n, ids, ards, self.mean_id, ctypes.byref(handle)), create)
+            periodic = [c[0] == "Periodic" for c in self.components]
+            ids = (ctypes.c_int * n)(*[KERNEL_PERIODIC if p else KERNEL_IDS[c[0]] for c, p in zip(self.components, periodic)])
+            ards = (ctypes.c_int * n)(*[int(c[1] > 1) for c in self.components])
+            if any(periodic):
+                bases = (ctypes.c_int * n)(*[KERNEL_IDS[c[2]] if p else 0 for c, p in zip(self.components, periodic)])
+                pards = (ctypes.c_int * n)(*[int(c[3] > 1) if p else 0 for c, p in zip(self.components, periodic)])
+                kind = 5 if kernel == "Sum" else 6
+                _check(lib, lib.gpso_create_combination(device, kind, n, ids, ards, bases, pards, self.mean_id, ctypes.byref(handle)),
+                       "gpso_create_combination")
+            else:
+                create = "gpso_create_sum" if kernel == "Sum" else "gpso_create_product"
+                _check(lib, getattr(lib, create)(device, n, ids, ards, self.mean_id, ctypes.byref(handle)), create)
+        elif kernel == "Periodic":
+            if not components or len(components) != 1 or components[0][0] not in ("SquaredExponential", "RationalQuadratic"):
+                raise ValueError(f"a Periodic session needs [(base family, n_periods)] with a SquaredExponential or RationalQuadratic "
+                                 f"base, got {components!r}")
+            base, n_periods = components[0]
+            self.components = [(base, int(n_periods))]
+            self.ard = n_lengthscales > 1
+            _check(lib, lib.gpso_create_periodic(device, KERNEL_IDS[base], int(self.ard), int(n_periods > 1), self.mean_id,
+                                                 ctypes.byref(handle)), "gpso_create_periodic")
         else:
             if kernel not in KERNEL_IDS:
                 raise ValueError(f"unsupported kernel {kernel!r}; choose from {sorted(KERNEL_IDS)}, Sum or Product")

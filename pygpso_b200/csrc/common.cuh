@@ -387,6 +387,14 @@ struct SumTable {
     double alpha[MAX_SUM]; // RationalQuadratic shape (read for KERNEL_RQ components only)
 };
 
+// The rows of a sum or product's components, read by the KERNEL_SUM_EMB / KERNEL_PRODUCT_EMB instantiations only (a sum or product
+// with periodic components; appended last to the covariance kernels, a separate argument so that the table above keeps its
+// layout): component c covers the rows [off[c], off[c] + rows[c]) of the scaled inputs and of the width-wide candidate rows
+// (rows[c] = 2d for a periodic component's embedded rows, d otherwise); pmask has bit c set for a periodic component.
+struct SumRows {
+    int off[MAX_SUM], rows[MAX_SUM], width, pmask;
+};
+
 __device__ __forceinline__ double sum_term(const SumTable& t, int c, double r2) {
     const double v = t.var[c], a = t.alpha[c];
     switch (t.fam[c]) {
@@ -403,10 +411,19 @@ __device__ __forceinline__ double sum_term(const SumTable& t, int c, double r2) 
 // (var_prod = prod_c var_c, fp64 in factor order): k = cov(r2_0; var_prod) * prod_{c>=1} cov(r2_c; 1), so k(x, x) is exactly
 // var_prod, small factor variances cannot underflow in fp32, and a one-factor product is its bare kernel's operations.
 constexpr int KERNEL_PRODUCT = 6;
-__host__ __device__ constexpr bool composite_kernel(int kid) { return kid == KERNEL_SUM || kid == KERNEL_PRODUCT; }
+// A sum / product with periodic components (gpflow.kernels.Periodic terms): the covariance kernels' instantiations for it read each
+// component's rows at the table's offsets (the rows of a periodic component are its embedded inputs, at unit lengthscale, and
+// its family is its base's), and the candidates as rows of the table's width.  Internal ids: the C ABI's id 7 is the periodic kernel.
+constexpr int KERNEL_SUM_EMB = 8;
+constexpr int KERNEL_PRODUCT_EMB = 9;
+__host__ __device__ constexpr bool embedded_composite(int kid) { return kid == KERNEL_SUM_EMB || kid == KERNEL_PRODUCT_EMB; }
+__host__ __device__ constexpr bool product_kernel(int kid) { return kid == KERNEL_PRODUCT || kid == KERNEL_PRODUCT_EMB; }
+__host__ __device__ constexpr bool composite_kernel(int kid) {
+    return kid == KERNEL_SUM || kid == KERNEL_PRODUCT || embedded_composite(kid);
+}
 // the running combination of the component values: added for a sum, multiplied for a product
 template <int KID>
-__device__ __forceinline__ double combine(double acc, double t) { return KID == KERNEL_PRODUCT ? acc * t : acc + t; }
+__device__ __forceinline__ double combine(double acc, double t) { return product_kernel(KID) ? acc * t : acc + t; }
 
 template <int W>
 __device__ __forceinline__ void sum_term_v(const SumTable& t, int c, const double (&r2)[W], double (&k)[W]) {

@@ -275,10 +275,24 @@ struct gpso_handle {
     // other kernels) and the ARD flag of each component.  `variance` then holds the prior variance var_tot = sum_c var_c, the fp64
     // sum in component order, and ls_host the lengthscales of every component expanded to d entries ([C][d], as on the device).
     SumTable sum = {};
+    SumRows srow = {};  // the components' rows (sum / product with periodic components)
     int sum_ard[MAX_SUM] = {0};
     // KERNEL_PRODUCT (gpso_create_product) shares that table and ARD flags.  `variance` holds var_prod = prod_c var_c (fp64,
     // factor order), the table's variances are {var_prod, 1, 1, 1}, and prod_var keeps the factor variances themselves.
     double prod_var[MAX_SUM] = {0};
+    // GPSO_KERNEL_PERIODIC (gpso_create_periodic): kernel_id is the base family (SE or RQ), whose covariance kernels run at unit
+    // lengthscale on the 2d embedded rows of kern_cov.cuh's periodic_embed_kernel.  ls_host keeps the base lengthscale(s) as
+    // packed and per_p the period(s); the device buffer ls holds the unit lengthscale, plp the embedding's [l(d), p(d)] (from
+    // plp_host), pX the embedded candidates of a window or of a joint call (row-major [M][2d]).
+    bool periodic = false;
+    int per_ard = 0;
+    double per_p[MAX_LS] = {0}, plp_host[MAX_SUM * 2 * MAX_LS] = {0}, unit_ls = 1.0;
+    // A sum / product with periodic components (gpso_create_combination): sum_per[c] marks component c as periodic (its fam is
+    // the base's) with the period ARD flag sum_per_ard[c] and its period(s) comp_p[c]; the table's off / rows / width give each
+    // component's rows (layout()).  ls then holds the unit lengthscale on a periodic component's rows, plp its [l(d), p(d)].
+    int sum_per[MAX_SUM] = {0}, sum_per_ard[MAX_SUM] = {0};
+    double comp_p[MAX_SUM][MAX_LS] = {{0}};
+    DevBuf plp, pX;
     bool have_data = false, factorized = false;
     double factor_nlml = 0.0;
     double* host_rec = nullptr;  // pinned: results of an evaluation come back in one record without staging copies
@@ -302,14 +316,33 @@ struct gpso_handle {
     bool is_sum() const { return kernel_id == KERNEL_SUM; }
     bool is_product() const { return kernel_id == KERNEL_PRODUCT; }
     bool composite() const { return composite_kernel(kernel_id); }  // a sum or a product: the component table is in force
-    int dx() const { return composite() ? sum.n * d : d; }  // rows of the scaled inputs Xs: [C][d] for a sum or a product
-    int n_ls() const { return composite() ? dx() : (ard ? d : 1); }
+    // rows of the scaled inputs Xs per input dimension: C for a sum or a product, 2 for a periodic kernel
+    bool emb() const { return composite() && srow.pmask != 0; }  // a sum / product with periodic components
+    bool embeds() const { return periodic || emb(); }           // the candidates are embedded before the covariance kernels
+    // the covariance kernels' instantiation: a sum / product with periodic components has its own
+    int cov_kid() const { return emb() ? (is_product() ? KERNEL_PRODUCT_EMB : KERNEL_SUM_EMB) : kernel_id; }
+    // rows of the scaled inputs Xs for input dimension dd: [C][d] for a sum or a product (2d for a periodic component), [2][d]
+    // for a periodic kernel
+    int rows_for(int dd) const {
+        if (!composite()) return periodic ? 2 * dd : dd;
+        int r = 0;
+        for (int c = 0; c < sum.n; c++) r += sum_per[c] ? 2 * dd : dd;
+        return r;
+    }
+    int dx() const { return rows_for(d); }
+    int cand_width() const { return emb() ? dx() : 2 * d; }  // columns of the embedded candidates (pX)
+    int comp_np(int c) const { return sum_per[c] ? (sum_per_ard[c] ? d : 1) : 0; }  // packed periods of component c
+    int kd() const { return periodic ? 2 * d : d; }  // the input dimension the covariance kernels are launched with
+    int n_ls() const { return composite() ? sum.n * d : (ard ? d : 1); }
+    int kern_nls() const { return periodic ? 1 : n_ls(); }  // lengthscales the covariance kernels read from ls
+    int n_per() const { return periodic ? (per_ard ? d : 1) : 0; }  // packed periods
     double comp_var(int c) const { return is_product() ? prod_var[c] : sum.var[c]; }  // component c's own variance
     int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
     int comp_ls(int c) const { return sum_ard[c] ? d : 1; }      // packed lengthscales of sum component c
-    int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + 1; }  // [alpha], lengthscale(s), variance
+    // [alpha], lengthscale(s), variance, [period(s)]
+    int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + 1 + comp_np(c); }
     int n_kernel_params() const {
-        if (!composite()) return n_rq() + n_ls() + 1;
+        if (!composite()) return n_rq() + n_ls() + 1 + n_per();
         int n = 0;
         for (int c = 0; c < sum.n; c++) n += comp_params(c);
         return n;
@@ -378,28 +411,30 @@ struct KernelIds {
         return rc;
     }
 };
-static_assert(GPSO_KERNEL_SUM == KERNEL_SUM && GPSO_KERNEL_PRODUCT == KERNEL_PRODUCT && GPSO_MAX_SUM == MAX_SUM,
+static_assert(GPSO_KERNEL_SUM == KERNEL_SUM && GPSO_KERNEL_PRODUCT == KERNEL_PRODUCT && GPSO_MAX_SUM == MAX_SUM && GPSO_KERNEL_SE == KERNEL_SE &&
+              GPSO_KERNEL_RQ == KERNEL_RQ,
               "sum and product kernel constants of the C ABI");
 using AllKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ>;
 // The covariance kernels also have KERNEL_SUM and KERNEL_PRODUCT instantiations; the gradient of a sum runs the families' own
 // kernel per component, a product's runs lml_grad_product_kernel.
-using CovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM, KERNEL_PRODUCT>;
+using CovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM, KERNEL_PRODUCT,
+                             KERNEL_SUM_EMB, KERNEL_PRODUCT_EMB>;
 
 static void launch_gram(gpso_handle* h, cudaStream_t st) {
     dim3 grid(h->Np / CT, h->Np / CT);
-    CovKernels::with(h->kernel_id, [&](auto kid) {
-        gram_kernel<kid><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->d, h->Np, h->variance, h->noise, h->K.as<double>(),
-                                               h->rq_alpha, h->sum);
+    CovKernels::with(h->cov_kid(), [&](auto kid) {
+        gram_kernel<kid><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->kd(), h->Np, h->variance, h->noise, h->K.as<double>(),
+                                               h->rq_alpha, h->sum, h->srow);
     });
 }
 
 static void launch_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long Mw_pad) {
     size_t sm = (size_t)(XG * h->dx() + 8 * XG) * sizeof(double);
-    CovKernels::with(h->kernel_id, [&](auto kid) {
-        crosscov_kernel<kid><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
+    CovKernels::with(h->cov_kid(), [&](auto kid) {
+        crosscov_kernel<kid><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->kd(), h->ls.as<double>(), h->kern_nls(), h->Xs.as<double>(),
                                                                       h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
                                                                       h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha,
-                                                                      h->sum);
+                                                                      h->sum, h->srow);
     });
 }
 
@@ -439,10 +474,10 @@ static size_t screen_xcov_smem(int d) {
 template <int S>
 static void launch_screen_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long ngroups, float bscale,
                                    uint8_t* B, double* wmean) {
-    CovKernels::with(h->kernel_id, [&](auto kid) {
+    CovKernels::with(h->cov_kid(), [&](auto kid) {
         crosscov_screen_kernel<kid, S, SCR_NT><<<(unsigned)ngroups, 256, screen_xcov_smem(h->dx()), st>>>(
-            Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs32.as<float>(), h->alpha32.as<float>(), h->N, h->Np, (float)h->variance,
-            h->c0, bscale, h->Np / 32, B, wmean, (float)h->rq_alpha, h->sum);
+            Xc, Mw, h->kd(), h->ls.as<double>(), h->kern_nls(), h->Xs32.as<float>(), h->alpha32.as<float>(), h->N, h->Np, (float)h->variance,
+            h->c0, bscale, h->Np / 32, B, wmean, (float)h->rq_alpha, h->sum, h->srow);
     });
 }
 
@@ -481,10 +516,10 @@ static size_t oz_xcov_smem(int d) { return (size_t)(OZ_NT * d + 2 * d * OZ_XK + 
 template <int S>
 static void launch_oz_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long nct, double bscale,
                                uint8_t* B, double* wmean) {
-    CovKernels::with(h->kernel_id, [&](auto kid) {
+    CovKernels::with(h->cov_kid(), [&](auto kid) {
         crosscov_slices_kernel<kid, S><<<(unsigned)nct, 256, oz_xcov_smem(h->dx()), st>>>(
-            Xc, Mw, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(), h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-            bscale, h->Np / 32, B, wmean, h->rq_alpha, h->sum);
+            Xc, Mw, h->kd(), h->ls.as<double>(), h->kern_nls(), h->Xs.as<double>(), h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
+            bscale, h->Np / 32, B, wmean, h->rq_alpha, h->sum, h->srow);
     });
 }
 
@@ -544,6 +579,9 @@ static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride, i
     });
 }
 
+static size_t periodic_grad_smem(int d) { return (size_t)(6 * d * CT + CT * CT) * sizeof(double); }
+static const int PERIODIC_GRAD_SMEM_MAX = (int)periodic_grad_smem(MAX_LS / 2);
+
 // Function attributes (dynamic shared-memory limits, carve-out preferences) belong to the device's primary context: set once per
 // device and process, not per handle (the ~90 cudaFuncSetAttribute calls cost 0.3 s per gpso_create).
 static bool g_configured[64] = {false};
@@ -569,6 +607,12 @@ static int configure_kernels() {
     // up to 64 scaled coordinate rows of the tile's rows and columns, and four ARD factors' pair weights
     CU_TRY(cudaFuncSetAttribute(lml_grad_product_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (2 * MAX_LS * CT + MAX_SUM * CT * CT) * (int)sizeof(double)));
+    // with periodic factors also 2 x 32 raw coordinate rows: 224 KB, within the 227 KB of a block
+    CU_TRY(cudaFuncSetAttribute(lml_grad_product_periodic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (2 * MAX_LS * CT + MAX_LS * CT + MAX_SUM * CT * CT) * (int)sizeof(double)));
+    // a periodic kernel of up to 32 dimensions: 64 embedded and 32 raw coordinate rows of the tile's rows and columns, the pair weights
+    CU_TRY(cudaFuncSetAttribute(lml_grad_periodic_kernel<KERNEL_SE>, cudaFuncAttributeMaxDynamicSharedMemorySize, PERIODIC_GRAD_SMEM_MAX));
+    CU_TRY(cudaFuncSetAttribute(lml_grad_periodic_kernel<KERNEL_RQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, PERIODIC_GRAD_SMEM_MAX));
     GP_TRY(CovKernels::each([](auto kid) -> int {
         CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<kid>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
         CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
@@ -598,8 +642,18 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     size_t mat = (size_t)Np * Np * sizeof(double);
     GP_TRY(h->X.ensure((size_t)N * d * sizeof(double)));
     GP_TRY(h->y.ensure((size_t)Np * sizeof(double)));
-    GP_TRY(h->Xs.ensure((size_t)(h->composite() ? h->sum.n : 1) * d * Np * sizeof(double)));
+    GP_TRY(h->Xs.ensure((size_t)h->rows_for(d) * Np * sizeof(double)));
     GP_TRY(h->ls.ensure(MAX_LS * sizeof(double)));
+    if (h->embeds()) GP_TRY(h->plp.ensure(MAX_SUM * 2 * MAX_LS * sizeof(double)));
+    if (h->composite()) {  // each component's rows: d, or 2d embedded rows for a periodic component
+        int off = 0;
+        for (int c = 0; c < h->sum.n; c++) {
+            h->srow.off[c] = off;
+            h->srow.rows[c] = h->sum_per[c] ? 2 * d : d;
+            off += h->srow.rows[c];
+        }
+        h->srow.width = off;
+    }
     if (h->linear()) GP_TRY(h->meanA.ensure(MAX_LS * sizeof(double)));
     GP_TRY(h->alpha.ensure((size_t)Np * sizeof(double)));
     GP_TRY(h->resid.ensure((size_t)Np * sizeof(double)));
@@ -627,21 +681,60 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     return 0;
 }
 
-// Xs[dim][Np] = X / ls; a sum: Xs_c = X / ls_c at Xs + c d Np, the division of the bare kernel (ls_c expanded to d entries)
+// Xs[dim][Np] = X / ls; a sum: Xs_c = X / ls_c at Xs + c d Np, the division of the bare kernel (ls_c expanded to d entries);
+// a periodic kernel: the embedded rows [cos rows; sin rows] = [2d][Np]
 static int scale_inputs(gpso_handle* h, cudaStream_t st, const double* X, int rows, int Np, double* Xs) {
+    if (h->periodic) {
+        periodic_embed_kernel<<<(unsigned)(((long long)Np * h->d + 255) / 256), 256, 0, st>>>(X, rows, Np, h->d, h->plp.as<double>(), 1,
+                                                                                              Np, Xs);
+        return check_launch(h, "periodic_embed");
+    }
     if (!h->composite()) {
         scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>(), h->n_ls(), rows, h->d, Np, Xs);
         return check_launch(h, "scale_inputs");
     }
     for (int c = 0; c < h->sum.n; c++) {
-        scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>() + (size_t)c * h->d, h->d, rows, h->d, Np,
-                                                              Xs + (size_t)c * h->d * Np);
-        GP_TRY(check_launch(h, "scale_inputs"));
+        double* out = Xs + (size_t)h->srow.off[c] * Np;
+        if (h->sum_per[c]) {
+            periodic_embed_kernel<<<(unsigned)(((long long)Np * h->d + 255) / 256), 256, 0, st>>>(
+                X, rows, Np, h->d, h->plp.as<double>() + (size_t)c * 2 * h->d, 1, Np, out);
+            GP_TRY(check_launch(h, "periodic_embed"));
+        } else {
+            scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>() + h->srow.off[c], h->d, rows, h->d, Np, out);
+            GP_TRY(check_launch(h, "scale_inputs"));
+        }
     }
     return 0;
 }
 
+// a periodic kernel: the unit lengthscale of the base kernel on the embedded rows, and [l, p] (each expanded to d entries) for
+// the embedding
 static int upload_lengthscales(gpso_handle* h, cudaStream_t st) {
+    if (h->periodic) {
+        for (int k = 0; k < h->d; k++) {
+            h->plp_host[k] = h->ls_host[h->ard ? k : 0];
+            h->plp_host[h->d + k] = h->per_p[h->per_ard ? k : 0];
+        }
+        CU_TRY(cudaMemcpyAsync(h->ls.p, &h->unit_ls, sizeof(double), cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(h->plp.p, h->plp_host, sizeof(double) * 2 * h->d, cudaMemcpyHostToDevice, st));
+        return 0;
+    }
+    if (h->emb()) {  // ls: [width], a periodic component's rows at unit lengthscale; plp: [C][l(d), p(d)]
+        double lsw[MAX_LS];
+        const int d = h->d;
+        for (int c = 0; c < h->sum.n; c++) {
+            const int o = h->srow.off[c];
+            for (int r = 0; r < h->srow.rows[c]; r++) lsw[o + r] = h->sum_per[c] ? 1.0 : h->ls_host[c * d + r];
+            for (int k = 0; k < d && h->sum_per[c]; k++) {
+                h->plp_host[c * 2 * d + k] = h->ls_host[c * d + k];
+                h->plp_host[c * 2 * d + d + k] = h->comp_p[c][h->sum_per_ard[c] ? k : 0];
+            }
+        }
+        CU_TRY(cudaMemcpyAsync(h->ls.p, lsw, sizeof(double) * h->dx(), cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(h->plp.p, h->plp_host, sizeof(double) * h->sum.n * 2 * d, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaStreamSynchronize(st));  // lsw is on this stack frame
+        return 0;
+    }
     CU_TRY(cudaMemcpyAsync(h->ls.p, h->ls_host, sizeof(double) * h->n_ls(), cudaMemcpyHostToDevice, st));
     return 0;
 }
@@ -1481,7 +1574,8 @@ static int init_handle(gpso_handle* h, int device, int kernel_id, int ard, int m
 
 extern "C" int gpso_destroy(gpso_handle* h);
 
-static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out);
+static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out,
+                         int pmask = 0);
 
 extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso_handle** out) {
     if (!out) return fail(GPSO_E_BADARG, "gpso_create: out is null");
@@ -1492,9 +1586,11 @@ extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso
     return create_handle(device, kernel_id, ard, mean_id, SumTable{}, nullptr, out);
 }
 
-// The arguments of gpso_create_sum and gpso_create_product: n components (1..MAX_SUM) of the five families, ARD flags 0 / 1.
+// The arguments of gpso_create_sum, gpso_create_product and gpso_create_combination: n components (1..MAX_SUM) of the five
+// families, ARD flags 0 / 1; with base_ids (gpso_create_combination only) a component of id GPSO_KERNEL_PERIODIC is periodic with
+// the base base_ids[c] (SE or RQ) and the period ARD flag period_ard[c].
 static int component_table(const char* who, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out,
-                           SumTable& tab) {
+                           SumTable& tab, const int* base_ids = nullptr, const int* period_ard = nullptr, int* pmask = nullptr) {
     const std::string w(who);
     if (!out) return fail(GPSO_E_BADARG, w + ": out is null");
     *out = nullptr;
@@ -1503,13 +1599,20 @@ static int component_table(const char* who, int n, const int* kernel_ids, const 
     if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, w + ": unknown mean id");
     tab = {};
     tab.n = n;
+    int pm = 0;
     for (int c = 0; c < n; c++) {
-        if (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ) return fail(GPSO_E_BADARG, w + ": unknown component kernel id");
-        if (ard[c] != 0 && ard[c] != 1) return fail(GPSO_E_BADARG, w + ": ard flags must be 0 or 1");
-        tab.fam[c] = kernel_ids[c];
+        const bool per = base_ids && kernel_ids[c] == GPSO_KERNEL_PERIODIC;
+        if (!per && (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ)) return fail(GPSO_E_BADARG, w + ": unknown component kernel id");
+        if (per && base_ids[c] != KERNEL_SE && base_ids[c] != KERNEL_RQ)
+            return fail(GPSO_E_BADARG, w + ": a periodic component's base must be SquaredExponential or RationalQuadratic");
+        if ((ard[c] != 0 && ard[c] != 1) || (per && period_ard[c] != 0 && period_ard[c] != 1))
+            return fail(GPSO_E_BADARG, w + ": ard flags must be 0 or 1");
+        tab.fam[c] = per ? base_ids[c] : kernel_ids[c];
+        pm |= per ? 1 << c : 0;
         tab.var[c] = 1.0;
         tab.alpha[c] = 1.0;
     }
+    if (pmask) *pmask = pm;
     return 0;
 }
 
@@ -1519,13 +1622,46 @@ extern "C" int gpso_create_sum(int device, int n, const int* kernel_ids, const i
     return create_handle(device, KERNEL_SUM, 0, mean_id, sum, ard, out);
 }
 
+extern "C" int gpso_create_combination(int device, int kind, int n, const int* kernel_ids, const int* ard, const int* base_ids,
+                                       const int* period_ard, int mean_id, gpso_handle** out) {
+    if (kind != KERNEL_SUM && kind != KERNEL_PRODUCT) {
+        if (out) *out = nullptr;
+        return fail(GPSO_E_BADARG, "gpso_create_combination: kind must be GPSO_KERNEL_SUM or GPSO_KERNEL_PRODUCT");
+    }
+    if (!base_ids || !period_ard) {
+        if (out) *out = nullptr;
+        return fail(GPSO_E_BADARG, "gpso_create_combination: null argument");
+    }
+    SumTable tab;
+    int pmask = 0;
+    GP_TRY(component_table("gpso_create_combination", n, kernel_ids, ard, mean_id, out, tab, base_ids, period_ard, &pmask));
+    GP_TRY(create_handle(device, kind, 0, mean_id, tab, ard, out, pmask));
+    for (int c = 0; c < n; c++) (*out)->sum_per_ard[c] = (pmask >> c & 1) ? period_ard[c] : 0;
+    return 0;
+}
+
 extern "C" int gpso_create_product(int device, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out) {
     SumTable tab;
     GP_TRY(component_table("gpso_create_product", n, kernel_ids, ard, mean_id, out, tab));
     return create_handle(device, KERNEL_PRODUCT, 0, mean_id, tab, ard, out);
 }
 
-static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out) {
+extern "C" int gpso_create_periodic(int device, int base_id, int ard, int period_ard, int mean_id, gpso_handle** out) {
+    if (!out) return fail(GPSO_E_BADARG, "gpso_create_periodic: out is null");
+    *out = nullptr;
+    if (base_id != KERNEL_SE && base_id != KERNEL_RQ)
+        return fail(GPSO_E_BADARG, "gpso_create_periodic: the base kernel must be SquaredExponential or RationalQuadratic");
+    if ((ard != 0 && ard != 1) || (period_ard != 0 && period_ard != 1))
+        return fail(GPSO_E_BADARG, "gpso_create_periodic: ard flags must be 0 or 1");
+    if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create_periodic: unknown mean id");
+    GP_TRY(create_handle(device, base_id, ard, mean_id, SumTable{}, nullptr, out));
+    (*out)->periodic = true;
+    (*out)->per_ard = period_ard;
+    return 0;
+}
+
+static int create_handle(int device, int kernel_id, int ard, int mean_id, const SumTable& sum, const int* sum_ard, gpso_handle** out,
+                         int pmask) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) return fail(GPSO_E_NOGPU, "gpso_create: no CUDA device available");
     if (device < 0 || device >= n) return fail(GPSO_E_BADARG, "gpso_create: device index out of range");
@@ -1540,8 +1676,10 @@ static int create_handle(int device, int kernel_id, int ard, int mean_id, const 
     CU_TRY(cudaSetDevice(device));
     gpso_handle* h = new gpso_handle();
     h->sum = sum;
+    h->srow.pmask = pmask;
     for (int c = 0; c < sum.n; c++) {
         h->sum_ard[c] = sum_ard[c];
+        h->sum_per[c] = pmask >> c & 1;
         h->prod_var[c] = sum.var[c];
     }
     int rc = init_handle(h, device, kernel_id, ard, mean_id, prop);
@@ -1591,6 +1729,10 @@ extern "C" int gpso_set_data(gpso_handle* h, const double* X_host, const double*
     if (h->composite() && h->sum.n * d > MAX_LS)
         return fail(GPSO_E_BADARG, h->is_sum() ? "gpso_set_data: a sum kernel supports components x input dimension up to 64"
                                                : "gpso_set_data: a product kernel supports factors x input dimension up to 64");
+    if (h->periodic && 2 * d > MAX_LS)
+        return fail(GPSO_E_BADARG, "gpso_set_data: a periodic kernel embeds each input dimension in 2 rows: input dimension up to 32");
+    if (h->emb() && h->rows_for(d) > MAX_LS)
+        return fail(GPSO_E_BADARG, "gpso_set_data: the rows of all components (d each, 2d for a periodic component) may not exceed 64");
     GP_TRY(set_device(h));
     CU_TRY(cudaStreamSynchronize(h->stream));
     GP_TRY(ensure_shape(h, N, d));
@@ -1640,7 +1782,11 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
                 h->sum.var[c] = theta[nl];
                 var_tot = (c == 0) ? theta[nl] : var_tot + theta[nl];
             }
-            theta += nl + 1;
+            for (int i = 0; i < h->comp_np(c); i++) {  // a periodic component's period(s) follow its variance
+                if (!positive(theta[nl + 1 + i])) return fail(GPSO_E_BADARG, std::string(who) + ": period must be positive");
+                h->comp_p[c][i] = theta[nl + 1 + i];
+            }
+            theta += nl + 1 + h->comp_np(c);
         }
         h->variance = var_tot;
         if (h->is_product())  // the table: var_prod on the first factor, unit variance on the others
@@ -1663,10 +1809,15 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
         h->ls_host[i] = theta[i];
     }
     h->variance = theta[nl];
-    h->noise = theta[nl + 1];
+    const int np = h->n_per();  // a periodic kernel's period(s) follow the variance ('base_kernel' < 'period')
+    for (int i = 0; i < np; i++) {
+        if (!positive(theta[nl + 1 + i])) return fail(GPSO_E_BADARG, std::string(who) + ": period must be positive");
+        h->per_p[i] = theta[nl + 1 + i];
+    }
+    h->noise = theta[nl + 1 + np];
     if (!(h->variance > 0.0 || (allow_zero && h->variance == 0.0)) || !(h->noise > 0.0))
         return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
-    load_mean(h, theta + nl + 2);
+    load_mean(h, theta + nl + 2 + np);
     return 0;
 }
 
@@ -1690,10 +1841,11 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
     const int nb64 = h->Np / CT;
     const int nblk = nb64 * (nb64 + 1) / 2;
     // where component c's entries sit in the reduced partial sums: its variance entry (s_K), lengthscales and alpha
+    // a periodic component's entries are per dimension for its lengthscales and its periods: 2d entries before its alpha
     int ik[MAX_SUM], il[MAX_SUM], ia[MAX_SUM], stride[MAX_SUM], off[MAX_SUM + 1] = {0};
     if (h->is_product()) off[0] = 2;
     for (int c = 0; c < h->sum.n; c++) {
-        const int nls = h->comp_ls(c), rq = h->sum.fam[c] == KERNEL_RQ;
+        const int nls = h->sum_per[c] ? 2 * h->d : h->comp_ls(c), rq = h->sum.fam[c] == KERNEL_RQ;
         stride[c] = (h->is_product() ? 0 : 2) + nls + rq;
         ik[c] = h->is_product() ? 0 : off[c];
         il[c] = h->is_product() ? off[c] : off[c] + 2;
@@ -1705,22 +1857,37 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
     GP_TRY(h->gpart.ensure((size_t)nblk * total * sizeof(double)));
     GP_TRY(h->gout.ensure((size_t)(total + 4 + nA) * sizeof(double)));
     if (h->is_product()) {
-        int ard_mask = 0, nard = 0;
+        int ard_mask = 0, nard = 0;  // a periodic factor always takes a weight slot
         for (int c = 0; c < h->sum.n; c++) {
-            ard_mask |= h->sum_ard[c] << c;
-            nard += h->sum_ard[c];
+            const int slot = h->sum_ard[c] | h->sum_per[c];
+            ard_mask |= slot << c;
+            nard += slot;
         }
-        const size_t smem = ((size_t)2 * h->dx() * CT + (size_t)nard * CT * CT) * sizeof(double);
-        lml_grad_product_kernel<<<nblk, 256, smem, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N, h->d,
-                                                         h->Np, ard_mask, h->gpart.as<double>(), total, h->sum);
+        const size_t smem = ((size_t)2 * h->dx() * CT + (h->emb() ? (size_t)2 * h->d * CT : 0) + (size_t)nard * CT * CT) * sizeof(double);
+        if (h->emb())
+            lml_grad_product_periodic_kernel<<<nblk, 256, smem, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(),
+                                                                      h->N, h->d, h->Np, ard_mask, h->gpart.as<double>(), total,
+                                                                      h->sum, h->X.as<double>(), h->srow);
+        else
+            lml_grad_product_kernel<<<nblk, 256, smem, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
+                                                             h->d, h->Np, ard_mask, h->gpart.as<double>(), total, h->sum);
         GP_TRY(check_launch(h, "lml_grad_product"));
         reduce_partials_kernel<<<total, 256, 0, st>>>(h->gpart.as<double>(), nblk, total, h->gout.as<double>());
         GP_TRY(check_launch(h, "reduce_partials"));
     } else {
         for (int c = 0; c < h->sum.n; c++) {
             double* part = h->gpart.as<double>() + (size_t)nblk * off[c];
-            launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], h->Xs.as<double>() + (size_t)c * h->d * h->Np,
-                        h->sum.var[c], h->sum.alpha[c], part);
+            const double* Xs_c = h->Xs.as<double>() + (size_t)h->srow.off[c] * h->Np;
+            if (h->sum_per[c]) {
+                KernelIds<KERNEL_SE, KERNEL_RQ>::with(h->sum.fam[c], [&](auto kid) {
+                    lml_grad_periodic_kernel<kid><<<nblk, 256, periodic_grad_smem(h->d), st>>>(
+                        Xs_c, h->X.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N, h->d, h->Np, h->sum.var[c],
+                        h->sum.alpha[c], part, stride[c]);
+                });
+                h->launches++;
+            } else {
+                launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], Xs_c, h->sum.var[c], h->sum.alpha[c], part);
+            }
             if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
             reduce_partials_kernel<<<stride[c], 256, 0, st>>>(part, nblk, stride[c], h->gout.as<double>() + off[c]);
             GP_TRY(check_launch(h, "reduce_partials"));
@@ -1752,12 +1919,26 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
             grad_host[pos] = h->sum.alpha[c] > 0.0 ? -(0.5 * g[ia[c]]) * sigmoid(u[pos]) : 0.0;
             pos++;
         }
-        const int nl = h->comp_ls(c);
-        for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[il[c] + i] / h->ls_host[c * h->d + i]) * sigmoid(u[pos + i]);
+        const int nl = h->comp_ls(c), np = h->comp_np(c), d = h->d;
+        if (h->sum_per[c]) {  // per-dimension entries L(d), Q(d) as for a bare periodic kernel (gpso_neg_lml_grad)
+            const double* L = g + il[c];
+            const double* Q = g + il[c] + d;
+            double Ls = 0.0, Qs = 0.0;
+            for (int k = 0; k < d; k++) {
+                Ls += L[k];
+                Qs += Q[k];
+            }
+            for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * (nl > 1 ? L[i] : Ls) / h->ls_host[c * d + i]) * sigmoid(u[pos + i]);
+            for (int i = 0; i < np; i++)
+                grad_host[pos + nl + 1 + i] =
+                    -(M_PI * (np > 1 ? Q[i] : Qs) / (h->comp_p[c][i] * h->comp_p[c][i])) * sigmoid(u[pos + nl + 1 + i]);
+        } else {
+            for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[il[c] + i] / h->ls_host[c * d + i]) * sigmoid(u[pos + i]);
+        }
         pos += nl;
         const double var_c = h->comp_var(c);
         grad_host[pos] = var_c > 0.0 ? -(0.5 * g[ik[c]] / var_c) * sigmoid(u[pos]) : 0.0;
-        pos++;
+        pos += 1 + np;
     }
     grad_host[pos] = -(0.5 * g[1]) * sigmoid(u[pos]);  // sum_i W_ii, taken from the first component's block
     if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[pos + 1] = -sc[2];
@@ -1774,15 +1955,16 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     if (p != h->n_params()) return fail(GPSO_E_BADARG, "gpso_neg_lml_grad: wrong number of hyper-parameters");
     GP_TRY(set_device(h));
     if (h->composite()) return neg_lml_grad_composite(h, u, p, f_host, grad_host);
-    const int nl = h->n_ls(), na = h->n_rq();
+    const int nl = h->n_ls(), na = h->n_rq(), np = h->n_per();
     std::vector<double> theta(p);
     for (int i = 0; i < na; i++) theta[i] = softplus(u[i]);  // alpha: positive, no floor
     grad_host += na;  // the shared layout after alpha
     u += na;
     for (int i = 0; i < nl; i++) theta[na + i] = softplus(u[i]);
     theta[na + nl] = softplus(u[nl]);
-    theta[na + nl + 1] = NOISE_FLOOR + softplus(u[nl + 1]);
-    for (int i = 0; i < h->n_mean(); i++) theta[na + nl + 2 + i] = u[nl + 2 + i];  // unconstrained
+    for (int i = 0; i < np; i++) theta[na + nl + 1 + i] = softplus(u[nl + 1 + i]);  // period(s): positive, no floor
+    theta[na + nl + 1 + np] = NOISE_FLOOR + softplus(u[nl + 1 + np]);
+    for (int i = 0; i < h->n_mean(); i++) theta[na + nl + 2 + np + i] = u[nl + 2 + np + i];  // unconstrained
     // softplus(u) underflows to exactly 0 for u < -745 and L-BFGS-B line searches do probe such points: like GPflow, evaluate
     // them (kernel variance 0 -> K_y = noise * I; lengthscale 0 -> NaN objective) instead of rejecting the call
     GP_TRY(load_theta(h, theta.data(), p, "gpso_neg_lml_grad", true));
@@ -1792,12 +1974,22 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     GP_TRY(factor_pipeline(h, st, true));
     const int nb64 = h->Np / CT;
     const int nblk = nb64 * (nb64 + 1) / 2;
-    const int stride = 2 + nl + na;
+    // a periodic kernel's partial sums are per dimension for the lengthscales and the periods alike: [s_K, tr, L(d), Q(d), (alpha)]
+    const int stride = 2 + (h->periodic ? 2 * h->d : nl) + na;
     const int nA = h->linear() ? h->d : 0;  // X^T alpha follows the reduced partial sums in gout
     GP_TRY(h->gpart.ensure((size_t)nblk * stride * sizeof(double)));
     GP_TRY(h->gout.ensure((size_t)(stride + 4 + nA) * sizeof(double)));
-    launch_grad(h, st, nblk, stride, h->kernel_id, h->ard, h->Xs.as<double>(), h->variance, h->rq_alpha, h->gpart.as<double>());
-    if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
+    if (h->periodic) {
+        KernelIds<KERNEL_SE, KERNEL_RQ>::with(h->kernel_id, [&](auto kid) {
+            lml_grad_periodic_kernel<kid><<<nblk, 256, periodic_grad_smem(h->d), st>>>(
+                h->Xs.as<double>(), h->X.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N, h->d, h->Np, h->variance,
+                h->rq_alpha, h->gpart.as<double>(), stride);
+        });
+        GP_TRY(check_launch(h, "lml_grad_periodic"));
+    } else {
+        launch_grad(h, st, nblk, stride, h->kernel_id, h->ard, h->Xs.as<double>(), h->variance, h->rq_alpha, h->gpart.as<double>());
+        if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
+    }
     reduce_partials_kernel<<<stride, 256, 0, st>>>(h->gpart.as<double>(), nblk, stride, h->gout.as<double>());
     GP_TRY(check_launch(h, "reduce_partials"));
     if (nA) {
@@ -1822,14 +2014,29 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
     GP_TRY(pivot_status(info, "Gram matrix"));
     *f_host = nlml_from_scalars(h, sc);
     // dLML/dtheta = 0.5 * sum W * dK/dtheta ; chain through softplus: dtheta/du = sigmoid(u)
-    for (int i = 0; i < nl; i++) grad_host[i] = -(0.5 * g[2 + i] / h->ls_host[i]) * sigmoid(u[i]);
+    if (h->periodic) {
+        // dK/dl_j = g r2_j / l_j and dK/dp_j = 2 pi g delta_j sin(2 pi delta_j / p_j) / (4 l_j^2) / p_j^2: dLML/dl_j = 0.5 L_j / l_j,
+        // dLML/dp_j = pi Q_j / p_j^2; a scalar lengthscale or period takes the sum over the dimensions
+        const double* L = g + 2;
+        const double* Q = g + 2 + h->d;
+        double Ls = 0.0, Qs = 0.0;
+        for (int k = 0; k < h->d; k++) {
+            Ls += L[k];
+            Qs += Q[k];
+        }
+        for (int i = 0; i < nl; i++) grad_host[i] = -(0.5 * (nl > 1 ? L[i] : Ls) / h->ls_host[i]) * sigmoid(u[i]);
+        for (int i = 0; i < np; i++)
+            grad_host[nl + 1 + i] = -(M_PI * (np > 1 ? Q[i] : Qs) / (h->per_p[i] * h->per_p[i])) * sigmoid(u[nl + 1 + i]);
+    } else {
+        for (int i = 0; i < nl; i++) grad_host[i] = -(0.5 * g[2 + i] / h->ls_host[i]) * sigmoid(u[i]);
+    }
     // variance == 0 only when softplus underflowed, where the chain factor sigmoid(u) is 0 too: the entry is 0, not 0/0
     grad_host[nl] = h->variance > 0.0 ? -(0.5 * g[0] / h->variance) * sigmoid(u[nl]) : 0.0;
-    grad_host[nl + 1] = -(0.5 * g[1]) * sigmoid(u[nl + 1]);
-    if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[nl + 2] = -sc[2];
+    grad_host[nl + 1 + np] = -(0.5 * g[1]) * sigmoid(u[nl + 1 + np]);
+    if (h->mean_id == GPSO_MEAN_CONSTANT) grad_host[nl + 2 + np] = -sc[2];
     if (nA) {  // d(-LML)/dA = -X^T alpha, d(-LML)/db = -sum(alpha)
-        for (int k = 0; k < nA; k++) grad_host[nl + 2 + k] = -g[stride + k];
-        grad_host[nl + 2 + nA] = -sc[2];
+        for (int k = 0; k < nA; k++) grad_host[nl + 2 + np + k] = -g[stride + k];
+        grad_host[nl + 2 + np + nA] = -sc[2];
     }
     // alpha (slot stride - 1 of the partial sums); alpha == 0 only when softplus underflowed: the entry is 0, as for the variance
     if (na) grad_host[-1] = h->rq_alpha > 0.0 ? -(0.5 * g[stride - 1]) * sigmoid(u[-1]) : 0.0;
@@ -1959,6 +2166,23 @@ struct WindowSpan {
     long long off, n;  // first candidate, candidates
 };
 
+// A periodic kernel: the embedded rows of M candidates, row-major [M][2d] in pX (the layout the cross-covariance kernels stage).
+// A sum / product with periodic components: rows of cand_width() columns, each component's at its offset -- the embedded rows of a
+// periodic component, the raw coordinates of the others.
+static int embed_candidates(gpso_handle* h, cudaStream_t st, const double* Xc, long long M) {
+    const unsigned grid = (unsigned)((M * h->d + 255) / 256);
+    if (h->periodic) {
+        periodic_embed_kernel<<<grid, 256, 0, st>>>(Xc, M, M, h->d, h->plp.as<double>(), 2 * h->d, 1, h->pX.as<double>());
+        return check_launch(h, "periodic_embed");
+    }
+    for (int c = 0; c < h->sum.n; c++) {
+        const double* lp = h->sum_per[c] ? h->plp.as<double>() + (size_t)c * 2 * h->d : nullptr;
+        periodic_embed_kernel<<<grid, 256, 0, st>>>(Xc, M, M, h->d, lp, h->cand_width(), 1, h->pX.as<double>() + h->srow.off[c]);
+        GP_TRY(check_launch(h, "periodic_embed"));
+    }
+    return 0;
+}
+
 static std::vector<WindowSpan> uniform_windows(long long M, long long W) {
     std::vector<WindowSpan> wins;
     for (long long off = 0; off < M; off += W) wins.push_back({off, std::min(W, M - off)});
@@ -1969,6 +2193,7 @@ struct Window {
     long long w, off, Mw;
     const double* src;  // the window's candidates on the device
     int b;              // digit-tile / mean buffer (0 without overlap)
+    const double* xk;   // what the covariance kernels read: src, or a periodic kernel's embedded candidates
 };
 
 // The work of one window.  xcov runs on the stream it is given, everything else on the product stream.  A pass without a
@@ -1989,6 +2214,8 @@ static int window_pipeline(gpso_handle* h, cudaStream_t st, const double* Xc_dev
         GP_TRY(h->cand[0].ensure((size_t)W * d * sizeof(double)));
         GP_TRY(h->cand[1].ensure((size_t)W * d * sizeof(double)));
     }
+    // one buffer: the embedding of window w + 1 follows the cross-covariance of window w on the same stream
+    if (h->embeds()) GP_TRY(h->pX.ensure((size_t)W * h->cand_width() * sizeof(double)));
     cudaStream_t user_st = st;
     cudaStream_t xs = overlap ? h->aux_stream : st;  // stream of the cross-covariance kernels
     cudaStream_t cs = h->copy_stream;
@@ -2005,7 +2232,7 @@ static int window_pipeline(gpso_handle* h, cudaStream_t st, const double* Xc_dev
     long long w = 0;
     for (bool stop = false; w < (long long)wins.size() && !stop; w++) {
         const int cb = (int)(w & 1);  // candidate staging buffer
-        Window win = {w, wins[(size_t)w].off, wins[(size_t)w].n, nullptr, overlap ? cb : 0};
+        Window win = {w, wins[(size_t)w].off, wins[(size_t)w].n, nullptr, overlap ? cb : 0, nullptr};
         h->last_windows++;
         // ---- 1. candidates of this window on the device
         if (host) {
@@ -2021,6 +2248,11 @@ static int window_pipeline(gpso_handle* h, cudaStream_t st, const double* Xc_dev
         if (overlap && buf_busy[win.b]) CU_TRY(cudaStreamWaitEvent(xs, h->ev_free[win.b], 0));  // window w-2 has released buffer b
         GP_TRY(prof_mark(h, xs));
         GP_TRY(trace_mark(h, xs, 1, w));
+        win.xk = win.src;
+        if (h->embeds()) {
+            GP_TRY(embed_candidates(h, xs, win.src, win.Mw));
+            win.xk = h->pX.as<double>();
+        }
         GP_TRY(body.xcov(win, xs));
         GP_TRY(trace_mark(h, xs, 2, w));
         if (host) {
@@ -2105,11 +2337,11 @@ static int full_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, cons
     WindowStages body;
     body.xcov = [&](const Window& win, cudaStream_t xs) {
         if (oz) {
-            DISPATCH_S(S, launch_oz_crosscov, h, xs, win.src, win.Mw, pad(win.Mw) / OZ_NT, bscale, h->ozBb[win.b].as<uint8_t>(),
+            DISPATCH_S(S, launch_oz_crosscov, h, xs, win.xk, win.Mw, pad(win.Mw) / OZ_NT, bscale, h->ozBb[win.b].as<uint8_t>(),
                        h->wmeanb[win.b].as<double>());
             GP_TRY(check_launch(h, "crosscov_slices"));
         } else {
-            launch_crosscov(h, xs, win.src, win.Mw, pad(win.Mw));
+            launch_crosscov(h, xs, win.xk, win.Mw, pad(win.Mw));
             GP_TRY(check_launch(h, "crosscov"));
         }
         return add_linear_offset(h, xs, win.src, win.Mw, 1.0, h->wmeanb[win.b].as<double>());
@@ -2282,6 +2514,11 @@ static bool screen_applicable(const gpso_handle* h, long long M) {
         if (h->sum.fam[c] == KERNEL_RQ && !(h->sum.alpha[c] > 1e-30 && h->sum.alpha[c] < 1e30)) return false;
     for (int i = 0; i < h->n_ls(); i++)
         if (!(h->ls_host[i] > 1e-30 && h->ls_host[i] < 1e30)) return false;
+    for (int i = 0; i < h->n_per(); i++)
+        if (!(h->per_p[i] > 1e-30 && h->per_p[i] < 1e30)) return false;
+    for (int c = 0; c < h->sum.n; c++)
+        for (int i = 0; i < h->comp_np(c); i++)
+            if (!(h->comp_p[c][i] > 1e-30 && h->comp_p[c][i] < 1e30)) return false;
     return true;
 }
 
@@ -2363,7 +2600,7 @@ static int screen_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, co
     auto pad = [](long long Mw) { return ((Mw + SCR_NT - 1) / SCR_NT) * SCR_NT; };
     WindowStages body;
     body.xcov = [&](const Window& win, cudaStream_t xs) {
-        DISPATCH_SCREEN_S(S, launch_screen_crosscov, h, xs, win.src, win.Mw, pad(win.Mw) / 64, bscale, h->ozBb[win.b].as<uint8_t>(),
+        DISPATCH_SCREEN_S(S, launch_screen_crosscov, h, xs, win.xk, win.Mw, pad(win.Mw) / 64, bscale, h->ozBb[win.b].as<uint8_t>(),
                           h->wmeanb[win.b].as<double>());
         GP_TRY(check_launch(h, "crosscov_screen"));
         return add_linear_offset(h, xs, win.src, win.Mw, 1.0, h->wmeanb[win.b].as<double>());  // the refine pass adds the same
@@ -2434,7 +2671,7 @@ static int bound_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, con
     CU_TRY(cudaMemsetAsync(h->scr_state.p, 0, 4 * sizeof(unsigned long long), st));
     WindowStages body;
     body.xcov = [&](const Window& win, cudaStream_t xs) {
-        launch_screen_crosscov<0>(h, xs, win.src, win.Mw, ((win.Mw + SCR_NT - 1) / SCR_NT) * SCR_NT / 64, 0.0f, nullptr,
+        launch_screen_crosscov<0>(h, xs, win.xk, win.Mw, ((win.Mw + SCR_NT - 1) / SCR_NT) * SCR_NT / 64, 0.0f, nullptr,
                                   h->wmeanb[0].as<double>());
         GP_TRY(check_launch(h, "crosscov_mean"));
         return add_linear_offset(h, xs, win.src, win.Mw, 1.0, h->wmeanb[0].as<double>());
@@ -2718,19 +2955,19 @@ static int joint_ready(gpso_handle* h, const char* who) {
 
 static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, int M, int Mp) {
     size_t sm = (size_t)(XG * h->dx() + 8 * XG) * sizeof(double);
-    CovKernels::with(h->kernel_id, [&](auto kid) {
-        crosscov_kernel<kid><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->d, h->ls.as<double>(), h->n_ls(), h->Xs.as<double>(),
+    CovKernels::with(h->cov_kid(), [&](auto kid) {
+        crosscov_kernel<kid><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->kd(), h->ls.as<double>(), h->kern_nls(), h->Xs.as<double>(),
                                                                   h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
-                                                                  h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha, h->sum);
+                                                                  h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha, h->sum, h->srow);
     });
 }
 
 static void launch_joint_syrk(gpso_handle* h, cudaStream_t st, int M, int Mp, double jitter) {
     const int mb = Mp / TB;
-    CovKernels::with(h->kernel_id, [&](auto kid) {
+    CovKernels::with(h->cov_kid(), [&](auto kid) {
         joint_syrk_kernel<kid><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp,
-                                                                                   h->Np, h->d, h->variance, jitter,
-                                                                                   h->jSigma.as<double>(), h->rq_alpha, h->sum);
+                                                                                   h->Np, h->kd(), h->variance, jitter,
+                                                                                   h->jSigma.as<double>(), h->rq_alpha, h->sum, h->srow);
     });
 }
 
@@ -2744,7 +2981,13 @@ static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M,
     GP_TRY(h->jSigma.ensure((size_t)Mp * Mp * sizeof(double)));
     GP_TRY(h->jcounter.ensure(sizeof(int)));
     GP_TRY(scale_inputs(h, st, Xc, M, Mp, h->jXcs.as<double>()));
-    launch_joint_crosscov(h, st, Xc, M, Mp);
+    const double* xk = Xc;
+    if (h->embeds()) {
+        GP_TRY(h->pX.ensure((size_t)M * h->cand_width() * sizeof(double)));
+        GP_TRY(embed_candidates(h, st, Xc, M));
+        xk = h->pX.as<double>();
+    }
+    launch_joint_crosscov(h, st, xk, M, Mp);
     GP_TRY(check_launch(h, "crosscov"));
     GP_TRY(add_linear_offset(h, st, Xc, M, 1.0, h->jmean.as<double>()));
     JointVParams P;
@@ -2969,21 +3212,32 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 // A sum kernel: slot 2 is the prior variance var_tot, Xs holds the C scaled copies (C*d*Np), the header's lengthscales are the
 // components' expanded to d entries each, and the component block is [C, then per component: family, lengthscale count,
 // variance, alpha, lengthscales].  A product kernel: the same, with slot 2 the prior variance var_prod and the factor variances
-// in the component block.
+// in the component block.  A periodic kernel: the kernel id is its base family's, slot 10 is 1 and slot 11 the period's ARD
+// flag, Xs holds the 2d embedded rows (2*d*Np) and the period(s) follow the lengthscale slots (STATE_PERIODS).
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int STATE_HEADER = 128;
+constexpr int STATE_PERIODS = 16 + MAX_LS;  // a periodic kernel's period(s); slot 10 = 1 marks it, slot 11 = the period's ARD flag
+
+// the family entry of a component in the state's component block: its family id, + 16 for a periodic component (its base's id)
+static int comp_code(const gpso_handle* h, int c) { return h->sum.fam[c] + (h->sum_per[c] ? 16 : 0); }
+// the block entries of component c: family, lengthscale count, variance, alpha, lengthscales, [period count, periods]
+static int comp_block(const gpso_handle* h, int c, int d) {
+    return 4 + (h->sum_ard[c] ? d : 1) + (h->sum_per[c] ? 1 + (h->sum_per_ard[c] ? d : 1) : 0);
+}
 
 static long long sum_block_size(const gpso_handle* h, int d) {
     if (!h->composite()) return 0;
     long long n = 1;
-    for (int c = 0; c < h->sum.n; c++) n += 4 + (h->sum_ard[c] ? d : 1);
+    for (int c = 0; c < h->sum.n; c++) n += 4 + (h->sum_ard[c] ? d : 1) + (h->sum_per[c] ? 1 + (h->sum_per_ard[c] ? d : 1) : 0);
     return n;
 }
 
 extern "C" int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes) {
     if (!h || !bytes || N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_state_bytes: bad argument");
     long long Np = ((N + TB - 1) / TB) * TB;
-    const long long dx = (long long)(h->composite() ? h->sum.n : 1) * d;
+    if (h->periodic && 2 * d > MAX_LS)
+        return fail(GPSO_E_BADARG, "gpso_state_bytes: a periodic kernel embeds each input dimension in 2 rows: input dimension up to 32");
+    const long long dx = h->rows_for(d);
     *bytes = (int64_t)sizeof(double) * (STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? d : 0) + sum_block_size(h, d));
     return 0;
 }
@@ -3008,6 +3262,11 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     if (h->n_rq()) hdr[8] = h->rq_alpha;
     hdr[9] = h->mean_id;
     for (int i = 0; i < h->n_ls(); i++) hdr[16 + i] = h->ls_host[i];
+    if (h->periodic) {
+        hdr[10] = 1.0;
+        hdr[11] = h->per_ard;
+        for (int i = 0; i < h->n_per(); i++) hdr[STATE_PERIODS + i] = h->per_p[i];
+    }
     double* dst = (double*)dst_dev;
     CU_TRY(cudaStreamSynchronize(h->stream));
     CU_TRY(cudaMemcpyAsync(dst, hdr, sizeof hdr, cudaMemcpyHostToDevice, st));
@@ -3023,8 +3282,12 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
         blk.push_back(h->sum.n);
         for (int c = 0; c < h->sum.n; c++) {
             const int nl = h->comp_ls(c);
-            blk.insert(blk.end(), {(double)h->sum.fam[c], (double)nl, h->comp_var(c), h->sum.alpha[c]});
+            blk.insert(blk.end(), {(double)comp_code(h, c), (double)nl, h->comp_var(c), h->sum.alpha[c]});
             for (int i = 0; i < nl; i++) blk.push_back(h->ls_host[c * h->d + i]);
+            if (h->sum_per[c]) {  // a periodic component: its period count and period(s)
+                blk.push_back(h->comp_np(c));
+                for (int i = 0; i < h->comp_np(c); i++) blk.push_back(h->comp_p[c][i]);
+            }
         }
         CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? h->d : 0), blk.data(),
                                sizeof(double) * blk.size(), cudaMemcpyHostToDevice, st));
@@ -3035,7 +3298,7 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
 
 extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_t bytes, int N, int d, void* stream) {
     if (!h || !src_dev) return fail(GPSO_E_BADARG, "gpso_import_state_dev: null argument");
-    if (N <= 0 || d <= 0 || d > MAX_LS || (h && h->composite() && h->sum.n * d > MAX_LS))
+    if (N <= 0 || d <= 0 || d > MAX_LS || (h && h->rows_for(d) > MAX_LS))
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: bad shape");
     GP_TRY(set_device(h));
     int64_t need = 0;
@@ -3050,6 +3313,8 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     CU_TRY(cudaStreamSynchronize(st));
     if ((int)hdr[0] != N || (int)hdr[1] != d) return fail(GPSO_E_BADARG, "gpso_import_state_dev: header shape mismatch");
     if ((int)hdr[6] != h->kernel_id || (int)hdr[7] != h->ard) return fail(GPSO_E_BADARG, "gpso_import_state_dev: kernel mismatch");
+    if ((hdr[10] == 1.0) != h->periodic || (h->periodic && (int)hdr[11] != h->per_ard))
+        return fail(GPSO_E_BADARG, "gpso_import_state_dev: periodic kernel mismatch");
     if (((int)hdr[9] == GPSO_MEAN_LINEAR) != h->linear())
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: linear mean function on one side only");
     const size_t dx = h->dx();
@@ -3060,12 +3325,14 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
                                sizeof(double) * blk.size(), cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
         bool same = (int)blk[0] == h->sum.n;
-        for (int c = 0, q = 1; same && c < h->sum.n; q += 4 + h->comp_ls(c), c++)
-            same = (int)blk[q] == h->sum.fam[c] && (int)blk[q + 1] == h->comp_ls(c);
+        for (int c = 0, q = 1; same && c < h->sum.n; q += comp_block(h, c, d), c++)
+            same = (int)blk[q] == comp_code(h, c) && (int)blk[q + 1] == (h->sum_ard[c] ? d : 1) &&
+                   (!h->sum_per[c] || (int)blk[q + 4 + (h->sum_ard[c] ? d : 1)] == (h->sum_per_ard[c] ? d : 1));
         if (!same)
             return fail(GPSO_E_BADARG, h->is_sum() ? "gpso_import_state_dev: sum kernel component mismatch"
                                                    : "gpso_import_state_dev: product kernel component mismatch");
-        for (int c = 0, q = 1; c < h->sum.n; q += 4 + h->comp_ls(c), c++) {
+        for (int c = 0, q = 1; c < h->sum.n; q += comp_block(h, c, d), c++) {
+            for (int i = 0; h->sum_per[c] && i < (h->sum_per_ard[c] ? d : 1); i++) h->comp_p[c][i] = blk[q + 5 + (h->sum_ard[c] ? d : 1) + i];
             if (h->is_product())  // the table's variances are {var_prod, 1, 1, 1}, var_prod from slot 2
                 h->prod_var[c] = blk[q + 2];
             else
@@ -3081,6 +3348,7 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     h->factor_nlml = hdr[5];
     if (h->n_rq()) h->rq_alpha = hdr[8];
     for (int i = 0; i < h->n_ls(); i++) h->ls_host[i] = hdr[16 + i];
+    for (int i = 0; i < h->n_per(); i++) h->per_p[i] = hdr[STATE_PERIODS + i];
     size_t Np = h->Np;
     CU_TRY(cudaMemcpyAsync(h->Xs.p, src + STATE_HEADER, sizeof(double) * dx * Np, cudaMemcpyDeviceToDevice, st));
     CU_TRY(cudaMemcpyAsync(h->alpha.p, src + STATE_HEADER + dx * Np, sizeof(double) * Np, cudaMemcpyDeviceToDevice, st));

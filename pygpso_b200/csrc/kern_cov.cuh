@@ -23,7 +23,7 @@ constexpr int CDCH = 32;  // dimensions staged in shared memory per pass
 
 template <int KID>
 __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs, int N, int d, int Np, double var,
-                                                   double noise, double* __restrict__ K, double rq_alpha, SumTable sum) {
+                                                   double noise, double* __restrict__ K, double rq_alpha, SumTable sum, SumRows srow) {
     const int bj = blockIdx.x, bi = blockIdx.y;
     if (bj > bi) return;
     __shared__ double sXi[CDCH][CT];
@@ -33,12 +33,13 @@ __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs
         // the loop below once per component (its own scaled inputs), the component values added (multiplied) in order
         double kv[16];
         for (int c = 0; c < sum.n; c++) {
-            const double* Xc = Xs + (size_t)c * d * Np;
+            const int rn = embedded_composite(KID) ? srow.rows[c] : d;
+            const double* Xc = (embedded_composite(KID) ? Xs + (size_t)srow.off[c] * Np : Xs + (size_t)c * d * Np);
             double r2[16];
 #pragma unroll
             for (int r = 0; r < 16; r++) r2[r] = 0.0;
-            for (int d0 = 0; d0 < d; d0 += CDCH) {
-                int dc = min(CDCH, d - d0);
+            for (int d0 = 0; d0 < rn; d0 += CDCH) {
+                int dc = min(CDCH, rn - d0);
                 __syncthreads();
                 for (int e = threadIdx.x; e < dc * CT; e += 256) sXi[e / CT][e % CT] = Xc[(size_t)(d0 + e / CT) * Np + bi * CT + e % CT];
                 __syncthreads();
@@ -115,13 +116,21 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
                                                        const double* __restrict__ ls, int n_ls,
                                                        const double* __restrict__ Xs, const double* __restrict__ alpha,
                                                        int N, int Np, double var, double c0, double* __restrict__ KsT,
-                                                       double* __restrict__ mean, double rq_alpha, SumTable sum) {
+                                                       double* __restrict__ mean, double rq_alpha, SumTable sum, SumRows srow) {
     extern __shared__ double sm[];  // [XG][d] scaled candidate coords (sum: [C][XG][d]), then [8 warps][XG] reduction scratch
     double* sC = sm;
     const int nsc = composite_kernel(KID) ? sum.n : 1;  // scaled copies of the candidates
-    double* sR = sm + nsc * XG * d;
+    double* sR = sm + (embedded_composite(KID) ? XG * srow.width : nsc * XG * d);
     const long long cbase = (long long)blockIdx.x * XG;
-    if constexpr (composite_kernel(KID)) {
+    if constexpr (embedded_composite(KID)) {
+        // [XG][width]: candidate row r divided by ls[r] (a periodic component's embedded rows by its unit lengthscale)
+        const int w = srow.width;
+        for (int e = threadIdx.x; e < XG * w; e += 256) {
+            const long long c = cbase + e / w;
+            const int r = e % w;
+            sC[e] = (c < Mw) ? Xc[c * w + r] / ls[r] : 0.0;
+        }
+    } else if constexpr (composite_kernel(KID)) {
         // component q divides by its own lengthscales (expanded to d entries at ls + q d): the bare kernel's division
         for (int e = threadIdx.x; e < nsc * XG * d; e += 256) {
             const int q = e / (XG * d), f = e - q * XG * d;
@@ -144,16 +153,18 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
         for (int j = threadIdx.x; j < Np; j += 256) {
             double kv[XG];
             for (int q = 0; q < sum.n; q++) {
-                const double* Xq = Xs + (size_t)q * d * Np;
-                const double* sq = sC + q * XG * d;
+                constexpr bool E = embedded_composite(KID);
+                const int rn = E ? srow.rows[q] : d, cs = E ? srow.width : d;  // rows of component q, candidate stride
+                const double* Xq = (E ? Xs + (size_t)srow.off[q] * Np : Xs + (size_t)q * d * Np);
+                const double* sq = E ? sC + srow.off[q] : sC + q * XG * d;
                 double r2[XG];
 #pragma unroll
                 for (int c = 0; c < XG; c++) r2[c] = 0.0;
-                for (int dim = 0; dim < d; dim++) {
+                for (int dim = 0; dim < rn; dim++) {
                     double xj = Xq[(size_t)dim * Np + j];
 #pragma unroll
                     for (int c = 0; c < XG; c++) {
-                        double df = xj - sq[c * d + dim];
+                        double df = xj - sq[c * cs + dim];
                         r2[c] = fma(df, df, r2[c]);
                     }
                 }
@@ -430,6 +441,282 @@ __global__ void __launch_bounds__(256) lml_grad_product_kernel(const double* __r
             slot++;
         }
         o += (ard ? d : 1) + (tab.fam[c] == KERNEL_RQ);
+    }
+}
+
+// A product with periodic factors (bit c of srow.pmask): lml_grad_product_kernel with factor c's rows [srow.off[c], + srow.rows[c])
+// -- a periodic factor's 2d embedded rows -- and X[N][d] holding the raw inputs (a separate kernel, so that the one above stays as
+// it is).  A periodic factor always takes a weight slot (set in ard_mask) and writes, like lml_grad_periodic_kernel, per dimension
+// j the lengthscale entry sum w ((De_j)^2 + (De_{d+j})^2) and the period entry sum w (x_j - x'_j) (e_{d+j} e'_j - e_j e'_{d+j}),
+// 2d entries before its alpha.
+__global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const double* __restrict__ Xs, const double* __restrict__ alpha,
+                                                                        const double* __restrict__ Kinv, int N, int d, int Np,
+                                                                        int ard_mask, double* __restrict__ part, int part_stride,
+                                                                        SumTable tab, const double* __restrict__ X, SumRows srow) {
+    int blk = blockIdx.x;
+    int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
+    while ((bi + 1) * (bi + 2) / 2 <= blk) bi++;
+    while (bi * (bi + 1) / 2 > blk) bi--;
+    int bj = blk - bi * (bi + 1) / 2;
+    const int n = tab.n, dx = srow.width;
+    extern __shared__ double smg[];
+    double* sXi = smg;                // [dx][64] scaled coordinates of the tile's rows
+    double* sXj = smg + dx * CT;      // [dx][64] ... and of its columns
+    double* sRi = sXj + dx * CT;      // [d][64] raw coordinates of the tile's rows, then of its columns
+    double* sRj = sRi + d * CT;
+    double* sW = sRj + d * CT;        // [ARD / periodic factors][64 * 64] per-pair weights W P_-c g_c
+    __shared__ double sRed[8];
+    for (int e = threadIdx.x; e < dx * CT; e += 256) {
+        const size_t row = (size_t)(e / CT) * Np;
+        sXi[e] = Xs[row + bi * CT + e % CT];
+        sXj[e] = Xs[row + bj * CT + e % CT];
+    }
+    for (int e = threadIdx.x; e < d * CT; e += 256) {
+        const int q = e / CT, t = e % CT, ri = bi * CT + t, rj = bj * CT + t;
+        sRi[e] = ri < N ? X[(size_t)ri * d + q] : 0.0;
+        sRj[e] = rj < N ? X[(size_t)rj * d + q] : 0.0;
+    }
+    __syncthreads();
+    const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
+    const int j = bj * CT + tx;
+    const double aj = alpha[j];
+    const double wsym = (bi == bj) ? 1.0 : 2.0;
+    double s_k = 0.0, s_tr = 0.0, s_l[MAX_SUM], s_a[MAX_SUM];
+#pragma unroll
+    for (int c = 0; c < MAX_SUM; c++) s_l[c] = s_a[c] = 0.0;
+#pragma unroll 1
+    for (int r = 0; r < 16; r++) {
+        const int il = ty + 4 * r, i = bi * CT + il;
+        const bool valid = i < N && j < N;
+        // diagonal tiles: the tile holds both triangles of a symmetric quantity, take every element once
+        double W = 0.0;
+        if (valid) W = fma(alpha[i], aj, -((j <= i) ? Kinv[(size_t)i * Np + j] : Kinv[(size_t)j * Np + i])) * wsym;
+        double r2[MAX_SUM], k[MAX_SUM], g[MAX_SUM], ka[MAX_SUM];
+#pragma unroll
+        for (int c = 0; c < MAX_SUM; c++) {
+            r2[c] = 0.0;
+            k[c] = 1.0;  // absent factors: the products below stay those of the n present ones
+            g[c] = ka[c] = 0.0;
+            if (c < n) {
+                const int r0 = srow.off[c], r1 = r0 + srow.rows[c];
+                for (int q = r0; q < r1; q++) {
+                    const double df = sXi[q * CT + il] - sXj[q * CT + tx];
+                    r2[c] = fma(df, df, r2[c]);
+                }
+                sum_term_radial(tab, c, r2[c], k[c], g[c], ka[c]);
+            }
+        }
+        double pre[MAX_SUM], suf[MAX_SUM];
+        pre[0] = 1.0;
+#pragma unroll
+        for (int c = 1; c < MAX_SUM; c++) pre[c] = pre[c - 1] * k[c - 1];
+        suf[MAX_SUM - 1] = 1.0;
+#pragma unroll
+        for (int c = MAX_SUM - 2; c >= 0; c--) suf[c] = suf[c + 1] * k[c + 1];
+        if (valid) {
+            s_k = fma(W, pre[MAX_SUM - 1] * k[MAX_SUM - 1], s_k);
+            if (i == j) s_tr += W;
+        }
+        int slot = 0;
+#pragma unroll
+        for (int c = 0; c < MAX_SUM; c++) {
+            if (c < n) {
+                const double pw = W * (pre[c] * suf[c]);
+                if (ard_mask >> c & 1) {
+                    sW[slot * CT * CT + il * CT + tx] = valid ? pw * g[c] : 0.0;
+                    slot++;
+                } else if (valid) {
+                    s_l[c] = fma(pw * g[c], fmax(r2[c], 0.0), s_l[c]);
+                }
+                if (valid && tab.fam[c] == KERNEL_RQ) s_a[c] = fma(pw, ka[c], s_a[c]);
+            }
+        }
+    }
+    double v = block_sum<256>(s_k, sRed);
+    if (threadIdx.x == 0) part[(size_t)blk * part_stride + 0] = v;
+    v = block_sum<256>(s_tr, sRed);
+    if (threadIdx.x == 0) part[(size_t)blk * part_stride + 1] = v;
+    int off = 2;
+#pragma unroll
+    for (int c = 0; c < MAX_SUM; c++) {
+        if (c >= n) break;
+        const bool ard = ard_mask >> c & 1, rq = tab.fam[c] == KERNEL_RQ;
+        if (!ard) {
+            v = block_sum<256>(s_l[c], sRed);
+            if (threadIdx.x == 0) part[(size_t)blk * part_stride + off] = v;
+        }
+        const int nl = (srow.pmask >> c & 1) ? 2 * d : (ard ? d : 1);
+        if (rq) {
+            v = block_sum<256>(s_a[c], sRed);
+            if (threadIdx.x == 0) part[(size_t)blk * part_stride + off + nl] = v;
+        }
+        off += nl + rq;
+    }
+    if (ard_mask == 0) return;
+    __syncthreads();  // the weights of every pair are in sW
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int c = 0, slot = 0, o = 2; c < n; c++) {
+        const bool ard = ard_mask >> c & 1, per = srow.pmask >> c & 1;
+        if (per) {
+            const double* ws = sW + slot * CT * CT;
+            for (int q = w; q < d; q += 8) {
+                const int r = srow.off[c] + q;
+                const double *ci = sXi + r * CT, *cj = sXj + r * CT, *si = sXi + (r + d) * CT, *sj = sXj + (r + d) * CT;
+                const double *xi = sRi + q * CT, *xj = sRj + q * CT;
+                double acc_l = 0.0, acc_p = 0.0;
+                for (int p = lane; p < CT * CT; p += 32) {
+                    const int a = p >> 6, b = p & 63;
+                    const double dc = ci[a] - cj[b], ds = si[a] - sj[b];
+                    acc_l = fma(ws[p], fma(dc, dc, ds * ds), acc_l);
+                    acc_p = fma(ws[p] * (xi[a] - xj[b]), fma(si[a], cj[b], -(ci[a] * sj[b])), acc_p);
+                }
+                acc_l = warp_sum(acc_l);
+                acc_p = warp_sum(acc_p);
+                if (lane == 0) {
+                    part[(size_t)blk * part_stride + o + q] = acc_l;
+                    part[(size_t)blk * part_stride + o + d + q] = acc_p;
+                }
+            }
+            slot++;
+        } else if (ard) {
+            const double* ws = sW + slot * CT * CT;
+            for (int q = w; q < d; q += 8) {
+                const int r = srow.off[c] + q;
+                const double* xi = sXi + r * CT;
+                const double* xj = sXj + r * CT;
+                double acc = 0.0;
+                for (int p = lane; p < CT * CT; p += 32) {
+                    const double df = xi[p >> 6] - xj[p & 63];
+                    acc = fma(ws[p], df * df, acc);
+                }
+                acc = warp_sum(acc);
+                if (lane == 0) part[(size_t)blk * part_stride + o + q] = acc;
+            }
+            slot++;
+        }
+        o += (per ? 2 * d : (ard ? d : 1)) + (tab.fam[c] == KERNEL_RQ);
+    }
+}
+
+// ---- periodic kernel (gpflow.kernels.Periodic with a SquaredExponential / RationalQuadratic base) ------------------------
+// k(x, x') = base.K_r2(r2), r2 = sum_j sin^2(pi (x_j - x'_j) / p_j) / l_j^2, is the base kernel at unit lengthscale on the
+// embedded rows  e_j(x) = cos(theta_j) / (2 l_j),  e_{d+j}(x) = sin(theta_j) / (2 l_j),  theta_j = 2 pi x_j / p_j
+// (chord: |e(x) - e(x')|^2 = (2 - 2 cos(theta - theta')) / (4 l^2) = sin^2((theta - theta') / 2) / l^2).  The phase is one fp64
+// sincospi(2 x / p) per coordinate; lp = [l expanded to d entries, p expanded to d entries].  out[i * s_row + r * s_dim] for rows
+// i < rows, zero for padding rows rows <= i < rows_pad (dimension-major training inputs [2d][Np], or row-major candidates
+// [M][2d]).  A NaN or infinite coordinate gives NaN rows.  lp == nullptr writes the raw coordinates to the d rows instead (the columns of
+// a sum / product's candidate rows that belong to a component that is not periodic).
+__global__ void __launch_bounds__(256) periodic_embed_kernel(const double* __restrict__ X, long long rows, long long rows_pad, int d,
+                                                             const double* __restrict__ lp, long long s_row, long long s_dim,
+                                                             double* __restrict__ out) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= rows_pad * d) return;
+    const long long i = e / d;
+    const int j = (int)(e - i * d);
+    if (!lp) {  // a plain component's columns of a sum / product's candidate rows: the raw coordinate (its kernel divides by l)
+        out[i * s_row + (long long)j * s_dim] = i < rows ? X[e] : 0.0;
+        return;
+    }
+    double c = 0.0, s = 0.0;
+    if (i < rows) {
+        const double l2 = 2.0 * lp[j];
+        sincospi(2.0 * X[e] / lp[d + j], &s, &c);
+        c /= l2;
+        s /= l2;
+    }
+    out[i * s_row + (long long)j * s_dim] = c;
+    out[i * s_row + (long long)(d + j) * s_dim] = s;
+}
+
+// LML gradient of a periodic kernel: every entry in one launch.  One block per lower 64x64 tile, the tile's embedded rows
+// (Xs[2d][Np]) and raw coordinates (X[N][d]) of its rows and columns in shared memory.  Per pair W, the base covariance k and
+// g = -2 dk/dr2 are formed once; W g goes to shared memory and a second pass gives warp w the dimensions j = w, w + 8, ...:
+//   part[blk][0]         = sum W k                                                (-> d/d variance after / variance)
+//   part[blk][1]         = sum_i W_ii                                             (-> d/d noise)
+//   part[blk][2 + j]     = sum W g ((e_j - e'_j)^2 + (e_{d+j} - e'_{d+j})^2)       (dK/dl_j = g r2_j / l_j)
+//   part[blk][2 + d + j] = sum W g (x_j - x'_j) (e_{d+j} e'_j - e_j e'_{d+j})       (dK/dp_j = 2 pi g delta_j sin(2 pi delta_j / p_j) / (4 l_j^2 p_j^2))
+//   part[blk][2 + 2d]    = sum W dk/dalpha                                        (RationalQuadratic base only)
+// Scalar lengthscales / periods are the sums of these entries over j (the host adds them).
+template <int KID>
+__global__ void __launch_bounds__(256) lml_grad_periodic_kernel(const double* __restrict__ Xs, const double* __restrict__ X,
+                                                                const double* __restrict__ alpha, const double* __restrict__ Kinv,
+                                                                int N, int d, int Np, double var, double rq_alpha,
+                                                                double* __restrict__ part, int part_stride) {
+    int blk = blockIdx.x;
+    int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
+    while ((bi + 1) * (bi + 2) / 2 <= blk) bi++;
+    while (bi * (bi + 1) / 2 > blk) bi--;
+    int bj = blk - bi * (bi + 1) / 2;
+    const int dx = 2 * d;
+    extern __shared__ double smg[];
+    double* sXi = smg;               // [2d][64] embedded rows of the tile's rows
+    double* sXj = sXi + dx * CT;     // [2d][64] ... and of its columns
+    double* sRi = sXj + dx * CT;     // [d][64]  raw coordinates of the tile's rows
+    double* sRj = sRi + d * CT;      // [d][64]  ... and of its columns
+    double* sW = sRj + d * CT;       // [64 * 64] W g per pair
+    __shared__ double sRed[8];
+    for (int e = threadIdx.x; e < dx * CT; e += 256) {
+        const size_t row = (size_t)(e / CT) * Np;
+        sXi[e] = Xs[row + bi * CT + e % CT];
+        sXj[e] = Xs[row + bj * CT + e % CT];
+    }
+    for (int e = threadIdx.x; e < d * CT; e += 256) {
+        const int q = e / CT, t = e % CT, ri = bi * CT + t, rj = bj * CT + t;
+        sRi[e] = ri < N ? X[(size_t)ri * d + q] : 0.0;
+        sRj[e] = rj < N ? X[(size_t)rj * d + q] : 0.0;
+    }
+    __syncthreads();
+    const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
+    const int j = bj * CT + tx;
+    const double aj = alpha[j];
+    const double wsym = (bi == bj) ? 1.0 : 2.0;
+    double s_k = 0.0, s_tr = 0.0, s_a = 0.0;
+#pragma unroll 1
+    for (int r = 0; r < 16; r++) {
+        const int il = ty + 4 * r, i = bi * CT + il;
+        double wg = 0.0;
+        if (i < N && j < N) {
+            const double W = fma(alpha[i], aj, -((j <= i) ? Kinv[(size_t)i * Np + j] : Kinv[(size_t)j * Np + i])) * wsym;
+            double r2 = 0.0;
+            for (int q = 0; q < dx; q++) {
+                const double df = sXi[q * CT + il] - sXj[q * CT + tx];
+                r2 = fma(df, df, r2);
+            }
+            double k, g, ka;
+            cov_and_radial<KID>(r2, var, rq_alpha, k, g, ka);
+            s_k = fma(W, k, s_k);
+            if (KID == KERNEL_RQ) s_a = fma(W, ka, s_a);
+            if (i == j) s_tr += W;
+            wg = W * g;
+        }
+        sW[il * CT + tx] = wg;
+    }
+    double v = block_sum<256>(s_k, sRed);
+    if (threadIdx.x == 0) part[(size_t)blk * part_stride + 0] = v;
+    v = block_sum<256>(s_tr, sRed);
+    if (threadIdx.x == 0) part[(size_t)blk * part_stride + 1] = v;
+    if (KID == KERNEL_RQ) {
+        v = block_sum<256>(s_a, sRed);
+        if (threadIdx.x == 0) part[(size_t)blk * part_stride + 2 + dx] = v;
+    }
+    __syncthreads();  // the weights of every pair are in sW
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int q = w; q < d; q += 8) {
+        const double *ci = sXi + q * CT, *cj = sXj + q * CT, *si = sXi + (d + q) * CT, *sj = sXj + (d + q) * CT;
+        const double *xi = sRi + q * CT, *xj = sRj + q * CT;
+        double acc_l = 0.0, acc_p = 0.0;
+        for (int p = lane; p < CT * CT; p += 32) {
+            const int a = p >> 6, b = p & 63;
+            const double dc = ci[a] - cj[b], ds = si[a] - sj[b];
+            acc_l = fma(sW[p], fma(dc, dc, ds * ds), acc_l);
+            acc_p = fma(sW[p] * (xi[a] - xj[b]), fma(si[a], cj[b], -(ci[a] * sj[b])), acc_p);
+        }
+        acc_l = warp_sum(acc_l);
+        acc_p = warp_sum(acc_p);
+        if (lane == 0) {
+            part[(size_t)blk * part_stride + 2 + q] = acc_l;
+            part[(size_t)blk * part_stride + 2 + d + q] = acc_p;
+        }
     }
 }
 

@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_v_kernel(JointVParams P) {
 template <int KID>
 __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* __restrict__ VT, const double* __restrict__ Xcs, int M,
                                                                  int Mp, int Np, int d, double var, double jitter,
-                                                                 double* __restrict__ Sigma, double rq_alpha, SumTable sum) {
+                                                                 double* __restrict__ Sigma, double rq_alpha, SumTable sum, SumRows srow) {
     extern __shared__ double smem[];
     int a, b;
     tri_index(blockIdx.x, a, b);
@@ -114,9 +114,10 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* _
             // sum_q var_q (a product: var_prod, its unit factors being exactly 1 at r = 0)
             double k = 0.0;
             for (int q = 0; q < sum.n; q++) {
-                const double* Xq = Xcs + (size_t)q * d * Mp;
+                const double* Xq = (embedded_composite(KID) ? Xcs + (size_t)srow.off[q] * Mp : Xcs + (size_t)q * d * Mp);
+                const int rn = embedded_composite(KID) ? srow.rows[q] : d;
                 double r2 = 0.0;
-                for (int dim = 0; dim < d; dim++) {
+                for (int dim = 0; dim < rn; dim++) {
                     const double df = Xq[(size_t)dim * Mp + gi] - Xq[(size_t)dim * Mp + gj];
                     r2 = fma(df, df, r2);
                 }

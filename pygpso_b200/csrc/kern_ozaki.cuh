@@ -380,9 +380,9 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                                                               const double* __restrict__ Xs, const double* __restrict__ alpha, int N,
                                                               int Np, double var, double c0, double bscale, int nks,
                                                               uint8_t* __restrict__ B, double* __restrict__ mean, double rq_alpha,
-                                                              SumTable sum) {
+                                                              SumTable sum, SumRows srow) {
     // sum / product: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs and in shared memory alike
-    const int dx = composite_kernel(KID) ? sum.n * d : d;
+    const int dx = embedded_composite(KID) ? srow.width : (composite_kernel(KID) ? sum.n * d : d);
     extern __shared__ double sm[];
     double* sC = sm;                      // [dx][64]      scaled candidate coordinates, dimension-major
     double* sX = sC + dx * OZ_NT;         // [2][dx][128]  scaled training coordinates of the current / next super-step
@@ -394,7 +394,8 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
         for (int e = tid; e < OZ_NT * dx; e += 256) {
             int cc = e / dx, qd = e - cc * dx, dim = qd % d;  // qd = q d + dim: component q divides by its own lengthscales
             long long cg = ct * OZ_NT + cc;
-            sC[qd * OZ_NT + cc] = (cg < Mw) ? Xc[cg * d + dim] / ls[qd] : 0.0;
+            // periodic components: candidate rows of the table's width, row qd divided by ls[qd]
+            sC[qd * OZ_NT + cc] = (cg < Mw) ? Xc[embedded_composite(KID) ? cg * dx + qd : cg * d + dim] / ls[qd] : 0.0;
         }
     } else {
         for (int e = tid; e < OZ_NT * d; e += 256) {
@@ -437,7 +438,8 @@ __global__ void __launch_bounds__(256, 2) crosscov_slices_kernel(const double* _
                     double r2[16];
 #pragma unroll
                     for (int i = 0; i < 16; i++) r2[i] = 0.0;
-                    for (int dim = q * d; dim < (q + 1) * d; dim++) {
+                    const int r0 = embedded_composite(KID) ? srow.off[q] : q * d, r1 = embedded_composite(KID) ? r0 + srow.rows[q] : (q + 1) * d;
+                    for (int dim = r0; dim < r1; dim++) {
                         const double xa = sC[dim * OZ_NT + cl + 32 * a];
                         const double2* xr = reinterpret_cast<const double2*>(x + dim * OZ_XK);
 #pragma unroll

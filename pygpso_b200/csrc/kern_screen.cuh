@@ -232,9 +232,9 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                                                                  const float* __restrict__ Xs32, const float* __restrict__ alpha32,
                                                                  int N, int Np, float var, double c0, float bscale, int nks,
                                                                  uint8_t* __restrict__ B, double* __restrict__ mean, float rq_alpha,
-                                                                 SumTable sum) {
+                                                                 SumTable sum, SumRows srow) {
     // sum / product: the C components' scaled coordinates are dx = C d rows ([C][d] component-major), in Xs32 and in shared memory alike
-    const int dx = composite_kernel(KID) ? sum.n * d : d;
+    const int dx = embedded_composite(KID) ? srow.width : (composite_kernel(KID) ? sum.n * d : d);
     extern __shared__ __align__(16) float smf[];
     float* sC = smf;                       // [dx][64]
     float* sX = sC + dx * 64;              // [2][dx][128]
@@ -251,7 +251,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
             const long long cg = blk * 64 + cc;
             double x = 0.0;
             if (cg < Mw) {
-                x = Xc[cg * d + dim] / ls[qd];
+                x = Xc[embedded_composite(KID) ? cg * dx + qd : cg * d + dim] / ls[qd];  // periodic components: rows of width dx
                 if (!(fabs(x) <= 1.0e15)) sBad[cc] = 1;
             }
             sC[qd * 64 + cc] = (float)x;
@@ -304,7 +304,8 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                 f32x2_t rq[16];
 #pragma unroll
                 for (int i = 0; i < 16; i++) rq[i] = 0ULL;
-                for (int dim = q * d; dim < (q + 1) * d; dim++) {
+                const int r0 = embedded_composite(KID) ? srow.off[q] : q * d, r1 = embedded_composite(KID) ? r0 + srow.rows[q] : (q + 1) * d;
+                for (int dim = r0; dim < r1; dim++) {
                     const f32x2_t xc = f2_pack(sC[dim * 64 + cl], sC[dim * 64 + cl + 32]);
                     const float4* xr = reinterpret_cast<const float4*>(x + dim * OZ_XK);
 #pragma unroll
@@ -329,7 +330,7 @@ __global__ void __launch_bounds__(256, 2) crosscov_screen_kernel(const double* _
                         case KERNEL_SE: t = cov32x2_from_r2<KERNEL_SE>(rq[g], v, al); break;
                         default: t = cov32x2_from_r2<KERNEL_RQ>(rq[g], v, al); break;
                     }
-                    kv[g] = (q == 0) ? t : (KID == KERNEL_PRODUCT ? f2_mul(kv[g], t) : f2_add(kv[g], t));
+                    kv[g] = (q == 0) ? t : (product_kernel(KID) ? f2_mul(kv[g], t) : f2_add(kv[g], t));
                 }
             }
         } else {

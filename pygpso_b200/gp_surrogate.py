@@ -601,9 +601,11 @@ class GPRSurrogate(GPSurrogate):
             dill.dump(params, handle)
         meanf = model.mean_function
         is_sum = isinstance(model.kernel, gpmodel.Combination)  # a Sum or a Product
+        periodic = isinstance(model.kernel, gpmodel.Periodic)
+        leaf = model.kernel.base_kernel if periodic else model.kernel
         save_info = {
             "gpr_kernel": model.kernel.__class__.__name__,
-            "gpr_kernel_shape": [] if is_sum else model.kernel.lengthscales.shape.as_list(),
+            "gpr_kernel_shape": [] if is_sum else leaf.lengthscales.shape.as_list(),
             "gpr_meanf": meanf.__class__.__name__,
             "gpr_meanf_shape": meanf.parameters[0].shape.as_list() if meanf.parameters else [],
             "gp_varsigma": self.gp_varsigma,
@@ -611,7 +613,13 @@ class GPRSurrogate(GPSurrogate):
             "optimiser": self._serialise_optimiser(),
         }
         if is_sum:  # component (factor) families and lengthscale shapes, in order
-            save_info["gpr_kernel_components"] = [[k.__class__.__name__, k.lengthscales.shape.as_list()] for k in model.kernel.kernels]
+            # a periodic term: ["Periodic", base lengthscale shape, base family, period shape]
+            save_info["gpr_kernel_components"] = [
+                ["Periodic", k.base_kernel.lengthscales.shape.as_list(), k.base_kernel.__class__.__name__, k.period.shape.as_list()]
+                if isinstance(k, gpmodel.Periodic) else [k.__class__.__name__, k.lengthscales.shape.as_list()]
+                for k in model.kernel.kernels]
+        if periodic:  # base family and the shape of the period; gpr_kernel_shape is the base lengthscales'
+            save_info["gpr_kernel_periodic"] = [leaf.__class__.__name__, model.kernel.period.shape.as_list()]
         with open(os.path.join(folder, self.GPR_INFO), "w") as handle:
             handle.write(json.dumps(save_info))
 
@@ -625,8 +633,16 @@ class GPRSurrogate(GPSurrogate):
         info = load_json(os.path.join(folder, cls.GPR_INFO))
         assert hasattr(gpmodel.kernels, info["gpr_kernel"])
         if info["gpr_kernel"] in ("Sum", "Product"):  # multiple_assign restores every component's parameters below
-            gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])([getattr(gpmodel.kernels, name)(lengthscales=np.ones(shape))
-                                                                     for name, shape in info["gpr_kernel_components"]])
+            def component(entry):
+                if entry[0] == "Periodic":
+                    return gpmodel.kernels.Periodic(getattr(gpmodel.kernels, entry[2])(lengthscales=np.ones(entry[1])),
+                                                    period=np.ones(entry[3]))
+                return getattr(gpmodel.kernels, entry[0])(lengthscales=np.ones(entry[1]))
+            gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])([component(e) for e in info["gpr_kernel_components"]])
+        elif info["gpr_kernel"] == "Periodic":
+            base, period_shape = info["gpr_kernel_periodic"]
+            gp_kernel = gpmodel.kernels.Periodic(getattr(gpmodel.kernels, base)(lengthscales=np.ones(info["gpr_kernel_shape"])),
+                                                 period=np.ones(period_shape))
         else:
             gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
         assert hasattr(gpmodel.mean_functions, info["gpr_meanf"])

@@ -20,7 +20,8 @@ Parameterisation follows GPflow 2: positive parameters are softplus-transformed,
 the 1e-6 floor, and ``trainable_variables`` are ordered kernel.lengthscales, kernel.variance, likelihood.variance,
 mean_function.c (or mean_function.A, mean_function.b for ``Linear``) -- preceded by kernel.alpha for ``RationalQuadratic``
 (tf.Module visits attributes in sorted name order).  A ``Sum`` (``Product``) kernel lists its components' (factors')
-parameters in component order, each component's in that same sorted order.
+parameters in component order, each component's in that same sorted order.  A ``Periodic`` kernel lists its base kernel's
+parameters, then kernel.period ('base_kernel' < 'period').
 """
 import types
 
@@ -181,7 +182,9 @@ class Combination(Kernel):
             if not isinstance(k, Kernel):
                 raise TypeError("can only combine Kernel instances")
             flat.extend(k.kernels if type(k) is type(self) else [k])
-        if any(flat[i] is flat[j] for i in range(len(flat)) for j in range(i)):
+        # a periodic term's base kernel holds the parameters: the same base object twice shares them too
+        leaves = [k.base_kernel if isinstance(k, Periodic) else k for k in flat]
+        if any(leaves[i] is leaves[j] for i in range(len(leaves)) for j in range(i)):
             raise ValueError(f"a kernel object appears twice in the {self._what}: GPflow would share its parameters between the "
                              "terms, which this model does not support; use two separate kernel objects")
         if not 1 <= len(flat) <= MAX_SUM:
@@ -222,6 +225,30 @@ class RationalQuadratic(Stationary):
         return (self.alpha, self.lengthscales, self.variance)
 
 
+class Periodic(Kernel):
+    """``gpflow.kernels.Periodic(base_kernel, period)``: ``k(x, x') = base.K_r2(r2)`` with
+    ``r2 = sum_j sin^2(pi (x_j - x'_j) / period_j) / lengthscales_j^2``, the base kernel's lengthscales and variance.  The base is a
+    ``SquaredExponential`` or a ``RationalQuadratic`` (GPflow evaluates a Matern base on a different distance, through its K_r); the
+    period (positive, softplus, no floor) is a scalar or one entry per input dimension.  The prior variance is the base variance.
+    It may also be a term of a ``Sum`` or a factor of a ``Product``."""
+
+    def __init__(self, base_kernel, period=1.0):
+        if isinstance(base_kernel, (Combination, Periodic)) or not isinstance(base_kernel, Kernel):
+            raise TypeError("the base kernel of a Periodic kernel must be a single stationary kernel (GPflow requires an "
+                            "IsotropicStationary base), not a Sum, Product or Periodic")
+        if not isinstance(base_kernel, (SquaredExponential, RationalQuadratic)):
+            raise TypeError(f"Periodic({type(base_kernel).__name__}(...)) is not supported: the base kernel must be SquaredExponential "
+                            "or RationalQuadratic (GPflow evaluates a Matern base on sum |sin| through its K_r, a different kernel)")
+        self.base_kernel = base_kernel
+        self.period = Parameter(period, positive=True, name="kernel.period")
+        if len(self.period.shape) > 1:
+            raise ValueError(f"period must be a scalar or a vector, got shape {tuple(self.period.shape)}")
+
+    @property
+    def parameters(self):
+        return tuple(self.base_kernel.parameters) + (self.period,)
+
+
 class MeanFunction:
     parameters = ()
 
@@ -259,6 +286,14 @@ class Linear(MeanFunction):
     @property
     def parameters(self):
         return (self.A, self.b)
+
+
+# a component of a Sum / Product as the backend takes it: (family, n_lengthscales), or ("Periodic", n_lengthscales, base family,
+# n_periods) for a periodic term
+def _component_spec(k):
+    if isinstance(k, Periodic):
+        return ("Periodic", k.base_kernel.lengthscales.size, type(k.base_kernel).__name__, k.period.size)
+    return (type(k).__name__, k.lengthscales.size)
 
 
 # mean id of the C ABI (GPSO_MEAN_*) passed to open_session: False / True for Zero / Constant, 2 for Linear
@@ -307,7 +342,7 @@ class GPR(GPModel):
         if isinstance(kernel, Combination) and any(isinstance(k, Combination) for k in parts):
             raise TypeError("sums of products and products of sums are not supported: the components of a Sum and the factors "
                             "of a Product must be Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic")
-        if not all(isinstance(k, Stationary) for k in parts):
+        if not all(isinstance(k, (Stationary, Periodic)) for k in parts):
             raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic, "
                             "or a Sum of them")
         self.kernel = kernel
@@ -319,7 +354,12 @@ class GPR(GPModel):
         if isinstance(kernel, Combination):
             self._session = self._backend.open_session(
                 kernel=type(kernel).__name__, n_lengthscales=0, has_mean=_mean_id(self.mean_function),
-                components=[(type(k).__name__, k.lengthscales.size) for k in parts],
+                components=[_component_spec(k) for k in parts],
+            )
+        elif isinstance(kernel, Periodic):  # components: [(base family, number of periods)]
+            self._session = self._backend.open_session(
+                kernel="Periodic", n_lengthscales=kernel.base_kernel.lengthscales.size, has_mean=_mean_id(self.mean_function),
+                components=[(type(kernel.base_kernel).__name__, kernel.period.size)],
             )
         else:
             self._session = self._backend.open_session(
@@ -344,6 +384,10 @@ class GPR(GPModel):
         if x.ndim != 2 or y.ndim != 2 or y.shape != (x.shape[0], 1):
             raise ValueError(f"data must be (X[N,d], Y[N,1]); got {x.shape}, {y.shape}")
         for k in self.kernel.kernels if isinstance(self.kernel, Combination) else [self.kernel]:
+            if isinstance(k, Periodic):
+                if k.period.size not in (1, x.shape[1]):
+                    raise ValueError("an ARD period must have one entry per input dimension")
+                k = k.base_kernel
             if k.lengthscales.size not in (1, x.shape[1]):
                 raise ValueError("ARD lengthscales must have one entry per input dimension")
         if isinstance(self.mean_function, Linear) and self.mean_function.A.shape[0] != x.shape[1]:
@@ -378,7 +422,8 @@ class GPR(GPModel):
             pos += p.size
 
     def _theta(self):
-        """Constrained vector in packing order: [alpha], lengthscale(s), kernel variance, noise variance, [mean c | A, b]."""
+        """Constrained vector in packing order: [alpha], lengthscale(s), kernel variance, [period(s)], noise variance,
+        [mean c | A, b]."""
         return np.concatenate([np.asarray(p, dtype=np.float64).reshape(-1) for p in self._ordered_parameters])
 
     # -- objective ----------------------------------------------------------------------------------------------------
@@ -509,6 +554,10 @@ class Scipy:
 # gpflow.utilities look-alikes (used by save / load)
 # ---------------------------------------------------------------------------------------------------------------------
 def _kernel_leaves(prefix, kernel):
+    if isinstance(kernel, Periodic):
+        out = _kernel_leaves(f"{prefix}.base_kernel", kernel.base_kernel)
+        out[f"{prefix}.period"] = kernel.period
+        return out
     out = {f"{prefix}.alpha": kernel.alpha} if isinstance(kernel, RationalQuadratic) else {}
     out.update({f"{prefix}.lengthscales": kernel.lengthscales, f"{prefix}.variance": kernel.variance})
     return out
@@ -553,7 +602,7 @@ def tabulate_module_summary(model):
 kernels = types.SimpleNamespace(
     Kernel=Kernel, Stationary=Stationary, Matern12=Matern12, Matern32=Matern32, Matern52=Matern52,
     SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic, Sum=Sum,
-    Product=Product,
+    Product=Product, Periodic=Periodic,
 )
 mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant, Linear=Linear)
 likelihoods = types.SimpleNamespace(Gaussian=Gaussian)
