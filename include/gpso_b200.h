@@ -29,7 +29,8 @@
  *     GPSO_KERNEL_PERIODIC (gpflow.kernels.Periodic(base, period)) packs its base kernel's block, then the period(s) ('base_kernel'
  *     < 'period' in tf.Module's sorted names):
  *         [ (alpha) , lengthscale(s) , kernel variance , period(s) (1, or d when period_ard) , likelihood (noise) variance , mean entries ]
- *     d is the input dimension of gpso_set_data, so the count is known from then on (as for ARD lengthscales).
+ *     d is the input dimension of gpso_set_data, so the count is known from then on (as for ARD lengthscales).  With an active
+ *     dims map (gpso_set_active_dims) an ARD flag of leaf c means counts[c] lengthscales, and counts[c] periods, instead of d.
  *     `u`     = unconstrained (softplus pre-image; noise variance has the 1e-6 floor of gpflow.likelihoods.Gaussian),
  *     `theta` = constrained values.
  */
@@ -99,6 +100,16 @@ int gpso_destroy(gpso_handle* h);
 
 /* model.data = (x, y), gp_surrogate.py:498.  X_host[N,d], y_host[N] are copied to the device. */
 int gpso_set_data(gpso_handle* h, const double* X_host, const double* y_host, int N, int d);
+
+/* Kernels on a subset of the inputs (GPflow's active_dims).  Leaf c -- the bare kernel, or component c of a sum / product; a
+ * periodic leaf means its base -- reads the counts[c] input columns listed next in dims (in that order, repeats allowed).  Call it
+ * after create and before gpso_set_data; n = 0 clears the map.  Any call drops the data: fit and predict calls return
+ * GPSO_E_STATE until gpso_set_data.  gpso_set_data checks that n is the leaf count (1 for a bare kernel), that every column is
+ * below d and that the rows (counts[c] per leaf, 2 counts[c] for a periodic one) do not exceed 64; the limit of d itself is
+ * still 64.  With a map, an ARD flag means counts[c] lengthscales (periods) instead of d.  The exported state of a handle with a
+ * map carries it, and gpso_import_state_dev accepts such a state only into a handle with the same map (and a state without a
+ * map only into a handle without one): otherwise GPSO_E_BADARG, "active dims mismatch". */
+int gpso_set_active_dims(gpso_handle* h, int n, const int* counts, const int* dims);
 
 /* ---- fit: the closure scipy's L-BFGS-B calls, i.e. model.training_loss + TF autodiff, gp_surrogate.py:500-503 -- */
 /* f = -log marginal likelihood at unconstrained u[p]; grad[p] = df/du.  Host in, host out, synchronous.            */

@@ -86,6 +86,7 @@ def load_library():
                                           ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(H)]),
         "gpso_destroy": (i32, [H]),
         "gpso_set_data": (i32, [H, _c_double_p, _c_double_p, i32, i32]),
+        "gpso_set_active_dims": (i32, [H, i32, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]),
         "gpso_neg_lml_grad": (i32, [H, _c_double_p, i32, _c_double_p, _c_double_p]),
         "gpso_factorize": (i32, [H, _c_double_p, i32]),
         "gpso_factor_lml": (i32, [H, _c_double_p]),
@@ -149,7 +150,7 @@ def load_library():
 
 
 EXPORTED_SYMBOLS = (
-    "gpso_version gpso_last_error gpso_device_count gpso_create gpso_create_sum gpso_create_product gpso_create_periodic gpso_create_combination gpso_destroy gpso_set_data gpso_neg_lml_grad "
+    "gpso_version gpso_last_error gpso_device_count gpso_create gpso_create_sum gpso_create_product gpso_create_periodic gpso_create_combination gpso_destroy gpso_set_data gpso_set_active_dims gpso_neg_lml_grad "
     "gpso_factorize gpso_factor_lml gpso_predict_y_host gpso_predict_y_dev gpso_ucb_argmax_host gpso_ucb_argmax_dev "
     "gpso_ucb_topk_host gpso_ucb_topk_dev "
     "gpso_predict_f_cov_host gpso_predict_f_cov_dev gpso_predict_f_samples_host gpso_predict_f_samples_dev "
@@ -242,6 +243,17 @@ class CudaSession:
         self.factorized = False
 
     # -- fit ----------------------------------------------------------------------------------------------------------
+    def set_active_dims(self, leaf_dims):
+        """The input columns of each leaf (the bare kernel, or each component / factor in order; a periodic one's base), or None
+        for every column in order.  Drops the data: call ``set_data`` next."""
+        dims = [] if leaf_dims is None else [[int(i) for i in cols] for cols in leaf_dims]
+        counts = (ctypes.c_int * max(len(dims), 1))(*[len(cols) for cols in dims])
+        flat = [i for cols in dims for i in cols]
+        cols = (ctypes.c_int * max(len(flat), 1))(*flat)
+        self.factorized = False
+        _check(self._lib, self._lib.gpso_set_active_dims(self._h, len(dims), counts, cols), "gpso_set_active_dims")
+        self.N = self.d = 0
+
     def set_data(self, x, y):
         x = np.ascontiguousarray(x, dtype=np.float64)
         y = np.ascontiguousarray(y, dtype=np.float64).reshape(-1)

@@ -286,13 +286,24 @@ struct gpso_handle {
     // plp_host), pX the embedded candidates of a window or of a joint call (row-major [M][2d]).
     bool periodic = false;
     int per_ard = 0;
-    double per_p[MAX_LS] = {0}, plp_host[MAX_SUM * 2 * MAX_LS] = {0}, unit_ls = 1.0;
+    double per_p[MAX_LS] = {0}, plp_host[2 * MAX_LS] = {0}, unit_ls = 1.0;
     // A sum / product with periodic components (gpso_create_combination): sum_per[c] marks component c as periodic (its fam is
-    // the base's) with the period ARD flag sum_per_ard[c] and its period(s) comp_p[c]; the table's off / rows / width give each
-    // component's rows (layout()).  ls then holds the unit lengthscale on a periodic component's rows, plp its [l(d), p(d)].
+    // the base's) with the period ARD flag sum_per_ard[c] and its period(s) comp_p[c]; srow's off / rows / width give each
+    // component's rows (ensure_shape).  ls then holds the unit lengthscale on a periodic component's rows, rmap its (l, p).
     int sum_per[MAX_SUM] = {0}, sum_per_ard[MAX_SUM] = {0};
     double comp_p[MAX_SUM][MAX_LS] = {{0}};
     DevBuf plp, pX;
+    // gpso_set_active_dims: leaf c (component c; a periodic leaf's base) reads the map_n[c] input columns map_cols[map_off[c] ..];
+    // nmap = 0 without a map.  A handle with a map always runs the row layout of a sum / product with periodic components: a bare
+    // kernel becomes a one-component sum (bare_kid keeps its kernel id, restored when the map is cleared).  ls_host then holds
+    // component c's lengthscales from ls_off(c), rmap describes the rows (stage_rows_kernel), Xg[N][raw.width] holds the
+    // periodic leaves' raw active columns for the gradient.
+    int nmap = 0, map_n[MAX_SUM] = {0}, map_off[MAX_SUM + 1] = {0};
+    std::vector<int> map_cols;
+    int bare_kid = -1, bare_ard = 0, bare_per_ard = 0;
+    RowMap rmap = {};
+    RawCols raw = {};
+    DevBuf Xg;
     bool have_data = false, factorized = false;
     double factor_nlml = 0.0;
     double* host_rec = nullptr;  // pinned: results of an evaluation come back in one record without staging copies
@@ -317,7 +328,7 @@ struct gpso_handle {
     bool is_product() const { return kernel_id == KERNEL_PRODUCT; }
     bool composite() const { return composite_kernel(kernel_id); }  // a sum or a product: the component table is in force
     // rows of the scaled inputs Xs per input dimension: C for a sum or a product, 2 for a periodic kernel
-    bool emb() const { return composite() && srow.pmask != 0; }  // a sum / product with periodic components
+    bool emb() const { return composite() && (srow.pmask != 0 || nmap != 0); }  // a sum / product with periodic components or a map
     bool embeds() const { return periodic || emb(); }           // the candidates are embedded before the covariance kernels
     // the covariance kernels' instantiation: a sum / product with periodic components has its own
     int cov_kid() const { return emb() ? (is_product() ? KERNEL_PRODUCT_EMB : KERNEL_SUM_EMB) : kernel_id; }
@@ -326,19 +337,21 @@ struct gpso_handle {
     int rows_for(int dd) const {
         if (!composite()) return periodic ? 2 * dd : dd;
         int r = 0;
-        for (int c = 0; c < sum.n; c++) r += sum_per[c] ? 2 * dd : dd;
+        for (int c = 0; c < sum.n; c++) r += sum_per[c] ? 2 * cdim(c, dd) : cdim(c, dd);
         return r;
     }
+    int cdim(int c, int dd) const { return nmap ? map_n[c] : dd; }  // input columns component c reads
+    int ls_off(int c) const { return nmap ? map_off[c] : c * d; }   // component c's lengthscales in ls_host
     int dx() const { return rows_for(d); }
     int cand_width() const { return emb() ? dx() : 2 * d; }  // columns of the embedded candidates (pX)
-    int comp_np(int c) const { return sum_per[c] ? (sum_per_ard[c] ? d : 1) : 0; }  // packed periods of component c
+    int comp_np(int c) const { return sum_per[c] ? (sum_per_ard[c] ? cdim(c, d) : 1) : 0; }  // packed periods of component c
     int kd() const { return periodic ? 2 * d : d; }  // the input dimension the covariance kernels are launched with
-    int n_ls() const { return composite() ? sum.n * d : (ard ? d : 1); }
+    int n_ls() const { return composite() ? ls_off(sum.n) : (ard ? d : 1); }
     int kern_nls() const { return periodic ? 1 : n_ls(); }  // lengthscales the covariance kernels read from ls
     int n_per() const { return periodic ? (per_ard ? d : 1) : 0; }  // packed periods
     double comp_var(int c) const { return is_product() ? prod_var[c] : sum.var[c]; }  // component c's own variance
     int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
-    int comp_ls(int c) const { return sum_ard[c] ? d : 1; }      // packed lengthscales of sum component c
+    int comp_ls(int c) const { return sum_ard[c] ? cdim(c, d) : 1; }  // packed lengthscales of sum component c
     // [alpha], lengthscale(s), variance, [period(s)]
     int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + 1 + comp_np(c); }
     int n_kernel_params() const {
@@ -558,20 +571,20 @@ static void launch_oz_slices(gpso_handle* h, cudaStream_t st) {
         default: fn<8>(__VA_ARGS__); break;    \
     }
 
-// The partial sums of one covariance family (a sum kernel calls this once per component, with the component's own scaled
-// inputs, variance and alpha, into its own block of partial sums).
-static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride, int kernel_id, int ard, const double* Xs, double var,
+// The partial sums of one covariance family on d scaled input rows (a sum kernel calls this once per component, with the
+// component's own scaled inputs, dimensions, variance and alpha, into its own block of partial sums).
+static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride, int kernel_id, int ard, const double* Xs, int d, double var,
                         double rq_alpha, double* part) {
     AllKernels::with(kernel_id, [&](auto kid) {
         if (!ard) {
             lml_grad_kernel<kid, false><<<nblk, 256, 0, st>>>(Xs, h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
-                                                             h->d, h->Np, var, 0, 1, part, stride, rq_alpha);
+                                                             d, h->Np, var, 0, 1, part, stride, rq_alpha);
             h->launches++;
         } else {
-            for (int dim0 = 0; dim0 < h->d; dim0 += GRAD_DCH) {
-                int nd = std::min(GRAD_DCH, h->d - dim0);
+            for (int dim0 = 0; dim0 < d; dim0 += GRAD_DCH) {
+                int nd = std::min(GRAD_DCH, d - dim0);
                 lml_grad_kernel<kid, true><<<nblk, 256, 0, st>>>(Xs, h->alpha.as<double>(), h->Kinv.as<double>(),
-                                                                h->N, h->d, h->Np, var, dim0, nd, part,
+                                                                h->N, d, h->Np, var, dim0, nd, part,
                                                                 stride, rq_alpha);
                 h->launches++;
             }
@@ -644,12 +657,12 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
     GP_TRY(h->y.ensure((size_t)Np * sizeof(double)));
     GP_TRY(h->Xs.ensure((size_t)h->rows_for(d) * Np * sizeof(double)));
     GP_TRY(h->ls.ensure(MAX_LS * sizeof(double)));
-    if (h->embeds()) GP_TRY(h->plp.ensure(MAX_SUM * 2 * MAX_LS * sizeof(double)));
-    if (h->composite()) {  // each component's rows: d, or 2d embedded rows for a periodic component
+    if (h->periodic) GP_TRY(h->plp.ensure(2 * MAX_LS * sizeof(double)));
+    if (h->composite()) {  // each component's rows: its d (active) columns, or 2d embedded rows for a periodic component
         int off = 0;
         for (int c = 0; c < h->sum.n; c++) {
             h->srow.off[c] = off;
-            h->srow.rows[c] = h->sum_per[c] ? 2 * d : d;
+            h->srow.rows[c] = h->sum_per[c] ? 2 * h->cdim(c, d) : h->cdim(c, d);
             off += h->srow.rows[c];
         }
         h->srow.width = off;
@@ -682,27 +695,26 @@ static int ensure_shape(gpso_handle* h, int N, int d) {
 }
 
 // Xs[dim][Np] = X / ls; a sum: Xs_c = X / ls_c at Xs + c d Np, the division of the bare kernel (ls_c expanded to d entries);
-// a periodic kernel: the embedded rows [cos rows; sin rows] = [2d][Np]
+// a periodic kernel: the embedded rows [cos rows; sin rows] = [2d][Np]; a sum / product with periodic components or a map: the
+// rows of rmap, one launch
 static int scale_inputs(gpso_handle* h, cudaStream_t st, const double* X, int rows, int Np, double* Xs) {
     if (h->periodic) {
         periodic_embed_kernel<<<(unsigned)(((long long)Np * h->d + 255) / 256), 256, 0, st>>>(X, rows, Np, h->d, h->plp.as<double>(), 1,
                                                                                               Np, Xs);
         return check_launch(h, "periodic_embed");
     }
+    if (h->emb()) {
+        stage_rows_kernel<<<(unsigned)(((long long)Np * h->rmap.n + 255) / 256), 256, 0, st>>>(X, rows, Np, h->d, h->rmap, 1, 1, Np, Xs);
+        return check_launch(h, "stage_rows");
+    }
     if (!h->composite()) {
         scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>(), h->n_ls(), rows, h->d, Np, Xs);
         return check_launch(h, "scale_inputs");
     }
     for (int c = 0; c < h->sum.n; c++) {
-        double* out = Xs + (size_t)h->srow.off[c] * Np;
-        if (h->sum_per[c]) {
-            periodic_embed_kernel<<<(unsigned)(((long long)Np * h->d + 255) / 256), 256, 0, st>>>(
-                X, rows, Np, h->d, h->plp.as<double>() + (size_t)c * 2 * h->d, 1, Np, out);
-            GP_TRY(check_launch(h, "periodic_embed"));
-        } else {
-            scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>() + h->srow.off[c], h->d, rows, h->d, Np, out);
-            GP_TRY(check_launch(h, "scale_inputs"));
-        }
+        scale_inputs_kernel<<<(Np + 255) / 256, 256, 0, st>>>(X, h->ls.as<double>() + c * h->d, h->d, rows, h->d, Np,
+                                                              Xs + (size_t)c * h->d * Np);
+        GP_TRY(check_launch(h, "scale_inputs"));
     }
     return 0;
 }
@@ -719,19 +731,23 @@ static int upload_lengthscales(gpso_handle* h, cudaStream_t st) {
         CU_TRY(cudaMemcpyAsync(h->plp.p, h->plp_host, sizeof(double) * 2 * h->d, cudaMemcpyHostToDevice, st));
         return 0;
     }
-    if (h->emb()) {  // ls: [width], a periodic component's rows at unit lengthscale; plp: [C][l(d), p(d)]
+    if (h->emb()) {  // ls: [width], a periodic component's rows at unit lengthscale; rmap: one slot per active column
         double lsw[MAX_LS];
-        const int d = h->d;
+        RowMap& m = h->rmap;
+        m.n = 0;
         for (int c = 0; c < h->sum.n; c++) {
-            const int o = h->srow.off[c];
-            for (int r = 0; r < h->srow.rows[c]; r++) lsw[o + r] = h->sum_per[c] ? 1.0 : h->ls_host[c * d + r];
-            for (int k = 0; k < d && h->sum_per[c]; k++) {
-                h->plp_host[c * 2 * d + k] = h->ls_host[c * d + k];
-                h->plp_host[c * 2 * d + d + k] = h->comp_p[c][h->sum_per_ard[c] ? k : 0];
+            const int o = h->srow.off[c], k = h->cdim(c, h->d), lo = h->ls_off(c);
+            for (int j = 0; j < k; j++, m.n++) {
+                m.src[m.n] = h->nmap ? h->map_cols[h->map_off[c] + j] : j;
+                m.r0[m.n] = o + j;
+                m.r1[m.n] = h->sum_per[c] ? o + k + j : -1;
+                m.l[m.n] = h->ls_host[lo + j];
+                m.p[m.n] = h->sum_per[c] ? h->comp_p[c][h->sum_per_ard[c] ? j : 0] : 0.0;
+                lsw[o + j] = h->sum_per[c] ? 1.0 : h->ls_host[lo + j];
+                if (h->sum_per[c]) lsw[o + k + j] = 1.0;
             }
         }
         CU_TRY(cudaMemcpyAsync(h->ls.p, lsw, sizeof(double) * h->dx(), cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(h->plp.p, h->plp_host, sizeof(double) * h->sum.n * 2 * d, cudaMemcpyHostToDevice, st));
         CU_TRY(cudaStreamSynchronize(st));  // lsw is on this stack frame
         return 0;
     }
@@ -1726,7 +1742,13 @@ extern "C" int gpso_set_data(gpso_handle* h, const double* X_host, const double*
     if (!h || !X_host || !y_host) return fail(GPSO_E_BADARG, "gpso_set_data: null argument");
     if (N <= 0 || d <= 0) return fail(GPSO_E_BADARG, "gpso_set_data: N and d must be positive");
     if (d > MAX_LS) return fail(GPSO_E_BADARG, "gpso_set_data: input dimension above the supported maximum (64)");
-    if (h->composite() && h->sum.n * d > MAX_LS)
+    if (h->nmap) {
+        if (h->nmap != h->sum.n) return fail(GPSO_E_BADARG, "gpso_set_data: the active dims map has a leaf count other than the kernel's");
+        for (int col : h->map_cols)
+            if (col >= d) return fail(GPSO_E_BADARG, "gpso_set_data: an active dim is not below the input dimension");
+        if (h->rows_for(d) > MAX_LS)
+            return fail(GPSO_E_BADARG, "gpso_set_data: the rows of all components (their active columns, twice for a periodic one) may not exceed 64");
+    } else if (h->composite() && h->sum.n * d > MAX_LS)
         return fail(GPSO_E_BADARG, h->is_sum() ? "gpso_set_data: a sum kernel supports components x input dimension up to 64"
                                                : "gpso_set_data: a product kernel supports factors x input dimension up to 64");
     if (h->periodic && 2 * d > MAX_LS)
@@ -1739,8 +1761,79 @@ extern "C" int gpso_set_data(gpso_handle* h, const double* X_host, const double*
     CU_TRY(cudaMemcpyAsync(h->X.p, X_host, sizeof(double) * (size_t)N * d, cudaMemcpyHostToDevice, h->stream));
     CU_TRY(cudaMemsetAsync(h->y.p, 0, sizeof(double) * h->Np, h->stream));
     CU_TRY(cudaMemcpyAsync(h->y.p, y_host, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, h->stream));
+    // the raw coordinates the periodic components' gradient reads: X itself, or with a map their active columns, gathered
+    h->raw = {};
+    h->raw.width = d;
+    std::vector<double> xg;
+    if (h->nmap) {
+        h->raw.width = 0;
+        for (int c = 0; c < h->sum.n; c++)
+            if (h->sum_per[c]) {
+                h->raw.off[c] = h->raw.width;
+                h->raw.width += h->map_n[c];
+            }
+        xg.resize((size_t)N * h->raw.width);
+        for (int i = 0; i < N; i++)
+            for (int c = 0; c < h->sum.n; c++)
+                for (int j = 0; h->sum_per[c] && j < h->map_n[c]; j++)
+                    xg[(size_t)i * h->raw.width + h->raw.off[c] + j] = X_host[(size_t)i * d + h->map_cols[h->map_off[c] + j]];
+        if (!xg.empty()) {
+            GP_TRY(h->Xg.ensure(xg.size() * sizeof(double)));
+            CU_TRY(cudaMemcpyAsync(h->Xg.p, xg.data(), xg.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        }
+    }
     CU_TRY(cudaStreamSynchronize(h->stream));
     h->have_data = true;
+    h->factorized = false;
+    return 0;
+}
+
+extern "C" int gpso_set_active_dims(gpso_handle* h, int n, const int* counts, const int* dims) {
+    if (!h) return fail(GPSO_E_BADARG, "gpso_set_active_dims: null handle");
+    if (n < 0 || n > MAX_SUM) return fail(GPSO_E_BADARG, "gpso_set_active_dims: the number of leaves must be in 0..4");
+    if (n > 0 && (!counts || !dims)) return fail(GPSO_E_BADARG, "gpso_set_active_dims: null argument");
+    int total = 0;
+    for (int c = 0; c < n; c++) {
+        if (counts[c] < 1 || counts[c] > MAX_LS) return fail(GPSO_E_BADARG, "gpso_set_active_dims: each leaf needs 1..64 columns");
+        total += counts[c];
+    }
+    for (int i = 0; i < total; i++)
+        if (dims[i] < 0) return fail(GPSO_E_BADARG, "gpso_set_active_dims: negative column index");
+    GP_TRY(set_device(h));
+    CU_TRY(cudaStreamSynchronize(h->stream));
+    if (n == 0 && h->bare_kid >= 0) {  // back to the bare kernel the map turned into a one-component sum
+        h->kernel_id = h->bare_kid;
+        h->ard = h->bare_ard;
+        h->periodic = h->sum_per[0] != 0;
+        h->per_ard = h->bare_per_ard;
+        h->sum = SumTable{};
+        h->srow = SumRows{};
+        h->sum_ard[0] = h->sum_per[0] = h->sum_per_ard[0] = 0;
+        h->bare_kid = -1;
+    } else if (n > 0 && !h->composite()) {  // a bare kernel: a one-component sum, which packs and computes as the bare kernel does
+        h->bare_kid = h->kernel_id;
+        h->bare_ard = h->ard;
+        h->bare_per_ard = h->per_ard;
+        h->sum = SumTable{};
+        h->sum.n = 1;
+        h->sum.fam[0] = h->kernel_id;
+        h->sum.var[0] = h->sum.alpha[0] = 1.0;
+        h->sum_ard[0] = h->ard;
+        h->sum_per[0] = h->periodic ? 1 : 0;
+        h->sum_per_ard[0] = h->periodic ? h->per_ard : 0;
+        h->srow.pmask = h->sum_per[0];
+        h->kernel_id = KERNEL_SUM;
+        h->ard = h->per_ard = 0;
+        h->periodic = false;
+    }
+    h->nmap = n;
+    h->map_cols.assign(dims, dims + (n ? total : 0));
+    for (int c = 0; c < MAX_SUM; c++) {
+        h->map_n[c] = c < n ? counts[c] : 0;
+        h->map_off[c + 1] = h->map_off[c] + h->map_n[c];
+    }
+    // the rows, the packed vector's length and the scaled inputs follow the map: the data has to be set again
+    h->have_data = false;
     h->factorized = false;
     return 0;
 }
@@ -1773,7 +1866,7 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
             const int nl = h->comp_ls(c);
             for (int i = 0; i < nl; i++)
                 if (!positive(theta[i])) return fail(GPSO_E_BADARG, std::string(who) + ": lengthscale must be positive");
-            for (int k = 0; k < h->d; k++) h->ls_host[c * h->d + k] = theta[nl > 1 ? k : 0];
+            for (int k = 0; k < h->cdim(c, h->d); k++) h->ls_host[h->ls_off(c) + k] = theta[nl > 1 ? k : 0];
             if (!positive(theta[nl])) return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
             if (h->is_product()) {
                 h->prod_var[c] = theta[nl];
@@ -1845,7 +1938,7 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
     int ik[MAX_SUM], il[MAX_SUM], ia[MAX_SUM], stride[MAX_SUM], off[MAX_SUM + 1] = {0};
     if (h->is_product()) off[0] = 2;
     for (int c = 0; c < h->sum.n; c++) {
-        const int nls = h->sum_per[c] ? 2 * h->d : h->comp_ls(c), rq = h->sum.fam[c] == KERNEL_RQ;
+        const int nls = h->sum_per[c] ? 2 * h->cdim(c, h->d) : h->comp_ls(c), rq = h->sum.fam[c] == KERNEL_RQ;
         stride[c] = (h->is_product() ? 0 : 2) + nls + rq;
         ik[c] = h->is_product() ? 0 : off[c];
         il[c] = h->is_product() ? off[c] : off[c] + 2;
@@ -1863,11 +1956,11 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
             ard_mask |= slot << c;
             nard += slot;
         }
-        const size_t smem = ((size_t)2 * h->dx() * CT + (h->emb() ? (size_t)2 * h->d * CT : 0) + (size_t)nard * CT * CT) * sizeof(double);
+        const size_t smem = ((size_t)2 * h->dx() * CT + (h->emb() ? (size_t)2 * h->raw.width * CT : 0) + (size_t)nard * CT * CT) * sizeof(double);
         if (h->emb())
             lml_grad_product_periodic_kernel<<<nblk, 256, smem, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(),
-                                                                      h->N, h->d, h->Np, ard_mask, h->gpart.as<double>(), total,
-                                                                      h->sum, h->X.as<double>(), h->srow);
+                                                                      h->N, h->Np, ard_mask, h->gpart.as<double>(), total, h->sum,
+                                                                      h->nmap ? h->Xg.as<double>() : h->X.as<double>(), h->srow, h->raw);
         else
             lml_grad_product_kernel<<<nblk, 256, smem, st>>>(h->Xs.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N,
                                                              h->d, h->Np, ard_mask, h->gpart.as<double>(), total, h->sum);
@@ -1878,15 +1971,17 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
         for (int c = 0; c < h->sum.n; c++) {
             double* part = h->gpart.as<double>() + (size_t)nblk * off[c];
             const double* Xs_c = h->Xs.as<double>() + (size_t)h->srow.off[c] * h->Np;
+            const int k = h->cdim(c, h->d);
             if (h->sum_per[c]) {
+                const double* Xr = h->nmap ? h->Xg.as<double>() + h->raw.off[c] : h->X.as<double>();
                 KernelIds<KERNEL_SE, KERNEL_RQ>::with(h->sum.fam[c], [&](auto kid) {
-                    lml_grad_periodic_kernel<kid><<<nblk, 256, periodic_grad_smem(h->d), st>>>(
-                        Xs_c, h->X.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N, h->d, h->Np, h->sum.var[c],
-                        h->sum.alpha[c], part, stride[c]);
+                    lml_grad_periodic_kernel<kid><<<nblk, 256, periodic_grad_smem(k), st>>>(
+                        Xs_c, Xr, h->alpha.as<double>(), h->Kinv.as<double>(), h->N, k, h->Np, h->sum.var[c], h->sum.alpha[c], part,
+                        stride[c], h->raw.width);
                 });
                 h->launches++;
             } else {
-                launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], Xs_c, h->sum.var[c], h->sum.alpha[c], part);
+                launch_grad(h, st, nblk, stride[c], h->sum.fam[c], h->sum_ard[c], Xs_c, k, h->sum.var[c], h->sum.alpha[c], part);
             }
             if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
             reduce_partials_kernel<<<stride[c], 256, 0, st>>>(part, nblk, stride[c], h->gout.as<double>() + off[c]);
@@ -1919,7 +2014,7 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
             grad_host[pos] = h->sum.alpha[c] > 0.0 ? -(0.5 * g[ia[c]]) * sigmoid(u[pos]) : 0.0;
             pos++;
         }
-        const int nl = h->comp_ls(c), np = h->comp_np(c), d = h->d;
+        const int nl = h->comp_ls(c), np = h->comp_np(c), d = h->cdim(c, h->d), lo = h->ls_off(c);
         if (h->sum_per[c]) {  // per-dimension entries L(d), Q(d) as for a bare periodic kernel (gpso_neg_lml_grad)
             const double* L = g + il[c];
             const double* Q = g + il[c] + d;
@@ -1928,12 +2023,12 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
                 Ls += L[k];
                 Qs += Q[k];
             }
-            for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * (nl > 1 ? L[i] : Ls) / h->ls_host[c * d + i]) * sigmoid(u[pos + i]);
+            for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * (nl > 1 ? L[i] : Ls) / h->ls_host[lo + i]) * sigmoid(u[pos + i]);
             for (int i = 0; i < np; i++)
                 grad_host[pos + nl + 1 + i] =
                     -(M_PI * (np > 1 ? Q[i] : Qs) / (h->comp_p[c][i] * h->comp_p[c][i])) * sigmoid(u[pos + nl + 1 + i]);
         } else {
-            for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[il[c] + i] / h->ls_host[c * d + i]) * sigmoid(u[pos + i]);
+            for (int i = 0; i < nl; i++) grad_host[pos + i] = -(0.5 * g[il[c] + i] / h->ls_host[lo + i]) * sigmoid(u[pos + i]);
         }
         pos += nl;
         const double var_c = h->comp_var(c);
@@ -1983,11 +2078,11 @@ extern "C" int gpso_neg_lml_grad(gpso_handle* h, const double* u, int p, double*
         KernelIds<KERNEL_SE, KERNEL_RQ>::with(h->kernel_id, [&](auto kid) {
             lml_grad_periodic_kernel<kid><<<nblk, 256, periodic_grad_smem(h->d), st>>>(
                 h->Xs.as<double>(), h->X.as<double>(), h->alpha.as<double>(), h->Kinv.as<double>(), h->N, h->d, h->Np, h->variance,
-                h->rq_alpha, h->gpart.as<double>(), stride);
+                h->rq_alpha, h->gpart.as<double>(), stride, h->d);
         });
         GP_TRY(check_launch(h, "lml_grad_periodic"));
     } else {
-        launch_grad(h, st, nblk, stride, h->kernel_id, h->ard, h->Xs.as<double>(), h->variance, h->rq_alpha, h->gpart.as<double>());
+        launch_grad(h, st, nblk, stride, h->kernel_id, h->ard, h->Xs.as<double>(), h->d, h->variance, h->rq_alpha, h->gpart.as<double>());
         if (cudaGetLastError() != cudaSuccess) return fail(GPSO_E_CUDA, "launch of lml_grad failed");
     }
     reduce_partials_kernel<<<stride, 256, 0, st>>>(h->gpart.as<double>(), nblk, stride, h->gout.as<double>());
@@ -2167,20 +2262,17 @@ struct WindowSpan {
 };
 
 // A periodic kernel: the embedded rows of M candidates, row-major [M][2d] in pX (the layout the cross-covariance kernels stage).
-// A sum / product with periodic components: rows of cand_width() columns, each component's at its offset -- the embedded rows of a
-// periodic component, the raw coordinates of the others.
+// A sum / product with periodic components or a map: rows of cand_width() columns, each component's at its offset -- the
+// embedded rows of a periodic component, the raw (active) coordinates of the others; one launch.
 static int embed_candidates(gpso_handle* h, cudaStream_t st, const double* Xc, long long M) {
-    const unsigned grid = (unsigned)((M * h->d + 255) / 256);
     if (h->periodic) {
-        periodic_embed_kernel<<<grid, 256, 0, st>>>(Xc, M, M, h->d, h->plp.as<double>(), 2 * h->d, 1, h->pX.as<double>());
+        periodic_embed_kernel<<<(unsigned)((M * h->d + 255) / 256), 256, 0, st>>>(Xc, M, M, h->d, h->plp.as<double>(), 2 * h->d, 1,
+                                                                                  h->pX.as<double>());
         return check_launch(h, "periodic_embed");
     }
-    for (int c = 0; c < h->sum.n; c++) {
-        const double* lp = h->sum_per[c] ? h->plp.as<double>() + (size_t)c * 2 * h->d : nullptr;
-        periodic_embed_kernel<<<grid, 256, 0, st>>>(Xc, M, M, h->d, lp, h->cand_width(), 1, h->pX.as<double>() + h->srow.off[c]);
-        GP_TRY(check_launch(h, "periodic_embed"));
-    }
-    return 0;
+    stage_rows_kernel<<<(unsigned)((M * h->rmap.n + 255) / 256), 256, 0, st>>>(Xc, M, M, h->d, h->rmap, 0, h->cand_width(), 1,
+                                                                               h->pX.as<double>());
+    return check_launch(h, "stage_rows");
 }
 
 static std::vector<WindowSpan> uniform_windows(long long M, long long W) {
@@ -3214,6 +3306,8 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 // variance, alpha, lengthscales].  A product kernel: the same, with slot 2 the prior variance var_prod and the factor variances
 // in the component block.  A periodic kernel: the kernel id is its base family's, slot 10 is 1 and slot 11 the period's ARD
 // flag, Xs holds the 2d embedded rows (2*d*Np) and the period(s) follow the lengthscale slots (STATE_PERIODS).
+// A handle with an active dims map (gpso_set_active_dims): slot 12 is its leaf count, the lengthscale and period counts of the
+// component block are those of the active columns, and the map block [leaf count, counts, columns] follows the component block.
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int STATE_HEADER = 128;
 constexpr int STATE_PERIODS = 16 + MAX_LS;  // a periodic kernel's period(s); slot 10 = 1 marks it, slot 11 = the period's ARD flag
@@ -3222,14 +3316,38 @@ constexpr int STATE_PERIODS = 16 + MAX_LS;  // a periodic kernel's period(s); sl
 static int comp_code(const gpso_handle* h, int c) { return h->sum.fam[c] + (h->sum_per[c] ? 16 : 0); }
 // the block entries of component c: family, lengthscale count, variance, alpha, lengthscales, [period count, periods]
 static int comp_block(const gpso_handle* h, int c, int d) {
-    return 4 + (h->sum_ard[c] ? d : 1) + (h->sum_per[c] ? 1 + (h->sum_per_ard[c] ? d : 1) : 0);
+    const int k = h->cdim(c, d);
+    return 4 + (h->sum_ard[c] ? k : 1) + (h->sum_per[c] ? 1 + (h->sum_per_ard[c] ? k : 1) : 0);
 }
 
 static long long sum_block_size(const gpso_handle* h, int d) {
     if (!h->composite()) return 0;
     long long n = 1;
-    for (int c = 0; c < h->sum.n; c++) n += 4 + (h->sum_ard[c] ? d : 1) + (h->sum_per[c] ? 1 + (h->sum_per_ard[c] ? d : 1) : 0);
+    for (int c = 0; c < h->sum.n; c++) n += comp_block(h, c, d);
     return n;
+}
+
+// slots 12..14 of the state header: leaf count, column count and a fingerprint of the map (exact in a double), so that a state with
+// another map is refused before its layout is read
+static void map_header(const gpso_handle* h, double* out3) {
+    long long f = 0;
+    const long long P = (1LL << 52) - 47;
+    for (int c = 0; c < h->nmap; c++) f = (f * 131 + h->map_n[c]) % P;
+    for (int col : h->map_cols) f = (f * 131 + col + 1) % P;
+    out3[0] = h->nmap;
+    out3[1] = h->nmap ? (double)h->map_cols.size() : 0.0;
+    out3[2] = (double)f;
+}
+
+static long long map_block_size(const gpso_handle* h) { return h->nmap ? 1 + h->nmap + (long long)h->map_cols.size() : 0; }
+
+static std::vector<double> map_block(const gpso_handle* h) {
+    std::vector<double> m;
+    if (!h->nmap) return m;
+    m.push_back(h->nmap);
+    for (int c = 0; c < h->nmap; c++) m.push_back(h->map_n[c]);
+    for (int col : h->map_cols) m.push_back(col);
+    return m;
 }
 
 extern "C" int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes) {
@@ -3238,7 +3356,8 @@ extern "C" int gpso_state_bytes(gpso_handle* h, int N, int d, int64_t* bytes) {
     if (h->periodic && 2 * d > MAX_LS)
         return fail(GPSO_E_BADARG, "gpso_state_bytes: a periodic kernel embeds each input dimension in 2 rows: input dimension up to 32");
     const long long dx = h->rows_for(d);
-    *bytes = (int64_t)sizeof(double) * (STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? d : 0) + sum_block_size(h, d));
+    *bytes = (int64_t)sizeof(double) * (STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? d : 0) + sum_block_size(h, d) +
+                                        map_block_size(h));
     return 0;
 }
 
@@ -3267,6 +3386,7 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
         hdr[11] = h->per_ard;
         for (int i = 0; i < h->n_per(); i++) hdr[STATE_PERIODS + i] = h->per_p[i];
     }
+    map_header(h, hdr + 12);
     double* dst = (double*)dst_dev;
     CU_TRY(cudaStreamSynchronize(h->stream));
     CU_TRY(cudaMemcpyAsync(dst, hdr, sizeof hdr, cudaMemcpyHostToDevice, st));
@@ -3283,12 +3403,14 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
         for (int c = 0; c < h->sum.n; c++) {
             const int nl = h->comp_ls(c);
             blk.insert(blk.end(), {(double)comp_code(h, c), (double)nl, h->comp_var(c), h->sum.alpha[c]});
-            for (int i = 0; i < nl; i++) blk.push_back(h->ls_host[c * h->d + i]);
+            for (int i = 0; i < nl; i++) blk.push_back(h->ls_host[h->ls_off(c) + i]);
             if (h->sum_per[c]) {  // a periodic component: its period count and period(s)
                 blk.push_back(h->comp_np(c));
                 for (int i = 0; i < h->comp_np(c); i++) blk.push_back(h->comp_p[c][i]);
             }
         }
+        const std::vector<double> mb = map_block(h);
+        blk.insert(blk.end(), mb.begin(), mb.end());
         CU_TRY(cudaMemcpyAsync(dst + STATE_HEADER + dx * Np + Np + Np * Np + (h->linear() ? h->d : 0), blk.data(),
                                sizeof(double) * blk.size(), cudaMemcpyHostToDevice, st));
     }
@@ -3301,16 +3423,22 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     if (N <= 0 || d <= 0 || d > MAX_LS || (h && h->rows_for(d) > MAX_LS))
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: bad shape");
     GP_TRY(set_device(h));
+    cudaStream_t st = (cudaStream_t)stream;
+    const double* src = (const double*)src_dev;
+    double hdr[STATE_HEADER];
+    if (bytes >= (int64_t)sizeof hdr) {  // the map decides the layout of the rest: compare it first
+        double mh[3];
+        map_header(h, mh);
+        CU_TRY(cudaMemcpyAsync(hdr, src, sizeof hdr, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
+        if (hdr[12] != mh[0] || hdr[13] != mh[1] || hdr[14] != mh[2])
+            return fail(GPSO_E_BADARG, "gpso_import_state_dev: active dims mismatch");
+    }
     int64_t need = 0;
     gpso_state_bytes(h, N, d, &need);
     if (bytes < need) return fail(GPSO_E_BADARG, "gpso_import_state_dev: source too small");
-    cudaStream_t st = (cudaStream_t)stream;
     CU_TRY(cudaStreamSynchronize(h->stream));
     GP_TRY(ensure_shape(h, N, d));
-    const double* src = (const double*)src_dev;
-    double hdr[STATE_HEADER];
-    CU_TRY(cudaMemcpyAsync(hdr, src, sizeof hdr, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
     if ((int)hdr[0] != N || (int)hdr[1] != d) return fail(GPSO_E_BADARG, "gpso_import_state_dev: header shape mismatch");
     if ((int)hdr[6] != h->kernel_id || (int)hdr[7] != h->ard) return fail(GPSO_E_BADARG, "gpso_import_state_dev: kernel mismatch");
     if ((hdr[10] == 1.0) != h->periodic || (h->periodic && (int)hdr[11] != h->per_ard))
@@ -3318,21 +3446,28 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     if (((int)hdr[9] == GPSO_MEAN_LINEAR) != h->linear())
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: linear mean function on one side only");
     const size_t dx = h->dx();
-    std::vector<double> blk(sum_block_size(h, d));
+    std::vector<double> blk(sum_block_size(h, d) + map_block_size(h));
     if (h->composite()) {
         // the component block: the same count, families and lengthscale counts (ARD flags) as this handle's, or no import
         CU_TRY(cudaMemcpyAsync(blk.data(), src + STATE_HEADER + dx * h->Np + h->Np + (size_t)h->Np * h->Np + (h->linear() ? d : 0),
                                sizeof(double) * blk.size(), cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
+        // a map: the same map as this handle's, or no import (the component block's counts depend on it, so it is compared first)
+        const std::vector<double> mb = map_block(h);
+        if (!std::equal(mb.begin(), mb.end(), blk.end() - mb.size()))
+            return fail(GPSO_E_BADARG, "gpso_import_state_dev: active dims mismatch");
         bool same = (int)blk[0] == h->sum.n;
-        for (int c = 0, q = 1; same && c < h->sum.n; q += comp_block(h, c, d), c++)
-            same = (int)blk[q] == comp_code(h, c) && (int)blk[q + 1] == (h->sum_ard[c] ? d : 1) &&
-                   (!h->sum_per[c] || (int)blk[q + 4 + (h->sum_ard[c] ? d : 1)] == (h->sum_per_ard[c] ? d : 1));
+        for (int c = 0, q = 1; same && c < h->sum.n; q += comp_block(h, c, d), c++) {
+            const int k = h->cdim(c, d);
+            same = (int)blk[q] == comp_code(h, c) && (int)blk[q + 1] == (h->sum_ard[c] ? k : 1) &&
+                   (!h->sum_per[c] || (int)blk[q + 4 + (h->sum_ard[c] ? k : 1)] == (h->sum_per_ard[c] ? k : 1));
+        }
         if (!same)
             return fail(GPSO_E_BADARG, h->is_sum() ? "gpso_import_state_dev: sum kernel component mismatch"
                                                    : "gpso_import_state_dev: product kernel component mismatch");
         for (int c = 0, q = 1; c < h->sum.n; q += comp_block(h, c, d), c++) {
-            for (int i = 0; h->sum_per[c] && i < (h->sum_per_ard[c] ? d : 1); i++) h->comp_p[c][i] = blk[q + 5 + (h->sum_ard[c] ? d : 1) + i];
+            const int k = h->cdim(c, d);
+            for (int i = 0; h->sum_per[c] && i < (h->sum_per_ard[c] ? k : 1); i++) h->comp_p[c][i] = blk[q + 5 + (h->sum_ard[c] ? k : 1) + i];
             if (h->is_product())  // the table's variances are {var_prod, 1, 1, 1}, var_prod from slot 2
                 h->prod_var[c] = blk[q + 2];
             else

@@ -444,37 +444,45 @@ __global__ void __launch_bounds__(256) lml_grad_product_kernel(const double* __r
     }
 }
 
-// A product with periodic factors (bit c of srow.pmask): lml_grad_product_kernel with factor c's rows [srow.off[c], + srow.rows[c])
-// -- a periodic factor's 2d embedded rows -- and X[N][d] holding the raw inputs (a separate kernel, so that the one above stays as
-// it is).  A periodic factor always takes a weight slot (set in ard_mask) and writes, like lml_grad_periodic_kernel, per dimension
-// j the lengthscale entry sum w ((De_j)^2 + (De_{d+j})^2) and the period entry sum w (x_j - x'_j) (e_{d+j} e'_j - e_j e'_{d+j}),
-// 2d entries before its alpha.
+// The raw coordinates of a product's periodic factors: X[N][width], factor c's from column off[c] (without active dims every
+// periodic factor reads all d columns of the inputs: width = d, off = 0).
+struct RawCols {
+    int off[MAX_SUM], width;
+};
+
+// A product on the rows of srow (periodic factors, or active dims): lml_grad_product_kernel with factor c's rows [srow.off[c],
+// + srow.rows[c]) over its k_c dimensions -- k_c rows, or a periodic factor's 2 k_c embedded rows -- and X[N][xw] holding the raw
+// coordinates the periodic factors read, factor c's k_c of them from column raw.off[c] (a separate kernel, so that the one above
+// stays as it is).  A periodic factor always takes a weight slot (set in ard_mask) and writes, like lml_grad_periodic_kernel, per
+// dimension j the lengthscale entry sum w ((De_j)^2 + (De_{k+j})^2) and the period entry sum w (x_j - x'_j) (e_{k+j} e'_j - e_j e'_{k+j}),
+// 2 k_c entries before its alpha.
 __global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const double* __restrict__ Xs, const double* __restrict__ alpha,
-                                                                        const double* __restrict__ Kinv, int N, int d, int Np,
+                                                                        const double* __restrict__ Kinv, int N, int Np,
                                                                         int ard_mask, double* __restrict__ part, int part_stride,
-                                                                        SumTable tab, const double* __restrict__ X, SumRows srow) {
+                                                                        SumTable tab, const double* __restrict__ X, SumRows srow,
+                                                                        RawCols raw) {
     int blk = blockIdx.x;
     int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
     while ((bi + 1) * (bi + 2) / 2 <= blk) bi++;
     while (bi * (bi + 1) / 2 > blk) bi--;
     int bj = blk - bi * (bi + 1) / 2;
-    const int n = tab.n, dx = srow.width;
+    const int n = tab.n, dx = srow.width, xw = raw.width;
     extern __shared__ double smg[];
     double* sXi = smg;                // [dx][64] scaled coordinates of the tile's rows
     double* sXj = smg + dx * CT;      // [dx][64] ... and of its columns
-    double* sRi = sXj + dx * CT;      // [d][64] raw coordinates of the tile's rows, then of its columns
-    double* sRj = sRi + d * CT;
-    double* sW = sRj + d * CT;        // [ARD / periodic factors][64 * 64] per-pair weights W P_-c g_c
+    double* sRi = sXj + dx * CT;      // [xw][64] raw coordinates of the tile's rows, then of its columns
+    double* sRj = sRi + xw * CT;
+    double* sW = sRj + xw * CT;       // [ARD / periodic factors][64 * 64] per-pair weights W P_-c g_c
     __shared__ double sRed[8];
     for (int e = threadIdx.x; e < dx * CT; e += 256) {
         const size_t row = (size_t)(e / CT) * Np;
         sXi[e] = Xs[row + bi * CT + e % CT];
         sXj[e] = Xs[row + bj * CT + e % CT];
     }
-    for (int e = threadIdx.x; e < d * CT; e += 256) {
+    for (int e = threadIdx.x; e < xw * CT; e += 256) {
         const int q = e / CT, t = e % CT, ri = bi * CT + t, rj = bj * CT + t;
-        sRi[e] = ri < N ? X[(size_t)ri * d + q] : 0.0;
-        sRj[e] = rj < N ? X[(size_t)rj * d + q] : 0.0;
+        sRi[e] = ri < N ? X[(size_t)ri * xw + q] : 0.0;
+        sRj[e] = rj < N ? X[(size_t)rj * xw + q] : 0.0;
     }
     __syncthreads();
     const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
@@ -545,7 +553,7 @@ __global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const do
             v = block_sum<256>(s_l[c], sRed);
             if (threadIdx.x == 0) part[(size_t)blk * part_stride + off] = v;
         }
-        const int nl = (srow.pmask >> c & 1) ? 2 * d : (ard ? d : 1);
+        const int nl = (srow.pmask >> c & 1) ? srow.rows[c] : (ard ? srow.rows[c] : 1);
         if (rq) {
             v = block_sum<256>(s_a[c], sRed);
             if (threadIdx.x == 0) part[(size_t)blk * part_stride + off + nl] = v;
@@ -557,12 +565,13 @@ __global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const do
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     for (int c = 0, slot = 0, o = 2; c < n; c++) {
         const bool ard = ard_mask >> c & 1, per = srow.pmask >> c & 1;
+        const int k = per ? srow.rows[c] / 2 : srow.rows[c];  // the factor's dimensions
         if (per) {
             const double* ws = sW + slot * CT * CT;
-            for (int q = w; q < d; q += 8) {
+            for (int q = w; q < k; q += 8) {
                 const int r = srow.off[c] + q;
-                const double *ci = sXi + r * CT, *cj = sXj + r * CT, *si = sXi + (r + d) * CT, *sj = sXj + (r + d) * CT;
-                const double *xi = sRi + q * CT, *xj = sRj + q * CT;
+                const double *ci = sXi + r * CT, *cj = sXj + r * CT, *si = sXi + (r + k) * CT, *sj = sXj + (r + k) * CT;
+                const double *xi = sRi + (raw.off[c] + q) * CT, *xj = sRj + (raw.off[c] + q) * CT;
                 double acc_l = 0.0, acc_p = 0.0;
                 for (int p = lane; p < CT * CT; p += 32) {
                     const int a = p >> 6, b = p & 63;
@@ -574,13 +583,13 @@ __global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const do
                 acc_p = warp_sum(acc_p);
                 if (lane == 0) {
                     part[(size_t)blk * part_stride + o + q] = acc_l;
-                    part[(size_t)blk * part_stride + o + d + q] = acc_p;
+                    part[(size_t)blk * part_stride + o + k + q] = acc_p;
                 }
             }
             slot++;
         } else if (ard) {
             const double* ws = sW + slot * CT * CT;
-            for (int q = w; q < d; q += 8) {
+            for (int q = w; q < k; q += 8) {
                 const int r = srow.off[c] + q;
                 const double* xi = sXi + r * CT;
                 const double* xj = sXj + r * CT;
@@ -594,7 +603,7 @@ __global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const do
             }
             slot++;
         }
-        o += (per ? 2 * d : (ard ? d : 1)) + (tab.fam[c] == KERNEL_RQ);
+        o += (per ? 2 * k : (ard ? k : 1)) + (tab.fam[c] == KERNEL_RQ);
     }
 }
 
@@ -604,8 +613,7 @@ __global__ void __launch_bounds__(256) lml_grad_product_periodic_kernel(const do
 // (chord: |e(x) - e(x')|^2 = (2 - 2 cos(theta - theta')) / (4 l^2) = sin^2((theta - theta') / 2) / l^2).  The phase is one fp64
 // sincospi(2 x / p) per coordinate; lp = [l expanded to d entries, p expanded to d entries].  out[i * s_row + r * s_dim] for rows
 // i < rows, zero for padding rows rows <= i < rows_pad (dimension-major training inputs [2d][Np], or row-major candidates
-// [M][2d]).  A NaN or infinite coordinate gives NaN rows.  lp == nullptr writes the raw coordinates to the d rows instead (the columns of
-// a sum / product's candidate rows that belong to a component that is not periodic).
+// [M][2d]).  A NaN or infinite coordinate gives NaN rows.
 __global__ void __launch_bounds__(256) periodic_embed_kernel(const double* __restrict__ X, long long rows, long long rows_pad, int d,
                                                              const double* __restrict__ lp, long long s_row, long long s_dim,
                                                              double* __restrict__ out) {
@@ -613,10 +621,6 @@ __global__ void __launch_bounds__(256) periodic_embed_kernel(const double* __res
     if (e >= rows_pad * d) return;
     const long long i = e / d;
     const int j = (int)(e - i * d);
-    if (!lp) {  // a plain component's columns of a sum / product's candidate rows: the raw coordinate (its kernel divides by l)
-        out[i * s_row + (long long)j * s_dim] = i < rows ? X[e] : 0.0;
-        return;
-    }
     double c = 0.0, s = 0.0;
     if (i < rows) {
         const double l2 = 2.0 * lp[j];
@@ -628,8 +632,44 @@ __global__ void __launch_bounds__(256) periodic_embed_kernel(const double* __res
     out[i * s_row + (long long)(d + j) * s_dim] = s;
 }
 
+// ---- the rows of a sum / product's components (KERNEL_SUM_EMB / KERNEL_PRODUCT_EMB) -------------------------------------
+// One slot per active column of each component, in component order: slot s reads input column src[s].  A plain slot writes row
+// r0[s]: the coordinate over l[s] (scale != 0: training inputs, a joint call's candidates) or the raw coordinate (scale == 0: a
+// window's candidates, which the covariance kernels divide themselves).  A periodic slot writes the embedded pair to the rows r0[s]
+// (cos) and r1[s] (sin) with periodic_embed_kernel's arithmetic, so that its rows are the same bits.
+constexpr int STAGE_SLOTS = 64;  // the rows of all components may not exceed 64, so neither may their slots
+struct RowMap {
+    int n;
+    int src[STAGE_SLOTS], r0[STAGE_SLOTS], r1[STAGE_SLOTS];  // r1 < 0: a plain slot
+    double l[STAGE_SLOTS], p[STAGE_SLOTS];
+};
+
+// out[i * s_row + r * s_dim] for the rows i < rows of X[.][d], zero for padding rows rows <= i < rows_pad
+__global__ void __launch_bounds__(256) stage_rows_kernel(const double* __restrict__ X, long long rows, long long rows_pad, int d,
+                                                         RowMap m, int scale, long long s_row, long long s_dim,
+                                                         double* __restrict__ out) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= rows_pad * m.n) return;
+    const long long i = e / m.n;
+    const int s = (int)(e - i * m.n);
+    const double x = i < rows ? X[i * d + m.src[s]] : 0.0;
+    if (m.r1[s] < 0) {
+        out[i * s_row + (long long)m.r0[s] * s_dim] = i < rows ? (scale ? x / m.l[s] : x) : 0.0;
+        return;
+    }
+    double c = 0.0, sn = 0.0;
+    if (i < rows) {
+        const double l2 = 2.0 * m.l[s];
+        sincospi(2.0 * x / m.p[s], &sn, &c);
+        c /= l2;
+        sn /= l2;
+    }
+    out[i * s_row + (long long)m.r0[s] * s_dim] = c;
+    out[i * s_row + (long long)m.r1[s] * s_dim] = sn;
+}
+
 // LML gradient of a periodic kernel: every entry in one launch.  One block per lower 64x64 tile, the tile's embedded rows
-// (Xs[2d][Np]) and raw coordinates (X[N][d]) of its rows and columns in shared memory.  Per pair W, the base covariance k and
+// (Xs[2d][Np]) and raw coordinates (the first d columns of X[N][xw]) of its rows and columns in shared memory.  Per pair W, the base covariance k and
 // g = -2 dk/dr2 are formed once; W g goes to shared memory and a second pass gives warp w the dimensions j = w, w + 8, ...:
 //   part[blk][0]         = sum W k                                                (-> d/d variance after / variance)
 //   part[blk][1]         = sum_i W_ii                                             (-> d/d noise)
@@ -641,7 +681,7 @@ template <int KID>
 __global__ void __launch_bounds__(256) lml_grad_periodic_kernel(const double* __restrict__ Xs, const double* __restrict__ X,
                                                                 const double* __restrict__ alpha, const double* __restrict__ Kinv,
                                                                 int N, int d, int Np, double var, double rq_alpha,
-                                                                double* __restrict__ part, int part_stride) {
+                                                                double* __restrict__ part, int part_stride, int xw) {
     int blk = blockIdx.x;
     int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
     while ((bi + 1) * (bi + 2) / 2 <= blk) bi++;
@@ -662,8 +702,8 @@ __global__ void __launch_bounds__(256) lml_grad_periodic_kernel(const double* __
     }
     for (int e = threadIdx.x; e < d * CT; e += 256) {
         const int q = e / CT, t = e % CT, ri = bi * CT + t, rj = bj * CT + t;
-        sRi[e] = ri < N ? X[(size_t)ri * d + q] : 0.0;
-        sRj[e] = rj < N ? X[(size_t)rj * d + q] : 0.0;
+        sRi[e] = ri < N ? X[(size_t)ri * xw + q] : 0.0;
+        sRj[e] = rj < N ? X[(size_t)rj * xw + q] : 0.0;
     }
     __syncthreads();
     const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;

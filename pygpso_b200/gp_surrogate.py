@@ -620,6 +620,10 @@ class GPRSurrogate(GPSurrogate):
                 for k in model.kernel.kernels]
         if periodic:  # base family and the shape of the period; gpr_kernel_shape is the base lengthscales'
             save_info["gpr_kernel_periodic"] = [leaf.__class__.__name__, model.kernel.period.shape.as_list()]
+        leaves = model.kernel.kernels if is_sum else [model.kernel]
+        if any(gpmodel._active_dims_given(k.active_dims) for k in leaves):  # per leaf: its resolved columns, or null
+            save_info["gpr_kernel_active_dims"] = [
+                list(dims) if gpmodel._active_dims_given(k.active_dims) else None for k, dims in zip(leaves, model._leaf_dims)]
         with open(os.path.join(folder, self.GPR_INFO), "w") as handle:
             handle.write(json.dumps(save_info))
 
@@ -645,6 +649,10 @@ class GPRSurrogate(GPSurrogate):
                                                  period=np.ones(period_shape))
         else:
             gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
+        if "gpr_kernel_active_dims" in info:
+            leaves = gp_kernel.kernels if isinstance(gp_kernel, gpmodel.Combination) else [gp_kernel]
+            for k, dims in zip(leaves, info["gpr_kernel_active_dims"]):
+                k.active_dims = dims
         assert hasattr(gpmodel.mean_functions, info["gpr_meanf"])
         meanf_cls = getattr(gpmodel.mean_functions, info["gpr_meanf"])
         if meanf_cls is gpmodel.Constant:

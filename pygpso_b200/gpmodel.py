@@ -22,6 +22,11 @@ mean_function.c (or mean_function.A, mean_function.b for ``Linear``) -- preceded
 (tf.Module visits attributes in sorted name order).  A ``Sum`` (``Product``) kernel lists its components' (factors')
 parameters in component order, each component's in that same sorted order.  A ``Periodic`` kernel lists its base kernel's
 parameters, then kernel.period ('base_kernel' < 'period').
+
+A stationary kernel acts on the input columns ``active_dims`` (GPflow's keyword: None for all of them, a slice, or a list of
+column indices in the order given, repeats allowed); a ``Periodic`` kernel's are its base kernel's.  ARD lengthscales (and an ARD
+period) then have one entry per active column.  ``active_dims`` is not a parameter: it is resolved against the inputs when data is
+set, and the model passes the column map to the backend only when some kernel does not read every column in order.
 """
 import types
 
@@ -123,6 +128,39 @@ class Parameter:
 # kernels / mean functions / likelihood
 # ---------------------------------------------------------------------------------------------------------------------
 MAX_SUM = 4  # GPSO_MAX_SUM: components of a Sum kernel, factors of a Product kernel
+MAX_ROWS = 64  # rows of a kernel with active dims: each component's active columns, twice for a periodic one
+
+
+def _active_dims_value(active_dims):
+    """``active_dims`` as GPflow stores it: a slice (None is ``slice(None)``) or a 1-D int ndarray."""
+    if active_dims is None:
+        return slice(None)
+    if isinstance(active_dims, slice):
+        return active_dims
+    dims = np.asarray(active_dims)
+    if dims.ndim != 1 or (dims.size and not np.issubdtype(dims.dtype, np.integer)):
+        raise ValueError(f"active_dims must be None, a slice or a 1-D list of integer column indices, got {active_dims!r}")
+    return dims.astype(np.int64)
+
+
+def _active_dims_given(active_dims):
+    """False for ``slice(None)``, the columns of a kernel that was given no ``active_dims``."""
+    return not (isinstance(active_dims, slice) and active_dims == slice(None))
+
+
+def _resolve_active_dims(active_dims, d):
+    """The column list a kernel reads from d-dimensional inputs (numpy slicing / tf.gather semantics); ValueError when empty or
+    out of range."""
+    if isinstance(active_dims, slice):
+        dims = list(range(d))[active_dims]
+    else:
+        dims = [int(i) for i in active_dims]
+        bad = [i for i in dims if not 0 <= i < d]
+        if bad:
+            raise ValueError(f"active_dims {dims} has entries outside [0, {d}) for {d}-dimensional inputs")
+    if not dims:
+        raise ValueError(f"active_dims {active_dims!r} selects no column of the {d}-dimensional inputs")
+    return dims
 
 
 class Kernel:
@@ -134,11 +172,20 @@ class Kernel:
 
 
 class Stationary(Kernel):
-    """Isotropic / ARD stationary kernel; ``lengthscales`` scalar or one per dimension."""
+    """Isotropic / ARD stationary kernel; ``lengthscales`` scalar or one per active dimension."""
 
-    def __init__(self, variance=1.0, lengthscales=1.0):
+    def __init__(self, variance=1.0, lengthscales=1.0, active_dims=None):
         self.variance = Parameter(variance, positive=True, name="kernel.variance")
         self.lengthscales = Parameter(lengthscales, positive=True, name="kernel.lengthscales")
+        self.active_dims = active_dims
+
+    @property
+    def active_dims(self):
+        return self._active_dims
+
+    @active_dims.setter
+    def active_dims(self, value):
+        self._active_dims = _active_dims_value(value)
 
     @property
     def ard(self):
@@ -214,8 +261,8 @@ class RationalQuadratic(Stationary):
     """``gpflow.kernels.RationalQuadratic``: ``variance * (1 + r2 / (2 alpha))^-alpha``, a scale mixture of squared
     exponentials; ``alpha`` (positive, softplus) sets how heavy the tail is, alpha -> inf gives the SquaredExponential."""
 
-    def __init__(self, variance=1.0, lengthscales=1.0, alpha=1.0):
-        super().__init__(variance=variance, lengthscales=lengthscales)
+    def __init__(self, variance=1.0, lengthscales=1.0, alpha=1.0, active_dims=None):
+        super().__init__(variance=variance, lengthscales=lengthscales, active_dims=active_dims)
         self.alpha = Parameter(alpha, positive=True, name="kernel.alpha")
         if self.alpha.size != 1:
             raise ValueError("alpha must be a scalar")
@@ -243,6 +290,15 @@ class Periodic(Kernel):
         self.period = Parameter(period, positive=True, name="kernel.period")
         if len(self.period.shape) > 1:
             raise ValueError(f"period must be a scalar or a vector, got shape {tuple(self.period.shape)}")
+
+    @property
+    def active_dims(self):
+        """The base kernel's (GPflow 2's Periodic has none of its own): the phase uses those columns only."""
+        return self.base_kernel.active_dims
+
+    @active_dims.setter
+    def active_dims(self, value):
+        self.base_kernel.active_dims = value
 
     @property
     def parameters(self):
@@ -369,6 +425,7 @@ class GPR(GPModel):
             )
         self._factor_key = None
         self.n_loss_evaluations = 0
+        self._active_map = None  # the column map in force in the session (None: every leaf reads all columns in order)
         self.data = data
 
     # -- data ---------------------------------------------------------------------------------------------------------
@@ -383,17 +440,32 @@ class GPR(GPModel):
         y = np.ascontiguousarray(y, dtype=np.float64)
         if x.ndim != 2 or y.ndim != 2 or y.shape != (x.shape[0], 1):
             raise ValueError(f"data must be (X[N,d], Y[N,1]); got {x.shape}, {y.shape}")
-        for k in self.kernel.kernels if isinstance(self.kernel, Combination) else [self.kernel]:
+        leaves = self.kernel.kernels if isinstance(self.kernel, Combination) else [self.kernel]
+        leaf_dims = [_resolve_active_dims(k.active_dims, x.shape[1]) for k in leaves]
+        for k, dims in zip(leaves, leaf_dims):
             if isinstance(k, Periodic):
-                if k.period.size not in (1, x.shape[1]):
-                    raise ValueError("an ARD period must have one entry per input dimension")
+                if k.period.size not in (1, len(dims)):
+                    raise ValueError("an ARD period must have one entry per input dimension"
+                                     + (f" ({len(dims)} active)" if len(dims) != x.shape[1] else ""))
                 k = k.base_kernel
-            if k.lengthscales.size not in (1, x.shape[1]):
-                raise ValueError("ARD lengthscales must have one entry per input dimension")
+            if k.lengthscales.size not in (1, len(dims)):
+                raise ValueError("ARD lengthscales must have one entry per input dimension"
+                                 + (f" ({len(dims)} active)" if len(dims) != x.shape[1] else ""))
+        identity = list(range(x.shape[1]))
+        active_map = None if all(dims == identity for dims in leaf_dims) else leaf_dims
+        if active_map is not None:
+            rows = sum(len(dims) * (2 if isinstance(k, Periodic) else 1) for k, dims in zip(leaves, leaf_dims))
+            if rows > MAX_ROWS:
+                raise ValueError(f"the kernel needs {rows} rows (the active columns of each component, twice for a periodic one); "
+                                 f"at most {MAX_ROWS} are supported")
         if isinstance(self.mean_function, Linear) and self.mean_function.A.shape[0] != x.shape[1]:
             raise ValueError(f"Linear mean function: A must have shape [{x.shape[1]}, 1] for {x.shape[1]}-dimensional inputs, "
                              f"got {list(self.mean_function.A.shape)}")
+        if active_map != self._active_map:  # a new map, or back to none (the session then drops its data)
+            self._session.set_active_dims(active_map)
+            self._active_map = active_map
         self._data = (x, y)
+        self._leaf_dims = leaf_dims
         self._session.set_data(x, y)
         self._factor_key = None
 
