@@ -71,6 +71,15 @@ enum { GPSO_KERNEL_PRODUCT = 6 };
  * over 2 l_j).  Created with gpso_create_periodic (gpso_create refuses it); the input dimension d may not exceed 32.  The prior
  * variance k(x, x) is the base variance. */
 enum { GPSO_KERNEL_PERIODIC = 7 };
+/* GPSO_KERNEL_LINEAR = gpflow.kernels.Linear: k(x, x') = sum_j var_j x_j x'_j over the (active) columns, one variance (ard = 0) or
+ * one per column (ard = 1); it packs [variance(s)] only.  gpso_create opens it bare; gpso_create_combination takes it as a
+ * component of kind GPSO_KERNEL_SUM and refuses it in a product.  It is not stationary: the prior variance k(x, x) differs per
+ * candidate, and the predict finalise, the arg-max and the joint posterior's diagonal read each candidate's own value.  A handle
+ * with a Linear term scores on the FP64 engines only: the automatic predict mode picks the FP64 DMMA product, and predict mode 2
+ * and screen modes 2..6 are refused with GPSO_E_BADARG (the int8 slices and the screen are scaled by a bound on |k*| that a
+ * Linear term does not have); screen mode 1 runs the exact unscreened pass.  The exported state of a bare Linear kernel carries
+ * this id in its kernel-id slot, a sum's component block the code 10 for a Linear component. */
+enum { GPSO_KERNEL_LINEAR = 10 };
 /* gpflow.mean_functions.*: None/Zero or Constant (:167, :427), or Linear (m(x) = x . A + b, A[d,1] and b unconstrained) */
 enum { GPSO_MEAN_ZERO = 0, GPSO_MEAN_CONSTANT = 1, GPSO_MEAN_LINEAR = 2 };
 

@@ -14,6 +14,7 @@ import numpy as np
 
 KERNEL_IDS = {"Matern12": 0, "Matern32": 1, "Matern52": 2, "SquaredExponential": 3, "RationalQuadratic": 4}
 KERNEL_PERIODIC = 7  # GPSO_KERNEL_PERIODIC
+KERNEL_LINEAR = 10  # GPSO_KERNEL_LINEAR (gpflow.kernels.Linear)
 _LIB_NAME = "libgpso_b200.so"
 _ABI_VERSION = 1
 
@@ -193,7 +194,8 @@ class CudaSession:
         """``components``: for ``kernel="Sum"`` (``"Product"``) the list ``[(family, n_lengthscales), ...]`` of the sum's
         components (the product's factors), ``("Periodic", n_lengthscales, base family, n_periods)`` for a periodic one; for
         ``kernel="Periodic"`` the one entry ``[(base family, n_periods)]``, the base
-        being SquaredExponential or RationalQuadratic with ``n_lengthscales`` lengthscales."""
+        being SquaredExponential or RationalQuadratic with ``n_lengthscales`` lengthscales.  A sum's component may be
+        ``("Linear", n_variances)``; ``kernel="Linear"`` is a bare Linear kernel with ``n_lengthscales`` variances."""
         self._lib = lib
         self.device = device
         self.kernel = kernel
@@ -203,16 +205,19 @@ class CudaSession:
         handle = ctypes.c_void_p()
         if kernel in ("Sum", "Product"):
             def known(c):
-                return c[0] in KERNEL_IDS or (c[0] == "Periodic" and len(c) == 4 and c[2] in ("SquaredExponential", "RationalQuadratic"))
+                return (c[0] in KERNEL_IDS or (c[0] == "Periodic" and len(c) == 4 and c[2] in ("SquaredExponential", "RationalQuadratic"))
+                        or (c[0] == "Linear" and len(c) == 2))
             if not components or not all(known(c) for c in components):
                 raise ValueError(f"a {kernel} session needs components from {sorted(KERNEL_IDS)} or periodic ones, got {components!r}")
             self.components = [tuple(c) for c in components]
             self.ard = False
             n = len(self.components)
             periodic = [c[0] == "Periodic" for c in self.components]
-            ids = (ctypes.c_int * n)(*[KERNEL_PERIODIC if p else KERNEL_IDS[c[0]] for c, p in zip(self.components, periodic)])
+            linear = [c[0] == "Linear" for c in self.components]
+            ids = (ctypes.c_int * n)(*[KERNEL_PERIODIC if p else KERNEL_LINEAR if lin else KERNEL_IDS[c[0]]
+                                       for c, p, lin in zip(self.components, periodic, linear)])
             ards = (ctypes.c_int * n)(*[int(c[1] > 1) for c in self.components])
-            if any(periodic):
+            if any(periodic) or any(linear):
                 bases = (ctypes.c_int * n)(*[KERNEL_IDS[c[2]] if p else 0 for c, p in zip(self.components, periodic)])
                 pards = (ctypes.c_int * n)(*[int(c[3] > 1) if p else 0 for c, p in zip(self.components, periodic)])
                 kind = 5 if kernel == "Sum" else 6
@@ -230,6 +235,9 @@ class CudaSession:
             self.ard = n_lengthscales > 1
             _check(lib, lib.gpso_create_periodic(device, KERNEL_IDS[base], int(self.ard), int(n_periods > 1), self.mean_id,
                                                  ctypes.byref(handle)), "gpso_create_periodic")
+        elif kernel == "Linear":
+            self.ard = n_lengthscales > 1
+            _check(lib, lib.gpso_create(device, KERNEL_LINEAR, int(self.ard), self.mean_id, ctypes.byref(handle)), "gpso_create")
         else:
             if kernel not in KERNEL_IDS:
                 raise ValueError(f"unsupported kernel {kernel!r}; choose from {sorted(KERNEL_IDS)}, Sum or Product")

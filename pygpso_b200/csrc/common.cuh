@@ -416,6 +416,13 @@ constexpr int KERNEL_PRODUCT = 6;
 // its family is its base's), and the candidates as rows of the table's width.  Internal ids: the C ABI's id 7 is the periodic kernel.
 constexpr int KERNEL_SUM_EMB = 8;
 constexpr int KERNEL_PRODUCT_EMB = 9;
+// A sum with Linear terms (gpflow.kernels.Linear, k(x, x') = sum_r var_r x_r x'_r: not stationary, so k(x, x) depends on x): the
+// row layout of KERNEL_SUM_EMB, its own instantiations of gram_kernel, crosscov_kernel and joint_syrk_kernel.  A Linear component
+// has the family KERNEL_LINEAR (the C ABI's GPSO_KERNEL_LINEAR) in the table, and its rows are its (active) columns divided by the
+// "lengthscale" 1 / sqrt(var_r), so that its covariance is the plain dot product of its rows (sum_r (x_r / l_r)(x'_r / l_r)) and
+// k(x, x) the squared norm of x's.
+constexpr int KERNEL_LINEAR = 10;
+constexpr int KERNEL_SUM_LIN = 11;
 __host__ __device__ constexpr bool embedded_composite(int kid) { return kid == KERNEL_SUM_EMB || kid == KERNEL_PRODUCT_EMB; }
 __host__ __device__ constexpr bool product_kernel(int kid) { return kid == KERNEL_PRODUCT || kid == KERNEL_PRODUCT_EMB; }
 __host__ __device__ constexpr bool composite_kernel(int kid) {

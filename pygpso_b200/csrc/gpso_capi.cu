@@ -301,6 +301,11 @@ struct gpso_handle {
     int nmap = 0, map_n[MAX_SUM] = {0}, map_off[MAX_SUM + 1] = {0};
     std::vector<int> map_cols;
     int bare_kid = -1, bare_ard = 0, bare_per_ard = 0;
+    // GPSO_KERNEL_LINEAR: a Linear component has the family KERNEL_LINEAR (bit c of lin_mask); ls_host holds its variance(s) where a
+    // stationary component's lengthscales go, and its rows are its (active) columns over 1 / sqrt(variance) (common.cuh).  A bare
+    // Linear kernel is a one-component sum from the start (bare_lin), with or without a map.
+    int lin_mask = 0;
+    bool bare_lin = false;
     RowMap rmap = {};
     RawCols raw = {};
     DevBuf Xg;
@@ -328,10 +333,12 @@ struct gpso_handle {
     bool is_product() const { return kernel_id == KERNEL_PRODUCT; }
     bool composite() const { return composite_kernel(kernel_id); }  // a sum or a product: the component table is in force
     // rows of the scaled inputs Xs per input dimension: C for a sum or a product, 2 for a periodic kernel
-    bool emb() const { return composite() && (srow.pmask != 0 || nmap != 0); }  // a sum / product with periodic components or a map
+    bool emb() const { return composite() && (srow.pmask != 0 || nmap != 0 || lin_mask != 0); }
+    bool has_lin() const { return lin_mask != 0; }
+    bool comp_lin(int c) const { return lin_mask >> c & 1; }  // a sum / product with periodic components or a map
     bool embeds() const { return periodic || emb(); }           // the candidates are embedded before the covariance kernels
     // the covariance kernels' instantiation: a sum / product with periodic components has its own
-    int cov_kid() const { return emb() ? (is_product() ? KERNEL_PRODUCT_EMB : KERNEL_SUM_EMB) : kernel_id; }
+    int cov_kid() const { return has_lin() ? KERNEL_SUM_LIN : emb() ? (is_product() ? KERNEL_PRODUCT_EMB : KERNEL_SUM_EMB) : kernel_id; }
     // rows of the scaled inputs Xs for input dimension dd: [C][d] for a sum or a product (2d for a periodic component), [2][d]
     // for a periodic kernel
     int rows_for(int dd) const {
@@ -351,9 +358,9 @@ struct gpso_handle {
     int n_per() const { return periodic ? (per_ard ? d : 1) : 0; }  // packed periods
     double comp_var(int c) const { return is_product() ? prod_var[c] : sum.var[c]; }  // component c's own variance
     int n_rq() const { return kernel_id == KERNEL_RQ ? 1 : 0; }  // alpha leads the packed vector (GPflow's sorted names)
-    int comp_ls(int c) const { return sum_ard[c] ? cdim(c, d) : 1; }  // packed lengthscales of sum component c
-    // [alpha], lengthscale(s), variance, [period(s)]
-    int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + 1 + comp_np(c); }
+    int comp_ls(int c) const { return sum_ard[c] ? cdim(c, d) : 1; }  // packed lengthscales of sum component c (Linear: variances)
+    // [alpha], lengthscale(s), variance, [period(s)]; a Linear component: variance(s)
+    int comp_params(int c) const { return (sum.fam[c] == KERNEL_RQ) + comp_ls(c) + (comp_lin(c) ? 0 : 1) + comp_np(c); }
     int n_kernel_params() const {
         if (!composite()) return n_rq() + n_ls() + 1 + n_per();
         int n = 0;
@@ -433,9 +440,14 @@ using AllKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, 
 using CovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM, KERNEL_PRODUCT,
                              KERNEL_SUM_EMB, KERNEL_PRODUCT_EMB>;
 
+// gram_kernel, crosscov_kernel and joint_syrk_kernel also have the KERNEL_SUM_LIN instantiation (a sum with Linear terms); the
+// other covariance kernels do not (such a handle never screens nor runs the int8 variance product)
+using FullCovKernels = KernelIds<KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SE, KERNEL_RQ, KERNEL_SUM, KERNEL_PRODUCT,
+                                 KERNEL_SUM_EMB, KERNEL_PRODUCT_EMB, KERNEL_SUM_LIN>;
+
 static void launch_gram(gpso_handle* h, cudaStream_t st) {
     dim3 grid(h->Np / CT, h->Np / CT);
-    CovKernels::with(h->cov_kid(), [&](auto kid) {
+    FullCovKernels::with(h->cov_kid(), [&](auto kid) {
         gram_kernel<kid><<<grid, 256, 0, st>>>(h->Xs.as<double>(), h->N, h->kd(), h->Np, h->variance, h->noise, h->K.as<double>(),
                                                h->rq_alpha, h->sum, h->srow);
     });
@@ -443,7 +455,7 @@ static void launch_gram(gpso_handle* h, cudaStream_t st) {
 
 static void launch_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, long long Mw, long long Mw_pad) {
     size_t sm = (size_t)(XG * h->dx() + 8 * XG) * sizeof(double);
-    CovKernels::with(h->cov_kid(), [&](auto kid) {
+    FullCovKernels::with(h->cov_kid(), [&](auto kid) {
         crosscov_kernel<kid><<<(unsigned)(Mw_pad / XG), 256, sm, st>>>(Xc, Mw, h->kd(), h->ls.as<double>(), h->kern_nls(), h->Xs.as<double>(),
                                                                       h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
                                                                       h->KsT.as<double>(), h->wmeanb[0].as<double>(), h->rq_alpha,
@@ -594,6 +606,8 @@ static void launch_grad(gpso_handle* h, cudaStream_t st, int nblk, int stride, i
 
 static size_t periodic_grad_smem(int d) { return (size_t)(6 * d * CT + CT * CT) * sizeof(double); }
 static const int PERIODIC_GRAD_SMEM_MAX = (int)periodic_grad_smem(MAX_LS / 2);
+static size_t linear_grad_smem(int k) { return (size_t)(2 * k * CT + CT * CT) * sizeof(double); }
+static const int LINEAR_GRAD_SMEM_MAX = (int)linear_grad_smem(MAX_LS);
 
 // Function attributes (dynamic shared-memory limits, carve-out preferences) belong to the device's primary context: set once per
 // device and process, not per handle (the ~90 cudaFuncSetAttribute calls cost 0.3 s per gpso_create).
@@ -626,6 +640,9 @@ static int configure_kernels() {
     // a periodic kernel of up to 32 dimensions: 64 embedded and 32 raw coordinate rows of the tile's rows and columns, the pair weights
     CU_TRY(cudaFuncSetAttribute(lml_grad_periodic_kernel<KERNEL_SE>, cudaFuncAttributeMaxDynamicSharedMemorySize, PERIODIC_GRAD_SMEM_MAX));
     CU_TRY(cudaFuncSetAttribute(lml_grad_periodic_kernel<KERNEL_RQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, PERIODIC_GRAD_SMEM_MAX));
+    CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<KERNEL_SUM_LIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    // a Linear component of up to 64 columns: its rows for the tile's rows and columns, the pair weights
+    CU_TRY(cudaFuncSetAttribute(lml_grad_linear_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LINEAR_GRAD_SMEM_MAX));
     GP_TRY(CovKernels::each([](auto kid) -> int {
         CU_TRY(cudaFuncSetAttribute(joint_syrk_kernel<kid>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
         CU_TRY(cudaFuncSetAttribute(crosscov_screen_kernel<kid, 0, SCR_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_XCOV_SMEM_MAX));
@@ -741,9 +758,11 @@ static int upload_lengthscales(gpso_handle* h, cudaStream_t st) {
                 m.src[m.n] = h->nmap ? h->map_cols[h->map_off[c] + j] : j;
                 m.r0[m.n] = o + j;
                 m.r1[m.n] = h->sum_per[c] ? o + k + j : -1;
-                m.l[m.n] = h->ls_host[lo + j];
+                // a Linear component's rows: its columns over 1 / sqrt(variance)
+                const double l = h->comp_lin(c) ? 1.0 / sqrt(h->ls_host[lo + j]) : h->ls_host[lo + j];
+                m.l[m.n] = l;
                 m.p[m.n] = h->sum_per[c] ? h->comp_p[c][h->sum_per_ard[c] ? j : 0] : 0.0;
-                lsw[o + j] = h->sum_per[c] ? 1.0 : h->ls_host[lo + j];
+                lsw[o + j] = h->sum_per[c] ? 1.0 : l;
                 if (h->sum_per[c]) lsw[o + k + j] = 1.0;
             }
         }
@@ -1492,7 +1511,8 @@ static int prepare_ozaki(gpso_handle* h, cudaStream_t st) {
     h->oz_est = 0.0;
     h->screen_ready = false;
     h->screen_built_S = 0;
-    bool want = h->predict_mode == 2 || (h->predict_mode == 0 && h->Np >= OZ_MIN_NP);
+    // a kernel with Linear terms: the FP64 DMMA product (the int8 slices are scaled by a bound on |k*| that it does not have)
+    bool want = !h->has_lin() && (h->predict_mode == 2 || (h->predict_mode == 0 && h->Np >= OZ_MIN_NP));
     if (!want || h->Np > OZ_MAX_NP) return 0;
     const int Np = h->Np;
     GP_TRY(h->rowscale.ensure((size_t)Np * sizeof(double)));
@@ -1597,8 +1617,19 @@ extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso
     if (!out) return fail(GPSO_E_BADARG, "gpso_create: out is null");
     *out = nullptr;
     // GPSO_KERNEL_SUM and GPSO_KERNEL_PRODUCT have components: gpso_create_sum, gpso_create_product
-    if (kernel_id < 0 || kernel_id > KERNEL_RQ) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
+    if ((kernel_id < 0 || kernel_id > KERNEL_RQ) && kernel_id != GPSO_KERNEL_LINEAR) return fail(GPSO_E_BADARG, "gpso_create: unknown kernel id");
     if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, "gpso_create: unknown mean id");
+    if (kernel_id == GPSO_KERNEL_LINEAR) {  // a one-component sum from the start: the row layout of a sum with Linear terms
+        if (ard != 0 && ard != 1) return fail(GPSO_E_BADARG, "gpso_create: the Linear kernel's ard flag must be 0 or 1");
+        SumTable tab = {};
+        tab.n = 1;
+        tab.fam[0] = KERNEL_LINEAR;
+        tab.var[0] = tab.alpha[0] = 1.0;
+        GP_TRY(create_handle(device, KERNEL_SUM, 0, mean_id, tab, &ard, out));
+        (*out)->lin_mask = 1;
+        (*out)->bare_lin = true;
+        return 0;
+    }
     return create_handle(device, kernel_id, ard, mean_id, SumTable{}, nullptr, out);
 }
 
@@ -1606,7 +1637,8 @@ extern "C" int gpso_create(int device, int kernel_id, int ard, int mean_id, gpso
 // families, ARD flags 0 / 1; with base_ids (gpso_create_combination only) a component of id GPSO_KERNEL_PERIODIC is periodic with
 // the base base_ids[c] (SE or RQ) and the period ARD flag period_ard[c].
 static int component_table(const char* who, int n, const int* kernel_ids, const int* ard, int mean_id, gpso_handle** out,
-                           SumTable& tab, const int* base_ids = nullptr, const int* period_ard = nullptr, int* pmask = nullptr) {
+                           SumTable& tab, const int* base_ids = nullptr, const int* period_ard = nullptr, int* pmask = nullptr,
+                           int* lmask = nullptr) {
     const std::string w(who);
     if (!out) return fail(GPSO_E_BADARG, w + ": out is null");
     *out = nullptr;
@@ -1615,20 +1647,23 @@ static int component_table(const char* who, int n, const int* kernel_ids, const 
     if (mean_id < GPSO_MEAN_ZERO || mean_id > GPSO_MEAN_LINEAR) return fail(GPSO_E_BADARG, w + ": unknown mean id");
     tab = {};
     tab.n = n;
-    int pm = 0;
+    int pm = 0, lm = 0;
     for (int c = 0; c < n; c++) {
         const bool per = base_ids && kernel_ids[c] == GPSO_KERNEL_PERIODIC;
-        if (!per && (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ)) return fail(GPSO_E_BADARG, w + ": unknown component kernel id");
+        const bool lin = lmask && kernel_ids[c] == GPSO_KERNEL_LINEAR;
+        if (!per && !lin && (kernel_ids[c] < 0 || kernel_ids[c] > KERNEL_RQ)) return fail(GPSO_E_BADARG, w + ": unknown component kernel id");
         if (per && base_ids[c] != KERNEL_SE && base_ids[c] != KERNEL_RQ)
             return fail(GPSO_E_BADARG, w + ": a periodic component's base must be SquaredExponential or RationalQuadratic");
         if ((ard[c] != 0 && ard[c] != 1) || (per && period_ard[c] != 0 && period_ard[c] != 1))
             return fail(GPSO_E_BADARG, w + ": ard flags must be 0 or 1");
         tab.fam[c] = per ? base_ids[c] : kernel_ids[c];
         pm |= per ? 1 << c : 0;
+        lm |= lin ? 1 << c : 0;
         tab.var[c] = 1.0;
         tab.alpha[c] = 1.0;
     }
     if (pmask) *pmask = pm;
+    if (lmask) *lmask = lm;
     return 0;
 }
 
@@ -1648,10 +1683,18 @@ extern "C" int gpso_create_combination(int device, int kind, int n, const int* k
         if (out) *out = nullptr;
         return fail(GPSO_E_BADARG, "gpso_create_combination: null argument");
     }
+    if (kind == KERNEL_PRODUCT && kernel_ids && n >= 1 && n <= MAX_SUM)
+        for (int c = 0; c < n; c++)
+            if (kernel_ids[c] == GPSO_KERNEL_LINEAR) {
+                if (out) *out = nullptr;
+                return fail(GPSO_E_BADARG, "gpso_create_combination: a Linear kernel cannot be a factor of a product");
+            }
     SumTable tab;
-    int pmask = 0;
-    GP_TRY(component_table("gpso_create_combination", n, kernel_ids, ard, mean_id, out, tab, base_ids, period_ard, &pmask));
+    int pmask = 0, lmask = 0;
+    GP_TRY(component_table("gpso_create_combination", n, kernel_ids, ard, mean_id, out, tab, base_ids, period_ard, &pmask,
+                           kind == KERNEL_SUM ? &lmask : nullptr));
     GP_TRY(create_handle(device, kind, 0, mean_id, tab, ard, out, pmask));
+    (*out)->lin_mask = lmask;
     for (int c = 0; c < n; c++) (*out)->sum_per_ard[c] = (pmask >> c & 1) ? period_ard[c] : 0;
     return 0;
 }
@@ -1864,6 +1907,14 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
                 h->sum.alpha[c] = *theta++;
             }
             const int nl = h->comp_ls(c);
+            if (h->comp_lin(c)) {  // variance(s) only, held on the component's rows; the constant part of the prior variance is the others'
+                for (int i = 0; i < nl; i++)
+                    if (!positive(theta[i])) return fail(GPSO_E_BADARG, std::string(who) + ": variances must be positive");
+                for (int k = 0; k < h->cdim(c, h->d); k++) h->ls_host[h->ls_off(c) + k] = theta[nl > 1 ? k : 0];
+                h->sum.var[c] = theta[0];
+                theta += nl;
+                continue;
+            }
             for (int i = 0; i < nl; i++)
                 if (!positive(theta[i])) return fail(GPSO_E_BADARG, std::string(who) + ": lengthscale must be positive");
             for (int k = 0; k < h->cdim(c, h->d); k++) h->ls_host[h->ls_off(c) + k] = theta[nl > 1 ? k : 0];
@@ -1873,7 +1924,7 @@ static int load_theta(gpso_handle* h, const double* theta, int p, const char* wh
                 var_tot = (c == 0) ? theta[nl] : var_tot * theta[nl];
             } else {
                 h->sum.var[c] = theta[nl];
-                var_tot = (c == 0) ? theta[nl] : var_tot + theta[nl];
+                var_tot = (var_tot == 0.0) ? theta[nl] : var_tot + theta[nl];
             }
             for (int i = 0; i < h->comp_np(c); i++) {  // a periodic component's period(s) follow its variance
                 if (!positive(theta[nl + 1 + i])) return fail(GPSO_E_BADARG, std::string(who) + ": period must be positive");
@@ -1938,7 +1989,9 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
     int ik[MAX_SUM], il[MAX_SUM], ia[MAX_SUM], stride[MAX_SUM], off[MAX_SUM + 1] = {0};
     if (h->is_product()) off[0] = 2;
     for (int c = 0; c < h->sum.n; c++) {
-        const int nls = h->sum_per[c] ? 2 * h->cdim(c, h->d) : h->comp_ls(c), rq = h->sum.fam[c] == KERNEL_RQ;
+        // a Linear component: one entry per column, [0, sum_i W_ii, x_j^T W x_j (j < k)] (lml_grad_linear_kernel)
+        const int nls = h->sum_per[c] ? 2 * h->cdim(c, h->d) : h->comp_lin(c) ? h->cdim(c, h->d) : h->comp_ls(c),
+                  rq = h->sum.fam[c] == KERNEL_RQ;
         stride[c] = (h->is_product() ? 0 : 2) + nls + rq;
         ik[c] = h->is_product() ? 0 : off[c];
         il[c] = h->is_product() ? off[c] : off[c] + 2;
@@ -1972,7 +2025,11 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
             double* part = h->gpart.as<double>() + (size_t)nblk * off[c];
             const double* Xs_c = h->Xs.as<double>() + (size_t)h->srow.off[c] * h->Np;
             const int k = h->cdim(c, h->d);
-            if (h->sum_per[c]) {
+            if (h->comp_lin(c)) {
+                lml_grad_linear_kernel<<<nblk, 256, linear_grad_smem(k), st>>>(Xs_c, h->alpha.as<double>(), h->Kinv.as<double>(), h->N, k,
+                                                                               h->Np, part, stride[c]);
+                h->launches++;
+            } else if (h->sum_per[c]) {
                 const double* Xr = h->nmap ? h->Xg.as<double>() + h->raw.off[c] : h->X.as<double>();
                 KernelIds<KERNEL_SE, KERNEL_RQ>::with(h->sum.fam[c], [&](auto kid) {
                     lml_grad_periodic_kernel<kid><<<nblk, 256, periodic_grad_smem(k), st>>>(
@@ -2015,6 +2072,19 @@ static int neg_lml_grad_composite(gpso_handle* h, const double* u, int p, double
             pos++;
         }
         const int nl = h->comp_ls(c), np = h->comp_np(c), d = h->cdim(c, h->d), lo = h->ls_off(c);
+        if (h->comp_lin(c)) {  // dK/dvar_j = x_j x_j^T: d(-LML)/dvar_j = -0.5 x_j^T W x_j; a scalar variance takes the sum over j
+            const double* Q = g + il[c];
+            // the rows are x_j / l_j with l_j^2 = 1 / var_j: x_j^T W x_j = Q_j / var_j (var_j = 0 only where softplus underflowed,
+            // with the chain factor sigmoid(u) 0 too: the entry is 0 there)
+            double Qs = 0.0;
+            for (int k = 0; k < d; k++) Qs += Q[k] / h->ls_host[lo + k];
+            for (int i = 0; i < nl; i++) {
+                const double v = h->ls_host[lo + i];
+                grad_host[pos + i] = v > 0.0 ? -(0.5 * (nl > 1 ? Q[i] / v : Qs)) * sigmoid(u[pos + i]) : 0.0;
+            }
+            pos += nl;
+            continue;
+        }
         if (h->sum_per[c]) {  // per-dimension entries L(d), Q(d) as for a bare periodic kernel (gpso_neg_lml_grad)
             const double* L = g + il[c];
             const double* Q = g + il[c] + d;
@@ -2407,7 +2477,8 @@ static int full_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, cons
     GP_TRY(h->part.ensure((size_t)W * h->nb * sizeof(double)));
     GP_TRY(h->blockbest.ensure((size_t)((W + 255) / 256) * sizeof(BestRec)));
     for (int b = 0; b < nbuf; b++) {
-        GP_TRY(h->wmeanb[b].ensure((size_t)W * sizeof(double)));
+        // Linear terms: the window's prior variances follow its (padded) means; W is a multiple of the padded window
+        GP_TRY(h->wmeanb[b].ensure((size_t)W * (h->has_lin() ? 2 : 1) * sizeof(double)));
         if (oz) GP_TRY(h->ozBb[b].ensure((size_t)W * h->Np * h->oz_S));
     }
     if (!oz) GP_TRY(h->KsT.ensure((size_t)W * h->Np * sizeof(double)));
@@ -2463,9 +2534,14 @@ static int full_pass(gpso_handle* h, cudaStream_t st, const double* Xc_dev, cons
         double* om = staged ? h->omean.as<double>() : out.mean ? out.mean + win.off : nullptr;
         double* ov = staged ? h->ovar.as<double>() : out.var ? out.var + win.off : nullptr;
         const int fb = (int)((win.Mw + 255) / 256);
-        predict_finalize_kernel<<<fb, 256, 0, ps>>>(h->part.as<double>(), h->wmeanb[win.b].as<double>(), h->nb, (int)pad(win.Mw), win.Mw,
-                                                    win.off, h->variance, h->noise, varsigma, argmax ? 1 : 0, om, ov,
-                                                    h->blockbest.as<BestRec>(), out.idx_map);
+        if (h->has_lin())
+            predict_finalize_kss_kernel<<<fb, 256, 0, ps>>>(h->part.as<double>(), h->wmeanb[win.b].as<double>(), h->nb, (int)pad(win.Mw),
+                                                            win.Mw, win.off, h->noise, varsigma, argmax ? 1 : 0, om, ov,
+                                                            h->blockbest.as<BestRec>(), out.idx_map);
+        else
+            predict_finalize_kernel<<<fb, 256, 0, ps>>>(h->part.as<double>(), h->wmeanb[win.b].as<double>(), h->nb, (int)pad(win.Mw), win.Mw,
+                                                        win.off, h->variance, h->noise, varsigma, argmax ? 1 : 0, om, ov,
+                                                        h->blockbest.as<BestRec>(), out.idx_map);
         GP_TRY(check_launch(h, "predict_finalize"));
         if (check) {
             screen_check_kernel<<<fb, 256, 0, ps>>>(om, ov, win.Mw, out.idx_map + win.off, varsigma, h->scr_ucb.as<double>(),
@@ -3047,7 +3123,7 @@ static int joint_ready(gpso_handle* h, const char* who) {
 
 static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double* Xc, int M, int Mp) {
     size_t sm = (size_t)(XG * h->dx() + 8 * XG) * sizeof(double);
-    CovKernels::with(h->cov_kid(), [&](auto kid) {
+    FullCovKernels::with(h->cov_kid(), [&](auto kid) {
         crosscov_kernel<kid><<<(unsigned)(Mp / XG), 256, sm, st>>>(Xc, M, h->kd(), h->ls.as<double>(), h->kern_nls(), h->Xs.as<double>(),
                                                                   h->alpha.as<double>(), h->N, h->Np, h->variance, h->c0,
                                                                   h->jKsT.as<double>(), h->jmean.as<double>(), h->rq_alpha, h->sum, h->srow);
@@ -3056,7 +3132,7 @@ static void launch_joint_crosscov(gpso_handle* h, cudaStream_t st, const double*
 
 static void launch_joint_syrk(gpso_handle* h, cudaStream_t st, int M, int Mp, double jitter) {
     const int mb = Mp / TB;
-    CovKernels::with(h->cov_kid(), [&](auto kid) {
+    FullCovKernels::with(h->cov_kid(), [&](auto kid) {
         joint_syrk_kernel<kid><<<mb * (mb + 1) / 2, GTHREADS, GEMM_SMEM_BYTES, st>>>(h->jVT.as<double>(), h->jXcs.as<double>(), M, Mp,
                                                                                    h->Np, h->kd(), h->variance, jitter,
                                                                                    h->jSigma.as<double>(), h->rq_alpha, h->sum, h->srow);
@@ -3068,7 +3144,7 @@ static int joint_sigma(gpso_handle* h, cudaStream_t st, const double* Xc, int M,
     const int Mp = (M + TB - 1) / TB * TB, Np = h->Np;
     GP_TRY(h->jXcs.ensure((size_t)h->dx() * Mp * sizeof(double)));
     GP_TRY(h->jKsT.ensure((size_t)Mp * Np * sizeof(double)));
-    GP_TRY(h->jmean.ensure((size_t)Mp * sizeof(double)));
+    GP_TRY(h->jmean.ensure((size_t)Mp * (h->has_lin() ? 2 : 1) * sizeof(double)));  // Linear terms: the prior variances follow
     GP_TRY(h->jVT.ensure((size_t)Mp * Np * sizeof(double)));
     GP_TRY(h->jSigma.ensure((size_t)Mp * Mp * sizeof(double)));
     GP_TRY(h->jcounter.ensure(sizeof(int)));
@@ -3312,7 +3388,8 @@ extern "C" int gpso_grow_ucb_argmax(gpso_handle* h, const double* bounds_host, i
 constexpr int STATE_HEADER = 128;
 constexpr int STATE_PERIODS = 16 + MAX_LS;  // a periodic kernel's period(s); slot 10 = 1 marks it, slot 11 = the period's ARD flag
 
-// the family entry of a component in the state's component block: its family id, + 16 for a periodic component (its base's id)
+// the family entry of a component in the state's component block: its family id, + 16 for a periodic component (its base's id),
+// KERNEL_LINEAR (10) for a Linear component, whose lengthscale slots hold its variance(s)
 static int comp_code(const gpso_handle* h, int c) { return h->sum.fam[c] + (h->sum_per[c] ? 16 : 0); }
 // the block entries of component c: family, lengthscale count, variance, alpha, lengthscales, [period count, periods]
 static int comp_block(const gpso_handle* h, int c, int d) {
@@ -3376,7 +3453,7 @@ extern "C" int gpso_export_state_dev(gpso_handle* h, void* dst_dev, int64_t byte
     hdr[3] = h->noise;
     hdr[4] = h->c0;
     hdr[5] = h->factor_nlml;
-    hdr[6] = h->kernel_id;
+    hdr[6] = h->bare_lin ? GPSO_KERNEL_LINEAR : h->kernel_id;
     hdr[7] = h->ard;
     if (h->n_rq()) hdr[8] = h->rq_alpha;
     hdr[9] = h->mean_id;
@@ -3440,7 +3517,8 @@ extern "C" int gpso_import_state_dev(gpso_handle* h, const void* src_dev, int64_
     CU_TRY(cudaStreamSynchronize(h->stream));
     GP_TRY(ensure_shape(h, N, d));
     if ((int)hdr[0] != N || (int)hdr[1] != d) return fail(GPSO_E_BADARG, "gpso_import_state_dev: header shape mismatch");
-    if ((int)hdr[6] != h->kernel_id || (int)hdr[7] != h->ard) return fail(GPSO_E_BADARG, "gpso_import_state_dev: kernel mismatch");
+    if ((int)hdr[6] != (h->bare_lin ? GPSO_KERNEL_LINEAR : h->kernel_id) || (int)hdr[7] != h->ard)
+        return fail(GPSO_E_BADARG, "gpso_import_state_dev: kernel mismatch");
     if ((hdr[10] == 1.0) != h->periodic || (h->periodic && (int)hdr[11] != h->per_ard))
         return fail(GPSO_E_BADARG, "gpso_import_state_dev: periodic kernel mismatch");
     if (((int)hdr[9] == GPSO_MEAN_LINEAR) != h->linear())
@@ -3559,6 +3637,8 @@ extern "C" int64_t gpso_last_windows(gpso_handle* h) { return h ? h->last_window
 extern "C" int gpso_set_predict_mode(gpso_handle* h, int mode, int slices) {
     if (!h || mode < 0 || mode > 2) return fail(GPSO_E_BADARG, "gpso_set_predict_mode: mode must be 0 (auto), 1 (fp64 DMMA) or 2 (int8 tcgen05)");
     if (slices != 0 && (slices < 5 || slices > 8)) return fail(GPSO_E_BADARG, "gpso_set_predict_mode: slices must be 0 (auto) or 5..8");
+    if (mode == 2 && h->has_lin())
+        return fail(GPSO_E_BADARG, "gpso_set_predict_mode: a kernel with a Linear term has no bound on |k*| for the int8 engine: modes 0 and 1 only");
     h->predict_mode = mode;
     h->oz_force_slices = slices;
     h->factorized = false;  // takes effect at the next gpso_factorize
@@ -3669,6 +3749,8 @@ extern "C" int gpso_predict_info(gpso_handle* h, double* out3) {
 extern "C" int gpso_set_screen_mode(gpso_handle* h, int mode) {
     if (!h || mode < 0 || mode > SCREEN_MODE_FULL2)
         return fail(GPSO_E_BADARG, "gpso_set_screen_mode: mode must be 0 (off), 1 (automatic), 2..4 (digits), 5 (mean bound first) or 6 (2 digits, all pairs)");
+    if (mode >= 2 && h->has_lin())
+        return fail(GPSO_E_BADARG, "gpso_set_screen_mode: a kernel with a Linear term is not screened (its prior variance differs per candidate): modes 0 and 1 only");
     h->screen_mode = mode;
     h->screen_S_cur = 0;
     if (h->nb > 0) g_screen_hint[std::min(h->nb, 64)] = ScreenHint();  // an explicit call restarts the ladder for this matrix size

@@ -29,7 +29,55 @@ __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs
     __shared__ double sXi[CDCH][CT];
     const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
     const int j = bj * CT + tx;
-    if constexpr (composite_kernel(KID)) {
+    if constexpr (KID == KERNEL_SUM_LIN) {
+        // a Linear component adds the dot product of its rows, the others their stationary value as KERNEL_SUM_EMB does
+        double kv[16];
+        for (int c = 0; c < sum.n; c++) {
+            const bool lin = sum.fam[c] == KERNEL_LINEAR;
+            const int rn = srow.rows[c];
+            const double* Xc = Xs + (size_t)srow.off[c] * Np;
+            double acc[16];
+#pragma unroll
+            for (int r = 0; r < 16; r++) acc[r] = 0.0;
+            for (int d0 = 0; d0 < rn; d0 += CDCH) {
+                int dc = min(CDCH, rn - d0);
+                __syncthreads();
+                for (int e = threadIdx.x; e < dc * CT; e += 256) sXi[e / CT][e % CT] = Xc[(size_t)(d0 + e / CT) * Np + bi * CT + e % CT];
+                __syncthreads();
+                for (int dd = 0; dd < dc; dd++) {
+                    const double xj = Xc[(size_t)(d0 + dd) * Np + j];
+                    if (lin) {
+#pragma unroll
+                        for (int r = 0; r < 16; r++) acc[r] = fma(sXi[dd][ty + 4 * r], xj, acc[r]);
+                    } else {
+#pragma unroll
+                        for (int r = 0; r < 16; r++) {
+                            const double df = sXi[dd][ty + 4 * r] - xj;
+                            acc[r] = fma(df, df, acc[r]);
+                        }
+                    }
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < 16; r++) {
+                const double t = lin ? acc[r] : sum_term(sum, c, acc[r]);
+                kv[r] = (c == 0) ? t : kv[r] + t;
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 16; r++) {
+            int i = bi * CT + ty + 4 * r;
+            double v;
+            if (i < N && j < N) {
+                v = kv[r];
+                if (i == j) v += noise;
+            } else {
+                v = (i == j) ? 1.0 : 0.0;
+            }
+            K[(size_t)i * Np + j] = v;
+        }
+        return;
+    } else if constexpr (composite_kernel(KID)) {
         // the loop below once per component (its own scaled inputs), the component values added (multiplied) in order
         double kv[16];
         for (int c = 0; c < sum.n; c++) {
@@ -111,6 +159,93 @@ __global__ void __launch_bounds__(256) gram_kernel(const double* __restrict__ Xs
 // of operations (position-independent results: duplicated candidates give bit-identical outputs).
 constexpr int XG = 8;
 
+// crosscov_kernel of a sum with Linear terms (KERNEL_SUM_LIN): the rows of KERNEL_SUM_EMB, and the prior variance k(x_c, x_c) of every
+// candidate c of the launch (grid XG-candidate blocks) after the means, at mean[gridDim.x XG + c]: the squared norm of a Linear
+// component's rows, the variance of the others, added in fp64 in component order (joint_syrk_kernel forms the same sum).
+__device__ __forceinline__ void crosscov_sum_lin(const double* __restrict__ Xc, long long Mw, const double* __restrict__ ls,
+                                                 const double* __restrict__ Xs, const double* __restrict__ alpha, int N, int Np,
+                                                 double c0, double* __restrict__ KsT, double* __restrict__ mean, const SumTable& sum,
+                                                 const SumRows& srow, double* sm) {
+    double* sC = sm;  // [XG][width]
+    double* sR = sm + XG * srow.width;
+    const long long cbase = (long long)blockIdx.x * XG;
+    const int w = srow.width;
+    for (int e = threadIdx.x; e < XG * w; e += 256) {
+        const long long c = cbase + e / w;
+        const int r = e % w;
+        sC[e] = (c < Mw) ? Xc[c * w + r] / ls[r] : 0.0;
+    }
+    __syncthreads();
+    double macc[XG];
+#pragma unroll
+    for (int c = 0; c < XG; c++) macc[c] = 0.0;
+    for (int j = threadIdx.x; j < Np; j += 256) {
+        double kv[XG];
+        for (int q = 0; q < sum.n; q++) {
+            const bool lin = sum.fam[q] == KERNEL_LINEAR;
+            const int rn = srow.rows[q];
+            const double* Xq = Xs + (size_t)srow.off[q] * Np;
+            const double* sq = sC + srow.off[q];
+            double acc[XG];
+#pragma unroll
+            for (int c = 0; c < XG; c++) acc[c] = 0.0;
+            if (lin) {
+                for (int dim = 0; dim < rn; dim++) {
+                    const double xj = Xq[(size_t)dim * Np + j];
+#pragma unroll
+                    for (int c = 0; c < XG; c++) acc[c] = fma(xj, sq[c * w + dim], acc[c]);
+                }
+            } else {
+                for (int dim = 0; dim < rn; dim++) {
+                    const double xj = Xq[(size_t)dim * Np + j];
+#pragma unroll
+                    for (int c = 0; c < XG; c++) {
+                        const double df = xj - sq[c * w + dim];
+                        acc[c] = fma(df, df, acc[c]);
+                    }
+                }
+#pragma unroll
+                for (int c = 0; c < XG; c++) acc[c] = sum_term(sum, q, acc[c]);
+            }
+#pragma unroll
+            for (int c = 0; c < XG; c++) kv[c] = (q == 0) ? acc[c] : kv[c] + acc[c];
+        }
+        const double a = alpha[j];
+#pragma unroll
+        for (int c = 0; c < XG; c++) {
+            const double k = (j < N && cbase + c < Mw) ? kv[c] : 0.0;
+            KsT[(size_t)(cbase + c) * Np + j] = k;
+            macc[c] = fma(k, a, macc[c]);
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < XG; c++) macc[c] = warp_sum(macc[c]);
+    const int wp = threadIdx.x >> 5, l = threadIdx.x & 31;
+    if (l == 0) {
+#pragma unroll
+        for (int c = 0; c < XG; c++) sR[wp * XG + c] = macc[c];
+    }
+    __syncthreads();
+    if (threadIdx.x < XG) {
+        double s = 0.0;
+#pragma unroll
+        for (int ww = 0; ww < 8; ww++) s += sR[ww * XG + threadIdx.x];
+        mean[cbase + threadIdx.x] = s + c0;
+    }
+    if (threadIdx.x < XG) {
+        double s = 0.0;
+        for (int q = 0; q < sum.n; q++) {
+            double t = sum.var[q];
+            if (sum.fam[q] == KERNEL_LINEAR) {
+                t = 0.0;
+                for (int r = srow.off[q]; r < srow.off[q] + srow.rows[q]; r++) t = fma(sC[threadIdx.x * w + r], sC[threadIdx.x * w + r], t);
+            }
+            s = (q == 0) ? t : s + t;
+        }
+        mean[(long long)gridDim.x * XG + cbase + threadIdx.x] = s;
+    }
+}
+
 template <int KID>
 __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict__ Xc, long long Mw, int d,
                                                        const double* __restrict__ ls, int n_ls,
@@ -122,7 +257,10 @@ __global__ void __launch_bounds__(256) crosscov_kernel(const double* __restrict_
     const int nsc = composite_kernel(KID) ? sum.n : 1;  // scaled copies of the candidates
     double* sR = sm + (embedded_composite(KID) ? XG * srow.width : nsc * XG * d);
     const long long cbase = (long long)blockIdx.x * XG;
-    if constexpr (embedded_composite(KID)) {
+    if constexpr (KID == KERNEL_SUM_LIN) {
+        crosscov_sum_lin(Xc, Mw, ls, Xs, alpha, N, Np, c0, KsT, mean, sum, srow, sm);
+        return;
+    } else if constexpr (embedded_composite(KID)) {
         // [XG][width]: candidate row r divided by ls[r] (a periodic component's embedded rows by its unit lengthscale)
         const int w = srow.width;
         for (int e = threadIdx.x; e < XG * w; e += 256) {
@@ -757,6 +895,60 @@ __global__ void __launch_bounds__(256) lml_grad_periodic_kernel(const double* __
             part[(size_t)blk * part_stride + 2 + q] = acc_l;
             part[(size_t)blk * part_stride + 2 + d + q] = acc_p;
         }
+    }
+}
+
+// LML gradient of a Linear component over its rows Xs[k][Np] (s_j = x_j / l_j, l_j = 1 / sqrt(var_j)): one block per lower 64x64 tile,
+// the tile's rows and columns and the pair weights W in shared memory, then warp w sums the columns j = w, w + 8, ...:
+//   part[blk][0] = 0, part[blk][1] = sum_i W_ii (-> d/d noise), part[blk][2 + j] = s_j^T W s_j over the tile
+// dK/dvar_j = x_j x_j^T, so dLML/dvar_j = 0.5 l_j^2 s_j^T W s_j; a scalar variance takes the sum over j (the host does both).
+__global__ void __launch_bounds__(256) lml_grad_linear_kernel(const double* __restrict__ Xs, const double* __restrict__ alpha,
+                                                              const double* __restrict__ Kinv, int N, int k, int Np,
+                                                              double* __restrict__ part, int part_stride) {
+    int blk = blockIdx.x;
+    int bi = (int)((sqrt(8.0 * blk + 1.0) - 1.0) * 0.5);
+    while ((bi + 1) * (bi + 2) / 2 <= blk) bi++;
+    while (bi * (bi + 1) / 2 > blk) bi--;
+    int bj = blk - bi * (bi + 1) / 2;
+    extern __shared__ double smg[];
+    double* sXi = smg;             // [k][64] the tile's rows
+    double* sXj = sXi + k * CT;    // [k][64] ... and its columns
+    double* sW = sXj + k * CT;     // [64 * 64] W per pair
+    __shared__ double sRed[8];
+    for (int e = threadIdx.x; e < k * CT; e += 256) {
+        const size_t row = (size_t)(e / CT) * Np;
+        sXi[e] = Xs[row + bi * CT + e % CT];
+        sXj[e] = Xs[row + bj * CT + e % CT];
+    }
+    const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
+    const int j = bj * CT + tx;
+    const double aj = alpha[j];
+    const double wsym = (bi == bj) ? 1.0 : 2.0;
+    double s_tr = 0.0;
+    for (int r = 0; r < 16; r++) {
+        const int il = ty + 4 * r, i = bi * CT + il;
+        double W = 0.0;
+        // diagonal tiles: the tile holds both triangles of a symmetric quantity, take every element once
+        if (i < N && j < N) {
+            W = fma(alpha[i], aj, -((j <= i) ? Kinv[(size_t)i * Np + j] : Kinv[(size_t)j * Np + i])) * wsym;
+            if (i == j) s_tr += W;
+        }
+        sW[il * CT + tx] = W;
+    }
+    const double v = block_sum<256>(s_tr, sRed);
+    if (threadIdx.x == 0) {
+        part[(size_t)blk * part_stride + 0] = 0.0;
+        part[(size_t)blk * part_stride + 1] = v;
+    }
+    __syncthreads();  // the weights of every pair are in sW
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int q = w; q < k; q += 8) {
+        const double* xi = sXi + q * CT;
+        const double* xj = sXj + q * CT;
+        double acc = 0.0;
+        for (int p = lane; p < CT * CT; p += 32) acc = fma(sW[p] * xi[p >> 6], xj[p & 63], acc);
+        acc = warp_sum(acc);
+        if (lane == 0) part[(size_t)blk * part_stride + 2 + q] = acc;
     }
 }
 

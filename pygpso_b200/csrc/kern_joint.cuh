@@ -109,6 +109,28 @@ __global__ void __launch_bounds__(GTHREADS, 1) joint_syrk_kernel(const double* _
             v = (gi == gj) ? 1.0 : 0.0;
         } else if (gj > gi) {
             v = 0.0;
+        } else if constexpr (KID == KERNEL_SUM_LIN) {
+            // a sum with Linear terms: a Linear component adds the dot product of its rows, the others their stationary value; the
+            // diagonal is the candidate's own prior variance, formed as crosscov_kernel forms it (the variances of the others)
+            double k = 0.0;
+            for (int q = 0; q < sum.n; q++) {
+                const double* Xq = Xcs + (size_t)srow.off[q] * Mp;
+                const bool lin = sum.fam[q] == KERNEL_LINEAR;
+                double acc = 0.0;
+                for (int dim = 0; dim < srow.rows[q] && (lin || gi != gj); dim++) {
+                    const double xi = Xq[(size_t)dim * Mp + gi], xj = Xq[(size_t)dim * Mp + gj];
+                    if (lin) {
+                        acc = fma(xi, xj, acc);
+                    } else {
+                        const double df = xi - xj;
+                        acc = fma(df, df, acc);
+                    }
+                }
+                const double t = lin ? acc : (gi == gj ? sum.var[q] : sum_term(sum, q, acc));
+                k = (q == 0) ? t : k + t;
+            }
+            v = k - smem[r * JST + c];
+            if (gi == gj) v += jitter;
         } else if constexpr (composite_kernel(KID)) {
             // Xcs[C][d][Mp]: component q's scaled candidates at Xcs + q d Mp; the diagonal starts from exactly
             // sum_q var_q (a product: var_prod, its unit factors being exactly 1 at r = 0)

@@ -164,6 +164,53 @@ __global__ void __launch_bounds__(256) predict_finalize_kernel(const double* __r
     }
 }
 
+// predict_finalize_kernel for a kernel with Linear terms: the prior variance of candidate c is its own, mean[ldp + c] (written after the
+// window's means by crosscov_kernel<KERNEL_SUM_LIN>), not one kernel variance; everything else as above
+__global__ void __launch_bounds__(256) predict_finalize_kss_kernel(const double* __restrict__ part, const double* __restrict__ mean,
+                                                                   int nb, int ldp, long long Mw, long long idx0, double noise,
+                                                                   double varsigma, int mode, double* __restrict__ out_mean,
+                                                                   double* __restrict__ out_var, BestRec* __restrict__ blockbest,
+                                                                   const long long* __restrict__ idx_map) {
+    long long c = (long long)blockIdx.x * 256 + threadIdx.x;
+    double m = 0.0, v = 0.0, u = 0.0;
+    bool valid = c < Mw;
+    if (valid) {
+        double ss = 0.0;
+        for (int I = 0; I < nb; I++) ss += part[(size_t)I * ldp + c];
+        m = mean[c];
+        v = __dadd_rn(__dsub_rn(mean[ldp + c], ss), noise);
+        u = __dadd_rn(m, __dmul_rn(varsigma, v));
+    }
+    if (out_mean != nullptr && valid) {
+        out_mean[c] = m;
+        out_var[c] = v;
+    }
+    if (mode == 0) return;
+    long long gi = valid ? (idx_map != nullptr ? idx_map[idx0 + c] : idx0 + c) : 0x7fffffffffffffffLL;
+    double bu = valid ? u : -INFINITY, bm = m, bv = v;
+    long long bi = gi;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        double ou = __shfl_xor_sync(0xffffffffu, bu, o);
+        double om = __shfl_xor_sync(0xffffffffu, bm, o);
+        double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (best_better(ou, oi, bu, bi)) {
+            bu = ou; bm = om; bv = ov; bi = oi;
+        }
+    }
+    __shared__ BestRec sb[8];
+    int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+    if (l == 0) sb[w] = BestRec{bu, bm, bv, bi};
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        BestRec b = sb[0];
+        for (int i = 1; i < 8; i++)
+            if (best_better(sb[i].ucb, sb[i].idx, b.ucb, b.idx)) b = sb[i];
+        blockbest[blockIdx.x] = b;
+    }
+}
+
 // running[0] = best of (running[0] if !first) and blockbest[0..n)
 __global__ void __launch_bounds__(256) best_merge_kernel(const BestRec* __restrict__ blockbest, int n, BestRec* __restrict__ running,
                                                          int first) {

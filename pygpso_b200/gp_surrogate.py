@@ -603,9 +603,10 @@ class GPRSurrogate(GPSurrogate):
         is_sum = isinstance(model.kernel, gpmodel.Combination)  # a Sum or a Product
         periodic = isinstance(model.kernel, gpmodel.Periodic)
         leaf = model.kernel.base_kernel if periodic else model.kernel
+        linear = isinstance(leaf, gpmodel.LinearKernel)  # no lengthscales: the shape saved is the variance's
         save_info = {
             "gpr_kernel": model.kernel.__class__.__name__,
-            "gpr_kernel_shape": [] if is_sum else leaf.lengthscales.shape.as_list(),
+            "gpr_kernel_shape": [] if is_sum else (leaf.variance if linear else leaf.lengthscales).shape.as_list(),
             "gpr_meanf": meanf.__class__.__name__,
             "gpr_meanf_shape": meanf.parameters[0].shape.as_list() if meanf.parameters else [],
             "gp_varsigma": self.gp_varsigma,
@@ -613,10 +614,11 @@ class GPRSurrogate(GPSurrogate):
             "optimiser": self._serialise_optimiser(),
         }
         if is_sum:  # component (factor) families and lengthscale shapes, in order
-            # a periodic term: ["Periodic", base lengthscale shape, base family, period shape]
+            # a periodic term: ["Periodic", base lengthscale shape, base family, period shape]; a Linear term: ["Linear", variance shape]
             save_info["gpr_kernel_components"] = [
                 ["Periodic", k.base_kernel.lengthscales.shape.as_list(), k.base_kernel.__class__.__name__, k.period.shape.as_list()]
-                if isinstance(k, gpmodel.Periodic) else [k.__class__.__name__, k.lengthscales.shape.as_list()]
+                if isinstance(k, gpmodel.Periodic) else ["Linear", k.variance.shape.as_list()] if isinstance(k, gpmodel.LinearKernel)
+                else [k.__class__.__name__, k.lengthscales.shape.as_list()]
                 for k in model.kernel.kernels]
         if periodic:  # base family and the shape of the period; gpr_kernel_shape is the base lengthscales'
             save_info["gpr_kernel_periodic"] = [leaf.__class__.__name__, model.kernel.period.shape.as_list()]
@@ -641,12 +643,16 @@ class GPRSurrogate(GPSurrogate):
                 if entry[0] == "Periodic":
                     return gpmodel.kernels.Periodic(getattr(gpmodel.kernels, entry[2])(lengthscales=np.ones(entry[1])),
                                                     period=np.ones(entry[3]))
+                if entry[0] == "Linear":
+                    return gpmodel.kernels.Linear(variance=np.ones(entry[1]))
                 return getattr(gpmodel.kernels, entry[0])(lengthscales=np.ones(entry[1]))
             gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])([component(e) for e in info["gpr_kernel_components"]])
         elif info["gpr_kernel"] == "Periodic":
             base, period_shape = info["gpr_kernel_periodic"]
             gp_kernel = gpmodel.kernels.Periodic(getattr(gpmodel.kernels, base)(lengthscales=np.ones(info["gpr_kernel_shape"])),
                                                  period=np.ones(period_shape))
+        elif info["gpr_kernel"] == "Linear":
+            gp_kernel = gpmodel.kernels.Linear(variance=np.ones(info["gpr_kernel_shape"]))
         else:
             gp_kernel = getattr(gpmodel.kernels, info["gpr_kernel"])(lengthscales=np.ones(info["gpr_kernel_shape"]))
         if "gpr_kernel_active_dims" in info:

@@ -21,7 +21,7 @@ the 1e-6 floor, and ``trainable_variables`` are ordered kernel.lengthscales, ker
 mean_function.c (or mean_function.A, mean_function.b for ``Linear``) -- preceded by kernel.alpha for ``RationalQuadratic``
 (tf.Module visits attributes in sorted name order).  A ``Sum`` (``Product``) kernel lists its components' (factors')
 parameters in component order, each component's in that same sorted order.  A ``Periodic`` kernel lists its base kernel's
-parameters, then kernel.period ('base_kernel' < 'period').
+parameters, then kernel.period ('base_kernel' < 'period').  A ``kernels.Linear`` kernel has kernel.variance only.
 
 A stationary kernel acts on the input columns ``active_dims`` (GPflow's keyword: None for all of them, a slice, or a list of
 column indices in the order given, repeats allowed); a ``Periodic`` kernel's are its base kernel's.  ARD lengthscales (and an ARD
@@ -215,6 +215,32 @@ class SquaredExponential(Stationary):
 RBF = SquaredExponential
 
 
+class LinearKernel(Kernel):
+    """``gpflow.kernels.Linear``: ``k(x, x') = sum_j variance_j x_j x'_j`` over the active columns, ``variance`` (positive,
+    softplus) a scalar or one entry per active column.  It is not stationary: the prior variance k(x, x) grows with |x|.  It is
+    ``kernels.Linear``; the top-level ``Linear`` is the mean function, as in GPflow.  Bare, or a term of a ``Sum``; not a factor of a
+    ``Product`` nor the base of a ``Periodic``."""
+
+    def __init__(self, variance=1.0, active_dims=None):
+        self.variance = Parameter(variance, positive=True, name="kernel.variance")
+        if len(self.variance.shape) > 1:
+            raise ValueError(f"variance must be a scalar or a vector, got shape {tuple(self.variance.shape)}")
+        self.active_dims = active_dims
+
+    active_dims = Stationary.active_dims
+
+    @property
+    def ard(self):
+        return self.variance.size > 1 or len(self.variance.shape) > 0 and self.variance.shape[0] > 1
+
+    @property
+    def parameters(self):
+        return (self.variance,)
+
+
+LinearKernel.__name__ = LinearKernel.__qualname__ = "Linear"  # GPflow's class name (saves record it)
+
+
 class Combination(Kernel):
     """GPflow's ``Combination``: 1..4 kernels combined in order.  Nested combinations of the same kind are flattened, so
     ``(a + b) + c`` and ``a + (b + c)`` are the same three-component sum (and likewise for products).  The same kernel object
@@ -347,6 +373,8 @@ class Linear(MeanFunction):
 # a component of a Sum / Product as the backend takes it: (family, n_lengthscales), or ("Periodic", n_lengthscales, base family,
 # n_periods) for a periodic term
 def _component_spec(k):
+    if isinstance(k, LinearKernel):
+        return ("Linear", k.variance.size)
     if isinstance(k, Periodic):
         return ("Periodic", k.base_kernel.lengthscales.size, type(k.base_kernel).__name__, k.period.size)
     return (type(k).__name__, k.lengthscales.size)
@@ -395,10 +423,13 @@ class GPR(GPModel):
 
     def __init__(self, data, kernel, mean_function=None, noise_variance=1.0, backend=None):
         parts = kernel.kernels if isinstance(kernel, Combination) else [kernel]
+        if isinstance(kernel, Product) and any(isinstance(k, LinearKernel) for k in parts):
+            raise TypeError("a Linear kernel cannot be a factor of a Product: its prior variance k(x, x) is not bounded by a "
+                            "constant, which the product path assumes; use it bare or as a term of a Sum")
         if isinstance(kernel, Combination) and any(isinstance(k, Combination) for k in parts):
             raise TypeError("sums of products and products of sums are not supported: the components of a Sum and the factors "
                             "of a Product must be Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic")
-        if not all(isinstance(k, (Stationary, Periodic)) for k in parts):
+        if not all(isinstance(k, (Stationary, Periodic, LinearKernel)) for k in parts):
             raise TypeError("kernel must be one of Matern12 / Matern32 / Matern52 / SquaredExponential / RationalQuadratic, "
                             "or a Sum of them")
         self.kernel = kernel
@@ -420,7 +451,7 @@ class GPR(GPModel):
         else:
             self._session = self._backend.open_session(
                 kernel=type(kernel).__name__,
-                n_lengthscales=self.kernel.lengthscales.size,
+                n_lengthscales=(kernel.variance if isinstance(kernel, LinearKernel) else kernel.lengthscales).size,
                 has_mean=_mean_id(self.mean_function),
             )
         self._factor_key = None
@@ -448,6 +479,11 @@ class GPR(GPModel):
                     raise ValueError("an ARD period must have one entry per input dimension"
                                      + (f" ({len(dims)} active)" if len(dims) != x.shape[1] else ""))
                 k = k.base_kernel
+            if isinstance(k, LinearKernel):
+                if k.variance.size not in (1, len(dims)):
+                    raise ValueError("ARD variances of a Linear kernel must have one entry per input dimension"
+                                     + (f" ({len(dims)} active)" if len(dims) != x.shape[1] else ""))
+                continue
             if k.lengthscales.size not in (1, len(dims)):
                 raise ValueError("ARD lengthscales must have one entry per input dimension"
                                  + (f" ({len(dims)} active)" if len(dims) != x.shape[1] else ""))
@@ -626,6 +662,8 @@ class Scipy:
 # gpflow.utilities look-alikes (used by save / load)
 # ---------------------------------------------------------------------------------------------------------------------
 def _kernel_leaves(prefix, kernel):
+    if isinstance(kernel, LinearKernel):
+        return {f"{prefix}.variance": kernel.variance}
     if isinstance(kernel, Periodic):
         out = _kernel_leaves(f"{prefix}.base_kernel", kernel.base_kernel)
         out[f"{prefix}.period"] = kernel.period
@@ -674,7 +712,7 @@ def tabulate_module_summary(model):
 kernels = types.SimpleNamespace(
     Kernel=Kernel, Stationary=Stationary, Matern12=Matern12, Matern32=Matern32, Matern52=Matern52,
     SquaredExponential=SquaredExponential, RBF=RBF, RationalQuadratic=RationalQuadratic, Sum=Sum,
-    Product=Product, Periodic=Periodic,
+    Product=Product, Periodic=Periodic, Linear=LinearKernel,
 )
 mean_functions = types.SimpleNamespace(MeanFunction=MeanFunction, Zero=Zero, Constant=Constant, Linear=Linear)
 likelihoods = types.SimpleNamespace(Gaussian=Gaussian)
